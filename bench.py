@@ -44,6 +44,8 @@ HBM_FALLBACK_GBS = 6650.0   # /opt/skills/guides/B200_PROFILING.md fallback
 BYTES_FULL = 285480         # SURVEY.md 8d: Z 9,720 + g 8,744 + grad 9,720 + f 8 + J 257,288
 KERNEL = "ql::eval_kernel<1, 1, 0>"     # JM_BLOCK, reciprocal-FMA division, strided rows (as ncu / cuobjdump print it)
 C4_CLASSES = [(N, kt, im) for (N, kt) in [(31, 11), (41, 14), (61, 21), (81, 27), (101, 34), (121, 41)] for im in (1, 2)]
+DUMP_ROWS = 128             # --dump-outputs: 128 x (1215 + 1093 + 32161) doubles = 35 MB per dump
+DUMP_SEED = 0
 
 
 def workload_config(n_gpus):
@@ -73,6 +75,22 @@ def make_inputs(prob, rank, nsets):
         Z[:, 19::20] = np.clip(Z[:, 19::20], 1e-3, 2e-2)
         out.append(np.ascontiguousarray(Z))
     return out
+
+
+def dump_outputs(path, outs):
+    """Writes what one step returned to the caller as float64 DIR/<name>.npy: f for every evaluation of the batch;
+    grad, g and jac for a fixed seeded sample of DUMP_ROWS evaluations (the whole Jacobian is 1.05 GB), whose batch
+    indices go to rows.npy.  Inputs are seeded too, so two builds can be compared file by file."""
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(len(outs["f"]), DUMP_ROWS, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "rows.npy"), rows.astype(np.float64))
+    for k, v in outs.items():
+        if not isinstance(v, np.ndarray):                   # a CUDA tensor: gather the sampled rows on the device
+            import torch
+            v = (v if k == "f" else v[torch.from_numpy(rows).to(v.device)]).cpu().numpy()
+        elif k != "f":
+            v = v[rows]
+        np.save(os.path.join(path, f"{k}.npy"), np.ascontiguousarray(v, dtype=np.float64))
 
 
 class ClockSampler:
@@ -202,12 +220,9 @@ def run_reference(args):
         nwarm += 1
         if nwarm >= 3:                                   # a CPU loop has no clocks to ramp: 3 passes warm the caches
             break
-    times = []
-    t_all = time.perf_counter()
-    for _ in range(args.steps):
-        times.append(runner.step())
-        if time.perf_counter() - t_all > 150:            # keep the whole run within minutes on any box
-            break
+    times = [runner.step() for _ in range(args.steps)]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("f", "grad", "g", "jac"), runner.bufs)))
     value = B_PER_GPU * len(times) / sum(times)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
@@ -547,6 +562,8 @@ def run_gpu(args):
     ms_step = cx.max_over_ranks(e0.elapsed_time(e1)) / args.steps
     value = B_PER_GPU * n_gpus / (ms_step * 1e-3)
     launch_info = nlp.launch_info()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)                 # rank 0's batch of the last timed step
 
     # ---- end to end through the C ABI with HOST buffers (pinned), copies inside the timed region -----------------
     # caller-side arrays come from the library's allocator (qlnlp_host_alloc: page-locked, 2 MB pages where granted)
@@ -728,6 +745,8 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extras", action="store_true", help="headline + e2e only (what the ncu captures run)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
     # the contract is ONE JSON line on stdout: libraries (e.g. NCCL's version banner) also write to fd 1, so
     # point fd 1 at stderr while running and emit the line on the real stdout at the end

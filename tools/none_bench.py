@@ -1,5 +1,5 @@
 import sys, os
-sys.path.insert(0, os.environ.get("REPO", "/root/repo"))
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import quadruped_landing_b200 as ql
 p = ql.default_problem(); nlp = ql.HybridNLP.from_problem(p)
