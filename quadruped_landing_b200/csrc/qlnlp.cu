@@ -79,12 +79,9 @@ struct HostLane {
 // single evaluations (the four MOI callbacks): one launch per decision vector, results cached
 struct OneEval {
     cudaStream_t stream = nullptr;
-    double* hx = nullptr;       // pinned: x | f grad g vals (packed, the layout of `dout`)
+    double* hx = nullptr;       // pinned, mapped: x(ldz_e) | f(2) grad(ldgrad_e) g(ldg_e) vals(ldv_e)
     double* hout = nullptr;
-    double* dx = nullptr;       // device: x (padded row)
-    double* dout = nullptr;     // device: f(2) | grad(ldz_e) | g(ldg_e) | vals(ldv_e)
-    bool zero_copy = false;     // the kernel reads x from / writes the results to the pinned block itself (mapped memory)
-    double* mx = nullptr;       // device-side addresses of hx / hout when zero_copy
+    double* mx = nullptr;       // device-side addresses of hx / hout: the kernel reads x and writes the results there
     double* mout = nullptr;
     int64_t o_grad = 0, o_g = 0, o_vals = 0, total = 0;
     bool valid = false;         // hout holds the results for the x stored in hx
@@ -397,12 +394,6 @@ int env_int(const char* name, int dflt)
     return dflt;
 }
 
-bool env_flag(const char* name, bool dflt)
-{
-    const char* e = std::getenv(name);
-    return (e && *e) ? std::atoi(e) != 0 : dflt;
-}
-
 // The worker pool of this handle: its share of the CPUs the process may use.  With one process per GPU (torchrun)
 // the ranks of a node split the cores (LOCAL_RANK of LOCAL_WORLD_SIZE); a multi-device handle splits its share
 // again between its devices; on a multi-socket host the share is taken from the CPUs next to the GPU.
@@ -427,8 +418,7 @@ int ensure_pool(qlnlp_handle h)
     if (h->opt_host_threads > 0) T = (int)h->opt_host_threads;
     T = env_int("QLNLP_HOST_THREADS", T);
     T = std::max(1, std::min(T, 256));
-    const bool pin = h->opt_pin_threads != 0 && env_flag("QLNLP_PIN_THREADS", true);
-    h->pool.reset(new (std::nothrow) qlhost::Pool(T, mine, pin));
+    h->pool.reset(new (std::nothrow) qlhost::Pool(T, mine, h->opt_pin_threads != 0));
     if (!h->pool) return fail(QLNLP_ENOMEM, "out of host memory");
     return QLNLP_OK;
 }
@@ -437,7 +427,6 @@ int ensure_pool(qlnlp_handle h)
 // kernel runs on (see launch(): programmatic dependent launch and spare CTA slots).
 size_t padded_smem(size_t smem_per_sm, size_t smem_optin, int per_sm, size_t smem)
 {
-    if (!env_flag("QLNLP_PAD_SMEM", true)) return smem;
     const size_t pad = (smem_per_sm / (size_t)(per_sm + 1) - 1024 + 128) & ~(size_t)127;
     if (pad > smem && (size_t)per_sm * (pad + 1024) <= smem_per_sm && pad <= smem_optin) return pad;
     return smem;
@@ -466,11 +455,32 @@ int set_carveout(const void* fn, int resident_blocks, size_t smem_per_block, siz
     // 132, 164, 196, 228 KB).  Ask for the smallest of those that holds `need`.  (Taking the percentage of the 228 KB
     // shared-memory maximum instead left the kernel without a Jacobian on 228 KB of shared memory and 28 KB of L1:
     // ncu launch__shared_mem_config_size; 46 % of its cost-table loads missed L1.  profiles/r02_kernel_ab.md)
-    int pct = carveout_pct(need, smem_per_sm);
-    pct = env_int("QLNLP_CARVEOUT_PCT", pct);          // tuning knob
-    if (!std::getenv("QLNLP_MAX_CARVEOUT"))
-        CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
+    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, carveout_pct(need, smem_per_sm)));
     return QLNLP_OK;
+}
+
+// Launch geometry of the eval kernel `fn` (value stream `wj`) at `smem` bytes of dynamic shared memory per CTA on the
+// handle's device: the resident CTAs per SM, and the L1 carve-out they leave.
+int kernel_geometry(const qlnlp_handle_s* h, const void* fn, int wj, size_t smem, int* blocks_per_sm)
+{
+    // the attributes are per FUNCTION, shared by every handle of the process: always raise the limit to the device's,
+    // never to this handle's own (possibly smaller) requirement
+    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
+    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    int nb = 0;
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, QL_LANES, smem));
+    if (nb < 1) return fail(QLNLP_ECUDA, "kernel does not fit on an SM");
+    // never more resident warps than the kernel was compiled for (its __launch_bounds__)
+    if (wj == ql::JM_NONE) nb = std::min(nb, QL_NONE_WARPS);
+    else if (wj != ql::JM_BLOCK) nb = std::min(nb, QL_TRUE_WARPS);
+    *blocks_per_sm = nb;
+    // Shared memory the resident warps really need: whatever the SM has beyond that serves as L1 (the cost table and
+    // the boundary states are re-read by every warp).  The attribute belongs to the FUNCTION, so it only ever grows
+    // (handles of other horizons share it).  launch() runs the SPARSE_BLOCK kernel on at most 6 CTAs per SM, each with
+    // its shared memory padded.
+    const int res = (wj == ql::JM_BLOCK) ? std::min(nb, 6) : nb;
+    const size_t per_block = (wj == ql::JM_BLOCK) ? padded_smem(h->smem_per_sm, h->smem_optin, res, smem) : smem;
+    return set_carveout(fn, res, per_block, h->smem_per_sm);
 }
 
 int check_handle(qlnlp_handle h)
@@ -515,36 +525,13 @@ int ensure_device(qlnlp_handle h)
 
     for (int wj = 0; wj < NJM; ++wj) {
         h->smem[wj] = ql::smem_bytes(h->cls.N, wj);
-        if (h->smem[wj] > (size_t)prop.sharedMemPerBlockOptin)
-            return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp (> %zu)", h->cls.N, h->smem[wj],
-                        (size_t)prop.sharedMemPerBlockOptin);
+        if (h->smem[wj] > h->smem_optin)
+            return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp (> %zu)", h->cls.N, h->smem[wj], h->smem_optin);
         for (int rg = 0; rg < 2; ++rg) {
             if (rg && wj == ql::JM_VALS) continue;
-            const void* fn = kernel_fn(wj, h->fastdiv, rg != 0);
-            // the attribute is per FUNCTION, shared by every handle of the process: always raise it to the device
-            // limit, never to this handle's own (possibly smaller) requirement
-            CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
-            CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
             int nb = 0;
-            CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, QL_LANES, h->smem[wj]));
-            if (nb < 1) return fail(QLNLP_ECUDA, "kernel does not fit on an SM");
-            // never more resident warps than the kernel was compiled for (its __launch_bounds__)
-            if (wj == ql::JM_NONE) nb = std::min(nb, QL_NONE_WARPS);
-            else if (wj != ql::JM_BLOCK) nb = std::min(nb, QL_TRUE_WARPS);
-            const char* env = std::getenv("QLNLP_BLOCKS_PER_SM");              // tuning knob: fewer resident warps per SM
-            if (env) {
-                const int cap = std::atoi(env);
-                if (cap >= 1 && cap < nb) nb = cap;
-            }
+            if (int rc = kernel_geometry(h, kernel_fn(wj, h->fastdiv, rg != 0), wj, h->smem[wj], &nb)) return rc;
             h->blocks_per_sm[wj] = rg ? std::min(h->blocks_per_sm[wj], nb) : nb;
-            // Shared memory the resident warps really need: whatever the SM has beyond that serves as L1 (the cost
-            // table and the boundary states are re-read by every warp).  The attribute belongs to the FUNCTION, so it
-            // only ever grows (handles of other horizons share it).
-            {
-                const int res = (wj == ql::JM_BLOCK && !env) ? std::min(nb, 6) : nb;
-                const size_t per_block = (wj == ql::JM_BLOCK) ? padded_smem(h->smem_per_sm, (size_t)prop.sharedMemPerBlockOptin, res, h->smem[wj]) : h->smem[wj];
-                if (int rc = set_carveout(fn, res, per_block, h->smem_per_sm)) return rc;
-            }
         }
     }
     for (auto& ln : h->lanes) {
@@ -650,17 +637,12 @@ int launch(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, cudaStream_t str
     int per_sm = rg ? table->blocks_per_sm[wj] : h->blocks_per_sm[wj];
     const size_t smem = rg ? table->smem[wj] : h->smem[wj];
     const bool fast = rg ? table->fastdiv : h->fastdiv;
-    if (wj == ql::JM_BLOCK && !std::getenv("QLNLP_BLOCKS_PER_SM")) {
+    if (wj == ql::JM_BLOCK) {
         const bool want_cost = io->f || io->grad;
         const bool short_batch = B < 8 * (int64_t)h->sm_count * 6;
         per_sm = std::min(per_sm, (want_cost && short_batch) ? 6 : 5);
     }
-    const int64_t resident = (int64_t)h->sm_count * per_sm;
-    int grid = (int)std::min<int64_t>(B, resident);
-    if (const char* e = std::getenv("QLNLP_GRID")) {                 // experiment knob: explicit grid size
-        const int gsz = std::atoi(e);
-        if (gsz >= 1 && gsz <= resident) grid = (int)std::min<int64_t>(B, gsz);
-    }
+    const int grid = (int)std::min<int64_t>(B, (int64_t)h->sm_count * per_sm);
     if (int rc = stream_ticket(h, stream, &P.ticket)) return rc;
     // With programmatic dependent launch the next grid's CTAs are placed as soon as an SM has room for one.  The
     // SPARSE_BLOCK kernel runs on fewer CTAs per SM than would fit (5 or 6 of up to 7 by shared memory): a spare slot
@@ -675,14 +657,14 @@ int launch(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, cudaStream_t str
     cfg.blockDim = dim3(QL_LANES);
     cfg.dynamicSmemBytes = smem_launch;
     cfg.stream = stream;
+    // programmatic dependent launch: back-to-back evaluations on a stream overlap the next grid's start-up with this
+    // grid's drain (B = 4,096: +1 % full evaluation, +4..6 % for the compact-output kernels; the kernel waits for its
+    // predecessors before it touches any data, see griddepcontrol.wait in eval_kernel)
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    // programmatic dependent launch: back-to-back evaluations on a stream overlap the next grid's start-up with this
-    // grid's drain (B = 4,096: +1 % full evaluation, +4..6 % for the compact-output kernels; the kernel waits for its
-    // predecessors before it touches any data, see griddepcontrol.wait in eval_kernel).  QLNLP_PDL=0 turns it off.
-    cfg.numAttrs = env_flag("QLNLP_PDL", true) ? 1 : 0;
+    cfg.numAttrs = 1;
     CUDA_TRY(cudaLaunchKernelExC(&cfg, kernel_fn(wj, fast, rg != nullptr), args));
     h->last_launch[0] = grid;
     h->last_launch[1] = QL_LANES;
@@ -733,23 +715,7 @@ int ragged_table(const qlnlp_handle* hs, int ncls, const RagTable** out)
         if (wj == ql::JM_VALS) continue;
         t.smem[wj] = ql::smem_bytes(t.layout.N, wj);
         if (t.smem[wj] > lead->smem_optin) return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp", t.layout.N, t.smem[wj]);
-        const void* fn = kernel_fn(wj, t.fastdiv, true);
-        int nb = 0;
-        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, QL_LANES, t.smem[wj]));
-        if (nb < 1) return fail(QLNLP_ECUDA, "kernel does not fit on an SM");
-        if (wj == ql::JM_NONE) nb = std::min(nb, QL_NONE_WARPS);
-        else if (wj != ql::JM_BLOCK) nb = std::min(nb, QL_TRUE_WARPS);
-        const char* env = std::getenv("QLNLP_BLOCKS_PER_SM");
-        if (env) {
-            const int cap = std::atoi(env);
-            if (cap >= 1 && cap < nb) nb = cap;
-        }
-        t.blocks_per_sm[wj] = nb;
-        {
-            const int res = (wj == ql::JM_BLOCK && !env) ? std::min(nb, 6) : nb;
-            const size_t per_block = (wj == ql::JM_BLOCK) ? padded_smem(lead->smem_per_sm, lead->smem_optin, res, t.smem[wj]) : t.smem[wj];
-            if (int rc = set_carveout(fn, res, per_block, lead->smem_per_sm)) return rc;
-        }
+        if (int rc = kernel_geometry(lead, kernel_fn(wj, t.fastdiv, true), wj, t.smem[wj], &t.blocks_per_sm[wj])) return rc;
     }
     *out = &lead->rag_tables.emplace(key, t).first->second;
     return QLNLP_OK;
@@ -942,27 +908,10 @@ bool is_registered(const qlnlp_handle_s* h, const double* jac, int64_t ldjac, in
 int eval_host_impl(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io)
 {
     const QlClass& c = h->cls;
-    const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(B, env_int("QLNLP_HOST_CHUNK", (int)h->opt_host_chunk)));
-    // Chunk schedule: uniform chunks.  QLNLP_HOST_RAMP=1 puts a quarter and a half chunk at either end (the first rows
-    // reach the row builder sooner, the last build is shorter); measured: no consistent gain (875 / 840 vs 856 / 855 k
-    // evals/s, profiles/r02_host_path.md) -- the D2H copies, not the fill, bound the pipeline -- so it is off.
-    std::vector<int64_t> c_start, c_size;
-    {
-        std::vector<int64_t> front, back;
-        if (B >= 3 * chunk && chunk >= 64 && env_flag("QLNLP_HOST_RAMP", false)) {
-            front = {chunk / 4, chunk / 2};
-            back = {chunk / 2, chunk / 4};
-        }
-        int64_t pos = 0, tail = 0;
-        for (int64_t v : back) tail += v;
-        for (int64_t v : front) { c_start.push_back(pos); c_size.push_back(v); pos += v; }
-        while (B - tail - pos > 0) {
-            const int64_t v = std::min(chunk, B - tail - pos);
-            c_start.push_back(pos); c_size.push_back(v); pos += v;
-        }
-        for (int64_t v : back) { c_start.push_back(pos); c_size.push_back(v); pos += v; }
-    }
-    const int64_t nchunks = (int64_t)c_start.size();
+    // Uniform chunks: chunk i is [i * chunk, min(B, (i + 1) * chunk)).  (Smaller chunks at either end measured no
+    // consistent gain, profiles/r02_host_path.md: the D2H copies, not the fill, bound the pipeline.)
+    const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(B, h->opt_host_chunk));
+    const int64_t nchunks = (B + chunk - 1) / chunk;
     const int nlanes = (int)std::min<int64_t>(MAX_LANES, nchunks);
     for (int l = 0; l < nlanes; ++l)
         if (int rc = reserve_lane(h, h->lanes[l], chunk)) return rc;
@@ -985,11 +934,10 @@ int eval_host_impl(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io)
     auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
     const double t_begin = now();
 
-    const bool vals_first = env_flag("QLNLP_HOST_VALS_FIRST", true);
     auto enqueue = [&](int64_t i) -> int {
         const double t0 = now();
         HostLane& ln = h->lanes[i % nlanes];
-        const int64_t b0 = c_start[(size_t)i], nb = c_size[(size_t)i];
+        const int64_t b0 = i * chunk, nb = std::min(chunk, B - b0);
         cudaStream_t s = ln.stream;
         CUDA_TRY(copy_rows(ln.Z, ldz_d, io->Z + b0 * io->ldz, io->ldz, c.n_nlp, nb, cudaMemcpyHostToDevice, s));
         if (io->x0) CUDA_TRY(cudaMemcpyAsync(ln.x0, io->x0 + b0 * QL_NX, sizeof(double) * nb * QL_NX, cudaMemcpyHostToDevice, s));
@@ -1006,19 +954,15 @@ int eval_host_impl(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io)
         if (int rc = h->kin ? launch_kin(h, nb, &d, s) : launch(h, nb, &d, s, compact ? ql::JM_VALS : -1)) return rc;
         // the staged values go first: the row builder only waits for them, f / grad / g land in the caller's arrays
         // by DMA while it works (the lanes are synchronised before the call returns)
-        if (compact && vals_first) {
+        if (compact) {
             CUDA_TRY(cudaMemcpyAsync(ln.stage, ln.jac, sizeof(double) * nb * h->ldv_e, cudaMemcpyDeviceToHost, s));
             CUDA_TRY(cudaEventRecord(ln.done, s));
         }
         if (io->f) CUDA_TRY(cudaMemcpyAsync(io->f + b0, ln.f, sizeof(double) * nb, cudaMemcpyDeviceToHost, s));
         if (io->grad) CUDA_TRY(copy_rows(io->grad + b0 * io->ldgrad, io->ldgrad, ln.grad, ldgrad_d, c.n_nlp, nb, cudaMemcpyDeviceToHost, s));
         if (io->g) CUDA_TRY(copy_rows(io->g + b0 * io->ldg, io->ldg, ln.g, ldg_d, m_out, nb, cudaMemcpyDeviceToHost, s));
-        if (compact && !vals_first) {
-            CUDA_TRY(cudaMemcpyAsync(ln.stage, ln.jac, sizeof(double) * nb * h->ldv_e, cudaMemcpyDeviceToHost, s));
-            CUDA_TRY(cudaEventRecord(ln.done, s));
-        } else if (!compact && io->jac) {
+        if (!compact && io->jac)
             CUDA_TRY(copy_rows(io->jac + b0 * io->ldjac, io->ldjac, ln.jac, ldjac_d, nnz_b, nb, cudaMemcpyDeviceToHost, s));
-        }
         h->stat_t_enqueue += now() - t0;
         return QLNLP_OK;
     };
@@ -1044,7 +988,7 @@ int eval_host_impl(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io)
             h->stat_t_wait += now() - t0;
             if (q == cudaErrorNotReady) return QLNLP_OK;
             if (q != cudaSuccess) return fail(QLNLP_ECUDA, "host pipeline: %s", cudaGetErrorString(q));
-            const int64_t b0 = c_start[(size_t)handed], nb = c_size[(size_t)handed];
+            const int64_t b0 = handed * chunk, nb = std::min(chunk, B - b0);
             double* rows = io->jac + b0 * io->ldjac;
             t_build0 = now();
             h->plan->build_async(h->pool.get(), ln.stage, h->ldv_e, rows, io->ldjac, nb, touched_only);
@@ -1125,37 +1069,29 @@ enum { HAVE_F = 1, HAVE_GRAD = 2, HAVE_G = 4, HAVE_J = 8 };
 int reserve_one(qlnlp_handle h)
 {
     OneEval& o = h->one;
-    if (o.hx) return QLNLP_OK;
+    if (o.mx) return QLNLP_OK;
     o.o_grad = 2;
     o.o_g = o.o_grad + h->ldgrad_e;
     o.o_vals = o.o_g + h->ldg_e;
     o.total = o.o_vals + h->ldv_e;
     // One decision vector is latency-bound: with mapped pinned memory the kernel fetches x and stores its 41 KB of
-    // results over PCIe itself, which saves the two copy calls (QLNLP_ONE_ZEROCOPY=0 goes back to explicit copies).
-    o.zero_copy = env_flag("QLNLP_ONE_ZEROCOPY", true);
-    CUDA_TRY(cudaHostAlloc(&o.hx, sizeof(double) * (h->ldz_e + o.total), o.zero_copy ? cudaHostAllocMapped : cudaHostAllocDefault));
+    // results over PCIe itself, which saves the two copy calls.
+    if (!o.hx) CUDA_TRY(cudaHostAlloc(&o.hx, sizeof(double) * (h->ldz_e + o.total), cudaHostAllocMapped));
     o.hout = o.hx + h->ldz_e;
-    if (o.zero_copy) {
-        void* dp = nullptr;
-        if (cudaHostGetDevicePointer(&dp, o.hx, 0) == cudaSuccess && dp) {
-            o.mx = static_cast<double*>(dp);
-            o.mout = o.mx + h->ldz_e;
-        } else {
-            cudaGetLastError();
-            o.zero_copy = false;
-        }
-    }
-    CUDA_TRY(cudaMalloc(&o.dx, sizeof(double) * h->ldz_e));
-    CUDA_TRY(cudaMalloc(&o.dout, sizeof(double) * o.total));
+    void* dp = nullptr;
+    CUDA_TRY(cudaHostGetDevicePointer(&dp, o.hx, 0));
+    o.mx = static_cast<double*>(dp);
+    o.mout = o.mx + h->ldz_e;
     o.valid = false;
     return QLNLP_OK;
 }
 
 // One decision vector on host pointers.  Ipopt asks for f, grad f, g and the Jacobian values of an iterate in four
 // separate callbacks (moi.jl:1-24): the first callback at a new x evaluates EVERYTHING with one launch (f, grad, g and
-// the value-dependent Jacobian entries: one H2D copy, one kernel, one D2H copy of 41 KB) and keeps the results; the
-// other callbacks at the same x (compared bit for bit, 9.7 KB) are served from that cache.  The Jacobian values are
-// assembled in the caller's array from the constant image of the pattern + the cached entries.
+// the value-dependent Jacobian entries: one kernel that reads x from and writes its 41 KB of results to mapped pinned
+// memory, see reserve_one) and keeps the results; the other callbacks at the same x (compared bit for bit, 9.7 KB) are
+// served from that cache.  The Jacobian values are assembled in the caller's array from the constant image of the
+// pattern + the cached entries.
 int eval_one(qlnlp_handle hh, const double* x, double* f, double* grad, double* g, double* vals)
 {
     if (int rc = check_handle(hh)) return rc;
@@ -1197,18 +1133,14 @@ int eval_one(qlnlp_handle hh, const double* x, double* f, double* grad, double* 
         o.valid = false;
         std::memcpy(o.hx, x, sizeof(double) * c.n_nlp);
         cudaStream_t s = o.stream;
-        double* const zin = o.zero_copy ? o.mx : o.dx;
-        double* const res = o.zero_copy ? o.mout : o.dout;
-        if (!o.zero_copy) CUDA_TRY(cudaMemcpyAsync(o.dx, o.hx, sizeof(double) * c.n_nlp, cudaMemcpyHostToDevice, s));
         qlnlp_batch_io d;
         std::memset(&d, 0, sizeof d);
-        d.Z = zin; d.ldz = o.zero_copy ? c.n_nlp : h->ldz_e;        // odd ld: plain (non-TMA) loads from host memory
-        d.f = res;
-        d.grad = res + o.o_grad; d.ldgrad = h->ldgrad_e;
-        d.g = res + o.o_g; d.ldg = h->ldg_e;
-        d.jac = res + o.o_vals; d.ldjac = o.zero_copy ? h->ldv_e + 1 : h->ldv_e;   // odd ld: plain stores into host memory
+        d.Z = o.mx; d.ldz = c.n_nlp;                                 // odd ld: plain (non-TMA) loads from host memory
+        d.f = o.mout;
+        d.grad = o.mout + o.o_grad; d.ldgrad = h->ldgrad_e;
+        d.g = o.mout + o.o_g; d.ldg = h->ldg_e;
+        d.jac = o.mout + o.o_vals; d.ldjac = h->ldv_e + 1;           // odd ld: plain stores into host memory
         if (int rc = launch(h, 1, &d, s, ql::JM_VALS)) return rc;
-        if (!o.zero_copy) CUDA_TRY(cudaMemcpyAsync(o.hout, o.dout, sizeof(double) * o.total, cudaMemcpyDeviceToHost, s));
         CUDA_TRY(cudaStreamSynchronize(s));
         o.valid = true;
     }
@@ -1281,7 +1213,6 @@ void destroy_device_state(qlnlp_handle h)
     }
     if (h->one.stream) cudaStreamDestroy(h->one.stream);
     if (h->one.hx) cudaFreeHost(h->one.hx);
-    cudaFree(h->one.dx); cudaFree(h->one.dout);
     cudaFree(h->d_hess_in); cudaFree(h->d_hess_out);
     cudaFree(h->d_kin_map);
     for (auto& kv : h->kin_scratch) cudaFree(kv.second.first);

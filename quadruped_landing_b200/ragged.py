@@ -26,10 +26,8 @@ class RaggedEvaluator:
         self.n = np.array([e.n_nlp for e in self.nlps], dtype=np.int64)
         self.m = np.array([e.m_nlp for e in self.nlps], dtype=np.int64)
         self.nnz = np.array([e.nnz_block for e in self.nlps], dtype=np.int64)
-        self._streams = None
         self._plan = None
         self.launches_per_eval = 1                     # one fused launch for the whole mixed batch
-        self.single_launch = True                      # False: one launch per class on its own stream (the older path)
 
     def offsets(self, class_of: np.ndarray) -> Dict[str, np.ndarray]:
         """Row starts (in doubles): problem b owns Z[z_off[b] : z_off[b] + n_b], g[g_off[b] : ...], jac[j_off[b] : ...].
@@ -49,25 +47,21 @@ class RaggedEvaluator:
         return Z
 
     def plan(self, class_of: np.ndarray, device=None) -> "RaggedPlan":
-        """Everything about a batch that does not depend on the decision vectors: the offset tables and each class's
-        problem list, uploaded once.  ``eval`` caches the plan of the last ``class_of`` it saw, so repeated
-        evaluations of one batch (solver iterations) do no per-call host work."""
+        """Everything about a batch that does not depend on the decision vectors: the offset tables and the launch
+        order, uploaded once.  ``eval`` caches the plan of the last ``class_of`` it saw, so repeated evaluations of
+        one batch (solver iterations) do no per-call host work."""
         import torch
 
         class_of = np.ascontiguousarray(class_of, dtype=np.int64)
         dev = torch.device("cuda", self.device) if device is None else device
         off = self.offsets(class_of)
         doff = {k: torch.from_numpy(v).to(dev) for k, v in off.items()}
-        index = []
-        for c in range(len(self.nlps)):
-            idx = np.nonzero(class_of == c)[0]
-            index.append(torch.from_numpy(idx).to(dev) if idx.size else None)
-        # single launch: all problems, ordered by class, largest horizon first (the long evaluations start first)
+        # all problems, ordered by class, largest horizon first (the long evaluations start first)
         by_class = sorted(range(len(self.nlps)), key=lambda c: -self.nlps[c].N)
         rank_of = np.empty(len(self.nlps), dtype=np.int64)
         rank_of[by_class] = np.arange(len(self.nlps))
         order = np.argsort(rank_of[class_of], kind="stable")
-        plan = RaggedPlan(class_of.copy(), off, doff, index)
+        plan = RaggedPlan(class_of.copy(), off, doff)
         plan.order = torch.from_numpy(order.astype(np.int64)).to(dev)
         plan.dclass = torch.from_numpy(class_of.astype(np.int32)).to(dev)
         return plan
@@ -78,8 +72,7 @@ class RaggedEvaluator:
         ``grad`` (Z layout), ``g``, ``jac`` and the offset tables; pass the returned dict back as ``out`` to reuse
         the output arrays.
 
-        The whole mixed batch is ONE ``qlnlp_eval_ragged_classes`` launch (``single_launch=False``: one
-        ``qlnlp_eval_ragged_device`` launch per class on its own stream); the kernel addresses each problem's rows
+        The whole mixed batch is ONE ``qlnlp_eval_ragged_classes`` launch; the kernel addresses each problem's rows
         through the offset tables, so nothing is gathered or scattered."""
         import torch
 
@@ -93,8 +86,6 @@ class RaggedEvaluator:
                 plan = self._plan = self.plan(class_of, dev)
         B = plan.class_of.shape[0]
         off = plan.off
-        if self._streams is None:
-            self._streams = [torch.cuda.Stream(device=dev) for _ in self.nlps]
         flat = {"Z": Z_flat}
         sizes = {"f": B, "grad": int(off["z_off"][-1]), "g": int(off["g_off"][-1]), "jac": int(off["j_off"][-1])}
         for name in ("f", "grad", "g", "jac"):
@@ -103,17 +94,7 @@ class RaggedEvaluator:
                 if t is None or t.numel() != sizes[name] or t.device != dev:
                     t = torch.empty(sizes[name], dtype=torch.float64, device=dev)
                 flat[name] = t
-        cur = torch.cuda.current_stream(dev)
-        if self.single_launch:
-            HybridNLP.eval_ragged_classes(self.nlps, plan.order, plan.dclass, flat, plan.doff, z_padded=True)
-        else:
-            for c, nlp in enumerate(self.nlps):
-                if plan.index[c] is None:
-                    continue
-                s = self._streams[c]
-                s.wait_stream(cur)
-                nlp.eval_ragged(plan.index[c], flat, plan.doff, stream=s, z_padded=True)
-                cur.wait_stream(s)
+        HybridNLP.eval_ragged_classes(self.nlps, plan.order, plan.dclass, flat, plan.doff, z_padded=True)
         res = {k: v for k, v in flat.items() if k != "Z"}
         res.update(off)
         self._keep = plan                  # alive until the next call: the launches are asynchronous
@@ -121,7 +102,7 @@ class RaggedEvaluator:
 
 
 class RaggedPlan:
-    """Offset tables (host + device) and per-class problem lists of one mixed batch (``RaggedEvaluator.plan``)."""
+    """Offset tables (host + device) and launch order of one mixed batch (``RaggedEvaluator.plan``)."""
 
-    def __init__(self, class_of, off, doff, index):
-        self.class_of, self.off, self.doff, self.index = class_of, off, doff, index
+    def __init__(self, class_of, off, doff):
+        self.class_of, self.off, self.doff = class_of, off, doff

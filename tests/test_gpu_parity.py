@@ -265,7 +265,7 @@ def test_c4_ragged_batch_of_mixed_horizons():
         assert_same_bits(ev.nlps[c], got, ref, f"problem {b} class {classes[c]}: ")
 
 
-def test_ragged_single_launch_equals_one_launch_per_class():
+def test_ragged_one_launch_equals_launch_per_class():
     """qlnlp_eval_ragged_classes (one launch, class records swapped per warp) against qlnlp_eval_ragged_device per class:
     identical bits, for a batch whose classes come in random order, including classes with a single problem."""
     classes = [(31, 11, 1), (2, 1, 2), (61, 21, 2), (121, 41, 1), (33, 33, 2), (65, 2, 1)]
@@ -282,14 +282,16 @@ def test_ragged_single_launch_equals_one_launch_per_class():
         v[19::20] = np.clip(v[19::20], 1e-3, 2e-2)
         vecs.append(v)
     Zd = torch.from_numpy(ev.pack(class_of, vecs)).cuda()
-    ev.single_launch = True
     one = {k: v.clone() for k, v in ev.eval(class_of, Zd).items() if isinstance(v, torch.Tensor)}
     torch.cuda.synchronize()
     assert ev.nlps[0].launch_info()["blocks"] > 0
-    ev.single_launch = False
-    per = ev.eval(class_of, Zd)
-    torch.cuda.synchronize()
+    # the reference: one qlnlp_eval_ragged_device launch per class over that class's problems
     off = ev.offsets(class_of)
+    doff = {k: torch.from_numpy(v).cuda() for k, v in off.items()}
+    per = {"Z": Zd, **{k: torch.empty_like(one[k]) for k in ("f", "grad", "g", "jac")}}
+    for c, nlp in enumerate(ev.nlps):
+        nlp.eval_ragged(torch.from_numpy(np.nonzero(class_of == c)[0]).cuda(), per, doff, z_padded=True)
+    torch.cuda.synchronize()
     for b in range(B):          # compare the rows themselves (the padding between rows is never written)
         e = ev.nlps[class_of[b]]
         for k, o, w in (("grad", "z_off", e.n_nlp), ("g", "g_off", e.m_nlp), ("jac", "j_off", e.nnz_block)):
@@ -297,7 +299,6 @@ def test_ragged_single_launch_equals_one_launch_per_class():
             assert torch.equal(one[k][lo:lo + w], per[k][lo:lo + w]), (b, k)
     assert torch.equal(one["f"], per["f"])
     # partial outputs through the single launch
-    ev.single_launch = True
     only = ev.eval(class_of, Zd, want=("g",))
     torch.cuda.synchronize()
     for b in range(0, B, 50):

@@ -15,19 +15,17 @@ Zf = ev.pack(class_of, [guesses[c] + 1e-2 * rng.standard_normal(probs[c].n_nlp) 
 Zd = torch.from_numpy(Zf).cuda()
 plan = ev.plan(class_of, Zd.device)
 bytes_total = 8 * int(sum(2 * ev.n[c] + ev.m[c] + ev.nnz[c] + 1 for c in class_of))
-for single in (True, False):
-    ev.single_launch = single
-    out = ev.eval(plan, Zd); torch.cuda.synchronize()
-    for want in (("f", "grad", "g", "jac"), ("g", "jac")):
-        for _ in range(2):
-            ev.eval(plan, Zd, out=out, want=want)
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        n = 8
-        e0.record()
-        for _ in range(n):
-            ev.eval(plan, Zd, out=out, want=want)
-        e1.record(); torch.cuda.synchronize()
-        dt = e0.elapsed_time(e1) / n * 1e-3
-        print(f"C4 ragged {'ONE launch' if single else 'launch per class'} {'+'.join(want):12s}: B={B}, {bytes_total / 1e9:.2f} GB per pass, "
-              f"{dt * 1e3:.2f} ms  {B / dt / 1e6:.2f} M evals/s  {bytes_total / dt / 1e12:.2f} TB/s  {ev.nlps[0].launch_info()}")
+out = ev.eval(plan, Zd); torch.cuda.synchronize()
+for want in (("f", "grad", "g", "jac"), ("g", "jac")):
+    for _ in range(2):
+        ev.eval(plan, Zd, out=out, want=want)
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    n = 8
+    e0.record()
+    for _ in range(n):
+        ev.eval(plan, Zd, out=out, want=want)
+    e1.record(); torch.cuda.synchronize()
+    dt = e0.elapsed_time(e1) / n * 1e-3
+    print(f"C4 ragged ONE launch {'+'.join(want):12s}: B={B}, {bytes_total / 1e9:.2f} GB per pass, "
+          f"{dt * 1e3:.2f} ms  {B / dt / 1e6:.2f} M evals/s  {bytes_total / dt / 1e12:.2f} TB/s  {ev.nlps[0].launch_info()}")

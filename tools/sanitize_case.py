@@ -53,8 +53,10 @@ zeros = lambda: {"f": torch.zeros(len(class_of), dtype=torch.float64, device="cu
                  "g": torch.zeros(int(off["g_off"][-1]), dtype=torch.float64, device="cuda"),
                  "jac": torch.zeros(int(off["j_off"][-1]), dtype=torch.float64, device="cuda")}
 a = ev.eval(class_of, Zd, out=zeros())           # (pre-zeroed: the padding element between rows is never written)
-ev.single_launch = False
-b = ev.eval(class_of, Zd, out=zeros())
+b = {"Z": Zd, **zeros()}                         # one qlnlp_eval_ragged_device launch per class
+doff = {k: torch.from_numpy(v).cuda() for k, v in off.items()}
+for c, nlp in enumerate(ev.nlps):
+    nlp.eval_ragged(torch.from_numpy(np.nonzero(class_of == c)[0]).cuda(), b, doff, z_padded=True)
 torch.cuda.synchronize()
 for kname in ("f", "grad", "g", "jac"):
     assert torch.equal(a[kname], b[kname]), kname
