@@ -102,68 +102,73 @@ struct RagTable {
     int blocks_per_sm[NJM] = {0, 0, 0, 0};
 };
 
-}  // namespace
-
-struct qlnlp_handle_s {
+// The problem a handle evaluates: built once when the handle is created, host memory only, read-only afterwards.
+struct Problem {
     QlClass cls;
-    int device = 0;
     int jac_mode = QLNLP_JAC_SPARSE_BLOCK;
+    // opt-in kinematic rows (qlnlp_kin.cuh): 2N more constraints, 8N more entries in either sparse pattern
+    bool kin = false;
+    double leg_reach = 0;              // l1 + l2 + lb/2
     double x0[QL_NX], xf[QL_NX];
     std::vector<double> cost;          // field-major [QL_NCOST][npad]
     int npad = 0;
     std::vector<QlSeg> segs;
     std::vector<int> seg_begin;
+    double rmb = 0, rmf = 0, rIb = 0;  // reciprocals of the divisors
+    bool fastdiv = false;              // reciprocal-FMA division verified exact for this model
+    uint64_t serial = 0;               // unique per handle ever created (addresses get reused)
+    int64_t ldz_e = 0, ldgrad_e = 0, ldg_e = 0, ldjac_e = 0, ldv_e = 0;   // even leading dimensions of the scratch
+};
 
-    // multi-device parent: one complete handle per device; the parent itself only answers the integer queries
-    std::vector<qlnlp_handle_s*> subs;
-    std::vector<std::unique_ptr<qlhost::Worker>> drivers;
-    int part = 0, nparts = 1;          // this handle's share of the host cores (multi-device handles split them)
-
-    // device state, created at the first evaluation
-    bool dev_ready = false;
+// What one device of a handle holds, created at its first evaluation (ensure_device).
+struct DeviceState {
+    int device = 0;
+    bool ready = false;
+    std::string pci_bus_id;
+    int sm_count = 0;
+    size_t smem_per_sm = 0, smem_optin = 0;
+    int blocks_per_sm[NJM] = {0, 0, 0, 0};
+    size_t smem[NJM] = {0, 0, 0, 0};
     double* d_cost = nullptr;
     double* d_x0xf = nullptr;          // x0[15] | xf[15]
     QlSeg* d_segs = nullptr;
     int* d_seg_begin = nullptr;
     long long* d_dense_lin = nullptr;  // DENSE mode: linear index of every SPARSE_BLOCK value
     double* d_dense = nullptr;         // DENSE mode: m x n grid
-    int sm_count = 0;
-    int blocks_per_sm[NJM] = {0, 0, 0, 0};
-    size_t smem[NJM] = {0, 0, 0, 0};
-    double rmb = 0, rmf = 0, rIb = 0;  // reciprocals of the divisors
-    bool fastdiv = false;              // reciprocal-FMA division verified exact for this model
-    int64_t last_launch[5] = {0, 0, 0, 0, 0};
     HostLane lanes[MAX_LANES];
     OneEval one;
-    std::map<cudaStream_t, unsigned*> tickets;   // work counters, one pair per stream the handle has launched on
+    std::map<cudaStream_t, unsigned*> tickets;   // work counters, one pair per stream the device has launched on
     unsigned* ticket_pool = nullptr;             // pre-zeroed counters (128 B apart) so that a launch needs no
     int ticket_pool_used = 0;                    // allocation: launches stay legal inside CUDA-graph capture
-    std::string pci_bus_id;
     // Lagrangian Hessian (single evaluations on host pointers): device scratch x | lambda | values
     double* d_hess_in = nullptr;
     double* d_hess_out = nullptr;
     int hess_blocks_per_sm = 0;
-    size_t smem_per_sm = 0, smem_optin = 0;
-    // opt-in kinematic rows (qlnlp_kin.cuh): 2N more constraints, 8N more entries in either sparse pattern
-    bool kin = false;
-    double leg_reach = 0;              // l1 + l2 + lb/2
-    std::vector<int32_t> kin_map;      // caller-visible value order of the batch pattern -> scratch position or -(entry + 1)
-    int* d_kin_map = nullptr;
+    int* d_kin_map = nullptr;          // caller-visible value order of the batch pattern -> scratch position or -(entry + 1)
     std::map<cudaStream_t, std::pair<double*, int64_t>> kin_scratch;   // per stream: reference-order rows (device), capacity
-    uint64_t serial = 0;               // unique per handle ever created (addresses get reused)
     std::map<std::vector<uint64_t>, RagTable> rag_tables;       // ragged launches led by this handle (key: the classes' serials)
-
-    // host-pointer path: row plan of the handle's batch pattern, worker pool, registered output buffers
-    std::unique_ptr<qlhost::RowPlan> plan;
-    std::unique_ptr<qlhost::Pool> pool;
-    std::vector<Registration> regs;
-    int64_t opt_host_chunk = 512;
-    int64_t opt_host_threads = 0;      // 0: this handle's share of the process's CPUs
-    int64_t opt_pin_threads = 1;
-    int64_t opt_x_cache = 1;
-    int64_t ldz_e = 0, ldgrad_e = 0, ldg_e = 0, ldjac_e = 0, ldv_e = 0;   // even leading dimensions of the scratch
+    int64_t last_launch[5] = {0, 0, 0, 0, 0};
+    std::unique_ptr<qlhost::Pool> pool;                                  // row builders of the host-pointer path
     int64_t stat_host_rows = 0, stat_host_lines = 0;                     // rows / 64-byte lines the row builder wrote
     double stat_t_enqueue = 0, stat_t_wait = 0, stat_t_build = 0, stat_t_total = 0;   // seconds, host-pointer batches
+};
+
+}  // namespace
+
+struct qlnlp_handle_s {
+    Problem prob;
+    std::vector<DeviceState> devs;     // one per device: a handle from qlnlp_create has one
+    bool multi = false;                // from qlnlp_create_multi: the single-device entry points refuse it
+    std::vector<std::unique_ptr<qlhost::Worker>> drivers;   // multi: one thread per device runs its host-pointer shard
+
+    // host-pointer path: row plan of the batch pattern, registered output buffers.  The driver threads share both and
+    // only read them: the plan is built before a shard is handed to a driver.
+    std::unique_ptr<qlhost::RowPlan> plan;
+    std::vector<Registration> regs;
+    int64_t opt_host_chunk = 512;
+    int64_t opt_host_threads = 0;      // 0: each device's share of the process's CPUs
+    int64_t opt_pin_threads = 1;
+    int64_t opt_x_cache = 1;
 };
 
 namespace {
@@ -265,12 +270,12 @@ const void* kernel_fn(int jm, bool fast, bool ragged)
     return kernel_fn_jm<ql::JM_NONE>(fast, ragged);
 }
 
-// the sparse pattern batched evaluations of this handle produce (DENSE handles batch in SPARSE_BLOCK)
-int batch_jm(const qlnlp_handle_s* h) { return h->jac_mode == QLNLP_JAC_SPARSE_TRUE ? ql::JM_TRUE : ql::JM_BLOCK; }
-int std_nnz(const qlnlp_handle_s* h) { return h->jac_mode == QLNLP_JAC_SPARSE_TRUE ? h->cls.nnz_true : h->cls.nnz; }
+// the sparse pattern batched evaluations of this problem produce (DENSE handles batch in SPARSE_BLOCK)
+int batch_jm(const Problem& p) { return p.jac_mode == QLNLP_JAC_SPARSE_TRUE ? ql::JM_TRUE : ql::JM_BLOCK; }
+int std_nnz(const Problem& p) { return p.jac_mode == QLNLP_JAC_SPARSE_TRUE ? p.cls.nnz_true : p.cls.nnz; }
 // what the caller sees: the kinematic rows add 8 entries per knot to either pattern and 2 rows per knot to g
-int batch_nnz(const qlnlp_handle_s* h) { return std_nnz(h) + (h->kin ? 8 * h->cls.N : 0); }
-int m_rows(const qlnlp_handle_s* h) { return h->cls.m_nlp + (h->kin ? 2 * h->cls.N : 0); }
+int batch_nnz(const Problem& p) { return std_nnz(p) + (p.kin ? 8 * p.cls.N : 0); }
+int m_rows(const Problem& p) { return p.cls.m_nlp + (p.kin ? 2 * p.cls.N : 0); }
 int jm_nnz(const QlClass& c, int jm) { return jm == ql::JM_TRUE ? c.nnz_true : jm == ql::JM_VALS ? c.nnz_vals : c.nnz; }
 
 // SPARSE_TRUE structure (1-based, value order): like sparse_block_structure restricted to structural non-zeros
@@ -357,29 +362,37 @@ void block_image_and_vals_map(const QlClass& c, std::vector<double>& image, std:
     }
 }
 
-// Row plan of the handle's batch pattern (SPARSE_BLOCK, or SPARSE_TRUE as a sub-sequence of it).
-int ensure_plan(qlnlp_handle h)
+// The constant image and the VALS positions of a row of the problem's batch pattern (SPARSE_BLOCK, or SPARSE_TRUE as a
+// sub-sequence of it).
+int batch_image_and_vals_map(const Problem& p, std::vector<double>& image, std::vector<int32_t>& pos)
 {
-    if (h->plan) return QLNLP_OK;
-    const QlClass& c = h->cls;
-    std::vector<double> image;
-    std::vector<int32_t> pos;
+    const QlClass& c = p.cls;
     block_image_and_vals_map(c, image, pos);
     if ((int)pos.size() != c.nnz_vals) return fail(QLNLP_ECUDA, "internal: VALS map has %zu entries, layout says %d", pos.size(), c.nnz_vals);
     for (size_t i = 1; i < pos.size(); ++i)
         if (pos[i] <= pos[i - 1]) return fail(QLNLP_ECUDA, "internal: VALS map is not ascending at %zu", i);
-    if (batch_jm(h) == ql::JM_TRUE) {
+    if (batch_jm(p) == ql::JM_TRUE) {
         const std::vector<int32_t> t2b = true_to_block(c);
         std::vector<int32_t> b2t((size_t)c.nnz, -1);
         for (size_t t = 0; t < t2b.size(); ++t) b2t[(size_t)t2b[t]] = (int32_t)t;
         std::vector<double> timage(t2b.size());
         for (size_t t = 0; t < t2b.size(); ++t) timage[t] = image[(size_t)t2b[t]];
-        for (auto& p : pos) {
-            if (b2t[(size_t)p] < 0) return fail(QLNLP_ECUDA, "internal: value-dependent entry outside SPARSE_TRUE");
-            p = b2t[(size_t)p];
+        for (auto& q : pos) {
+            if (b2t[(size_t)q] < 0) return fail(QLNLP_ECUDA, "internal: value-dependent entry outside SPARSE_TRUE");
+            q = b2t[(size_t)q];
         }
         image.swap(timage);
     }
+    return QLNLP_OK;
+}
+
+// Row plan of the handle's batch pattern.
+int ensure_plan(qlnlp_handle h)
+{
+    if (h->plan) return QLNLP_OK;
+    std::vector<double> image;
+    std::vector<int32_t> pos;
+    if (int rc = batch_image_and_vals_map(h->prob, image, pos)) return rc;
     h->plan.reset(new (std::nothrow) qlhost::RowPlan((int64_t)image.size(), image.data(), (int64_t)pos.size(), pos.data()));
     if (!h->plan) return fail(QLNLP_ENOMEM, "out of host memory");
     return QLNLP_OK;
@@ -394,17 +407,18 @@ int env_int(const char* name, int dflt)
     return dflt;
 }
 
-// The worker pool of this handle: its share of the CPUs the process may use.  With one process per GPU (torchrun)
-// the ranks of a node split the cores (LOCAL_RANK of LOCAL_WORLD_SIZE); a multi-device handle splits its share
-// again between its devices; on a multi-socket host the share is taken from the CPUs next to the GPU.
-int ensure_pool(qlnlp_handle h)
+// The worker pool of device i of the handle: its share of the CPUs the process may use.  With one process per GPU
+// (torchrun) the ranks of a node split the cores (LOCAL_RANK of LOCAL_WORLD_SIZE); a multi-device handle splits its
+// share again between its devices; on a multi-socket host the share is taken from the CPUs next to the GPU.
+int ensure_pool(qlnlp_handle h, int i)
 {
-    if (h->pool) return QLNLP_OK;
+    DeviceState& ds = h->devs[(size_t)i];
+    if (ds.pool) return QLNLP_OK;
     const int lws = env_int("LOCAL_WORLD_SIZE", 1);
     const int lr = std::getenv("LOCAL_RANK") ? std::atoi(std::getenv("LOCAL_RANK")) : 0;
     const std::vector<int> all = qlhost::affinity_cpus();
-    std::vector<int> near = qlhost::cpus_near_pci_device(h->pci_bus_id.c_str());
-    const int nparts = lws * h->nparts, part = lr * h->nparts + h->part;
+    std::vector<int> near = qlhost::cpus_near_pci_device(ds.pci_bus_id.c_str());
+    const int ndev = (int)h->devs.size(), nparts = lws * ndev, part = lr * ndev + i;
     std::vector<int> mine;
     if (near.size() == all.size() || near.empty()) {
         mine = qlhost::cpu_slice(all, part, nparts);
@@ -418,8 +432,8 @@ int ensure_pool(qlnlp_handle h)
     if (h->opt_host_threads > 0) T = (int)h->opt_host_threads;
     T = env_int("QLNLP_HOST_THREADS", T);
     T = std::max(1, std::min(T, 256));
-    h->pool.reset(new (std::nothrow) qlhost::Pool(T, mine, h->opt_pin_threads != 0));
-    if (!h->pool) return fail(QLNLP_ENOMEM, "out of host memory");
+    ds.pool.reset(new (std::nothrow) qlhost::Pool(T, mine, h->opt_pin_threads != 0));
+    if (!ds.pool) return fail(QLNLP_ENOMEM, "out of host memory");
     return QLNLP_OK;
 }
 
@@ -460,12 +474,12 @@ int set_carveout(const void* fn, int resident_blocks, size_t smem_per_block, siz
 }
 
 // Launch geometry of the eval kernel `fn` (value stream `wj`) at `smem` bytes of dynamic shared memory per CTA on the
-// handle's device: the resident CTAs per SM, and the L1 carve-out they leave.
-int kernel_geometry(const qlnlp_handle_s* h, const void* fn, int wj, size_t smem, int* blocks_per_sm)
+// device `ds`: the resident CTAs per SM, and the L1 carve-out they leave.
+int kernel_geometry(const DeviceState& ds, const void* fn, int wj, size_t smem, int* blocks_per_sm)
 {
     // the attributes are per FUNCTION, shared by every handle of the process: always raise the limit to the device's,
     // never to this handle's own (possibly smaller) requirement
-    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
+    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ds.smem_optin));
     CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     int nb = 0;
     CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, QL_LANES, smem));
@@ -479,8 +493,8 @@ int kernel_geometry(const qlnlp_handle_s* h, const void* fn, int wj, size_t smem
     // (handles of other horizons share it).  launch() runs the SPARSE_BLOCK kernel on at most 6 CTAs per SM, each with
     // its shared memory padded.
     const int res = (wj == ql::JM_BLOCK) ? std::min(nb, 6) : nb;
-    const size_t per_block = (wj == ql::JM_BLOCK) ? padded_smem(h->smem_per_sm, h->smem_optin, res, smem) : smem;
-    return set_carveout(fn, res, per_block, h->smem_per_sm);
+    const size_t per_block = (wj == ql::JM_BLOCK) ? padded_smem(ds.smem_per_sm, ds.smem_optin, res, smem) : smem;
+    return set_carveout(fn, res, per_block, ds.smem_per_sm);
 }
 
 int check_handle(qlnlp_handle h)
@@ -488,79 +502,71 @@ int check_handle(qlnlp_handle h)
     if (!h) return fail(QLNLP_EINVAL, "null handle");
     return QLNLP_OK;
 }
-// the handle that owns device state: a multi-device parent forwards single-device work to its first device
-qlnlp_handle first(qlnlp_handle h) { return h->subs.empty() ? h : h->subs[0]; }
 
-// Binds the handle to its device (first call: tables, occupancy, streams).  The caller holds a DeviceGuard.
-int ensure_device(qlnlp_handle h)
+// Binds one device of a handle (first call: tables, occupancy, streams).  The caller holds a DeviceGuard.
+int ensure_device(const Problem& p, DeviceState& ds)
 {
-    if (h->dev_ready) return QLNLP_OK;
+    if (ds.ready) return QLNLP_OK;
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
     if (e != cudaSuccess || ndev == 0)
         return fail(QLNLP_ENODEVICE, "no CUDA device available (%s); this library has no CPU path",
                     e == cudaSuccess ? "device count 0" : cudaGetErrorString(e));
-    if (h->device < 0 || h->device >= ndev) return fail(QLNLP_EINVAL, "device %d out of range (0..%d)", h->device, ndev - 1);
-    CUDA_TRY(cudaSetDevice(h->device));
+    if (ds.device < 0 || ds.device >= ndev) return fail(QLNLP_EINVAL, "device %d out of range (0..%d)", ds.device, ndev - 1);
+    CUDA_TRY(cudaSetDevice(ds.device));
     cudaDeviceProp prop;
-    CUDA_TRY(cudaGetDeviceProperties(&prop, h->device));
+    CUDA_TRY(cudaGetDeviceProperties(&prop, ds.device));
     if (prop.major != 10)
-        return fail(QLNLP_ENODEVICE, "device %d is sm_%d%d; this build targets sm_100a (B200) only", h->device, prop.major,
+        return fail(QLNLP_ENODEVICE, "device %d is sm_%d%d; this build targets sm_100a (B200) only", ds.device, prop.major,
                     prop.minor);
-    h->sm_count = prop.multiProcessorCount;
-    h->smem_per_sm = prop.sharedMemPerMultiprocessor;
-    h->smem_optin = prop.sharedMemPerBlockOptin;
+    ds.sm_count = prop.multiProcessorCount;
+    ds.smem_per_sm = prop.sharedMemPerMultiprocessor;
+    ds.smem_optin = prop.sharedMemPerBlockOptin;
     char bus[32] = {0};
-    if (cudaDeviceGetPCIBusId(bus, sizeof bus, h->device) == cudaSuccess) h->pci_bus_id = bus;
+    if (cudaDeviceGetPCIBusId(bus, sizeof bus, ds.device) == cudaSuccess) ds.pci_bus_id = bus;
 
-    CUDA_TRY(cudaMalloc(&h->d_cost, h->cost.size() * sizeof(double)));
-    CUDA_TRY(cudaMemcpy(h->d_cost, h->cost.data(), h->cost.size() * sizeof(double), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMalloc(&h->d_x0xf, 2 * QL_NX * sizeof(double)));
-    CUDA_TRY(cudaMemcpy(h->d_x0xf, h->x0, QL_NX * sizeof(double), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(h->d_x0xf + QL_NX, h->xf, QL_NX * sizeof(double), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMalloc(&h->d_segs, h->segs.size() * sizeof(QlSeg)));
-    CUDA_TRY(cudaMemcpy(h->d_segs, h->segs.data(), h->segs.size() * sizeof(QlSeg), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMalloc(&h->d_seg_begin, h->seg_begin.size() * sizeof(int)));
-    CUDA_TRY(cudaMemcpy(h->d_seg_begin, h->seg_begin.data(), h->seg_begin.size() * sizeof(int), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMalloc(&ds.d_cost, p.cost.size() * sizeof(double)));
+    CUDA_TRY(cudaMemcpy(ds.d_cost, p.cost.data(), p.cost.size() * sizeof(double), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMalloc(&ds.d_x0xf, 2 * QL_NX * sizeof(double)));
+    CUDA_TRY(cudaMemcpy(ds.d_x0xf, p.x0, QL_NX * sizeof(double), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(ds.d_x0xf + QL_NX, p.xf, QL_NX * sizeof(double), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMalloc(&ds.d_segs, p.segs.size() * sizeof(QlSeg)));
+    CUDA_TRY(cudaMemcpy(ds.d_segs, p.segs.data(), p.segs.size() * sizeof(QlSeg), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMalloc(&ds.d_seg_begin, p.seg_begin.size() * sizeof(int)));
+    CUDA_TRY(cudaMemcpy(ds.d_seg_begin, p.seg_begin.data(), p.seg_begin.size() * sizeof(int), cudaMemcpyHostToDevice));
 
     for (int wj = 0; wj < NJM; ++wj) {
-        h->smem[wj] = ql::smem_bytes(h->cls.N, wj);
-        if (h->smem[wj] > h->smem_optin)
-            return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp (> %zu)", h->cls.N, h->smem[wj], h->smem_optin);
+        ds.smem[wj] = ql::smem_bytes(p.cls.N, wj);
+        if (ds.smem[wj] > ds.smem_optin)
+            return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp (> %zu)", p.cls.N, ds.smem[wj], ds.smem_optin);
         for (int rg = 0; rg < 2; ++rg) {
             if (rg && wj == ql::JM_VALS) continue;
             int nb = 0;
-            if (int rc = kernel_geometry(h, kernel_fn(wj, h->fastdiv, rg != 0), wj, h->smem[wj], &nb)) return rc;
-            h->blocks_per_sm[wj] = rg ? std::min(h->blocks_per_sm[wj], nb) : nb;
+            if (int rc = kernel_geometry(ds, kernel_fn(wj, p.fastdiv, rg != 0), wj, ds.smem[wj], &nb)) return rc;
+            ds.blocks_per_sm[wj] = rg ? std::min(ds.blocks_per_sm[wj], nb) : nb;
         }
     }
-    for (auto& ln : h->lanes) {
+    for (auto& ln : ds.lanes) {
         CUDA_TRY(cudaStreamCreateWithFlags(&ln.stream, cudaStreamNonBlocking));
         CUDA_TRY(cudaEventCreateWithFlags(&ln.done, cudaEventDisableTiming));
     }
-    CUDA_TRY(cudaStreamCreateWithFlags(&h->one.stream, cudaStreamNonBlocking));
-    CUDA_TRY(cudaMalloc(&h->ticket_pool, 128 * TICKET_POOL));
-    CUDA_TRY(cudaMemset(h->ticket_pool, 0, 128 * TICKET_POOL));
-    const QlClass& c = h->cls;
-    h->ldz_e = (c.n_nlp + 1) & ~1;
-    h->ldgrad_e = h->ldz_e;
-    h->ldg_e = (m_rows(h) + 1) & ~1;
-    h->ldjac_e = (batch_nnz(h) + 1) & ~1;
-    h->ldv_e = (c.nnz_vals + 1) & ~1;
+    CUDA_TRY(cudaStreamCreateWithFlags(&ds.one.stream, cudaStreamNonBlocking));
+    CUDA_TRY(cudaMalloc(&ds.ticket_pool, 128 * TICKET_POOL));
+    CUDA_TRY(cudaMemset(ds.ticket_pool, 0, 128 * TICKET_POOL));
     // the set-up copies above ran on the legacy default stream and may still be in flight when cudaMemcpy returns
     // (pageable source); launches go to arbitrary, possibly non-blocking streams, so finish the set-up first
     CUDA_TRY(cudaDeviceSynchronize());
-    h->dev_ready = true;
+    ds.ready = true;
     return QLNLP_OK;
 }
 
 // Work counter of a stream (launches on one stream are ordered, so they can share it; the kernel's last CTA re-arms
-// it).  Concurrent launches of the handle on different streams get different counters.
-int stream_ticket(qlnlp_handle h, cudaStream_t stream, unsigned** out)
+// it).  Concurrent launches on the device on different streams get different counters.
+int stream_ticket(DeviceState& ds, cudaStream_t stream, unsigned** out)
 {
-    auto it = h->tickets.find(stream);
-    if (it == h->tickets.end()) {
-        if (h->ticket_pool_used >= TICKET_POOL) {
+    auto it = ds.tickets.find(stream);
+    if (it == ds.tickets.end()) {
+        if (ds.ticket_pool_used >= TICKET_POOL) {
             // Every counter of the pre-zeroed pool belongs to a stream.  Streams come and go (torch pools), so wait
             // for the handle's outstanding launches and start the pool over rather than allocating (an allocation
             // here would make the launch illegal inside a CUDA-graph capture, and a faulted kernel could leave a
@@ -570,22 +576,22 @@ int stream_ticket(qlnlp_handle h, cudaStream_t stream, unsigned** out)
             if (cap != cudaStreamCaptureStatusNone)
                 return fail(QLNLP_EINVAL, "more than %d streams used with this handle: cannot recycle work counters during a graph capture", TICKET_POOL);
             CUDA_TRY(cudaDeviceSynchronize());
-            CUDA_TRY(cudaMemset(h->ticket_pool, 0, 128 * TICKET_POOL));
+            CUDA_TRY(cudaMemset(ds.ticket_pool, 0, 128 * TICKET_POOL));
             CUDA_TRY(cudaDeviceSynchronize());
-            h->tickets.clear();
-            h->ticket_pool_used = 0;
+            ds.tickets.clear();
+            ds.ticket_pool_used = 0;
         }
-        unsigned* d = h->ticket_pool + 32 * h->ticket_pool_used++;      // zeroed (and synchronised) at set-up
-        it = h->tickets.emplace(stream, d).first;
+        unsigned* d = ds.ticket_pool + 32 * ds.ticket_pool_used++;      // zeroed (and synchronised) at set-up
+        it = ds.tickets.emplace(stream, d).first;
     }
     *out = it->second;
     return QLNLP_OK;
 }
 
-int launch(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, cudaStream_t stream, int jm_force = -1,
+int launch(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* io, cudaStream_t stream, int jm_force = -1,
            const qlnlp_ragged_io* rg = nullptr, const RagTable* table = nullptr, const int32_t* class_of = nullptr)
 {
-    const QlClass& c = h->cls;
+    const QlClass& c = p.cls;
     if (rg && !table) return fail(QLNLP_EINVAL, "internal: ragged launch without a class table");
     if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
     if (B == 0) return QLNLP_OK;          // an empty shard is not an error (its pointers may be NULL)
@@ -598,7 +604,7 @@ int launch(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, cudaStream_t str
         if (io->grad && io->ldgrad < c.n_nlp) return fail(QLNLP_EINVAL, "ldgrad %lld < n_nlp %d", (long long)io->ldgrad, c.n_nlp);
         if (io->g && io->ldg < c.m_nlp) return fail(QLNLP_EINVAL, "ldg %lld < m_nlp %d", (long long)io->ldg, c.m_nlp);
     }
-    const int jm_jac = jm_force >= 0 ? jm_force : batch_jm(h);
+    const int jm_jac = jm_force >= 0 ? jm_force : batch_jm(p);
     const int nnz_jac = jm_nnz(c, jm_jac);
     if (!rg && io->jac && io->ldjac < nnz_jac) return fail(QLNLP_EINVAL, "ldjac %lld < nnz %d", (long long)io->ldjac, nnz_jac);
     if ((reinterpret_cast<uintptr_t>(io->Z) & 7) != 0) return fail(QLNLP_EINVAL, "Z must be 8-byte aligned");
@@ -607,14 +613,14 @@ int launch(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, cudaStream_t str
     P.c = rg ? table->layout : c;
     P.classes = rg ? table->d_classes : nullptr;
     P.cls_of = rg ? reinterpret_cast<const int*>(class_of) : nullptr;
-    P.rmb = h->rmb; P.rmf = h->rmf; P.rIb = h->rIb;
-    P.cost = h->d_cost;
-    P.npad = h->npad;
-    P.nseg = (int)h->segs.size();
-    P.x0_def = h->d_x0xf;
-    P.xf_def = h->d_x0xf + QL_NX;
-    P.segs = h->d_segs;
-    P.seg_begin = h->d_seg_begin;
+    P.rmb = p.rmb; P.rmf = p.rmf; P.rIb = p.rIb;
+    P.cost = ds.d_cost;
+    P.npad = p.npad;
+    P.nseg = (int)p.segs.size();
+    P.x0_def = ds.d_x0xf;
+    P.xf_def = ds.d_x0xf + QL_NX;
+    P.segs = ds.d_segs;
+    P.seg_begin = ds.d_seg_begin;
     P.Z = io->Z; P.ldz = io->ldz;
     P.x0 = io->x0; P.xf = io->xf;
     P.f = io->f;
@@ -634,23 +640,23 @@ int launch(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, cudaStream_t str
     // Resident warps per SM.  The SPARSE_BLOCK stream is store-bound and the memory system takes the output of a
     // few fast warps better than that of all 8 that fit (occupancy sweeps in profiles/r01_ablation.md, section 7):
     // 5 per SM, 6 for short batches that also want the cost/gradient.
-    int per_sm = rg ? table->blocks_per_sm[wj] : h->blocks_per_sm[wj];
-    const size_t smem = rg ? table->smem[wj] : h->smem[wj];
-    const bool fast = rg ? table->fastdiv : h->fastdiv;
+    int per_sm = rg ? table->blocks_per_sm[wj] : ds.blocks_per_sm[wj];
+    const size_t smem = rg ? table->smem[wj] : ds.smem[wj];
+    const bool fast = rg ? table->fastdiv : p.fastdiv;
     if (wj == ql::JM_BLOCK) {
         const bool want_cost = io->f || io->grad;
-        const bool short_batch = B < 8 * (int64_t)h->sm_count * 6;
+        const bool short_batch = B < 8 * (int64_t)ds.sm_count * 6;
         per_sm = std::min(per_sm, (want_cost && short_batch) ? 6 : 5);
     }
-    const int grid = (int)std::min<int64_t>(B, (int64_t)h->sm_count * per_sm);
-    if (int rc = stream_ticket(h, stream, &P.ticket)) return rc;
+    const int grid = (int)std::min<int64_t>(B, (int64_t)ds.sm_count * per_sm);
+    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
     // With programmatic dependent launch the next grid's CTAs are placed as soon as an SM has room for one.  The
     // SPARSE_BLOCK kernel runs on fewer CTAs per SM than would fit (5 or 6 of up to 7 by shared memory): a spare slot
     // would take a CTA of the next grid while this grid is still running at full strength, and the next grid would
     // start out unevenly spread over the SMs (measured: -5 % on the headline once another handle had raised the
     // kernel's carve-out to 228 KB).  Ask for enough shared memory per CTA that per_sm + 1 of them never fit.
     // (Only that kernel: the others are capped by their registers, and padding them would cost L1.)
-    const size_t smem_launch = (wj == ql::JM_BLOCK) ? padded_smem(h->smem_per_sm, h->smem_optin, per_sm, smem) : smem;
+    const size_t smem_launch = (wj == ql::JM_BLOCK) ? padded_smem(ds.smem_per_sm, ds.smem_optin, per_sm, smem) : smem;
     void* args[] = {&P};
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid);
@@ -666,42 +672,44 @@ int launch(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, cudaStream_t str
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     CUDA_TRY(cudaLaunchKernelExC(&cfg, kernel_fn(wj, fast, rg != nullptr), args));
-    h->last_launch[0] = grid;
-    h->last_launch[1] = QL_LANES;
-    h->last_launch[2] = (int64_t)smem_launch;
-    h->last_launch[3] = per_sm;
-    h->last_launch[4] = h->sm_count;
+    ds.last_launch[0] = grid;
+    ds.last_launch[1] = QL_LANES;
+    ds.last_launch[2] = (int64_t)smem_launch;
+    ds.last_launch[3] = per_sm;
+    ds.last_launch[4] = ds.sm_count;
     return QLNLP_OK;
 }
 
-// The class table of a ragged launch over the handles `hs` (all on one device, already bound to it), cached in hs[0].
+// The class table of a ragged launch over the single-device handles `hs` (all on one device, already bound to it),
+// cached in the device state of hs[0].
 int ragged_table(const qlnlp_handle* hs, int ncls, const RagTable** out)
 {
-    qlnlp_handle lead = hs[0];
+    DeviceState& lead = hs[0]->devs[0];
     std::vector<uint64_t> key((size_t)ncls);
-    for (int i = 0; i < ncls; ++i) key[(size_t)i] = hs[i]->serial;
-    auto it = lead->rag_tables.find(key);
-    if (it != lead->rag_tables.end()) { *out = &it->second; return QLNLP_OK; }
+    for (int i = 0; i < ncls; ++i) key[(size_t)i] = hs[i]->prob.serial;
+    auto it = lead.rag_tables.find(key);
+    if (it != lead.rag_tables.end()) { *out = &it->second; return QLNLP_OK; }
     RagTable t;
     t.ncls = ncls;
     t.fastdiv = true;
-    t.layout = hs[0]->cls;
+    t.layout = hs[0]->prob.cls;
     std::vector<ql::QlRagClass> host((size_t)ncls);
     for (int i = 0; i < ncls; ++i) {
-        qlnlp_handle h = hs[i];
+        const Problem& p = hs[i]->prob;
+        const DeviceState& ds = hs[i]->devs[0];
         ql::QlRagClass& r = host[(size_t)i];
         std::memset(&r, 0, sizeof r);
-        r.c = h->cls;
-        r.rmb = h->rmb; r.rmf = h->rmf; r.rIb = h->rIb;
-        r.cost = h->d_cost;
-        r.x0_def = h->d_x0xf;
-        r.xf_def = h->d_x0xf + QL_NX;
-        r.segs = h->d_segs;
-        r.seg_begin = h->d_seg_begin;
-        r.npad = h->npad;
-        r.nseg = (int)h->segs.size();
-        t.fastdiv = t.fastdiv && h->fastdiv;
-        if (h->cls.N > t.layout.N) t.layout = h->cls;
+        r.c = p.cls;
+        r.rmb = p.rmb; r.rmf = p.rmf; r.rIb = p.rIb;
+        r.cost = ds.d_cost;
+        r.x0_def = ds.d_x0xf;
+        r.xf_def = ds.d_x0xf + QL_NX;
+        r.segs = ds.d_segs;
+        r.seg_begin = ds.d_seg_begin;
+        r.npad = p.npad;
+        r.nseg = (int)p.segs.size();
+        t.fastdiv = t.fastdiv && p.fastdiv;
+        if (p.cls.N > t.layout.N) t.layout = p.cls;
     }
     // device records are QL_RAGCLASS_BYTES apart (the kernel copies whole slots)
     std::vector<unsigned char> packed((size_t)ncls * QL_RAGCLASS_BYTES, 0);
@@ -714,22 +722,22 @@ int ragged_table(const qlnlp_handle* hs, int ncls, const RagTable** out)
     for (int wj = 0; wj < NJM; ++wj) {
         if (wj == ql::JM_VALS) continue;
         t.smem[wj] = ql::smem_bytes(t.layout.N, wj);
-        if (t.smem[wj] > lead->smem_optin) return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp", t.layout.N, t.smem[wj]);
+        if (t.smem[wj] > lead.smem_optin) return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp", t.layout.N, t.smem[wj]);
         if (int rc = kernel_geometry(lead, kernel_fn(wj, t.fastdiv, true), wj, t.smem[wj], &t.blocks_per_sm[wj])) return rc;
     }
-    *out = &lead->rag_tables.emplace(key, t).first->second;
+    *out = &lead.rag_tables.emplace(key, t).first->second;
     return QLNLP_OK;
 }
 
 // ---- opt-in kinematic rows (qlnlp_kin.cuh) ---------------------------------------------------------------------
-// The caller-visible structure of a handle with kinematic rows: the reference's entries + 8 per knot, column-major.
+// The caller-visible structure of a problem with kinematic rows: the reference's entries + 8 per knot, column-major.
 // map[o] = position in the reference-order row, or -(8 (k-1) + e + 1) for a kinematic entry.
-void kin_structure(const qlnlp_handle_s* h, std::vector<int64_t>& rows, std::vector<int64_t>& cols, std::vector<int32_t>& map)
+void kin_structure(const Problem& p, std::vector<int64_t>& rows, std::vector<int64_t>& cols, std::vector<int32_t>& map)
 {
-    const QlClass& c = h->cls;
-    const int n0 = std_nnz(h);
+    const QlClass& c = p.cls;
+    const int n0 = std_nnz(p);
     std::vector<int64_t> r0((size_t)n0), c0((size_t)n0);
-    if (h->jac_mode == QLNLP_JAC_SPARSE_TRUE) sparse_true_structure(c, r0.data(), c0.data());
+    if (p.jac_mode == QLNLP_JAC_SPARSE_TRUE) sparse_true_structure(c, r0.data(), c0.data());
     else sparse_block_structure(c, r0.data(), c0.data());
     struct Ent { int64_t col, row; int32_t src; };
     std::vector<Ent> all;
@@ -744,32 +752,33 @@ void kin_structure(const qlnlp_handle_s* h, std::vector<int64_t>& rows, std::vec
     for (size_t i = 0; i < all.size(); ++i) { rows[i] = all[i].row; cols[i] = all[i].col; map[i] = all[i].src; }
 }
 
-int ensure_kin(qlnlp_handle h)
+int ensure_kin(const Problem& p, DeviceState& ds)
 {
-    if (h->d_kin_map) return QLNLP_OK;
+    if (ds.d_kin_map) return QLNLP_OK;
     std::vector<int64_t> rows, cols;
-    kin_structure(h, rows, cols, h->kin_map);
-    CUDA_TRY(cudaMalloc(&h->d_kin_map, sizeof(int) * h->kin_map.size()));
-    CUDA_TRY(cudaMemcpy(h->d_kin_map, h->kin_map.data(), sizeof(int) * h->kin_map.size(), cudaMemcpyHostToDevice));
+    std::vector<int32_t> map;
+    kin_structure(p, rows, cols, map);
+    CUDA_TRY(cudaMalloc(&ds.d_kin_map, sizeof(int) * map.size()));
+    CUDA_TRY(cudaMemcpy(ds.d_kin_map, map.data(), sizeof(int) * map.size(), cudaMemcpyHostToDevice));
     CUDA_TRY(cudaDeviceSynchronize());
     return QLNLP_OK;
 }
 
-// launch() for a handle with kinematic rows: io describes the CALLER's arrays (g rows of m_nlp + 2N, jac rows of
+// launch() for a problem with kinematic rows: io describes the CALLER's arrays (g rows of m_nlp + 2N, jac rows of
 // nnz + 8N).  The fused kernel writes the reference's g rows in place and its Jacobian values into a scratch row per
 // evaluation; two small kernels append / interleave the kinematic part.
-int launch_kin(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, cudaStream_t stream)
+int launch_kin(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* io, cudaStream_t stream)
 {
-    const QlClass& c = h->cls;
+    const QlClass& c = p.cls;
     if (B == 0) return QLNLP_OK;
     if (!io || !io->Z) return fail(QLNLP_EINVAL, "io->Z is required");
-    if (io->g && io->ldg < m_rows(h)) return fail(QLNLP_EINVAL, "ldg %lld < m_nlp %d", (long long)io->ldg, m_rows(h));
-    if (io->jac && io->ldjac < batch_nnz(h)) return fail(QLNLP_EINVAL, "ldjac %lld < nnz %d", (long long)io->ldjac, batch_nnz(h));
-    if (int rc = ensure_kin(h)) return rc;
+    if (io->g && io->ldg < m_rows(p)) return fail(QLNLP_EINVAL, "ldg %lld < m_nlp %d", (long long)io->ldg, m_rows(p));
+    if (io->jac && io->ldjac < batch_nnz(p)) return fail(QLNLP_EINVAL, "ldjac %lld < nnz %d", (long long)io->ldjac, batch_nnz(p));
+    if (int rc = ensure_kin(p, ds)) return rc;
     qlnlp_batch_io d = *io;
-    const int64_t lds = (std_nnz(h) + 1) & ~1;
+    const int64_t lds = (std_nnz(p) + 1) & ~1;
     if (io->jac) {
-        auto& sc = h->kin_scratch[stream];
+        auto& sc = ds.kin_scratch[stream];
         if (sc.second < B * lds) {
             cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
             cudaStreamIsCapturing(stream, &cap);
@@ -781,7 +790,7 @@ int launch_kin(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, cudaStream_t
         d.jac = sc.first;
         d.ldjac = lds;
     }
-    if (int rc = launch(h, B, &d, stream)) return rc;
+    if (int rc = launch(p, ds, B, &d, stream)) return rc;
     const int threads = 256;
     if (io->g) {
         const long long total = (long long)B * 2 * c.N;
@@ -789,10 +798,10 @@ int launch_kin(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, cudaStream_t
         CUDA_TRY(cudaGetLastError());
     }
     if (io->jac) {
-        const int nnz_out = batch_nnz(h);
+        const int nnz_out = batch_nnz(p);
         const long long total = (long long)B * nnz_out;
         ql::kin_expand_kernel<<<(unsigned)((total + threads - 1) / threads), threads, 0, stream>>>(
-            h->d_kin_map, nnz_out, d.jac, lds, io->Z, io->ldz, io->jac, io->ldjac, B);
+            ds.d_kin_map, nnz_out, d.jac, lds, io->Z, io->ldz, io->jac, io->ldjac, B);
         CUDA_TRY(cudaGetLastError());
     }
     return QLNLP_OK;
@@ -816,29 +825,29 @@ void hessian_structure(const QlClass& c, int64_t* rows, int64_t* cols)
     }
 }
 
-int launch_hessian(qlnlp_handle h, int64_t B, const double* Z, int64_t ldz, const double* sigma, double sigma0,
-                   const double* lam, int64_t ldlam, double* H, int64_t ldh, cudaStream_t stream)
+int launch_hessian(const Problem& p, DeviceState& ds, int64_t B, const double* Z, int64_t ldz, const double* sigma,
+                   double sigma0, const double* lam, int64_t ldlam, double* H, int64_t ldh, cudaStream_t stream)
 {
-    const QlClass& c = h->cls;
+    const QlClass& c = p.cls;
     if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
     if (B == 0) return QLNLP_OK;
     if (!Z || !lam || !H) return fail(QLNLP_EINVAL, "Z, lambda and H are required");
     if (ldz < c.n_nlp || ldlam < c.m_nlp || ldh < ql_hess_nnz(c)) return fail(QLNLP_EINVAL, "leading dimension too small");
-    const void* fn = h->fastdiv ? (const void*)ql::hess_kernel<true> : (const void*)ql::hess_kernel<false>;
+    const void* fn = p.fastdiv ? (const void*)ql::hess_kernel<true> : (const void*)ql::hess_kernel<false>;
     const size_t smem = ql::hess_smem_bytes(c.N);
-    if (!h->hess_blocks_per_sm) {
-        if (smem > h->smem_optin) return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp", c.N, smem);
-        CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
+    if (!ds.hess_blocks_per_sm) {
+        if (smem > ds.smem_optin) return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp", c.N, smem);
+        CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ds.smem_optin));
         int nb = 0;
         CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, QL_LANES, smem));
         if (nb < 1) return fail(QLNLP_ECUDA, "Hessian kernel does not fit on an SM");
-        h->hess_blocks_per_sm = nb;
-        if (int rc = set_carveout(fn, nb, smem, h->smem_per_sm)) return rc;      // the rest of the SM's memory is L1 (cost table)
+        ds.hess_blocks_per_sm = nb;
+        if (int rc = set_carveout(fn, nb, smem, ds.smem_per_sm)) return rc;      // the rest of the SM's memory is L1 (cost table)
     }
     ql::HessLaunch P;
     P.c = c;
-    P.rmb = h->rmb; P.rmf = h->rmf; P.rIb = h->rIb;
-    P.cost = h->d_cost; P.npad = h->npad;
+    P.rmb = p.rmb; P.rmf = p.rmf; P.rIb = p.rIb;
+    P.cost = ds.d_cost; P.npad = p.npad;
     P.Z = Z; P.ldz = ldz;
     P.lam = lam; P.ldlam = ldlam;
     P.sigma = sigma; P.sigma0 = sigma0;
@@ -846,8 +855,8 @@ int launch_hessian(qlnlp_handle h, int64_t B, const double* Z, int64_t ldz, cons
     P.B = B;
     P.bulk = ((reinterpret_cast<uintptr_t>(H) & 15) == 0 && (ldh & 1) == 0) ? 1 : 0;
     P.zbulk = ((reinterpret_cast<uintptr_t>(Z) & 15) == 0 && (ldz & 1) == 0) ? 1 : 0;
-    if (int rc = stream_ticket(h, stream, &P.ticket)) return rc;
-    const int grid = (int)std::min<int64_t>(B, (int64_t)h->sm_count * h->hess_blocks_per_sm);
+    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
+    const int grid = (int)std::min<int64_t>(B, (int64_t)ds.sm_count * ds.hess_blocks_per_sm);
     void* args[] = {&P};
     CUDA_TRY(cudaLaunchKernel(fn, dim3(grid), dim3(QL_LANES), args, smem, stream));
     return QLNLP_OK;
@@ -862,18 +871,18 @@ void free_lane(HostLane& ln)
     ln.cap = 0;
 }
 
-int reserve_lane(qlnlp_handle h, HostLane& ln, int64_t cap)
+int reserve_lane(const Problem& p, HostLane& ln, int64_t cap)
 {
     if (ln.cap >= cap) return QLNLP_OK;
     free_lane(ln);
-    CUDA_TRY(cudaMalloc(&ln.Z, sizeof(double) * cap * h->ldz_e));
+    CUDA_TRY(cudaMalloc(&ln.Z, sizeof(double) * cap * p.ldz_e));
     CUDA_TRY(cudaMalloc(&ln.x0, sizeof(double) * cap * QL_NX));
     CUDA_TRY(cudaMalloc(&ln.xf, sizeof(double) * cap * QL_NX));
     CUDA_TRY(cudaMalloc(&ln.f, sizeof(double) * cap));
-    CUDA_TRY(cudaMalloc(&ln.grad, sizeof(double) * cap * h->ldgrad_e));
-    CUDA_TRY(cudaMalloc(&ln.g, sizeof(double) * cap * h->ldg_e));
-    CUDA_TRY(cudaMalloc(&ln.jac, sizeof(double) * cap * std::max(h->ldjac_e, h->ldv_e)));
-    CUDA_TRY(cudaHostAlloc(&ln.stage, sizeof(double) * cap * h->ldv_e, cudaHostAllocDefault));
+    CUDA_TRY(cudaMalloc(&ln.grad, sizeof(double) * cap * p.ldgrad_e));
+    CUDA_TRY(cudaMalloc(&ln.g, sizeof(double) * cap * p.ldg_e));
+    CUDA_TRY(cudaMalloc(&ln.jac, sizeof(double) * cap * std::max(p.ldjac_e, p.ldv_e)));
+    CUDA_TRY(cudaHostAlloc(&ln.stage, sizeof(double) * cap * p.ldv_e, cudaHostAllocDefault));
     ln.cap = cap;
     return QLNLP_OK;
 }
@@ -902,41 +911,43 @@ bool is_registered(const qlnlp_handle_s* h, const double* jac, int64_t ldjac, in
 // Pipeline over up to MAX_LANES streams, `chunk` evaluations per stage: H2D of the decision vectors, one fused launch,
 // D2H of f / grad / g straight into the caller's arrays.  The Jacobian rows cross PCIe as the VALS stream (only the
 // value-dependent entries: 2,794 of the 32,161 SPARSE_BLOCK values at the default instance) into a pinned staging
-// buffer; while the next chunks are in flight the handle's worker pool assembles the caller's rows from the constant
+// buffer; while the next chunks are in flight the device's worker pool assembles the caller's rows from the constant
 // image of the pattern and those values (hostrows.cpp) -- every 64-byte line of a row, or, when the caller has
 // registered the output buffer (qlnlp_host_output_register), only the lines that hold a value-dependent entry.
-int eval_host_impl(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io)
+int eval_host_impl(qlnlp_handle h, int dev, int64_t B, const qlnlp_batch_io* io)
 {
-    const QlClass& c = h->cls;
+    const Problem& p = h->prob;
+    DeviceState& ds = h->devs[(size_t)dev];
+    const QlClass& c = p.cls;
     // Uniform chunks: chunk i is [i * chunk, min(B, (i + 1) * chunk)).  (Smaller chunks at either end measured no
     // consistent gain, profiles/r02_host_path.md: the D2H copies, not the fill, bound the pipeline.)
     const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(B, h->opt_host_chunk));
     const int64_t nchunks = (B + chunk - 1) / chunk;
     const int nlanes = (int)std::min<int64_t>(MAX_LANES, nchunks);
     for (int l = 0; l < nlanes; ++l)
-        if (int rc = reserve_lane(h, h->lanes[l], chunk)) return rc;
-    const bool compact = io->jac && B >= COMPACT_MIN_B && !h->kin;      // kinematic rows: the rows come back as they are
+        if (int rc = reserve_lane(p, ds.lanes[l], chunk)) return rc;
+    const bool compact = io->jac && B >= COMPACT_MIN_B && !p.kin;      // kinematic rows: the rows come back as they are
     bool touched_only = false;
     if (compact) {
         if (int rc = ensure_plan(h)) return rc;
-        if (int rc = ensure_pool(h)) return rc;
+        if (int rc = ensure_pool(h, dev)) return rc;
         touched_only = is_registered(h, io->jac, io->ldjac, B);
     }
-    const int nnz_b = batch_nnz(h);
+    const int nnz_b = batch_nnz(p);
     // Device-side leading dimensions.  Padded (even) rows give the kernel its TMA / 16-byte paths, but when the caller's
     // rows are tightly packed a padded device copy needs a PITCHED transfer (one DMA descriptor per 9.7 KB row: 36 GB/s
     // instead of 50+).  PCIe is what bounds this path, not the kernel: mirror the caller's packing.
-    const int64_t ldz_d = (io->ldz == c.n_nlp) ? c.n_nlp : h->ldz_e;
-    const int64_t ldgrad_d = (io->grad && io->ldgrad == c.n_nlp) ? c.n_nlp : h->ldgrad_e;
-    const int m_out = m_rows(h);
-    const int64_t ldg_d = (io->g && io->ldg == m_out) ? m_out : h->ldg_e;
-    const int64_t ldjac_d = (io->jac && io->ldjac == nnz_b) ? nnz_b : h->ldjac_e;      // uncompacted rows only
+    const int64_t ldz_d = (io->ldz == c.n_nlp) ? c.n_nlp : p.ldz_e;
+    const int64_t ldgrad_d = (io->grad && io->ldgrad == c.n_nlp) ? c.n_nlp : p.ldgrad_e;
+    const int m_out = m_rows(p);
+    const int64_t ldg_d = (io->g && io->ldg == m_out) ? m_out : p.ldg_e;
+    const int64_t ldjac_d = (io->jac && io->ldjac == nnz_b) ? nnz_b : p.ldjac_e;      // uncompacted rows only
     auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
     const double t_begin = now();
 
     auto enqueue = [&](int64_t i) -> int {
         const double t0 = now();
-        HostLane& ln = h->lanes[i % nlanes];
+        HostLane& ln = ds.lanes[i % nlanes];
         const int64_t b0 = i * chunk, nb = std::min(chunk, B - b0);
         cudaStream_t s = ln.stream;
         CUDA_TRY(copy_rows(ln.Z, ldz_d, io->Z + b0 * io->ldz, io->ldz, c.n_nlp, nb, cudaMemcpyHostToDevice, s));
@@ -950,12 +961,12 @@ int eval_host_impl(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io)
         d.f = io->f ? ln.f : nullptr;
         d.grad = io->grad ? ln.grad : nullptr; d.ldgrad = ldgrad_d;
         d.g = io->g ? ln.g : nullptr; d.ldg = ldg_d;
-        d.jac = io->jac ? ln.jac : nullptr; d.ldjac = compact ? h->ldv_e : ldjac_d;
-        if (int rc = h->kin ? launch_kin(h, nb, &d, s) : launch(h, nb, &d, s, compact ? ql::JM_VALS : -1)) return rc;
+        d.jac = io->jac ? ln.jac : nullptr; d.ldjac = compact ? p.ldv_e : ldjac_d;
+        if (int rc = p.kin ? launch_kin(p, ds, nb, &d, s) : launch(p, ds, nb, &d, s, compact ? ql::JM_VALS : -1)) return rc;
         // the staged values go first: the row builder only waits for them, f / grad / g land in the caller's arrays
         // by DMA while it works (the lanes are synchronised before the call returns)
         if (compact) {
-            CUDA_TRY(cudaMemcpyAsync(ln.stage, ln.jac, sizeof(double) * nb * h->ldv_e, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(cudaMemcpyAsync(ln.stage, ln.jac, sizeof(double) * nb * p.ldv_e, cudaMemcpyDeviceToHost, s));
             CUDA_TRY(cudaEventRecord(ln.done, s));
         }
         if (io->f) CUDA_TRY(cudaMemcpyAsync(io->f + b0, ln.f, sizeof(double) * nb, cudaMemcpyDeviceToHost, s));
@@ -963,7 +974,7 @@ int eval_host_impl(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io)
         if (io->g) CUDA_TRY(copy_rows(io->g + b0 * io->ldg, io->ldg, ln.g, ldg_d, m_out, nb, cudaMemcpyDeviceToHost, s));
         if (!compact && io->jac)
             CUDA_TRY(copy_rows(io->jac + b0 * io->ldjac, io->ldjac, ln.jac, ldjac_d, nnz_b, nb, cudaMemcpyDeviceToHost, s));
-        h->stat_t_enqueue += now() - t0;
+        ds.stat_t_enqueue += now() - t0;
         return QLNLP_OK;
     };
     // Row assembly runs on the pool's workers while this thread keeps the device fed: chunk j is handed to the pool
@@ -974,27 +985,27 @@ int eval_host_impl(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io)
     auto progress = [&](bool may_block) -> int {
         if (!compact) { handed = built = enq; return QLNLP_OK; }
         if (handed > built) {                                   // a build is running
-            if (h->pool->busy()) {
+            if (ds.pool->busy()) {
                 if (!may_block) return QLNLP_OK;
-                h->pool->finish();
+                ds.pool->finish();
             }
             ++built;
-            h->stat_t_build += now() - t_build0;
+            ds.stat_t_build += now() - t_build0;
         }
         if (handed == built && handed < enq) {
-            HostLane& ln = h->lanes[handed % nlanes];
+            HostLane& ln = ds.lanes[handed % nlanes];
             const double t0 = now();
             cudaError_t q = may_block ? cudaEventSynchronize(ln.done) : cudaEventQuery(ln.done);
-            h->stat_t_wait += now() - t0;
+            ds.stat_t_wait += now() - t0;
             if (q == cudaErrorNotReady) return QLNLP_OK;
             if (q != cudaSuccess) return fail(QLNLP_ECUDA, "host pipeline: %s", cudaGetErrorString(q));
             const int64_t b0 = handed * chunk, nb = std::min(chunk, B - b0);
             double* rows = io->jac + b0 * io->ldjac;
             t_build0 = now();
-            h->plan->build_async(h->pool.get(), ln.stage, h->ldv_e, rows, io->ldjac, nb, touched_only);
+            h->plan->build_async(ds.pool.get(), ln.stage, p.ldv_e, rows, io->ldjac, nb, touched_only);
             ++handed;
-            h->stat_host_rows += nb;
-            h->stat_host_lines += nb * (touched_only ? h->plan->touched_lines((int)((reinterpret_cast<uintptr_t>(rows) >> 3) & 7))
+            ds.stat_host_rows += nb;
+            ds.stat_host_lines += nb * (touched_only ? h->plan->touched_lines((int)((reinterpret_cast<uintptr_t>(rows) >> 3) & 7))
                                                      : (h->plan->nnz() + 7) / 8);
         }
         return QLNLP_OK;
@@ -1009,32 +1020,34 @@ int eval_host_impl(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io)
     while (built < enq)
         if (int rc = progress(true)) return rc;
     const double t_sync = now();
-    for (int l = 0; l < nlanes; ++l) CUDA_TRY(cudaStreamSynchronize(h->lanes[l].stream));
-    h->stat_t_wait += now() - t_sync;
-    h->stat_t_total += now() - t_begin;
+    for (int l = 0; l < nlanes; ++l) CUDA_TRY(cudaStreamSynchronize(ds.lanes[l].stream));
+    ds.stat_t_wait += now() - t_sync;
+    ds.stat_t_total += now() - t_begin;
     return QLNLP_OK;
 }
 
-int eval_host(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io)
+int eval_host(qlnlp_handle h, int dev, int64_t B, const qlnlp_batch_io* io)
 {
-    const QlClass& c = h->cls;
+    const Problem& p = h->prob;
+    DeviceState& ds = h->devs[(size_t)dev];
+    const QlClass& c = p.cls;
     if (B == 0) return QLNLP_OK;
     if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
     if (!io || !io->Z) return fail(QLNLP_EINVAL, "io->Z is required");
     if (io->ldz < c.n_nlp) return fail(QLNLP_EINVAL, "ldz < n_nlp");
     if (io->grad && io->ldgrad < c.n_nlp) return fail(QLNLP_EINVAL, "ldgrad < n_nlp");
-    if (io->g && io->ldg < m_rows(h)) return fail(QLNLP_EINVAL, "ldg < m_nlp");
-    if (io->jac && io->ldjac < batch_nnz(h)) return fail(QLNLP_EINVAL, "ldjac < nnz");
+    if (io->g && io->ldg < m_rows(p)) return fail(QLNLP_EINVAL, "ldg < m_nlp");
+    if (io->jac && io->ldjac < batch_nnz(p)) return fail(QLNLP_EINVAL, "ldjac < nnz");
     if (io->jac && (reinterpret_cast<uintptr_t>(io->jac) & 7) != 0) return fail(QLNLP_EINVAL, "jac must be 8-byte aligned");
-    DeviceGuard guard(h->device);
-    if (int rc = ensure_device(h)) return rc;
-    const int rc = eval_host_impl(h, B, io);
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(p, ds)) return rc;
+    const int rc = eval_host_impl(h, dev, B, io);
     if (rc != QLNLP_OK) {
         // copies into caller-owned host memory (and out of the pinned stage) may still be in flight: finish them
         // before the caller gets its buffers back
         const std::string msg = g_err;
-        if (h->pool) h->pool->finish();
-        for (auto& ln : h->lanes)
+        if (ds.pool) ds.pool->finish();
+        for (auto& ln : ds.lanes)
             if (ln.stream) cudaStreamSynchronize(ln.stream);
         cudaGetLastError();
         g_err = msg;
@@ -1066,22 +1079,21 @@ qlnlp_batch_io shard_io(const QlClass&, const qlnlp_batch_io& io, int64_t lo)
 // ---- single evaluations -------------------------------------------------------------------------------------
 enum { HAVE_F = 1, HAVE_GRAD = 2, HAVE_G = 4, HAVE_J = 8 };
 
-int reserve_one(qlnlp_handle h)
+int reserve_one(const Problem& p, OneEval& o)
 {
-    OneEval& o = h->one;
     if (o.mx) return QLNLP_OK;
     o.o_grad = 2;
-    o.o_g = o.o_grad + h->ldgrad_e;
-    o.o_vals = o.o_g + h->ldg_e;
-    o.total = o.o_vals + h->ldv_e;
+    o.o_g = o.o_grad + p.ldgrad_e;
+    o.o_vals = o.o_g + p.ldg_e;
+    o.total = o.o_vals + p.ldv_e;
     // One decision vector is latency-bound: with mapped pinned memory the kernel fetches x and stores its 41 KB of
     // results over PCIe itself, which saves the two copy calls.
-    if (!o.hx) CUDA_TRY(cudaHostAlloc(&o.hx, sizeof(double) * (h->ldz_e + o.total), cudaHostAllocMapped));
-    o.hout = o.hx + h->ldz_e;
+    if (!o.hx) CUDA_TRY(cudaHostAlloc(&o.hx, sizeof(double) * (p.ldz_e + o.total), cudaHostAllocMapped));
+    o.hout = o.hx + p.ldz_e;
     void* dp = nullptr;
     CUDA_TRY(cudaHostGetDevicePointer(&dp, o.hx, 0));
     o.mx = static_cast<double*>(dp);
-    o.mout = o.mx + h->ldz_e;
+    o.mout = o.mx + p.ldz_e;
     o.valid = false;
     return QLNLP_OK;
 }
@@ -1091,34 +1103,35 @@ int reserve_one(qlnlp_handle h)
 // the value-dependent Jacobian entries: one kernel that reads x from and writes its 41 KB of results to mapped pinned
 // memory, see reserve_one) and keeps the results; the other callbacks at the same x (compared bit for bit, 9.7 KB) are
 // served from that cache.  The Jacobian values are assembled in the caller's array from the constant image of the
-// pattern + the cached entries.
-int eval_one(qlnlp_handle hh, const double* x, double* f, double* grad, double* g, double* vals)
+// pattern + the cached entries.  Runs on the handle's first device.
+int eval_one(qlnlp_handle h, const double* x, double* f, double* grad, double* g, double* vals)
 {
-    if (int rc = check_handle(hh)) return rc;
+    if (int rc = check_handle(h)) return rc;
     if (!x) return fail(QLNLP_EINVAL, "null x");
-    qlnlp_handle h = first(hh);
-    const QlClass& c = h->cls;
-    DeviceGuard guard(h->device);
-    if (int rc = ensure_device(h)) return rc;
-    if (h->kin) {
+    const Problem& p = h->prob;
+    DeviceState& ds = h->devs[0];
+    const QlClass& c = p.cls;
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(p, ds)) return rc;
+    if (p.kin) {
         // kinematic rows: the plain route -- copy x in, evaluate what was asked for, copy it out (no x cache)
-        HostLane& ln = h->lanes[0];
-        if (int rc = reserve_lane(h, ln, 1)) return rc;
+        HostLane& ln = ds.lanes[0];
+        if (int rc = reserve_lane(p, ln, 1)) return rc;
         cudaStream_t s = ln.stream;
         CUDA_TRY(cudaMemcpyAsync(ln.Z, x, sizeof(double) * c.n_nlp, cudaMemcpyHostToDevice, s));
         qlnlp_batch_io d;
         std::memset(&d, 0, sizeof d);
-        d.Z = ln.Z; d.ldz = h->ldz_e;
+        d.Z = ln.Z; d.ldz = p.ldz_e;
         d.f = f ? ln.f : nullptr;
-        d.grad = grad ? ln.grad : nullptr; d.ldgrad = h->ldgrad_e;
-        d.g = g ? ln.g : nullptr; d.ldg = h->ldg_e;
-        d.jac = vals ? ln.jac : nullptr; d.ldjac = h->ldjac_e;
-        int rc = launch_kin(h, 1, &d, s);
+        d.grad = grad ? ln.grad : nullptr; d.ldgrad = p.ldgrad_e;
+        d.g = g ? ln.g : nullptr; d.ldg = p.ldg_e;
+        d.jac = vals ? ln.jac : nullptr; d.ldjac = p.ldjac_e;
+        int rc = launch_kin(p, ds, 1, &d, s);
         cudaError_t e = cudaSuccess;
         if (rc == QLNLP_OK && f) e = cudaMemcpyAsync(f, ln.f, sizeof(double), cudaMemcpyDeviceToHost, s);
         if (rc == QLNLP_OK && e == cudaSuccess && grad) e = cudaMemcpyAsync(grad, ln.grad, sizeof(double) * c.n_nlp, cudaMemcpyDeviceToHost, s);
-        if (rc == QLNLP_OK && e == cudaSuccess && g) e = cudaMemcpyAsync(g, ln.g, sizeof(double) * m_rows(h), cudaMemcpyDeviceToHost, s);
-        if (rc == QLNLP_OK && e == cudaSuccess && vals) e = cudaMemcpyAsync(vals, ln.jac, sizeof(double) * batch_nnz(h), cudaMemcpyDeviceToHost, s);
+        if (rc == QLNLP_OK && e == cudaSuccess && g) e = cudaMemcpyAsync(g, ln.g, sizeof(double) * m_rows(p), cudaMemcpyDeviceToHost, s);
+        if (rc == QLNLP_OK && e == cudaSuccess && vals) e = cudaMemcpyAsync(vals, ln.jac, sizeof(double) * batch_nnz(p), cudaMemcpyDeviceToHost, s);
         if (rc == QLNLP_OK && e != cudaSuccess) rc = fail(QLNLP_ECUDA, "single evaluation: %s", cudaGetErrorString(e));
         const std::string msg = g_err;
         const cudaError_t es = cudaStreamSynchronize(s);
@@ -1126,8 +1139,8 @@ int eval_one(qlnlp_handle hh, const double* x, double* f, double* grad, double* 
         g_err = msg;
         return rc;
     }
-    if (int rc = reserve_one(h)) return rc;
-    OneEval& o = h->one;
+    OneEval& o = ds.one;
+    if (int rc = reserve_one(p, o)) return rc;
     const bool hit = h->opt_x_cache && o.valid && std::memcmp(o.hx, x, sizeof(double) * c.n_nlp) == 0;
     if (!hit) {
         o.valid = false;
@@ -1137,10 +1150,10 @@ int eval_one(qlnlp_handle hh, const double* x, double* f, double* grad, double* 
         std::memset(&d, 0, sizeof d);
         d.Z = o.mx; d.ldz = c.n_nlp;                                 // odd ld: plain (non-TMA) loads from host memory
         d.f = o.mout;
-        d.grad = o.mout + o.o_grad; d.ldgrad = h->ldgrad_e;
-        d.g = o.mout + o.o_g; d.ldg = h->ldg_e;
-        d.jac = o.mout + o.o_vals; d.ldjac = h->ldv_e + 1;           // odd ld: plain stores into host memory
-        if (int rc = launch(h, 1, &d, s, ql::JM_VALS)) return rc;
+        d.grad = o.mout + o.o_grad; d.ldgrad = p.ldgrad_e;
+        d.g = o.mout + o.o_g; d.ldg = p.ldg_e;
+        d.jac = o.mout + o.o_vals; d.ldjac = p.ldv_e + 1;            // odd ld: plain stores into host memory
+        if (int rc = launch(p, ds, 1, &d, s, ql::JM_VALS)) return rc;
         CUDA_TRY(cudaStreamSynchronize(s));
         o.valid = true;
     }
@@ -1149,48 +1162,47 @@ int eval_one(qlnlp_handle hh, const double* x, double* f, double* grad, double* 
     if (g) std::memcpy(g, o.hout + o.o_g, sizeof(double) * c.m_nlp);
     if (vals) {
         if (int rc = ensure_plan(h)) return rc;
-        h->plan->build_rows(o.hout + o.o_vals, h->ldv_e, vals, h->plan->nnz(), 0, 1, false);
+        h->plan->build_rows(o.hout + o.o_vals, p.ldv_e, vals, h->plan->nnz(), 0, 1, false);
     }
     return QLNLP_OK;
 }
 
 // DENSE: evaluate SPARSE_BLOCK on the device, scatter into the zeroed m x n grid, copy back
-int eval_dense_jacobian(qlnlp_handle hh, const double* x, double* vals)
+int eval_dense_jacobian(const Problem& p, DeviceState& ds, const double* x, double* vals)
 {
     if (!x) return fail(QLNLP_EINVAL, "null x");
-    qlnlp_handle h = first(hh);
-    DeviceGuard guard(h->device);
-    if (int rc = ensure_device(h)) return rc;
-    const QlClass& c = h->cls;
-    const int m = m_rows(h), nz = batch_nnz(h);          // DENSE handles batch in SPARSE_BLOCK (+ the kinematic entries)
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(p, ds)) return rc;
+    const QlClass& c = p.cls;
+    const int m = m_rows(p), nz = batch_nnz(p);          // DENSE handles batch in SPARSE_BLOCK (+ the kinematic entries)
     const size_t dense_n = (size_t)m * c.n_nlp;
-    if (!h->d_dense_lin) {
+    if (!ds.d_dense_lin) {
         std::vector<int64_t> rows((size_t)nz), cols((size_t)nz);
-        if (h->kin) { std::vector<int32_t> map; kin_structure(h, rows, cols, map); }
+        if (p.kin) { std::vector<int32_t> map; kin_structure(p, rows, cols, map); }
         else sparse_block_structure(c, rows.data(), cols.data());
         std::vector<long long> lin((size_t)nz);
         for (int i = 0; i < nz; ++i) lin[(size_t)i] = (rows[(size_t)i] - 1) + (long long)m * (cols[(size_t)i] - 1);
-        CUDA_TRY(cudaMalloc(&h->d_dense_lin, sizeof(long long) * nz));
-        CUDA_TRY(cudaMemcpy(h->d_dense_lin, lin.data(), sizeof(long long) * nz, cudaMemcpyHostToDevice));
-        CUDA_TRY(cudaMalloc(&h->d_dense, sizeof(double) * dense_n));
+        CUDA_TRY(cudaMalloc(&ds.d_dense_lin, sizeof(long long) * nz));
+        CUDA_TRY(cudaMemcpy(ds.d_dense_lin, lin.data(), sizeof(long long) * nz, cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMalloc(&ds.d_dense, sizeof(double) * dense_n));
         CUDA_TRY(cudaDeviceSynchronize());     // set-up copy on the default stream before work on the lane's stream
     }
-    HostLane& ln = h->lanes[0];
-    if (int rc = reserve_lane(h, ln, 1)) return rc;
+    HostLane& ln = ds.lanes[0];
+    if (int rc = reserve_lane(p, ln, 1)) return rc;
     cudaStream_t s = ln.stream;
     CUDA_TRY(cudaMemcpyAsync(ln.Z, x, sizeof(double) * c.n_nlp, cudaMemcpyHostToDevice, s));
     qlnlp_batch_io d;
     std::memset(&d, 0, sizeof d);
-    d.Z = ln.Z; d.ldz = h->ldz_e;
-    d.jac = ln.jac; d.ldjac = h->ldjac_e;
-    int rc = h->kin ? launch_kin(h, 1, &d, s) : launch(h, 1, &d, s);
+    d.Z = ln.Z; d.ldz = p.ldz_e;
+    d.jac = ln.jac; d.ldjac = p.ldjac_e;
+    int rc = p.kin ? launch_kin(p, ds, 1, &d, s) : launch(p, ds, 1, &d, s);
     if (rc == QLNLP_OK) {
-        cudaError_t e = cudaMemsetAsync(h->d_dense, 0, sizeof(double) * dense_n, s);
+        cudaError_t e = cudaMemsetAsync(ds.d_dense, 0, sizeof(double) * dense_n, s);
         if (e == cudaSuccess) {
-            ql::scatter_dense_kernel<<<(nz + 255) / 256, 256, 0, s>>>(ln.jac, h->d_dense_lin, h->d_dense, nz);
+            ql::scatter_dense_kernel<<<(nz + 255) / 256, 256, 0, s>>>(ln.jac, ds.d_dense_lin, ds.d_dense, nz);
             e = cudaGetLastError();
         }
-        if (e == cudaSuccess) e = cudaMemcpyAsync(vals, h->d_dense, sizeof(double) * dense_n, cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(vals, ds.d_dense, sizeof(double) * dense_n, cudaMemcpyDeviceToHost, s);
         if (e != cudaSuccess) rc = fail(QLNLP_ECUDA, "dense Jacobian: %s", cudaGetErrorString(e));
     }
     const std::string msg = g_err;
@@ -1200,62 +1212,71 @@ int eval_dense_jacobian(qlnlp_handle hh, const double* x, double* vals)
     return rc;
 }
 
-void destroy_device_state(qlnlp_handle h)
+void destroy_device_state(DeviceState& ds)
 {
-    if (!h->dev_ready) return;
-    DeviceGuard guard(h->device);
+    if (!ds.ready) return;
+    DeviceGuard guard(ds.device);
     cudaDeviceSynchronize();     // launches on caller streams may still use the handle's tables and counters
-    for (auto& ln : h->lanes) {
+    for (auto& ln : ds.lanes) {
         if (ln.stream) cudaStreamSynchronize(ln.stream);
         free_lane(ln);
         if (ln.stream) cudaStreamDestroy(ln.stream);
         if (ln.done) cudaEventDestroy(ln.done);
     }
-    if (h->one.stream) cudaStreamDestroy(h->one.stream);
-    if (h->one.hx) cudaFreeHost(h->one.hx);
-    cudaFree(h->d_hess_in); cudaFree(h->d_hess_out);
-    cudaFree(h->d_kin_map);
-    for (auto& kv : h->kin_scratch) cudaFree(kv.second.first);
-    for (auto& kv : h->rag_tables) cudaFree(kv.second.d_classes);
-    cudaFree(h->ticket_pool);
-    cudaFree(h->d_cost); cudaFree(h->d_x0xf); cudaFree(h->d_segs); cudaFree(h->d_seg_begin);
-    cudaFree(h->d_dense_lin); cudaFree(h->d_dense);
+    if (ds.one.stream) cudaStreamDestroy(ds.one.stream);
+    if (ds.one.hx) cudaFreeHost(ds.one.hx);
+    cudaFree(ds.d_hess_in); cudaFree(ds.d_hess_out);
+    cudaFree(ds.d_kin_map);
+    for (auto& kv : ds.kin_scratch) cudaFree(kv.second.first);
+    for (auto& kv : ds.rag_tables) cudaFree(kv.second.d_classes);
+    cudaFree(ds.ticket_pool);
+    cudaFree(ds.d_cost); cudaFree(ds.d_x0xf); cudaFree(ds.d_segs); cudaFree(ds.d_seg_begin);
+    cudaFree(ds.d_dense_lin); cudaFree(ds.d_dense);
 }
 
-int create_one(const qlnlp_problem_desc* d, int device, int jac_mode, qlnlp_handle* out)
+// The problem of `d` on the devices `devices[0 .. ndev)`, which share the host cores.
+int create_one(const qlnlp_problem_desc* d, const int* devices, int ndev, int jac_mode, qlnlp_handle* out)
 {
     qlnlp_handle h = new (std::nothrow) qlnlp_handle_s();
     if (!h) return fail(QLNLP_ENOMEM, "out of host memory");
+    Problem& p = h->prob;
     static std::atomic<uint64_t> g_serial{0};
-    h->serial = ++g_serial;
-    ql_class_init(&h->cls, (int)d->N, (int)d->k_trans, (int)d->init_mode, d->model.g, d->model.mb, d->model.mf, d->model.lb);
-    ql_class_finish(&h->cls);
-    h->device = device;
-    h->jac_mode = jac_mode & ~QLNLP_WITH_KINEMATICS;
-    h->kin = (jac_mode & QLNLP_WITH_KINEMATICS) != 0;
-    h->leg_reach = d->model.l1 + d->model.l2 + d->model.lb / 2;
-    std::memcpy(h->x0, d->x0, sizeof h->x0);
-    std::memcpy(h->xf, d->xf, sizeof h->xf);
-    const int N = h->cls.N;
-    h->npad = (N + 31) & ~31;
-    h->cost.assign((size_t)QL_NCOST * h->npad, 0.0);
+    p.serial = ++g_serial;
+    ql_class_init(&p.cls, (int)d->N, (int)d->k_trans, (int)d->init_mode, d->model.g, d->model.mb, d->model.mf, d->model.lb);
+    ql_class_finish(&p.cls);
+    p.jac_mode = jac_mode & ~QLNLP_WITH_KINEMATICS;
+    p.kin = (jac_mode & QLNLP_WITH_KINEMATICS) != 0;
+    p.leg_reach = d->model.l1 + d->model.l2 + d->model.lb / 2;
+    std::memcpy(p.x0, d->x0, sizeof p.x0);
+    std::memcpy(p.xf, d->xf, sizeof p.xf);
+    const QlClass& c = p.cls;
+    const int N = c.N;
+    p.npad = (N + 31) & ~31;
+    p.cost.assign((size_t)QL_NCOST * p.npad, 0.0);
     for (int k = 0; k < N; ++k) {
         for (int i = 0; i < QL_NX; ++i) {
-            h->cost[(size_t)i * h->npad + k] = d->Q[k * QL_NX + i];
-            h->cost[(size_t)(15 + i) * h->npad + k] = d->q[k * QL_NX + i];
+            p.cost[(size_t)i * p.npad + k] = d->Q[k * QL_NX + i];
+            p.cost[(size_t)(15 + i) * p.npad + k] = d->q[k * QL_NX + i];
         }
         for (int i = 0; i < QL_NU; ++i) {
-            h->cost[(size_t)(30 + i) * h->npad + k] = d->R[k * QL_NU + i];
-            h->cost[(size_t)(35 + i) * h->npad + k] = d->r[k * QL_NU + i];
+            p.cost[(size_t)(30 + i) * p.npad + k] = d->R[k * QL_NU + i];
+            p.cost[(size_t)(35 + i) * p.npad + k] = d->r[k * QL_NU + i];
         }
-        h->cost[(size_t)40 * h->npad + k] = d->c[k];
+        p.cost[(size_t)40 * p.npad + k] = d->c[k];
     }
-    plan_segments(h->cls, h->segs, h->seg_begin);
-    h->rmb = 1.0 / h->cls.mb;
-    h->rmf = 1.0 / h->cls.mf;
-    h->rIb = 1.0 / h->cls.Ib;
-    h->fastdiv = fastdiv_is_exact(h->cls.mb) && fastdiv_is_exact(h->cls.mf) && fastdiv_is_exact(h->cls.Ib) &&
-                 fastdiv_is_exact(6.0) && !std::getenv("QLNLP_IEEE_DIV");   // env: force the IEEE-division kernels
+    plan_segments(c, p.segs, p.seg_begin);
+    p.rmb = 1.0 / c.mb;
+    p.rmf = 1.0 / c.mf;
+    p.rIb = 1.0 / c.Ib;
+    p.fastdiv = fastdiv_is_exact(c.mb) && fastdiv_is_exact(c.mf) && fastdiv_is_exact(c.Ib) &&
+                fastdiv_is_exact(6.0) && !std::getenv("QLNLP_IEEE_DIV");   // env: force the IEEE-division kernels
+    p.ldz_e = (c.n_nlp + 1) & ~1;
+    p.ldgrad_e = p.ldz_e;
+    p.ldg_e = (m_rows(p) + 1) & ~1;
+    p.ldjac_e = (batch_nnz(p) + 1) & ~1;
+    p.ldv_e = (c.nnz_vals + 1) & ~1;
+    h->devs.resize((size_t)ndev);
+    for (int i = 0; i < ndev; ++i) h->devs[(size_t)i].device = devices[i];
     *out = h;
     return QLNLP_OK;
 }
@@ -1285,7 +1306,7 @@ int qlnlp_create(const qlnlp_problem_desc* d, int device, int jac_mode, qlnlp_ha
     if (!d || !out) return fail(QLNLP_EINVAL, "null argument");
     *out = nullptr;
     if (int rc = check_desc(d, jac_mode)) return rc;
-    return create_one(d, device, jac_mode, out);
+    return create_one(d, &device, 1, jac_mode, out);
 }
 
 int qlnlp_create_multi(const qlnlp_problem_desc* d, const int* devices, int ndev, int jac_mode, qlnlp_handle* out)
@@ -1297,17 +1318,9 @@ int qlnlp_create_multi(const qlnlp_problem_desc* d, const int* devices, int ndev
         for (int j = 0; j < i; ++j)
             if (devices[i] == devices[j]) return fail(QLNLP_EINVAL, "device %d listed twice", devices[i]);
     if (int rc = check_desc(d, jac_mode)) return rc;
-    qlnlp_handle parent = nullptr;
-    if (int rc = create_one(d, devices[0], jac_mode, &parent)) return rc;
-    for (int i = 0; i < ndev; ++i) {
-        qlnlp_handle sub = nullptr;
-        if (int rc = create_one(d, devices[i], jac_mode, &sub)) { qlnlp_destroy(parent); return rc; }
-        sub->part = i;
-        sub->nparts = ndev;
-        parent->subs.push_back(sub);
-        parent->drivers.emplace_back(new qlhost::Worker());
-    }
-    *out = parent;
+    if (int rc = create_one(d, devices, ndev, jac_mode, out)) return rc;
+    (*out)->multi = true;
+    for (int i = 0; i < ndev; ++i) (*out)->drivers.emplace_back(new qlhost::Worker());
     return QLNLP_OK;
 }
 
@@ -1316,8 +1329,7 @@ int qlnlp_destroy(qlnlp_handle h)
     if (!h) return QLNLP_OK;
     for (auto& w : h->drivers) w->wait();
     h->drivers.clear();
-    for (qlnlp_handle s : h->subs) qlnlp_destroy(s);
-    destroy_device_state(h);
+    for (DeviceState& ds : h->devs) destroy_device_state(ds);
     delete h;
     return QLNLP_OK;
 }
@@ -1325,20 +1337,21 @@ int qlnlp_destroy(qlnlp_handle h)
 int qlnlp_dims(qlnlp_handle h, int64_t* n_nlp, int64_t* m_nlp, int64_t* nnz, int64_t* nnz_block)
 {
     if (int rc = check_handle(h)) return rc;
-    if (n_nlp) *n_nlp = h->cls.n_nlp;
-    if (m_nlp) *m_nlp = m_rows(h);
-    if (nnz) *nnz = (h->jac_mode == QLNLP_JAC_DENSE) ? (int64_t)m_rows(h) * h->cls.n_nlp : batch_nnz(h);
-    if (nnz_block) *nnz_block = h->cls.nnz + (h->kin ? 8 * h->cls.N : 0);
+    const Problem& p = h->prob;
+    if (n_nlp) *n_nlp = p.cls.n_nlp;
+    if (m_nlp) *m_nlp = m_rows(p);
+    if (nnz) *nnz = (p.jac_mode == QLNLP_JAC_DENSE) ? (int64_t)m_rows(p) * p.cls.n_nlp : batch_nnz(p);
+    if (nnz_block) *nnz_block = p.cls.nnz + (p.kin ? 8 * p.cls.N : 0);
     return QLNLP_OK;
 }
 
 int qlnlp_devices(qlnlp_handle h, int* devices, int cap, int* ndev)
 {
     if (int rc = check_handle(h)) return rc;
-    const int n = h->subs.empty() ? 1 : (int)h->subs.size();
+    const int n = (int)h->devs.size();
     if (ndev) *ndev = n;
     if (devices)
-        for (int i = 0; i < n && i < cap; ++i) devices[i] = h->subs.empty() ? h->device : h->subs[i]->device;
+        for (int i = 0; i < n && i < cap; ++i) devices[i] = h->devs[(size_t)i].device;
     return QLNLP_OK;
 }
 
@@ -1353,21 +1366,22 @@ int qlnlp_jacobian_structure(qlnlp_handle h, int64_t* rows, int64_t* cols)
 {
     if (int rc = check_handle(h)) return rc;
     if (!rows || !cols) return fail(QLNLP_EINVAL, "null output");
-    if (h->jac_mode == QLNLP_JAC_DENSE) {
+    const Problem& p = h->prob;
+    if (p.jac_mode == QLNLP_JAC_DENSE) {
         // vec(Tuple.(CartesianIndices(zeros(m, n)))): column-major, row fastest (moi.jl:31-33)
         int64_t n = 0;
-        for (int64_t col = 1; col <= h->cls.n_nlp; ++col)
-            for (int64_t row = 1; row <= m_rows(h); ++row) { rows[n] = row; cols[n] = col; ++n; }
-    } else if (h->kin) {
+        for (int64_t col = 1; col <= p.cls.n_nlp; ++col)
+            for (int64_t row = 1; row <= m_rows(p); ++row) { rows[n] = row; cols[n] = col; ++n; }
+    } else if (p.kin) {
         std::vector<int64_t> r, c;
         std::vector<int32_t> map;
-        kin_structure(h, r, c, map);
+        kin_structure(p, r, c, map);
         std::copy(r.begin(), r.end(), rows);
         std::copy(c.begin(), c.end(), cols);
-    } else if (h->jac_mode == QLNLP_JAC_SPARSE_TRUE) {
-        sparse_true_structure(h->cls, rows, cols);
+    } else if (p.jac_mode == QLNLP_JAC_SPARSE_TRUE) {
+        sparse_true_structure(p.cls, rows, cols);
     } else {
-        sparse_block_structure(h->cls, rows, cols);
+        sparse_block_structure(p.cls, rows, cols);
     }
     return QLNLP_OK;
 }
@@ -1376,10 +1390,11 @@ int qlnlp_constraint_bounds(qlnlp_handle h, double* lb, double* ub)
 {
     if (int rc = check_handle(h)) return rc;
     if (!lb || !ub) return fail(QLNLP_EINVAL, "null output");
-    for (int i = 0; i < m_rows(h); ++i) { lb[i] = 0.0; ub[i] = 0.0; }            // nlp.jl:66-67
-    for (int i = 0; i < h->cls.N; ++i) ub[h->cls.c_body + i] = INFINITY;          // nlp.jl:69
-    if (h->kin)                                                                   // nlp.jl:70 (commented out upstream)
-        for (int i = 0; i < 2 * h->cls.N; ++i) ub[h->cls.m_nlp + i] = h->leg_reach;
+    const Problem& p = h->prob;
+    for (int i = 0; i < m_rows(p); ++i) { lb[i] = 0.0; ub[i] = 0.0; }            // nlp.jl:66-67
+    for (int i = 0; i < p.cls.N; ++i) ub[p.cls.c_body + i] = INFINITY;            // nlp.jl:69
+    if (p.kin)                                                                    // nlp.jl:70 (commented out upstream)
+        for (int i = 0; i < 2 * p.cls.N; ++i) ub[p.cls.m_nlp + i] = p.leg_reach;
     return QLNLP_OK;
 }
 
@@ -1387,9 +1402,9 @@ int qlnlp_variable_bounds(qlnlp_handle h, double* xl, double* xu)
 {
     if (int rc = check_handle(h)) return rc;
     if (!xl || !xu) return fail(QLNLP_EINVAL, "null output");
-    const int N = h->cls.N;
+    const int N = h->prob.cls.N;
     const double half_pi = 3.14159265358979323846 / 2;
-    for (int i = 0; i < h->cls.n_nlp; ++i) { xl[i] = -INFINITY; xu[i] = INFINITY; }
+    for (int i = 0; i < h->prob.cls.n_nlp; ++i) { xl[i] = -INFINITY; xu[i] = INFINITY; }
     for (int k = 1; k <= N; ++k) {                                                // moi.jl:53-67, 1-based as written
         xl[3 + 20 * (k - 1) - 1] = -half_pi;
         xu[3 + 20 * (k - 1) - 1] = half_pi;
@@ -1407,44 +1422,41 @@ int qlnlp_set_option(qlnlp_handle h, const char* name, int64_t value)
 {
     if (int rc = check_handle(h)) return rc;
     if (!name) return fail(QLNLP_EINVAL, "null option name");
-    auto apply = [&](qlnlp_handle t) -> int {
-        const std::string n(name);
-        if (n == "host_chunk") { if (value < 1) return fail(QLNLP_EINVAL, "host_chunk must be >= 1"); t->opt_host_chunk = value; }
-        else if (n == "host_threads") { if (value < 0) return fail(QLNLP_EINVAL, "host_threads must be >= 0"); t->opt_host_threads = value; t->pool.reset(); }
-        else if (n == "pin_threads") { t->opt_pin_threads = value != 0; t->pool.reset(); }
-        else if (n == "x_cache") { t->opt_x_cache = value != 0; t->one.valid = false; }
-        else return fail(QLNLP_EINVAL, "unknown option '%s'", name);
-        return QLNLP_OK;
-    };
-    if (int rc = apply(h)) return rc;
-    for (qlnlp_handle s : h->subs)
-        if (int rc = apply(s)) return rc;
+    const std::string n(name);
+    if (n == "host_chunk") { if (value < 1) return fail(QLNLP_EINVAL, "host_chunk must be >= 1"); h->opt_host_chunk = value; }
+    else if (n == "host_threads") { if (value < 0) return fail(QLNLP_EINVAL, "host_threads must be >= 0"); h->opt_host_threads = value; }
+    else if (n == "pin_threads") h->opt_pin_threads = value != 0;
+    else if (n == "x_cache") { h->opt_x_cache = value != 0; h->devs[0].one.valid = false; }
+    else return fail(QLNLP_EINVAL, "unknown option '%s'", name);
+    if (n == "host_threads" || n == "pin_threads")          // the pools take both when they are made
+        for (DeviceState& ds : h->devs) ds.pool.reset();
     return QLNLP_OK;
 }
 
 int qlnlp_eval_batch_device(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, void* stream)
 {
     if (int rc = check_handle(h)) return rc;
-    if (!h->subs.empty()) return fail(QLNLP_EINVAL, "multi-device handle: use qlnlp_eval_batch_device_multi");
+    if (h->multi) return fail(QLNLP_EINVAL, "multi-device handle: use qlnlp_eval_batch_device_multi");
     if (B == 0) return QLNLP_OK;
-    DeviceGuard guard(h->device);
-    if (int rc = ensure_device(h)) return rc;
-    if (h->kin) return launch_kin(h, B, io, static_cast<cudaStream_t>(stream));
-    return launch(h, B, io, static_cast<cudaStream_t>(stream));
+    DeviceState& ds = h->devs[0];
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(h->prob, ds)) return rc;
+    if (h->prob.kin) return launch_kin(h->prob, ds, B, io, static_cast<cudaStream_t>(stream));
+    return launch(h->prob, ds, B, io, static_cast<cudaStream_t>(stream));
 }
 
 int qlnlp_eval_batch_device_multi(qlnlp_handle h, const int64_t* B, const qlnlp_batch_io* io, void* const* streams)
 {
     if (int rc = check_handle(h)) return rc;
     if (!B || !io) return fail(QLNLP_EINVAL, "null argument");
-    const int n = h->subs.empty() ? 1 : (int)h->subs.size();
-    for (int i = 0; i < n; ++i) {
-        qlnlp_handle s = h->subs.empty() ? h : h->subs[i];
+    const Problem& p = h->prob;
+    for (size_t i = 0; i < h->devs.size(); ++i) {
+        DeviceState& ds = h->devs[i];
         if (B[i] == 0) continue;
-        DeviceGuard guard(s->device);
-        if (int rc = ensure_device(s)) return rc;
+        DeviceGuard guard(ds.device);
+        if (int rc = ensure_device(p, ds)) return rc;
         cudaStream_t st = streams ? static_cast<cudaStream_t>(streams[i]) : nullptr;
-        if (int rc = s->kin ? launch_kin(s, B[i], io + i, st) : launch(s, B[i], io + i, st)) return rc;
+        if (int rc = p.kin ? launch_kin(p, ds, B[i], io + i, st) : launch(p, ds, B[i], io + i, st)) return rc;
     }
     return QLNLP_OK;
 }
@@ -1452,11 +1464,9 @@ int qlnlp_eval_batch_device_multi(qlnlp_handle h, const int64_t* B, const qlnlp_
 int qlnlp_synchronize(qlnlp_handle h)
 {
     if (int rc = check_handle(h)) return rc;
-    const int n = h->subs.empty() ? 1 : (int)h->subs.size();
-    for (int i = 0; i < n; ++i) {
-        qlnlp_handle s = h->subs.empty() ? h : h->subs[i];
-        if (!s->dev_ready) continue;
-        DeviceGuard guard(s->device);
+    for (const DeviceState& ds : h->devs) {
+        if (!ds.ready) continue;
+        DeviceGuard guard(ds.device);
         CUDA_TRY(cudaDeviceSynchronize());
     }
     return QLNLP_OK;
@@ -1465,15 +1475,16 @@ int qlnlp_synchronize(qlnlp_handle h)
 int qlnlp_eval_ragged_device(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, const qlnlp_ragged_io* rg, void* stream)
 {
     if (int rc = check_handle(h)) return rc;
-    if (!h->subs.empty()) return fail(QLNLP_EINVAL, "multi-device handle: ragged launches take a single-device handle");
+    if (h->multi) return fail(QLNLP_EINVAL, "multi-device handle: ragged launches take a single-device handle");
     if (!rg) return fail(QLNLP_EINVAL, "null ragged descriptor");
-    if (h->kin) return fail(QLNLP_EINVAL, "ragged launches do not carry the kinematic rows");
+    if (h->prob.kin) return fail(QLNLP_EINVAL, "ragged launches do not carry the kinematic rows");
     if (B == 0) return QLNLP_OK;
-    DeviceGuard guard(h->device);
-    if (int rc = ensure_device(h)) return rc;
+    DeviceState& ds = h->devs[0];
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(h->prob, ds)) return rc;
     const RagTable* table = nullptr;
     if (int rc = ragged_table(&h, 1, &table)) return rc;
-    return launch(h, B, io, static_cast<cudaStream_t>(stream), -1, rg, table, nullptr);
+    return launch(h->prob, ds, B, io, static_cast<cudaStream_t>(stream), -1, rg, table, nullptr);
 }
 
 int qlnlp_eval_ragged_classes(const qlnlp_handle* hs, int ncls, int64_t B, const qlnlp_batch_io* io,
@@ -1484,44 +1495,46 @@ int qlnlp_eval_ragged_classes(const qlnlp_handle* hs, int ncls, int64_t B, const
     if (ncls > 1 && !class_of) return fail(QLNLP_EINVAL, "class_of is required with more than one class");
     for (int i = 0; i < ncls; ++i) {
         if (int rc = check_handle(hs[i])) return rc;
-        if (!hs[i]->subs.empty()) return fail(QLNLP_EINVAL, "multi-device handle: ragged launches take single-device handles");
-        if (hs[i]->device != hs[0]->device) return fail(QLNLP_EINVAL, "the classes of a ragged launch must share one device");
-        if (batch_jm(hs[i]) != batch_jm(hs[0])) return fail(QLNLP_EINVAL, "the classes of a ragged launch must share one Jacobian pattern");
-        if (hs[i]->kin) return fail(QLNLP_EINVAL, "ragged launches do not carry the kinematic rows");
+        if (hs[i]->multi) return fail(QLNLP_EINVAL, "multi-device handle: ragged launches take single-device handles");
+        if (hs[i]->devs[0].device != hs[0]->devs[0].device) return fail(QLNLP_EINVAL, "the classes of a ragged launch must share one device");
+        if (batch_jm(hs[i]->prob) != batch_jm(hs[0]->prob)) return fail(QLNLP_EINVAL, "the classes of a ragged launch must share one Jacobian pattern");
+        if (hs[i]->prob.kin) return fail(QLNLP_EINVAL, "ragged launches do not carry the kinematic rows");
     }
     if (B == 0) return QLNLP_OK;
-    DeviceGuard guard(hs[0]->device);
+    DeviceGuard guard(hs[0]->devs[0].device);
     for (int i = 0; i < ncls; ++i)
-        if (int rc = ensure_device(hs[i])) return rc;
+        if (int rc = ensure_device(hs[i]->prob, hs[i]->devs[0])) return rc;
     const RagTable* table = nullptr;
     if (int rc = ragged_table(hs, ncls, &table)) return rc;
-    return launch(hs[0], B, io, static_cast<cudaStream_t>(stream), -1, rg, table, class_of);
+    return launch(hs[0]->prob, hs[0]->devs[0], B, io, static_cast<cudaStream_t>(stream), -1, rg, table, class_of);
 }
 
 int qlnlp_eval_batch_host(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io)
 {
     if (int rc = check_handle(h)) return rc;
-    if (h->subs.empty()) return eval_host(h, B, io);
+    if (!h->multi) return eval_host(h, 0, B, io);
     if (B == 0) return QLNLP_OK;
     if (B < 0 || !io) return fail(QLNLP_EINVAL, "bad batch");
+    // the drivers share the row plan: build it before any of them may need it
+    if (io->jac && !h->prob.kin)
+        if (int rc = ensure_plan(h)) return rc;
     // contiguous shards, one driver thread per device, no exchange between the devices
-    const int n = (int)h->subs.size();
+    const int n = (int)h->devs.size();
     std::vector<int> rcs(n, QLNLP_OK);
     std::vector<std::string> msgs(n);
     for (int i = 0; i < n; ++i) {
         int64_t lo, hi;
         shard_bounds(B, n, i, &lo, &hi);
         if (hi == lo) continue;
-        const qlnlp_batch_io d = shard_io(h->cls, *io, lo);
-        qlnlp_handle s = h->subs[i];
-        h->drivers[i]->submit([s, d, lo, hi, i, &rcs, &msgs] {
-            rcs[i] = eval_host(s, hi - lo, &d);
+        const qlnlp_batch_io d = shard_io(h->prob.cls, *io, lo);
+        h->drivers[i]->submit([h, d, lo, hi, i, &rcs, &msgs] {
+            rcs[i] = eval_host(h, i, hi - lo, &d);
             if (rcs[i]) msgs[i] = g_err;        // g_err is per thread
         });
     }
     for (auto& w : h->drivers) w->wait();
     for (int i = 0; i < n; ++i)
-        if (rcs[i]) return fail(rcs[i], "device %d: %s", h->subs[i]->device, msgs[i].c_str());
+        if (rcs[i]) return fail(rcs[i], "device %d: %s", h->devs[(size_t)i].device, msgs[i].c_str());
     return QLNLP_OK;
 }
 
@@ -1530,33 +1543,22 @@ int qlnlp_host_output_register(qlnlp_handle h, double* jac, int64_t ldjac, int64
     if (int rc = check_handle(h)) return rc;
     if (!jac || B < 1) return fail(QLNLP_EINVAL, "bad buffer");
     if ((reinterpret_cast<uintptr_t>(jac) & 7) != 0) return fail(QLNLP_EINVAL, "jac must be 8-byte aligned");
-    if (ldjac < batch_nnz(h)) return fail(QLNLP_EINVAL, "ldjac < nnz");
-    if (h->kin) return fail(QLNLP_EINVAL, "registered output rows are not available with the kinematic rows");
-    const int n = h->subs.empty() ? 1 : (int)h->subs.size();
-    // every device's handle may be asked for any slice of the buffer: all of them learn the registration; the
-    // constant image is written once, by the first handle's pool
-    for (int i = 0; i < n; ++i) {
-        qlnlp_handle s = h->subs.empty() ? h : h->subs[i];
-        if (int rc = ensure_plan(s)) return rc;
-        for (auto it = s->regs.begin(); it != s->regs.end();)
-            it = (it->ptr == jac) ? s->regs.erase(it) : it + 1;
-        s->regs.push_back({jac, ldjac, B});
-    }
-    qlnlp_handle s0 = first(h);
-    if (int rc = ensure_pool(s0)) return rc;
-    s0->plan->build(s0->pool.get(), nullptr, 0, jac, ldjac, B, false);
+    if (ldjac < batch_nnz(h->prob)) return fail(QLNLP_EINVAL, "ldjac < nnz");
+    if (h->prob.kin) return fail(QLNLP_EINVAL, "registered output rows are not available with the kinematic rows");
+    if (int rc = ensure_plan(h)) return rc;
+    qlnlp_host_output_unregister(h, jac);
+    h->regs.push_back({jac, ldjac, B});
+    // the constant image is written once, by the first device's pool
+    if (int rc = ensure_pool(h, 0)) return rc;
+    h->plan->build(h->devs[0].pool.get(), nullptr, 0, jac, ldjac, B, false);
     return QLNLP_OK;
 }
 
 int qlnlp_host_output_unregister(qlnlp_handle h, double* jac)
 {
     if (int rc = check_handle(h)) return rc;
-    const int n = h->subs.empty() ? 1 : (int)h->subs.size();
-    for (int i = 0; i < n; ++i) {
-        qlnlp_handle s = h->subs.empty() ? h : h->subs[i];
-        for (auto it = s->regs.begin(); it != s->regs.end();)
-            it = (it->ptr == jac) ? s->regs.erase(it) : it + 1;
-    }
+    for (auto it = h->regs.begin(); it != h->regs.end();)
+        it = (it->ptr == jac) ? h->regs.erase(it) : it + 1;
     return QLNLP_OK;
 }
 
@@ -1625,7 +1627,7 @@ int qlnlp_hessian_nnz(qlnlp_handle h, int64_t* nnz)
 {
     if (int rc = check_handle(h)) return rc;
     if (!nnz) return fail(QLNLP_EINVAL, "null output");
-    *nnz = ql_hess_nnz(h->cls);
+    *nnz = ql_hess_nnz(h->prob.cls);
     return QLNLP_OK;
 }
 
@@ -1633,7 +1635,7 @@ int qlnlp_hessian_structure(qlnlp_handle h, int64_t* rows, int64_t* cols)
 {
     if (int rc = check_handle(h)) return rc;
     if (!rows || !cols) return fail(QLNLP_EINVAL, "null output");
-    hessian_structure(h->cls, rows, cols);
+    hessian_structure(h->prob.cls, rows, cols);
     return QLNLP_OK;
 }
 
@@ -1641,34 +1643,36 @@ int qlnlp_eval_hessian_batch_device(qlnlp_handle h, int64_t B, const double* Z, 
                                     const double* lambda, int64_t ldlambda, double* H, int64_t ldh, void* stream)
 {
     if (int rc = check_handle(h)) return rc;
-    if (!h->subs.empty()) return fail(QLNLP_EINVAL, "multi-device handle: the Hessian takes a single-device handle");
-    if (h->kin) return fail(QLNLP_EINVAL, "the Hessian does not cover the kinematic rows");
+    if (h->multi) return fail(QLNLP_EINVAL, "multi-device handle: the Hessian takes a single-device handle");
+    if (h->prob.kin) return fail(QLNLP_EINVAL, "the Hessian does not cover the kinematic rows");
     if (B == 0) return QLNLP_OK;
-    DeviceGuard guard(h->device);
-    if (int rc = ensure_device(h)) return rc;
-    return launch_hessian(h, B, Z, ldz, sigma, 1.0, lambda, ldlambda, H, ldh, static_cast<cudaStream_t>(stream));
+    DeviceState& ds = h->devs[0];
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(h->prob, ds)) return rc;
+    return launch_hessian(h->prob, ds, B, Z, ldz, sigma, 1.0, lambda, ldlambda, H, ldh, static_cast<cudaStream_t>(stream));
 }
 
-int qlnlp_eval_hessian_lagrangian(qlnlp_handle hh, const double* x, double sigma, const double* lambda, double* vals)
+int qlnlp_eval_hessian_lagrangian(qlnlp_handle h, const double* x, double sigma, const double* lambda, double* vals)
 {
-    if (int rc = check_handle(hh)) return rc;
+    if (int rc = check_handle(h)) return rc;
     if (!x || !lambda || !vals) return fail(QLNLP_EINVAL, "null argument");
-    if (hh->kin) return fail(QLNLP_EINVAL, "the Hessian does not cover the kinematic rows");
-    qlnlp_handle h = first(hh);
-    const QlClass& c = h->cls;
-    DeviceGuard guard(h->device);
-    if (int rc = ensure_device(h)) return rc;
+    const Problem& p = h->prob;
+    if (p.kin) return fail(QLNLP_EINVAL, "the Hessian does not cover the kinematic rows");
+    DeviceState& ds = h->devs[0];
+    const QlClass& c = p.cls;
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(p, ds)) return rc;
     const int64_t ldl = (c.m_nlp + 1) & ~1, ldh = (ql_hess_nnz(c) + 1) & ~1;
-    if (!h->d_hess_in) {
-        CUDA_TRY(cudaMalloc(&h->d_hess_in, sizeof(double) * (h->ldz_e + ldl)));
-        CUDA_TRY(cudaMalloc(&h->d_hess_out, sizeof(double) * ldh));
+    if (!ds.d_hess_in) {
+        CUDA_TRY(cudaMalloc(&ds.d_hess_in, sizeof(double) * (p.ldz_e + ldl)));
+        CUDA_TRY(cudaMalloc(&ds.d_hess_out, sizeof(double) * ldh));
     }
-    cudaStream_t s = h->one.stream;
-    CUDA_TRY(cudaMemcpyAsync(h->d_hess_in, x, sizeof(double) * c.n_nlp, cudaMemcpyHostToDevice, s));
-    CUDA_TRY(cudaMemcpyAsync(h->d_hess_in + h->ldz_e, lambda, sizeof(double) * c.m_nlp, cudaMemcpyHostToDevice, s));
-    int rc = launch_hessian(h, 1, h->d_hess_in, h->ldz_e, nullptr, sigma, h->d_hess_in + h->ldz_e, ldl, h->d_hess_out, ldh, s);
+    cudaStream_t s = ds.one.stream;
+    CUDA_TRY(cudaMemcpyAsync(ds.d_hess_in, x, sizeof(double) * c.n_nlp, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(ds.d_hess_in + p.ldz_e, lambda, sizeof(double) * c.m_nlp, cudaMemcpyHostToDevice, s));
+    int rc = launch_hessian(p, ds, 1, ds.d_hess_in, p.ldz_e, nullptr, sigma, ds.d_hess_in + p.ldz_e, ldl, ds.d_hess_out, ldh, s);
     if (rc == QLNLP_OK) {
-        cudaError_t e = cudaMemcpyAsync(vals, h->d_hess_out, sizeof(double) * ql_hess_nnz(c), cudaMemcpyDeviceToHost, s);
+        cudaError_t e = cudaMemcpyAsync(vals, ds.d_hess_out, sizeof(double) * ql_hess_nnz(c), cudaMemcpyDeviceToHost, s);
         if (e != cudaSuccess) rc = fail(QLNLP_ECUDA, "Hessian: %s", cudaGetErrorString(e));
     }
     const std::string msg = g_err;
@@ -1680,20 +1684,21 @@ int qlnlp_eval_hessian_lagrangian(qlnlp_handle hh, const double* x, double sigma
 
 /* Batched initial guesses on the device (SURVEY.md 8f N2; main.ipynb:181-196): Z[b] = the class guess `base` with the
  * first 14 states of knots 1..k_trans interpolated from x0[b] to the handle's terminal state.  All device pointers. */
-int qlnlp_initial_guess_batch_device(qlnlp_handle hh, int64_t B, const double* base, const double* x0, double* Z,
+int qlnlp_initial_guess_batch_device(qlnlp_handle h, int64_t B, const double* base, const double* x0, double* Z,
                                      int64_t ldz, void* stream)
 {
-    if (int rc = check_handle(hh)) return rc;
+    if (int rc = check_handle(h)) return rc;
     if (B == 0) return QLNLP_OK;
     if (B < 0 || !base || !x0 || !Z) return fail(QLNLP_EINVAL, "bad arguments");
-    qlnlp_handle h = first(hh);
-    if (ldz < h->cls.n_nlp) return fail(QLNLP_EINVAL, "ldz < n_nlp");
-    DeviceGuard guard(h->device);
-    if (int rc = ensure_device(h)) return rc;
-    const long long total = (long long)B * h->cls.n_nlp;
+    const QlClass& c = h->prob.cls;
+    DeviceState& ds = h->devs[0];
+    if (ldz < c.n_nlp) return fail(QLNLP_EINVAL, "ldz < n_nlp");
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(h->prob, ds)) return rc;
+    const long long total = (long long)B * c.n_nlp;
     const int threads = 256;
     ql::initial_guess_kernel<<<(unsigned)((total + threads - 1) / threads), threads, 0, static_cast<cudaStream_t>(stream)>>>(
-        base, x0, h->d_x0xf + QL_NX, Z, ldz, B, h->cls.n_nlp, h->cls.k_trans);
+        base, x0, ds.d_x0xf + QL_NX, Z, ldz, B, c.n_nlp, c.k_trans);
     CUDA_TRY(cudaGetLastError());
     return QLNLP_OK;
 }
@@ -1701,9 +1706,9 @@ int qlnlp_initial_guess_batch_device(qlnlp_handle hh, int64_t B, const double* b
 int qlnlp_eval_all(qlnlp_handle h, const double* x, double* f, double* grad, double* g, double* vals)
 {
     if (int rc = check_handle(h)) return rc;
-    if (vals && h->jac_mode == QLNLP_JAC_DENSE) {
+    if (vals && h->prob.jac_mode == QLNLP_JAC_DENSE) {
         if (int rc = eval_one(h, x, f, grad, g, nullptr)) return rc;
-        return eval_dense_jacobian(h, x, vals);
+        return eval_dense_jacobian(h->prob, h->devs[0], x, vals);
     }
     return eval_one(h, x, f, grad, g, vals);
 }
@@ -1730,15 +1735,15 @@ int qlnlp_eval_constraint_jacobian(qlnlp_handle h, const double* x, double* vals
 {
     if (int rc = check_handle(h)) return rc;
     if (!vals) return fail(QLNLP_EINVAL, "null output");
-    if (h->jac_mode != QLNLP_JAC_DENSE) return eval_one(h, x, nullptr, nullptr, nullptr, vals);
-    return eval_dense_jacobian(h, x, vals);
+    if (h->prob.jac_mode != QLNLP_JAC_DENSE) return eval_one(h, x, nullptr, nullptr, nullptr, vals);
+    return eval_dense_jacobian(h->prob, h->devs[0], x, vals);
 }
 
 int qlnlp_launch_info(qlnlp_handle h, int64_t info[5])
 {
     if (int rc = check_handle(h)) return rc;
     if (!info) return fail(QLNLP_EINVAL, "null output");
-    for (int i = 0; i < 5; ++i) info[i] = first(h)->last_launch[i];
+    for (int i = 0; i < 5; ++i) info[i] = h->devs[0].last_launch[i];
     return QLNLP_OK;
 }
 
@@ -1746,20 +1751,18 @@ int qlnlp_host_path_info(qlnlp_handle h, int64_t info[8])
 {
     if (int rc = check_handle(h)) return rc;
     if (!info) return fail(QLNLP_EINVAL, "null output");
-    qlnlp_handle s = first(h);
-    if (int rc = ensure_plan(s)) return rc;
+    if (int rc = ensure_plan(h)) return rc;
     int64_t rows = 0, lines = 0;
-    const int n = h->subs.empty() ? 1 : (int)h->subs.size();
-    for (int i = 0; i < n; ++i) {
-        const qlnlp_handle t = h->subs.empty() ? h : h->subs[i];
-        rows += t->stat_host_rows;
-        lines += t->stat_host_lines;
+    for (const DeviceState& ds : h->devs) {
+        rows += ds.stat_host_rows;
+        lines += ds.stat_host_lines;
     }
-    info[0] = s->pool ? s->pool->size() : 0;          // worker threads per device (0: pool not started yet)
-    info[1] = s->cls.nnz_vals;                        // doubles per evaluation that cross PCIe for the Jacobian
-    info[2] = s->plan->nnz();                         // doubles per row of the batch pattern
-    info[3] = s->plan->touched_lines(0);              // 64-byte lines rewritten per registered row (aligned row)
-    info[4] = (s->plan->nnz() + 7) / 8;               // 64-byte lines per row
+    const DeviceState& d0 = h->devs[0];
+    info[0] = d0.pool ? d0.pool->size() : 0;          // worker threads per device (0: pool not started yet)
+    info[1] = h->prob.cls.nnz_vals;                   // doubles per evaluation that cross PCIe for the Jacobian
+    info[2] = h->plan->nnz();                         // doubles per row of the batch pattern
+    info[3] = h->plan->touched_lines(0);              // 64-byte lines rewritten per registered row (aligned row)
+    info[4] = (h->plan->nnz() + 7) / 8;               // 64-byte lines per row
     info[5] = qlhost::RowPlan::have_avx512() ? 1 : 0;
     info[6] = rows;                                   // rows assembled so far
     info[7] = lines;                                  // lines written so far
@@ -1771,8 +1774,8 @@ int qlnlp_host_path_info(qlnlp_handle h, int64_t info[8])
 int qlnlp_debug_host_times(qlnlp_handle h, double out[4])
 {
     if (int rc = check_handle(h)) return rc;
-    qlnlp_handle s = first(h);
-    out[0] = s->stat_t_total; out[1] = s->stat_t_enqueue; out[2] = s->stat_t_wait; out[3] = s->stat_t_build;
+    const DeviceState& ds = h->devs[0];
+    out[0] = ds.stat_t_total; out[1] = ds.stat_t_enqueue; out[2] = ds.stat_t_wait; out[3] = ds.stat_t_build;
     return QLNLP_OK;
 }
 
@@ -1793,10 +1796,11 @@ int qlnlp_debug_launch_geometry(int64_t smem_per_sm, int64_t smem_optin, int per
 int qlnlp_debug_segments(qlnlp_handle h, int64_t* out, int64_t cap, int64_t* nseg)
 {
     if (int rc = check_handle(h)) return rc;
-    if (nseg) *nseg = (int64_t)h->segs.size();
+    const std::vector<QlSeg>& segs = h->prob.segs;
+    if (nseg) *nseg = (int64_t)segs.size();
     if (out) {
-        for (size_t i = 0; i < h->segs.size() && (int64_t)i < cap; ++i) {
-            const QlSeg& s = h->segs[i];
+        for (size_t i = 0; i < segs.size() && (int64_t)i < cap; ++i) {
+            const QlSeg& s = segs[i];
             int64_t* o = out + 6 * i;
             o[0] = s.k0; o[1] = s.nk; o[2] = s.start; o[3] = s.end; o[4] = s.tmpl; o[5] = ql_seg_buffer((unsigned)i);
         }
@@ -1808,16 +1812,9 @@ int qlnlp_debug_segments(qlnlp_handle h, int64_t* out, int64_t cap, int64_t* nse
 int qlnlp_debug_vals_map(qlnlp_handle h, int32_t* pos, int64_t cap, int64_t* n)
 {
     if (int rc = check_handle(h)) return rc;
-    const QlClass& c = h->cls;
     std::vector<double> image;
     std::vector<int32_t> p;
-    block_image_and_vals_map(c, image, p);
-    if (batch_jm(h) == ql::JM_TRUE) {
-        const std::vector<int32_t> t2b = true_to_block(c);
-        std::vector<int32_t> b2t((size_t)c.nnz, -1);
-        for (size_t t = 0; t < t2b.size(); ++t) b2t[(size_t)t2b[t]] = (int32_t)t;
-        for (auto& q : p) q = b2t[(size_t)q];
-    }
+    if (int rc = batch_image_and_vals_map(h->prob, image, p)) return rc;
     if (n) *n = (int64_t)p.size();
     if (pos)
         for (size_t i = 0; i < p.size() && (int64_t)i < cap; ++i) pos[i] = p[i];
@@ -1829,18 +1826,18 @@ int qlnlp_debug_build_rows(qlnlp_handle h, const double* vals, int64_t ldv, doub
                            int touched_only, int threads)
 {
     if (int rc = check_handle(h)) return rc;
-    qlnlp_handle s = first(h);
-    if (int rc = ensure_plan(s)) return rc;
-    if (threads == 1) { s->plan->build_rows(vals, ldv, jac, ldjac, 0, rows, touched_only != 0); return QLNLP_OK; }
+    if (int rc = ensure_plan(h)) return rc;
+    if (threads == 1) { h->plan->build_rows(vals, ldv, jac, ldjac, 0, rows, touched_only != 0); return QLNLP_OK; }
     const bool async = threads < -1;           // negative: the workers-only path the host pipeline uses (Pool::start)
     if (async) threads = -threads;
-    if (threads > 1) { s->opt_host_threads = threads; s->pool.reset(); }
-    if (int rc = ensure_pool(s)) return rc;
+    DeviceState& ds = h->devs[0];
+    if (threads > 1) { h->opt_host_threads = threads; ds.pool.reset(); }
+    if (int rc = ensure_pool(h, 0)) return rc;
     if (async) {
-        s->plan->build_async(s->pool.get(), vals, ldv, jac, ldjac, rows, touched_only != 0);
-        s->pool->finish();
+        h->plan->build_async(ds.pool.get(), vals, ldv, jac, ldjac, rows, touched_only != 0);
+        ds.pool->finish();
     } else {
-        s->plan->build(s->pool.get(), vals, ldv, jac, ldjac, rows, touched_only != 0);
+        h->plan->build(ds.pool.get(), vals, ldv, jac, ldjac, rows, touched_only != 0);
     }
     return QLNLP_OK;
 }

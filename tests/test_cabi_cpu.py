@@ -105,6 +105,50 @@ def test_evaluation_fails_loudly_without_a_gpu():
     assert e.value.code == ev.QLNLP_ENODEVICE and "no CPU path" in str(e.value)
     with pytest.raises(ql.QlnlpError):
         nlp.eval_batch_host(np.zeros((2, 1215)))
+    for devices in ([0], [0, 1]):                           # multi-device handles: the failing shard is named
+        multi = ql.HybridNLP.from_problem(nlp.prob, devices=devices)
+        with pytest.raises(ql.QlnlpError) as e:
+            multi.eval_batch_host(np.zeros((2, 1215)))
+        assert e.value.code == ev.QLNLP_ENODEVICE and f"error {ev.QLNLP_ENODEVICE}: device 0: no CUDA device" in str(e.value)
+
+
+@pytest.mark.parametrize("devices", [[0], [0, 1]])
+def test_multi_device_handle_answers_like_a_plain_handle(devices):
+    """qlnlp_create_multi needs no device until it evaluates: its host-side answers equal those of a plain handle, its
+    devices split the host cores, and the entry points that take a single-device handle refuse it."""
+    p = ql.default_problem()
+    L = ql.load_library()
+    one = ql.HybridNLP.from_problem(p)
+    multi = ql.HybridNLP.from_problem(p, devices=devices)
+    ids, n = (C.c_int * 4)(), C.c_int()
+    assert L.qlnlp_devices(multi._h, ids, 4, C.byref(n)) == 0 and list(ids[:n.value]) == devices
+    assert (multi.n_nlp, multi.m_nlp, multi.nnz, multi.nnz_block) == (one.n_nlp, one.m_nlp, one.nnz, one.nnz_block)
+    for a, b in zip(multi.jacobian_structure_arrays(), one.jacobian_structure_arrays()):
+        assert np.array_equal(a, b)
+    assert np.array_equal(multi._debug_segments(), one._debug_segments())
+    assert np.array_equal(multi._debug_vals_map(), one._debug_vals_map())
+    jm, j1 = np.full((5, multi.nnz_batch), np.nan), np.full((5, one.nnz_batch), np.nan)
+    multi.register_host_output(jm)
+    one.register_host_output(j1)
+    assert not np.isnan(jm).any() and np.array_equal(jm, j1)
+    threads = one.host_path_info()["threads_per_device"]
+    assert multi.host_path_info()["threads_per_device"] == max(1, threads // len(devices))
+    with pytest.raises(ql.QlnlpError) as e:
+        multi.set_option("bogus", 1)
+    assert e.value.code == ev.QLNLP_EINVAL
+    io, rg = ev._BatchIO(), ev._RaggedIO()
+    refusals = [
+        (lambda: L.qlnlp_eval_batch_device(multi._h, 1, C.byref(io), None),
+         "multi-device handle: use qlnlp_eval_batch_device_multi"),
+        (lambda: L.qlnlp_eval_ragged_device(multi._h, 1, C.byref(io), C.byref(rg), None),
+         "multi-device handle: ragged launches take a single-device handle"),
+        (lambda: L.qlnlp_eval_ragged_classes((C.c_void_p * 1)(multi._h.value), 1, 1, C.byref(io), C.byref(rg), None, None),
+         "multi-device handle: ragged launches take single-device handles"),
+        (lambda: L.qlnlp_eval_hessian_batch_device(multi._h, 1, None, 0, None, None, 0, None, 0, None),
+         "multi-device handle: the Hessian takes a single-device handle"),
+    ]
+    for call, msg in refusals:
+        assert call() == ev.QLNLP_EINVAL and L.qlnlp_last_error().decode() == msg
 
 
 def _build_demo(tmp_path):

@@ -661,11 +661,13 @@ def test_calls_leave_the_current_device_alone(dflt):
     assert torch.cuda.current_device() == 0
 
 
-def test_multi_device_handle_shards_the_batch(golden):
+@pytest.mark.parametrize("all_devices", [False, True], ids=["one_device", "all_devices"])
+def test_multi_device_handle_shards_the_batch(golden, all_devices):
     """qlnlp_create_multi: one call spreads a host batch (contiguous shards, one pipeline per device) or launches one
-    device-resident shard per GPU; results must equal the single-device ones bit for bit."""
-    nd = torch.cuda.device_count()
-    if nd < 2:
+    device-resident shard per GPU; results must equal the single-device ones bit for bit.  A multi-device handle over
+    one device takes the same paths."""
+    nd = torch.cuda.device_count() if all_devices else 1
+    if all_devices and nd < 2:
         pytest.skip("needs at least 2 devices")
     p = ql.default_problem()
     one = ql.HybridNLP.from_problem(p)
