@@ -24,35 +24,12 @@ def _point(prob, seed):
 
 def test_rk4_hessian_against_extended_precision():
     """sum_r lam_r Hess(rk4_r): the oracle's second-order forward mode vs central second differences of the RK4 map
-    evaluated in 50-digit arithmetic (mpmath), all three modes."""
+    evaluated in 50-digit arithmetic (the mpmath restatement in tests/mp_nlp.py), all three modes."""
     mp = pytest.importorskip("mpmath")
+    from mp_nlp import rk4
     mp.mp.dps = 50
     model = PlanarQuadruped()
     rng = np.random.default_rng(5)
-
-    def field(mode, x, u):
-        g, mb, mf, lb = (mp.mpf(v) for v in (model.g, model.mb, model.mf, model.lb))
-        Ib = mb * lb * lb / 12
-        xb, yb, x1, y1, x2, y2 = x[0], x[1], x[3], x[4], x[5], x[6]
-        F1x, F1y, F2x, F2y = u[0], u[1], u[2], u[3]
-        tau = -F1x * (y1 - yb) + F1y * (x1 - xb) - F2x * (y2 - yb) + F2y * (x2 - xb)
-        xd = [mp.mpf(0)] * 14
-        xd[0], xd[1], xd[2] = x[7], x[8], x[9]
-        xd[7], xd[8], xd[9] = (F1x + F2x) / mb, (F1y + F2y) / mb + g, tau / Ib
-        if mode == 1:
-            xd[5], xd[6], xd[12], xd[13] = x[12], x[13], -F2x / mf, -F2y / mf + g
-        elif mode == 2:
-            xd[3], xd[4], xd[10], xd[11] = x[10], x[11], -F1x / mf, -F1y / mf + g
-        return xd
-
-    def rk4(mode, z):
-        x, u = z[:15], z[15:]
-        h = u[4]
-        f1 = field(mode, x[:14], u)
-        f2 = field(mode, [x[i] + h / 2 * f1[i] for i in range(14)], u)
-        f3 = field(mode, [x[i] + h / 2 * f2[i] for i in range(14)], u)
-        f4 = field(mode, [x[i] + h * f3[i] for i in range(14)], u)
-        return [x[i] + h / 6 * (f1[i] + 2 * f2[i] + 2 * f3[i] + f4[i]) for i in range(14)] + [x[14] + h]
 
     for mode in (1, 2, 3):
         x = rng.standard_normal(15)
@@ -62,7 +39,7 @@ def test_rk4_hessian_against_extended_precision():
         assert np.array_equal(H, H.T)
         z0 = [mp.mpf(float(v)) for v in np.concatenate([x, u])]
         lm = [mp.mpf(float(v)) for v in lam]
-        phi = lambda z: sum(l * o for l, o in zip(lm, rk4(mode, z)))
+        phi = lambda z: sum(l * o for l, o in zip(lm, rk4(mode, model, z[:15], z[15:])))
         e = mp.mpf(10) ** -12
         scale = max(1.0, np.abs(H).max())
         for (i, j) in [(19, 19), (19, 16), (19, 2), (16, 1), (15, 4), (19, 9), (17, 5), (18, 6), (19, 12), (0, 0), (3, 19), (9, 9)]:

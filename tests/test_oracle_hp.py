@@ -2,8 +2,8 @@
 
 The reference records no gradient/Jacobian values ("parity unpinned", DESIGN.md section 2), so the oracle's
 `qlo_rk4_jacobian` (dense ForwardDiff-style duals in fp64) is checked here against the MATHEMATICAL
-derivative of the reference's RK4 map (planar_quadruped.jl:36-221), obtained from a separate mpmath
-restatement by central differences at 60 digits (truncation error ~1e-36)."""
+derivative of the reference's RK4 map (planar_quadruped.jl:36-221), obtained from the mpmath restatement in
+tests/mp_nlp.py by central differences at 60 digits (truncation error ~1e-36)."""
 import numpy as np
 import pytest
 
@@ -12,34 +12,12 @@ from quadruped_landing_b200 import PlanarQuadruped
 
 mp = pytest.importorskip("mpmath")
 mp.mp.dps = 60
-
-
-def f_mp(mode, m, x, u):
-    """contact{1,2,3}_dynamics, planar_quadruped.jl:36-185, on mpmath numbers (x: 14, u: 5)."""
-    g, mb, mf, lb = (mp.mpf(v) for v in (m.g, m.mb, m.mf, m.lb))
-    Ib = mb * lb ** 2 / 12
-    xb, yb, x1, y1, x2, y2 = x[0], x[1], x[3], x[4], x[5], x[6]
-    F1x, F1y, F2x, F2y = u[0], u[1], u[2], u[3]
-    ax, ay = (F1x + F2x) / mb, (F1y + F2y) / mb + g
-    tau = -F1x * (y1 - yb) + F1y * (x1 - xb) - F2x * (y2 - yb) + F2y * (x2 - xb)
-    z = mp.mpf(0)
-    v1 = [x[10], x[11]] if mode == 2 else [z, z]
-    v2 = [x[12], x[13]] if mode == 1 else [z, z]
-    a1 = [-F1x / mf, -F1y / mf + g] if mode == 2 else [z, z]
-    a2 = [-F2x / mf, -F2y / mf + g] if mode == 1 else [z, z]
-    return [x[7], x[8], x[9]] + v1 + v2 + [ax, ay, tau / Ib] + a1 + a2
+from mp_nlp import rk4  # noqa: E402
 
 
 def rk4_mp(mode, m, z):
-    """contactM_dynamics_rk4, planar_quadruped.jl:189-221, z = [x(15); u(5)]."""
-    x, u = z[:15], z[15:]
-    h = u[4]
-    x14 = x[:14]
-    f1 = f_mp(mode, m, x14, u)
-    f2 = f_mp(mode, m, [a + h / 2 * b for a, b in zip(x14, f1)], u)
-    f3 = f_mp(mode, m, [a + h / 2 * b for a, b in zip(x14, f2)], u)
-    f4 = f_mp(mode, m, [a + h * b for a, b in zip(x14, f3)], u)
-    return [a + h / 6 * (b + 2 * c + 2 * d + e) for a, b, c, d, e in zip(x14, f1, f2, f3, f4)] + [x[14] + h]
+    """contactM_dynamics_rk4, planar_quadruped.jl:189-221, z = [x(15); u(5)] (the restatement in tests/mp_nlp.py)."""
+    return rk4(mode, m, z[:15], z[15:])
 
 
 @pytest.mark.parametrize("mode", [1, 2, 3])
