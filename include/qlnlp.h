@@ -185,6 +185,40 @@ typedef struct {
  * synchronising.  One fused kernel evaluates everything requested. */
 int qlnlp_eval_batch_device(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io, void* stream);
 
+/* ---- matrix-free products: what MOI.eval_constraint_jacobian_product, eval_constraint_jacobian_transpose_product and
+ * eval_hessian_lagrangian_product need to offer [:JacVec] / [:HessVec].  NOT in the reference (moi.jl:26-28).
+ *   J     the Jacobian the handle reports, quirks included (Q2: the zeroed time row at the jump knot, Q4: the body
+ *         row's d/dtheta branches on theta > 0), with the 2N kinematic rows on a QLNLP_WITH_KINEMATICS handle; w and
+ *         J'y have n_nlp entries, y and Jw m_nlp (kinematic rows included).  The same for every jac_mode.
+ *   H     the matrix qlnlp_eval_hessian_* returns (its lower triangle, mirrored), same sigma / lambda conventions;
+ *         handles with kinematic rows are refused, as by the Hessian.
+ * Summation order (the bits are defined): every output entry is the left fold, starting from the first term, of
+ * RN(entry * vector) terms added with RN(a + b), no fused multiply-add, over the structurally non-zero entries (the
+ * SPARSE_TRUE pattern; for H the entries of qlnlp_hessian_structure and their mirror images):
+ *   (J w)_r   row r's entries in ascending column order (a defect row: the RK4 block's 20 columns, then -w_(k+1));
+ *   (J'y)_c   column c's entries in ascending row order (the order of the column inside the SPARSE_BLOCK values);
+ *   (H v)_i   row i of the knot's symmetric block in ascending column order.
+ * The result does not depend on B, the batch position, leading dimensions, alignment or the entry point used. */
+typedef struct {
+    const double* w;  int64_t ldw;     /* [B][ldw >= n_nlp]   or NULL: no J w */
+    double* jw;       int64_t ldjw;    /* [B][ldjw >= m_nlp]  required iff w */
+    const double* y;  int64_t ldy;     /* [B][ldy >= m_nlp]   or NULL: no J'y */
+    double* jty;      int64_t ldjty;   /* [B][ldjty >= n_nlp] required iff y */
+} qlnlp_product_io;
+/* DEVICE pointers, enqueued on `stream`, not synchronised.  io->jac must be NULL; io->Z, x0, xf, f, grad, g as in
+ * qlnlp_eval_batch_device: one fused launch evaluates everything requested.  Single-device handles only. */
+int qlnlp_eval_jacobian_products_batch_device(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io,
+                                              const qlnlp_product_io* pv, void* stream);
+/* DEVICE pointers: Z[B][ldz], sigma[B] (NULL: 1.0), lambda[B][ldlambda], V[B][ldv], HV[B][ldhv >= n_nlp] */
+int qlnlp_eval_hessian_product_batch_device(qlnlp_handle h, int64_t B, const double* Z, int64_t ldz, const double* sigma,
+                                            const double* lambda, int64_t ldlambda, const double* V, int64_t ldv,
+                                            double* HV, int64_t ldhv, void* stream);
+/* the MOI callbacks: HOST pointers, synchronous, one evaluation on the handle's first device */
+int qlnlp_eval_constraint_jacobian_product(qlnlp_handle h, const double* x, const double* w, double* jw);
+int qlnlp_eval_constraint_jacobian_transpose_product(qlnlp_handle h, const double* x, const double* y, double* jty);
+int qlnlp_eval_hessian_lagrangian_product(qlnlp_handle h, const double* x, const double* v, double sigma,
+                                          const double* lambda, double* hv);
+
 /* Ragged batches: problems of different size (several handles = several (N, k_trans, init_mode) classes) packed
  * back to back in flat arrays.  One call evaluates the B problems of THIS handle's class; the b-th of them is problem
  * number i = index[b] (or b when index is NULL) of the flat batch and its rows start at

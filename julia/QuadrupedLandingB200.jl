@@ -136,6 +136,22 @@ function gpu_hessian_lagrangian_structure(ev::GpuEvaluator)
     check(ccall((:qlnlp_hessian_structure, LIBQLNLP), Cint, (Ptr{Cvoid}, Ptr{Int64}, Ptr{Int64}), ev.handle, rows, cols))
     return collect(zip(rows, cols))                                           # lower triangle, 1-based
 end
+# matrix-free products (MOI :JacVec / :HessVec; NOT in the reference); used when install!(...; products=true)
+function gpu_eval_constraint_jacobian_product(ev::GpuEvaluator, y, x, w)
+    check(ccall((:qlnlp_eval_constraint_jacobian_product, LIBQLNLP), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}),
+                ev.handle, x, w, y))
+    return y
+end
+function gpu_eval_constraint_jacobian_transpose_product(ev::GpuEvaluator, y, x, w)
+    check(ccall((:qlnlp_eval_constraint_jacobian_transpose_product, LIBQLNLP), Cint,
+                (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}), ev.handle, x, w, y))
+    return y
+end
+function gpu_eval_hessian_lagrangian_product(ev::GpuEvaluator, h, x, v, sigma, mu)
+    check(ccall((:qlnlp_eval_hessian_lagrangian_product, LIBQLNLP), Cint,
+                (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Cdouble, Ptr{Cdouble}, Ptr{Cdouble}), ev.handle, x, v, sigma, mu, h))
+    return h
+end
 function gpu_eval_hessian_lagrangian(ev::GpuEvaluator, H, x, sigma, mu)
     check(ccall((:qlnlp_eval_hessian_lagrangian, LIBQLNLP), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Cdouble, Ptr{Cdouble}, Ptr{Cdouble}),
                 ev.handle, x, sigma, mu, H))
@@ -186,16 +202,20 @@ evaluator(nlp) = get(HANDLES, nlp) do
 end
 
 """
-    install!(nlp; sparse=false, pattern=:block, device=0, devices=nothing, hessian=false, into=Main)
+    install!(nlp; sparse=false, pattern=:block, device=0, devices=nothing, hessian=false, products=false, into=Main)
 
 Make `nlp` (a `HybridNLP` of the reference) evaluate on the GPU.  Re-defines, in module `into` (where the reference's
 src/nlp.jl and src/moi.jl were included), the seven MOI methods of src/moi.jl:1-33 for `::HybridNLP`; afterwards
 `solve(Z0, nlp; c_tol=1e-3, tol=1e-3)` (src/main.ipynb:742-744, src/moi.jl:46-103) runs without any edit.
 Every `HybridNLP` handed to MOI after this call needs its own `install!`.
+`products=true` also defines the matrix-free MOI methods `eval_constraint_jacobian_product` and
+`eval_constraint_jacobian_transpose_product` (`:JacVec`), and with `hessian=true` `eval_hessian_lagrangian_product`
+(`:HessVec`); the summation order of every product is fixed (include/qlnlp.h).
 """
-function install!(nlp; into::Module=Main, hessian::Bool=false, kwargs...)
+function install!(nlp; into::Module=Main, hessian::Bool=false, products::Bool=false, kwargs...)
     HANDLES[nlp] = GpuEvaluator(nlp; kwargs...)
     feats = hessian ? [:Grad, :Jac, :Hess] : [:Grad, :Jac]
+    products && append!(feats, hessian ? [:JacVec, :HessVec] : [:JacVec])
     Core.eval(into, quote
         $MOI.eval_objective(prob::HybridNLP, x) =
             $gpu_eval_objective($evaluator(prob), x)                                          # moi.jl:1-3
@@ -211,6 +231,16 @@ function install!(nlp; into::Module=Main, hessian::Bool=false, kwargs...)
             $gpu_eval_hessian_lagrangian($evaluator(prob), H, x, sigma, mu)
         $MOI.initialize(prob::HybridNLP, features) = nothing                                   # moi.jl:30
         $MOI.jacobian_structure(prob::HybridNLP) = $gpu_jacobian_structure($evaluator(prob))   # moi.jl:31-33
+    end)
+    products && Core.eval(into, quote
+        $MOI.eval_constraint_jacobian_product(prob::HybridNLP, y, x, w) =
+            $gpu_eval_constraint_jacobian_product($evaluator(prob), y, x, w)                  # y = J(x) w
+        $MOI.eval_constraint_jacobian_transpose_product(prob::HybridNLP, y, x, w) =
+            $gpu_eval_constraint_jacobian_transpose_product($evaluator(prob), y, x, w)        # y = J(x)' w
+    end)
+    products && hessian && Core.eval(into, quote
+        $MOI.eval_hessian_lagrangian_product(prob::HybridNLP, h, x, v, sigma, mu) =
+            $gpu_eval_hessian_lagrangian_product($evaluator(prob), h, x, v, sigma, mu)        # h = Hess L(x, sigma, mu) v
     end)
     return HANDLES[nlp]
 end

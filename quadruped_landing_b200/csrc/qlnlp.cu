@@ -144,6 +144,9 @@ struct DeviceState {
     double* d_hess_in = nullptr;
     double* d_hess_out = nullptr;
     int hess_blocks_per_sm = 0;
+    int prod_blocks_per_sm = 0;        // matrix-free products: resident CTAs of eval_prod_kernel / hess_prod_kernel
+    int hprod_blocks_per_sm = 0;
+    double* d_prod_one = nullptr;      // scratch of the three product callbacks: 5 rows
     int* d_kin_map = nullptr;          // caller-visible value order of the batch pattern -> scratch position or -(entry + 1)
     std::map<cudaStream_t, std::pair<double*, int64_t>> kin_scratch;   // per stream: reference-order rows (device), capacity
     std::map<std::vector<uint64_t>, RagTable> rag_tables;       // ragged launches led by this handle (key: the classes' serials)
@@ -862,6 +865,155 @@ int launch_hessian(const Problem& p, DeviceState& ds, int64_t B, const double* Z
     return QLNLP_OK;
 }
 
+// ---- matrix-free products (MOI :JacVec / :HessVec) ---------------------------------------------------------------
+// Argument checks of the batched product entry points: host logic only, before any device is touched.
+int check_products(const Problem& p, int64_t B, const qlnlp_batch_io* io, const qlnlp_product_io* pv)
+{
+    const QlClass& c = p.cls;
+    const int m = m_rows(p);
+    if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
+    if (!io || !pv || !io->Z) return fail(QLNLP_EINVAL, "io, pv and io->Z are required");
+    if (io->jac) return fail(QLNLP_EINVAL, "io->jac must be NULL: the product launch writes no Jacobian values");
+    if (!pv->w && !pv->y) return fail(QLNLP_EINVAL, "pv->w or pv->y is required");
+    if (!pv->w != !pv->jw) return fail(QLNLP_EINVAL, "pv->jw is required iff pv->w is set");
+    if (!pv->y != !pv->jty) return fail(QLNLP_EINVAL, "pv->jty is required iff pv->y is set");
+    if (io->ldz < c.n_nlp) return fail(QLNLP_EINVAL, "ldz %lld < n_nlp %d", (long long)io->ldz, c.n_nlp);
+    if (io->grad && io->ldgrad < c.n_nlp) return fail(QLNLP_EINVAL, "ldgrad %lld < n_nlp %d", (long long)io->ldgrad, c.n_nlp);
+    if (io->g && io->ldg < m) return fail(QLNLP_EINVAL, "ldg %lld < m_nlp %d", (long long)io->ldg, m);
+    if (pv->w && (pv->ldw < c.n_nlp || pv->ldjw < m))
+        return fail(QLNLP_EINVAL, "ldw %lld < n_nlp %d or ldjw %lld < m_nlp %d", (long long)pv->ldw, c.n_nlp, (long long)pv->ldjw, m);
+    if (pv->y && (pv->ldy < m || pv->ldjty < c.n_nlp))
+        return fail(QLNLP_EINVAL, "ldy %lld < m_nlp %d or ldjty %lld < n_nlp %d", (long long)pv->ldy, m, (long long)pv->ldjty, c.n_nlp);
+    for (const void* a : {(const void*)io->Z, (const void*)pv->w, (const void*)pv->jw, (const void*)pv->y, (const void*)pv->jty})
+        if ((reinterpret_cast<uintptr_t>(a) & 7) != 0) return fail(QLNLP_EINVAL, "arrays must be 8-byte aligned");
+    return QLNLP_OK;
+}
+
+// One fused launch of eval_prod_kernel: what launch() does for a plain batch, with J w / J' y in place of a value stream.
+int launch_products(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* io, const qlnlp_product_io* pv,
+                    cudaStream_t stream)
+{
+    const QlClass& c = p.cls;
+    const void* fn = p.fastdiv ? (const void*)ql::eval_prod_kernel<true> : (const void*)ql::eval_prod_kernel<false>;
+    const size_t smem = ql::smem_bytes(c.N, ql::JM_PROD);
+    if (!ds.prod_blocks_per_sm) {
+        if (smem > ds.smem_optin) return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp", c.N, smem);
+        if (int rc = kernel_geometry(ds, fn, ql::JM_PROD, smem, &ds.prod_blocks_per_sm)) return rc;
+    }
+    ql::ProdLaunch P;
+    std::memset(&P, 0, sizeof P);
+    P.c = c;
+    P.rmb = p.rmb; P.rmf = p.rmf; P.rIb = p.rIb;
+    P.cost = ds.d_cost;
+    P.npad = p.npad;
+    P.x0_def = ds.d_x0xf;
+    P.xf_def = ds.d_x0xf + QL_NX;
+    P.Z = io->Z; P.ldz = io->ldz;
+    P.x0 = io->x0; P.xf = io->xf;
+    P.f = io->f;
+    P.grad = io->grad; P.ldgrad = io->ldgrad;
+    P.g = io->g; P.ldg = io->ldg;
+    P.B = B;
+    P.zbulk = ((reinterpret_cast<uintptr_t>(io->Z) & 15) == 0 && (io->ldz & 1) == 0) ? 1 : 0;
+    P.w = pv->w; P.ldw = pv->ldw;
+    P.jw = pv->jw; P.ldjw = pv->ldjw;
+    P.y = pv->y; P.ldy = pv->ldy;
+    P.jty = pv->jty; P.ldjty = pv->ldjty;
+    P.kin = p.kin ? 1 : 0;
+    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
+    const int grid = (int)std::min<int64_t>(B, (int64_t)ds.sm_count * ds.prod_blocks_per_sm);
+    void* args[] = {&P};
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(QL_LANES);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];         // programmatic dependent launch, as in launch()
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    CUDA_TRY(cudaLaunchKernelExC(&cfg, fn, args));
+    return QLNLP_OK;
+}
+
+int check_hess_products(const Problem& p, int64_t B, const double* Z, int64_t ldz, const double* lam, int64_t ldlam,
+                        const double* V, int64_t ldv, const double* HV, int64_t ldhv)
+{
+    const QlClass& c = p.cls;
+    if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
+    if (!Z || !lam || !V || !HV) return fail(QLNLP_EINVAL, "Z, lambda, V and HV are required");
+    if (ldz < c.n_nlp || ldlam < c.m_nlp || ldv < c.n_nlp || ldhv < c.n_nlp) return fail(QLNLP_EINVAL, "leading dimension too small");
+    for (const void* a : {(const void*)Z, (const void*)lam, (const void*)V, (const void*)HV})
+        if ((reinterpret_cast<uintptr_t>(a) & 7) != 0) return fail(QLNLP_EINVAL, "arrays must be 8-byte aligned");
+    return QLNLP_OK;
+}
+
+int launch_hess_products(const Problem& p, DeviceState& ds, int64_t B, const double* Z, int64_t ldz, const double* sigma,
+                         double sigma0, const double* lam, int64_t ldlam, const double* V, int64_t ldv, double* HV,
+                         int64_t ldhv, cudaStream_t stream)
+{
+    const QlClass& c = p.cls;
+    const void* fn = p.fastdiv ? (const void*)ql::hess_prod_kernel<true> : (const void*)ql::hess_prod_kernel<false>;
+    const size_t smem = ql::hess_smem_bytes(c.N);
+    if (!ds.hprod_blocks_per_sm) {
+        if (smem > ds.smem_optin) return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp", c.N, smem);
+        CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ds.smem_optin));
+        int nb = 0;
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, QL_LANES, smem));
+        if (nb < 1) return fail(QLNLP_ECUDA, "Hessian-product kernel does not fit on an SM");
+        if (int rc = set_carveout(fn, nb, smem, ds.smem_per_sm)) return rc;
+        ds.hprod_blocks_per_sm = nb;
+    }
+    ql::HessProdLaunch P;
+    std::memset(&P, 0, sizeof P);
+    P.c = c;
+    P.rmb = p.rmb; P.rmf = p.rmf; P.rIb = p.rIb;
+    P.cost = ds.d_cost; P.npad = p.npad;
+    P.Z = Z; P.ldz = ldz;
+    P.lam = lam; P.ldlam = ldlam;
+    P.sigma = sigma; P.sigma0 = sigma0;
+    P.B = B;
+    P.zbulk = ((reinterpret_cast<uintptr_t>(Z) & 15) == 0 && (ldz & 1) == 0) ? 1 : 0;
+    P.V = V; P.ldv = ldv;
+    P.HV = HV; P.ldhv = ldhv;
+    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
+    const int grid = (int)std::min<int64_t>(B, (int64_t)ds.sm_count * ds.hprod_blocks_per_sm);
+    void* args[] = {&P};
+    CUDA_TRY(cudaLaunchKernel(fn, dim3(grid), dim3(QL_LANES), args, smem, stream));
+    return QLNLP_OK;
+}
+
+// The three MOI product callbacks: copy in, one launch of B = 1, copy out, on the single-evaluation stream of the
+// handle's first device.  `in[0..nin)` go to device slots 1.., x to slot 0; the result comes back from the last slot.
+template <typename RUN>
+int product_one(qlnlp_handle h, const double* x, const double* const* in, const int64_t* nin, int nslots, double* out,
+                int64_t nout, RUN run)
+{
+    const Problem& p = h->prob;
+    DeviceState& ds = h->devs[0];
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(p, ds)) return rc;
+    const int64_t ld = std::max(p.ldz_e, p.ldg_e);           // every slot holds a row of n_nlp or m_nlp (+ 2N) doubles
+    if (!ds.d_prod_one) CUDA_TRY(cudaMalloc(&ds.d_prod_one, sizeof(double) * 5 * ld));
+    double* slot[5];
+    for (int i = 0; i < 5; ++i) slot[i] = ds.d_prod_one + i * ld;
+    cudaStream_t s = ds.one.stream;
+    cudaError_t e = cudaMemcpyAsync(slot[0], x, sizeof(double) * p.cls.n_nlp, cudaMemcpyHostToDevice, s);
+    for (int i = 0; i < nslots - 2 && e == cudaSuccess; ++i)
+        e = cudaMemcpyAsync(slot[1 + i], in[i], sizeof(double) * nin[i], cudaMemcpyHostToDevice, s);
+    int rc = e == cudaSuccess ? run(p, ds, slot, ld, s) : fail(QLNLP_ECUDA, "product: %s", cudaGetErrorString(e));
+    if (rc == QLNLP_OK) {
+        e = cudaMemcpyAsync(out, slot[nslots - 1], sizeof(double) * nout, cudaMemcpyDeviceToHost, s);
+        if (e != cudaSuccess) rc = fail(QLNLP_ECUDA, "product: %s", cudaGetErrorString(e));
+    }
+    const std::string msg = g_err;
+    const cudaError_t es = cudaStreamSynchronize(s);      // also on the error path: the host arrays are caller-owned
+    if (rc == QLNLP_OK && es != cudaSuccess) return fail(QLNLP_ECUDA, "product: %s", cudaGetErrorString(es));
+    g_err = msg;
+    return rc;
+}
+
 void free_lane(HostLane& ln)
 {
     if (ln.stage) cudaFreeHost(ln.stage);
@@ -1225,7 +1377,7 @@ void destroy_device_state(DeviceState& ds)
     }
     if (ds.one.stream) cudaStreamDestroy(ds.one.stream);
     if (ds.one.hx) cudaFreeHost(ds.one.hx);
-    cudaFree(ds.d_hess_in); cudaFree(ds.d_hess_out);
+    cudaFree(ds.d_hess_in); cudaFree(ds.d_hess_out); cudaFree(ds.d_prod_one);
     cudaFree(ds.d_kin_map);
     for (auto& kv : ds.kin_scratch) cudaFree(kv.second.first);
     for (auto& kv : ds.rag_tables) cudaFree(kv.second.d_classes);
@@ -1680,6 +1832,83 @@ int qlnlp_eval_hessian_lagrangian(qlnlp_handle h, const double* x, double sigma,
     if (rc == QLNLP_OK && es != cudaSuccess) return fail(QLNLP_ECUDA, "Hessian: %s", cudaGetErrorString(es));
     g_err = msg;
     return rc;
+}
+
+/* ---- matrix-free products (MOI :JacVec / :HessVec) ---- */
+int qlnlp_eval_jacobian_products_batch_device(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io,
+                                              const qlnlp_product_io* pv, void* stream)
+{
+    if (int rc = check_handle(h)) return rc;
+    if (h->multi) return fail(QLNLP_EINVAL, "multi-device handle: the Jacobian products take a single-device handle");
+    if (B == 0) return QLNLP_OK;
+    if (int rc = check_products(h->prob, B, io, pv)) return rc;
+    DeviceState& ds = h->devs[0];
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(h->prob, ds)) return rc;
+    return launch_products(h->prob, ds, B, io, pv, static_cast<cudaStream_t>(stream));
+}
+
+int qlnlp_eval_hessian_product_batch_device(qlnlp_handle h, int64_t B, const double* Z, int64_t ldz, const double* sigma,
+                                            const double* lambda, int64_t ldlambda, const double* V, int64_t ldv,
+                                            double* HV, int64_t ldhv, void* stream)
+{
+    if (int rc = check_handle(h)) return rc;
+    if (h->multi) return fail(QLNLP_EINVAL, "multi-device handle: the Hessian takes a single-device handle");
+    if (h->prob.kin) return fail(QLNLP_EINVAL, "the Hessian does not cover the kinematic rows");
+    if (B == 0) return QLNLP_OK;
+    if (int rc = check_hess_products(h->prob, B, Z, ldz, lambda, ldlambda, V, ldv, HV, ldhv)) return rc;
+    DeviceState& ds = h->devs[0];
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(h->prob, ds)) return rc;
+    return launch_hess_products(h->prob, ds, B, Z, ldz, sigma, 1.0, lambda, ldlambda, V, ldv, HV, ldhv,
+                                static_cast<cudaStream_t>(stream));
+}
+
+// J w (transpose: J' y) at x for one evaluation: slot 1 holds the vector, slot 2 the result
+static int jacobian_product_one(qlnlp_handle h, const double* x, const double* v, double* out, bool transpose)
+{
+    if (int rc = check_handle(h)) return rc;
+    if (!x || !v || !out) return fail(QLNLP_EINVAL, "null argument");
+    const Problem& p = h->prob;
+    const int64_t n = p.cls.n_nlp, m = m_rows(p);
+    const int64_t nin = transpose ? m : n;
+    return product_one(h, x, &v, &nin, 3, out, transpose ? n : m,
+                       [&](const Problem& pp, DeviceState& ds, double* const* slot, int64_t ld, cudaStream_t s) {
+                           qlnlp_batch_io io;
+                           std::memset(&io, 0, sizeof io);
+                           io.Z = slot[0]; io.ldz = ld;
+                           qlnlp_product_io pv;
+                           std::memset(&pv, 0, sizeof pv);
+                           if (transpose) { pv.y = slot[1]; pv.ldy = ld; pv.jty = slot[2]; pv.ldjty = ld; }
+                           else { pv.w = slot[1]; pv.ldw = ld; pv.jw = slot[2]; pv.ldjw = ld; }
+                           return launch_products(pp, ds, 1, &io, &pv, s);
+                       });
+}
+
+int qlnlp_eval_constraint_jacobian_product(qlnlp_handle h, const double* x, const double* w, double* jw)
+{
+    return jacobian_product_one(h, x, w, jw, false);
+}
+
+int qlnlp_eval_constraint_jacobian_transpose_product(qlnlp_handle h, const double* x, const double* y, double* jty)
+{
+    return jacobian_product_one(h, x, y, jty, true);
+}
+
+int qlnlp_eval_hessian_lagrangian_product(qlnlp_handle h, const double* x, const double* v, double sigma,
+                                          const double* lambda, double* hv)
+{
+    if (int rc = check_handle(h)) return rc;
+    if (!x || !v || !lambda || !hv) return fail(QLNLP_EINVAL, "null argument");
+    const Problem& p = h->prob;
+    if (p.kin) return fail(QLNLP_EINVAL, "the Hessian does not cover the kinematic rows");
+    const double* in[2] = {lambda, v};
+    const int64_t nin[2] = {p.cls.m_nlp, p.cls.n_nlp};
+    return product_one(h, x, in, nin, 4, hv, p.cls.n_nlp,
+                       [&](const Problem& pp, DeviceState& ds, double* const* slot, int64_t ld, cudaStream_t s) {
+                           return launch_hess_products(pp, ds, 1, slot[0], ld, nullptr, sigma, slot[1], ld, slot[2], ld,
+                                                       slot[3], ld, s);
+                       });
 }
 
 /* Batched initial guesses on the device (SURVEY.md 8f N2; main.ipynb:181-196): Z[b] = the class guess `base` with the

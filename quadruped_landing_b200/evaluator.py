@@ -39,6 +39,9 @@ EXPORTED_SYMBOLS = (
     "qlnlp_eval_ragged_classes",
     "qlnlp_hessian_nnz", "qlnlp_hessian_structure", "qlnlp_eval_hessian_lagrangian", "qlnlp_eval_hessian_batch_device",
     "qlnlp_initial_guess_batch_device",
+    "qlnlp_eval_jacobian_products_batch_device", "qlnlp_eval_hessian_product_batch_device",
+    "qlnlp_eval_constraint_jacobian_product", "qlnlp_eval_constraint_jacobian_transpose_product",
+    "qlnlp_eval_hessian_lagrangian_product",
 )
 _DEBUG_SYMBOLS = ("qlnlp_debug_segments", "qlnlp_debug_vals_map", "qlnlp_debug_build_rows", "qlnlp_debug_host_times",
                   "qlnlp_debug_launch_geometry")
@@ -67,6 +70,11 @@ class _BatchIO(C.Structure):
                 ("grad", C.c_void_p), ("ldgrad", C.c_int64),
                 ("g", C.c_void_p), ("ldg", C.c_int64),
                 ("jac", C.c_void_p), ("ldjac", C.c_int64)]
+
+
+class _ProductIO(C.Structure):
+    _fields_ = [("w", C.c_void_p), ("ldw", C.c_int64), ("jw", C.c_void_p), ("ldjw", C.c_int64),
+                ("y", C.c_void_p), ("ldy", C.c_int64), ("jty", C.c_void_p), ("ldjty", C.c_int64)]
 
 
 class _RaggedIO(C.Structure):
@@ -130,6 +138,12 @@ def load_library(rebuild_if_stale: bool = True):
     L.qlnlp_eval_hessian_lagrangian.argtypes = [vp, vp, C.c_double, vp, vp]
     L.qlnlp_eval_hessian_batch_device.argtypes = [vp, C.c_int64, vp, C.c_int64, vp, vp, C.c_int64, vp, C.c_int64, vp]
     L.qlnlp_initial_guess_batch_device.argtypes = [vp, C.c_int64, vp, vp, vp, C.c_int64, vp]
+    L.qlnlp_eval_jacobian_products_batch_device.argtypes = [vp, C.c_int64, C.POINTER(_BatchIO), C.POINTER(_ProductIO), vp]
+    L.qlnlp_eval_hessian_product_batch_device.argtypes = [vp, C.c_int64, vp, C.c_int64, vp, vp, C.c_int64, vp, C.c_int64,
+                                                          vp, C.c_int64, vp]
+    L.qlnlp_eval_constraint_jacobian_product.argtypes = [vp, vp, vp, vp]
+    L.qlnlp_eval_constraint_jacobian_transpose_product.argtypes = [vp, vp, vp, vp]
+    L.qlnlp_eval_hessian_lagrangian_product.argtypes = [vp, vp, vp, C.c_double, vp, vp]
     L.qlnlp_host_alloc.argtypes = [C.c_int64, C.POINTER(vp)]
     L.qlnlp_host_free.argtypes = [vp, C.c_int64]
     for name in [n for n in EXPORTED_SYMBOLS if n not in ("qlnlp_version", "qlnlp_last_error")] + list(_DEBUG_SYMBOLS):
@@ -204,24 +218,27 @@ class HybridNLP:
     def __init__(self, model: PlanarQuadruped, obj: Sequence[QuadraticCost], init_mode: int, k_trans: int,
                  N: int, x0, xf, integration: str = "RK4", *, use_sparse_jacobian: bool = False,
                  pattern: str = "block", device: int = 0, devices: Optional[Sequence[int]] = None,
-                 hessian: bool = False, kinematics: bool = False):
+                 hessian: bool = False, kinematics: bool = False, products: bool = False):
         if integration != "RK4":
             raise ValueError("only RK4 is implemented (as in the reference)")
         self._init(ProblemData.from_costs(model, obj, init_mode, k_trans, N, x0, xf), use_sparse_jacobian, device, pattern,
                    devices, kinematics)
         self.hessian = bool(hessian)
+        self.products = bool(products)
 
     @classmethod
     def from_problem(cls, prob: ProblemData, *, use_sparse_jacobian: bool = True, pattern: str = "block",
                      device: int = 0, devices: Optional[Sequence[int]] = None, hessian: bool = False,
-                     kinematics: bool = False) -> "HybridNLP":
+                     kinematics: bool = False, products: bool = False) -> "HybridNLP":
         """``devices=[0, 1, ...]`` builds a multi-device evaluator (``qlnlp_create_multi``): host-pointer batches are
         sharded over the listed GPUs by the library, ``eval_batch_multi`` launches one shard per device.
         ``hessian=True`` advertises ``"Hess"`` (the reference does not, src/moi.jl:26-28).  ``kinematics=True`` switches
-        on the leg-length rows the reference keeps commented out (nlp.jl:60,70; constraints.jl:115-138,276-288)."""
+        on the leg-length rows the reference keeps commented out (nlp.jl:60,70; constraints.jl:115-138,276-288).
+        ``products=True`` advertises the matrix-free products: ``"JacVec"``, and ``"HessVec"`` with ``hessian=True``."""
         self = cls.__new__(cls)
         self._init(prob, use_sparse_jacobian, device, pattern, devices, kinematics)
         self.hessian = bool(hessian)
+        self.products = bool(products)
         return self
 
     def _init(self, prob: ProblemData, use_sparse_jacobian: bool, device: int, pattern: str = "block",
@@ -258,6 +275,7 @@ class HybridNLP:
             _check(L.qlnlp_create_multi(C.byref(d), arr, len(self.devices), flags, C.byref(self._h)))
         self._registered = {}
         self.hessian = False
+        self.products = False
         nh = C.c_int64()
         _check(L.qlnlp_hessian_nnz(self._h, C.byref(nh)))
         self.nnz_hess = nh.value
@@ -302,7 +320,10 @@ class HybridNLP:
 
     # ---- MOI surface, moi.jl:1-33
     def features_available(self) -> List[str]:
-        return ["Grad", "Jac", "Hess"] if self.hessian else ["Grad", "Jac"]      # moi.jl:26-28 (+ opt-in :Hess)
+        feats = ["Grad", "Jac", "Hess"] if self.hessian else ["Grad", "Jac"]     # moi.jl:26-28 (+ opt-in :Hess)
+        if self.products:                                                         # opt-in :JacVec / :HessVec
+            feats += ["JacVec", "HessVec"] if self.hessian else ["JacVec"]
+        return feats
 
     # ---- Lagrangian Hessian (MOI.hessian_lagrangian_structure / eval_hessian_lagrangian; not in the reference)
     def hessian_lagrangian_structure(self) -> List[Tuple[int, int]]:
@@ -338,6 +359,104 @@ class HybridNLP:
             self._h, B, C.c_void_p(Z.data_ptr()), Z.stride(0) if B > 1 else self.n_nlp,
             None if sigma is None else C.c_void_p(sigma.data_ptr()), C.c_void_p(mu.data_ptr()),
             mu.stride(0) if B > 1 else self.m_nlp, C.c_void_p(out.data_ptr()), ld(out, self.nnz_hess), C.c_void_p(s.cuda_stream)))
+        return out
+
+    # ---- matrix-free products (MOI :JacVec / :HessVec; not in the reference).  The summation order is fixed
+    # (include/qlnlp.h): each entry is the left fold of entry * vector over the structural non-zeros.
+    def eval_constraint_jacobian_product(self, y: np.ndarray, x, w) -> None:
+        """``y[m_nlp]`` <- J(x) w (MOI.eval_constraint_jacobian_product)."""
+        self._out(y, self.m_nlp, "y")
+        _check(load_library().qlnlp_eval_constraint_jacobian_product(
+            self._h, _np_ptr(self._x(x, self.n_nlp)), _np_ptr(self._x(w, self.n_nlp)), _np_ptr(y)))
+
+    def eval_constraint_jacobian_transpose_product(self, y: np.ndarray, x, w) -> None:
+        """``y[n_nlp]`` <- J(x)' w (MOI.eval_constraint_jacobian_transpose_product; ``w`` has m_nlp entries)."""
+        self._out(y, self.n_nlp, "y")
+        _check(load_library().qlnlp_eval_constraint_jacobian_transpose_product(
+            self._h, _np_ptr(self._x(x, self.n_nlp)), _np_ptr(self._x(w, self.m_nlp)), _np_ptr(y)))
+
+    def eval_hessian_lagrangian_product(self, h: np.ndarray, x, v, sigma: float, mu) -> None:
+        """``h[n_nlp]`` <- (sigma Hess f(x) + sum_r mu_r Hess g_r(x)) v (MOI.eval_hessian_lagrangian_product)."""
+        self._out(h, self.n_nlp, "h")
+        _check(load_library().qlnlp_eval_hessian_lagrangian_product(
+            self._h, _np_ptr(self._x(x, self.n_nlp)), _np_ptr(self._x(v, self.n_nlp)), float(sigma),
+            _np_ptr(self._x(mu, self.m_nlp)), _np_ptr(h)))
+
+    def eval_products_batch(self, Z, *, w=None, y=None, want: Sequence[str] = (), x0=None, xf=None,
+                            out: Optional[Dict[str, "object"]] = None, stream=None) -> Dict[str, "object"]:
+        """One fused launch over ``Z[B, n_nlp]``: ``jw = J w`` (``w[B, n_nlp]``) and / or ``jty = J' y`` (``y[B, m_nlp]``),
+        plus whichever of ``f``, ``grad``, ``g`` are in ``want`` (as ``eval_batch``).  Device tensors, rows padded to an
+        even length; enqueued on the current torch stream and not synchronised."""
+        import torch
+
+        if w is None and y is None:
+            raise ValueError("need w and / or y")
+        B = Z.shape[0]
+        for t, wd, name in ((Z, self.n_nlp, "Z"), (w, self.n_nlp, "w"), (y, self.m_nlp, "y")):
+            if t is not None and not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64
+                                      and t.dim() == 2 and t.shape == (B, wd) and t.stride(1) == 1):
+                raise ValueError(f"{name} must be a float64 CUDA tensor [B, {wd}] with unit inner stride")
+        if Z.device.index != self.device:
+            raise ValueError(f"Z lives on cuda:{Z.device.index}, the evaluator on cuda:{self.device}")
+        out = {} if out is None else out
+        dev = Z.device
+
+        def buf(name, width):
+            t = out.get(name)
+            if t is None:
+                t = torch.empty((B, even_ld(width)), dtype=torch.float64, device=dev)[:, :width]
+                out[name] = t
+            if not (t.is_cuda and t.dtype == torch.float64 and t.shape == (B, width) and t.stride(1) == 1):
+                raise ValueError(f"out[{name!r}] must be a float64 CUDA tensor of shape ({B}, {width})")
+            return t
+
+        ld = lambda t, width: t.stride(0) if B > 1 else width
+        io = _BatchIO()
+        io.Z, io.ldz = Z.data_ptr(), ld(Z, self.n_nlp)
+        for name, arr in (("x0", x0), ("xf", xf)):
+            if arr is not None:
+                if not (arr.is_cuda and arr.dtype == torch.float64 and arr.shape == (B, NX) and arr.is_contiguous()):
+                    raise ValueError(f"{name} must be a contiguous float64 CUDA tensor [B, 15]")
+                setattr(io, name, arr.data_ptr())
+        if "f" in want:
+            if out.get("f") is None:
+                out["f"] = torch.empty(B, dtype=torch.float64, device=dev)
+            io.f = out["f"].data_ptr()
+        if "grad" in want:
+            t = buf("grad", self.n_nlp)
+            io.grad, io.ldgrad = t.data_ptr(), ld(t, even_ld(self.n_nlp))
+        if "g" in want:
+            t = buf("g", self.m_nlp)
+            io.g, io.ldg = t.data_ptr(), ld(t, even_ld(self.m_nlp))
+        pv = _ProductIO()
+        if w is not None:
+            t = buf("jw", self.m_nlp)
+            pv.w, pv.ldw, pv.jw, pv.ldjw = w.data_ptr(), ld(w, self.n_nlp), t.data_ptr(), ld(t, even_ld(self.m_nlp))
+        if y is not None:
+            t = buf("jty", self.n_nlp)
+            pv.y, pv.ldy, pv.jty, pv.ldjty = y.data_ptr(), ld(y, self.m_nlp), t.data_ptr(), ld(t, even_ld(self.n_nlp))
+        s = torch.cuda.current_stream(dev) if stream is None else stream
+        _check(load_library().qlnlp_eval_jacobian_products_batch_device(self._h, B, C.byref(io), C.byref(pv),
+                                                                        C.c_void_p(s.cuda_stream)))
+        return out
+
+    def eval_hessian_product_batch(self, Z, mu, V, sigma=None, out=None, stream=None):
+        """Device tensors: ``Z[B, n_nlp]``, ``mu[B, m_nlp]``, ``V[B, n_nlp]``, optional ``sigma[B]`` (default 1) ->
+        ``HV[B, n_nlp]`` (rows padded to an even length)."""
+        import torch
+
+        B = Z.shape[0]
+        for t, wd, name in ((Z, self.n_nlp, "Z"), (mu, self.m_nlp, "mu"), (V, self.n_nlp, "V")):
+            if not (t.is_cuda and t.dtype == torch.float64 and t.dim() == 2 and t.shape == (B, wd) and t.stride(1) == 1):
+                raise ValueError(f"{name} must be a float64 CUDA tensor [B, {wd}]")
+        if out is None:
+            out = torch.empty((B, even_ld(self.n_nlp)), dtype=torch.float64, device=Z.device)[:, :self.n_nlp]
+        s = torch.cuda.current_stream(Z.device) if stream is None else stream
+        ld = lambda t, wd: t.stride(0) if B > 1 else wd
+        _check(load_library().qlnlp_eval_hessian_product_batch_device(
+            self._h, B, C.c_void_p(Z.data_ptr()), ld(Z, self.n_nlp), None if sigma is None else C.c_void_p(sigma.data_ptr()),
+            C.c_void_p(mu.data_ptr()), ld(mu, self.m_nlp), C.c_void_p(V.data_ptr()), ld(V, self.n_nlp),
+            C.c_void_p(out.data_ptr()), ld(out, even_ld(self.n_nlp)), C.c_void_p(s.cuda_stream)))
         return out
 
     def initialize(self, features: Iterable[str] = ()) -> None:

@@ -394,6 +394,83 @@ def rk4_offset(i, j):
     return 450 + 15 * (j - NX) + i
 
 
+def fold(terms):
+    """Left fold of the terms with QL_ADD, starting from the first term."""
+    expr = terms[0]
+    for t in terms[1:]:
+        expr = f"QL_ADD({expr}, {t})"
+    return expr
+
+
+def emit_products(w, mode, g, xn, pat, var, keep, union, hidx, obj):
+    """Matrix-free products of one mode (matrix times vector, no matrix in memory).  Every output entry is the left
+    fold of entry * vector terms over the structurally non-zero entries (the SPARSE_TRUE pattern / the Hessian's union
+    pattern), in ascending column order for J w and the Hessian, ascending row order for J' y.  Structural constants
+    are folded in: a +1 entry contributes the vector element itself, a -1 entry its negation (both exact)."""
+    w = w.append
+    vidx = {e: n for n, e in enumerate(var)}
+
+    def term(i, j, vec):
+        if (i, j) in vidx:
+            return f"QL_MUL(jv[{vidx[(i, j)]}], {vec})"
+        c = g.cval(xn[i].part(j))
+        if c == 1.0:
+            return vec
+        if c == -1.0:
+            return f"-{vec}"
+        return f"QL_MUL({c!r}, {vec})"
+
+    for jump in ((0, 1) if mode != 3 else (0,)):
+        pj = [(i, j) for (i, j) in pat if not (jump and not keep[i])]
+        fn = f"mode{mode}" + ("_jump" if jump else "")
+        w(f"// J w for the 15 defect rows of a knot in {fn}: the RK4 block (jv + constants) times w = [x_k; u_k] in")
+        w(f"// ascending column order, then the -I block times wn = x_(k+1) (a + (-b) is a - b bit for bit)")
+        w(f"QL_FN void ql_rk4_jvp_{fn}(const double* jv, const double* w, const double* wn, double* out)")
+        w("{")
+        for i in range(NX):
+            terms = [term(i, j, f"w[{j}]") for (ii, j) in sorted(pj, key=lambda e: e[1]) if ii == i]
+            w(f"    out[{i}] = {f'QL_SUB({fold(terms)}, wn[{i}])' if terms else f'-wn[{i}]'};")
+        w("}")
+        w("")
+        w(f"// J' y over the 20 columns of a knot's RK4 block in {fn}: y = the knot's 15 defect multipliers, rows in")
+        w(f"// ascending order.  State column j continues the fold a[j] of the rows above the block (init / term / -I).")
+        w(f"QL_FN void ql_rk4_vjp_{fn}(const double* jv, const double* y, const double* a, double* out)")
+        w("{")
+        for j in range(NP):
+            terms = [term(i, j, f"y[{i}]") for (i, jj) in pj if jj == j]
+            if j < NX:
+                terms = [f"a[{j}]"] + terms
+            assert terms, (fn, j)
+            w(f"    out[{j}] = {fold(terms)};")
+        w("}")
+        w("")
+    w(f"// Hessian block of a knot in mode {mode} times v (the knot's 20 variables): row i of the symmetric block in")
+    w(f"// ascending column order; each entry formed exactly as ql_hess_store_mode{mode} forms it")
+    w(f"QL_FN void ql_hess_prod_mode{mode}(const double* hv, const double* ox, const double* ou, const double* hx,")
+    w(f"                                  const double* hu, double hh, double tt, const double* v, double* out)")
+    w("{")
+    pos_of = {}
+    for pos, k in enumerate(union):
+        terms = []
+        if k in hidx:
+            terms.append(f"hv[{hidx[k]}]")
+        if k in obj:
+            terms.append(obj[k])
+        if k == (2, 2):
+            terms.append("tt")
+        w(f"    const double e{pos} = {fold(terms)};")
+        pos_of[k] = pos
+    for i in range(NP):
+        terms = []
+        for c in range(NP):
+            k = (i, c) if c <= i else (c, i)
+            if k in pos_of:
+                terms.append(f"QL_MUL(e{pos_of[k]}, v[{c}])")
+        w(f"    out[{i}] = {fold(terms)};")
+    w("}")
+    w("")
+
+
 def main():
     out = []
     w = out.append
@@ -413,6 +490,7 @@ def main():
     w("#pragma once")
     w("")
     summary = []
+    prod = []           # the product routines go after everything else: the routines above stay as they were
     for mode in (1, 2, 3):
         # primal only
         g, xn = build(mode, False)
@@ -587,6 +665,8 @@ def main():
         w("}")
         w("")
         summary.append((mode, "hess", cnt, len(hkeys), len(union)))
+        emit_products(prod, mode, g, xn, pat, var, keep, union, hidx, obj)
+    out.extend(prod)
     text = "\n".join(out) + "\n"
     with open(OUT, "w") as f:
         f.write(text)
