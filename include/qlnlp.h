@@ -219,6 +219,42 @@ int qlnlp_eval_constraint_jacobian_transpose_product(qlnlp_handle h, const doubl
 int qlnlp_eval_hessian_lagrangian_product(qlnlp_handle h, const double* x, const double* v, double sigma,
                                           const double* lambda, double* hv);
 
+/* ---- batched Newton step: the regularised KKT system of each problem (no reference counterpart; the reference hands
+ * it to Ipopt's sparse factorisation).  For every problem b of a SPARSE_TRUE handle, solve
+ *     [ W + diag(sx)   J'       ] [ px ]   [ r1 ]
+ *     [ J             -diag(dc) ] [ pl ] = [ r2 ]
+ *   W    hess[b]: the values qlnlp_eval_hessian_batch_device writes (lower triangle in qlnlp_hessian_structure
+ *        order), used mirrored;
+ *   J    jac[b]: SPARSE_TRUE values in qlnlp_jacobian_structure order, as qlnlp_eval_batch_device writes them on a
+ *        SPARSE_TRUE handle, used as given (quirks Q2 and Q4 included);
+ *   sx   [n_nlp] >= 0, the primal diagonal (barrier term + delta_w), or NULL: 0;
+ *   dc   [m_nlp] > 0 on EVERY row, the constraint diagonal (delta_c + slack terms; equality rows carry a
+ *        regularisation: the quasi-definite form).
+ * Method: M = W + diag(sx) + J' diag(dc)^-1 J is block tridiagonal with 20x20 blocks (15x15 at knot N); its Cholesky
+ * factor is formed knot by knot, then M px = r1 + J' (r2 ./ dc) and pl = (J px - r2) ./ dc.
+ * status[b]:  0  success;
+ *             k  (1-based knot) the diagonal block of knot k in the factorisation had a pivot <= 0 or not finite.
+ *                With dc > 0, M is positive definite exactly when the KKT matrix has inertia (n_nlp, m_nlp, 0)
+ *                (Haynsworth), so k > 0 is the "wrong inertia" signal: raise delta_w and solve again;
+ *            -1  a dc entry is <= 0 or not finite.
+ *   px[b] and pl[b] of a problem with status != 0 are written as NaN.
+ * One fixed operation order per problem: the bits do not depend on B, the batch position, leading dimensions,
+ * alignment or the stream.  DEVICE pointers, 8-byte aligned (status 4-byte); enqueued on `stream`, not
+ * synchronised.  Refused (QLNLP_EINVAL): SPARSE_BLOCK / DENSE handles, QLNLP_WITH_KINEMATICS handles, multi-device
+ * handles.  The factor scratch (1,840 B per knot per resident warp) is allocated at the first call on a stream. */
+typedef struct {
+    const double* hess; int64_t ldhess;   /* [B][ldhess >= nnz_hess] */
+    const double* jac;  int64_t ldjac;    /* [B][ldjac  >= nnz (SPARSE_TRUE)] */
+    const double* sx;   int64_t ldsx;     /* [B][ldsx   >= n_nlp]   or NULL */
+    const double* dc;   int64_t lddc;     /* [B][lddc   >= m_nlp] */
+    const double* r1;   int64_t ldr1;     /* [B][ldr1   >= n_nlp] */
+    const double* r2;   int64_t ldr2;     /* [B][ldr2   >= m_nlp] */
+    double* px;         int64_t ldpx;     /* [B][ldpx   >= n_nlp] */
+    double* pl;         int64_t ldpl;     /* [B][ldpl   >= m_nlp] */
+    int32_t* status;                      /* [B] */
+} qlnlp_kkt_io;
+int qlnlp_kkt_solve_batch_device(qlnlp_handle h, int64_t B, const qlnlp_kkt_io* io, void* stream);
+
 /* Ragged batches: problems of different size (several handles = several (N, k_trans, init_mode) classes) packed
  * back to back in flat arrays.  One call evaluates the B problems of THIS handle's class; the b-th of them is problem
  * number i = index[b] (or b when index is NULL) of the flat batch and its rows start at

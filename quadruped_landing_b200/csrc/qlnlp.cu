@@ -23,6 +23,7 @@
 #include "layout.h"
 #include "qlnlp_hess.cuh"
 #include "qlnlp_kin.cuh"
+#include "qlnlp_kkt.cuh"
 
 namespace {
 
@@ -150,6 +151,9 @@ struct DeviceState {
     int* d_kin_map = nullptr;          // caller-visible value order of the batch pattern -> scratch position or -(entry + 1)
     std::map<cudaStream_t, std::pair<double*, int64_t>> kin_scratch;   // per stream: reference-order rows (device), capacity
     std::map<std::vector<uint64_t>, RagTable> rag_tables;       // ragged launches led by this handle (key: the classes' serials)
+    unsigned short* d_kkt_tab = nullptr;   // KKT solve: slot / column of every SPARSE_TRUE value, then row / column of every W value
+    int kkt_blocks_per_sm = 0;
+    std::map<cudaStream_t, double*> kkt_scratch;                 // per stream: factor scratch of every resident warp
     int64_t last_launch[5] = {0, 0, 0, 0, 0};
     std::unique_ptr<qlhost::Pool> pool;                                  // row builders of the host-pointer path
     int64_t stat_host_rows = 0, stat_host_lines = 0;                     // rows / 64-byte lines the row builder wrote
@@ -984,6 +988,120 @@ int launch_hess_products(const Problem& p, DeviceState& ds, int64_t B, const dou
     return QLNLP_OK;
 }
 
+// ---- batched KKT solve (qlnlp_kkt.cuh) --------------------------------------------------------------------------
+// Argument checks: host logic only, before any device is touched.
+int check_kkt(const Problem& p, int64_t B, const qlnlp_kkt_io* io)
+{
+    const QlClass& c = p.cls;
+    if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
+    if (!io || !io->hess || !io->jac || !io->dc || !io->r1 || !io->r2 || !io->px || !io->pl || !io->status)
+        return fail(QLNLP_EINVAL, "io, hess, jac, dc, r1, r2, px, pl and status are required");
+    const int64_t n = c.n_nlp, m = c.m_nlp;
+    if (io->ldhess < ql_hess_nnz(c)) return fail(QLNLP_EINVAL, "ldhess %lld < nnz_hess %d", (long long)io->ldhess, ql_hess_nnz(c));
+    if (io->ldjac < c.nnz_true) return fail(QLNLP_EINVAL, "ldjac %lld < nnz %d", (long long)io->ldjac, c.nnz_true);
+    if (io->sx && io->ldsx < n) return fail(QLNLP_EINVAL, "ldsx %lld < n_nlp %lld", (long long)io->ldsx, (long long)n);
+    if (io->ldr1 < n || io->ldpx < n)
+        return fail(QLNLP_EINVAL, "ldr1 %lld / ldpx %lld < n_nlp %lld", (long long)io->ldr1, (long long)io->ldpx, (long long)n);
+    if (io->lddc < m || io->ldr2 < m || io->ldpl < m)
+        return fail(QLNLP_EINVAL, "lddc %lld / ldr2 %lld / ldpl %lld < m_nlp %lld", (long long)io->lddc, (long long)io->ldr2,
+                    (long long)io->ldpl, (long long)m);
+    for (const void* a : {(const void*)io->hess, (const void*)io->jac, (const void*)io->sx, (const void*)io->dc,
+                          (const void*)io->r1, (const void*)io->r2, (const void*)io->px, (const void*)io->pl})
+        if ((reinterpret_cast<uintptr_t>(a) & 7) != 0) return fail(QLNLP_EINVAL, "arrays must be 8-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(io->status) & 3) != 0) return fail(QLNLP_EINVAL, "status must be 4-byte aligned");
+    return QLNLP_OK;
+}
+
+// Per-value tables of the kernel, from the host structures: for every SPARSE_TRUE value its slot in the local Jacobian
+// of its knot (ql::kkt_slot_row) and its column inside the knot; then for every Hessian value its row and column inside
+// the knot (lower triangle).
+int ensure_kkt_tables(const Problem& p, DeviceState& ds)
+{
+    if (ds.d_kkt_tab) return QLNLP_OK;
+    const QlClass& c = p.cls;
+    const int nh = ql_hess_nnz(c);
+    std::vector<int64_t> rows(std::max(c.nnz_true, nh)), cols(rows.size());
+    std::vector<unsigned short> tab((size_t)c.nnz_true + nh);
+    sparse_true_structure(c, rows.data(), cols.data());
+    for (int e = 0; e < c.nnz_true; ++e) {
+        const int k = (int)((cols[e] - 1) / QL_NZK) + 1, j = (int)((cols[e] - 1) % QL_NZK);
+        int s = 0;
+        while (s < ql::KKT_SLOTS && ql::kkt_slot_row(c, k, s) != rows[e] - 1) ++s;
+        if (s == ql::KKT_SLOTS) return fail(QLNLP_ECUDA, "internal: Jacobian row %lld has no slot at knot %d", (long long)rows[e], k);
+        tab[e] = (unsigned short)(s | j << 8);
+    }
+    hessian_structure(c, rows.data(), cols.data());
+    for (int e = 0; e < nh; ++e) {
+        const int r = (int)((rows[e] - 1) % QL_NZK), q = (int)((cols[e] - 1) % QL_NZK);
+        tab[(size_t)c.nnz_true + e] = (unsigned short)(std::max(r, q) | std::min(r, q) << 8);
+    }
+    CUDA_TRY(cudaMalloc(&ds.d_kkt_tab, sizeof(unsigned short) * tab.size()));
+    CUDA_TRY(cudaMemcpy(ds.d_kkt_tab, tab.data(), sizeof(unsigned short) * tab.size(), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaDeviceSynchronize());
+    return QLNLP_OK;
+}
+
+int launch_kkt(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_kkt_io* io, cudaStream_t stream)
+{
+    const QlClass& c = p.cls;
+    const void* fn = (const void*)ql::kkt_kernel;
+    if (int rc = ensure_kkt_tables(p, ds)) return rc;
+    if (!ds.kkt_blocks_per_sm) {
+        int nb = 0;
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, QL_LANES, 0));
+        if (nb < 1) return fail(QLNLP_ECUDA, "KKT kernel does not fit on an SM");
+        ds.kkt_blocks_per_sm = nb;
+    }
+    const int64_t slots = (int64_t)ds.sm_count * ds.kkt_blocks_per_sm;
+    // the scratch holds one factor per resident warp (the most a launch of any B uses), allocated at the first call on
+    // a stream and never grown
+    double*& scratch = ds.kkt_scratch[stream];
+    if (!scratch) {
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        cudaStreamIsCapturing(stream, &cap);
+        if (cap != cudaStreamCaptureStatusNone) {
+            ds.kkt_scratch.erase(stream);
+            return fail(QLNLP_EINVAL, "KKT solve: the factor scratch of this stream would have to be allocated during a graph capture");
+        }
+        cudaError_t e = cudaMalloc(&scratch, sizeof(double) * (size_t)slots * c.N * ql::KKT_FSTRIDE);
+        if (e != cudaSuccess) {
+            ds.kkt_scratch.erase(stream);
+            return fail(e == cudaErrorMemoryAllocation ? QLNLP_ENOMEM : QLNLP_ECUDA, "KKT scratch: %s", cudaGetErrorString(e));
+        }
+    }
+    ql::KktLaunch P;
+    std::memset(&P, 0, sizeof P);
+    P.c = c;
+    P.jtab = ds.d_kkt_tab;
+    P.htab = ds.d_kkt_tab + c.nnz_true;
+    P.hess = io->hess; P.ldhess = io->ldhess;
+    P.jac = io->jac; P.ldjac = io->ldjac;
+    P.sx = io->sx; P.ldsx = io->ldsx;
+    P.dc = io->dc; P.lddc = io->lddc;
+    P.r1 = io->r1; P.ldr1 = io->ldr1;
+    P.r2 = io->r2; P.ldr2 = io->ldr2;
+    P.px = io->px; P.ldpx = io->ldpx;
+    P.pl = io->pl; P.ldpl = io->ldpl;
+    P.status = io->status;
+    P.scratch = scratch;
+    P.B = B;
+    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
+    const int grid = (int)std::min<int64_t>(B, slots);
+    void* args[] = {&P};
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(QL_LANES);
+    cfg.dynamicSmemBytes = 0;
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];         // programmatic dependent launch, as in launch()
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    CUDA_TRY(cudaLaunchKernelExC(&cfg, fn, args));
+    return QLNLP_OK;
+}
+
 // The three MOI product callbacks: copy in, one launch of B = 1, copy out, on the single-evaluation stream of the
 // handle's first device.  `in[0..nin)` go to device slots 1.., x to slot 0; the result comes back from the last slot.
 template <typename RUN>
@@ -1380,6 +1498,8 @@ void destroy_device_state(DeviceState& ds)
     cudaFree(ds.d_hess_in); cudaFree(ds.d_hess_out); cudaFree(ds.d_prod_one);
     cudaFree(ds.d_kin_map);
     for (auto& kv : ds.kin_scratch) cudaFree(kv.second.first);
+    cudaFree(ds.d_kkt_tab);
+    for (auto& kv : ds.kkt_scratch) cudaFree(kv.second);
     for (auto& kv : ds.rag_tables) cudaFree(kv.second.d_classes);
     cudaFree(ds.ticket_pool);
     cudaFree(ds.d_cost); cudaFree(ds.d_x0xf); cudaFree(ds.d_segs); cudaFree(ds.d_seg_begin);
@@ -1862,6 +1982,21 @@ int qlnlp_eval_hessian_product_batch_device(qlnlp_handle h, int64_t B, const dou
     if (int rc = ensure_device(h->prob, ds)) return rc;
     return launch_hess_products(h->prob, ds, B, Z, ldz, sigma, 1.0, lambda, ldlambda, V, ldv, HV, ldhv,
                                 static_cast<cudaStream_t>(stream));
+}
+
+/* ---- batched KKT solve (qlnlp_kkt.cuh) ---- */
+int qlnlp_kkt_solve_batch_device(qlnlp_handle h, int64_t B, const qlnlp_kkt_io* io, void* stream)
+{
+    if (int rc = check_handle(h)) return rc;
+    if (h->multi) return fail(QLNLP_EINVAL, "multi-device handle: the KKT solve takes a single-device handle");
+    if (h->prob.kin) return fail(QLNLP_EINVAL, "the KKT solve does not cover the kinematic rows");
+    if (h->prob.jac_mode != QLNLP_JAC_SPARSE_TRUE) return fail(QLNLP_EINVAL, "the KKT solve takes a SPARSE_TRUE handle");
+    if (B == 0) return QLNLP_OK;
+    if (int rc = check_kkt(h->prob, B, io)) return rc;
+    DeviceState& ds = h->devs[0];
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(h->prob, ds)) return rc;
+    return launch_kkt(h->prob, ds, B, io, static_cast<cudaStream_t>(stream));
 }
 
 // J w (transpose: J' y) at x for one evaluation: slot 1 holds the vector, slot 2 the result

@@ -42,6 +42,7 @@ EXPORTED_SYMBOLS = (
     "qlnlp_eval_jacobian_products_batch_device", "qlnlp_eval_hessian_product_batch_device",
     "qlnlp_eval_constraint_jacobian_product", "qlnlp_eval_constraint_jacobian_transpose_product",
     "qlnlp_eval_hessian_lagrangian_product",
+    "qlnlp_kkt_solve_batch_device",
 )
 _DEBUG_SYMBOLS = ("qlnlp_debug_segments", "qlnlp_debug_vals_map", "qlnlp_debug_build_rows", "qlnlp_debug_host_times",
                   "qlnlp_debug_launch_geometry")
@@ -75,6 +76,14 @@ class _BatchIO(C.Structure):
 class _ProductIO(C.Structure):
     _fields_ = [("w", C.c_void_p), ("ldw", C.c_int64), ("jw", C.c_void_p), ("ldjw", C.c_int64),
                 ("y", C.c_void_p), ("ldy", C.c_int64), ("jty", C.c_void_p), ("ldjty", C.c_int64)]
+
+
+class _KktIO(C.Structure):
+    _fields_ = [("hess", C.c_void_p), ("ldhess", C.c_int64), ("jac", C.c_void_p), ("ldjac", C.c_int64),
+                ("sx", C.c_void_p), ("ldsx", C.c_int64), ("dc", C.c_void_p), ("lddc", C.c_int64),
+                ("r1", C.c_void_p), ("ldr1", C.c_int64), ("r2", C.c_void_p), ("ldr2", C.c_int64),
+                ("px", C.c_void_p), ("ldpx", C.c_int64), ("pl", C.c_void_p), ("ldpl", C.c_int64),
+                ("status", C.c_void_p)]
 
 
 class _RaggedIO(C.Structure):
@@ -144,6 +153,7 @@ def load_library(rebuild_if_stale: bool = True):
     L.qlnlp_eval_constraint_jacobian_product.argtypes = [vp, vp, vp, vp]
     L.qlnlp_eval_constraint_jacobian_transpose_product.argtypes = [vp, vp, vp, vp]
     L.qlnlp_eval_hessian_lagrangian_product.argtypes = [vp, vp, vp, C.c_double, vp, vp]
+    L.qlnlp_kkt_solve_batch_device.argtypes = [vp, C.c_int64, C.POINTER(_KktIO), vp]
     L.qlnlp_host_alloc.argtypes = [C.c_int64, C.POINTER(vp)]
     L.qlnlp_host_free.argtypes = [vp, C.c_int64]
     for name in [n for n in EXPORTED_SYMBOLS if n not in ("qlnlp_version", "qlnlp_last_error")] + list(_DEBUG_SYMBOLS):
@@ -458,6 +468,48 @@ class HybridNLP:
             C.c_void_p(mu.data_ptr()), ld(mu, self.m_nlp), C.c_void_p(V.data_ptr()), ld(V, self.n_nlp),
             C.c_void_p(out.data_ptr()), ld(out, even_ld(self.n_nlp)), C.c_void_p(s.cuda_stream)))
         return out
+
+    # ---- batched Newton step (not in the reference): the regularised KKT system of each problem, include/qlnlp.h
+    def kkt_solve_batch(self, hess, jac, dc, r1, r2, sx=None, out=None, stream=None):
+        """Device tensors, one row per problem: ``hess[B, nnz_hess]`` (``eval_hessian_batch``), ``jac[B, nnz]``
+        (SPARSE_TRUE values, ``eval_batch``), ``dc[B, m_nlp] > 0``, ``r1[B, n_nlp]``, ``r2[B, m_nlp]``, optional
+        ``sx[B, n_nlp] >= 0`` (default 0) -> ``(px[B, n_nlp], pl[B, m_nlp], status[B] int32)``.  ``out`` may give the
+        three outputs.  Enqueued on the current torch stream (or ``stream``), not synchronised."""
+        import torch
+
+        B = hess.shape[0]
+        n, m = self.n_nlp, self.m_nlp
+        for t, wd, name in ((hess, self.nnz_hess, "hess"), (jac, self.nnz, "jac"), (dc, m, "dc"), (r1, n, "r1"),
+                            (r2, m, "r2"), (sx, n, "sx")):
+            if t is not None and not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64
+                                      and t.dim() == 2 and t.shape == (B, wd) and t.stride(1) == 1):
+                raise ValueError(f"{name} must be a float64 CUDA tensor [B, {wd}] with unit inner stride")
+        dev = hess.device
+        if out is None:
+            out = (torch.empty((B, even_ld(n)), dtype=torch.float64, device=dev)[:, :n],
+                   torch.empty((B, even_ld(m)), dtype=torch.float64, device=dev)[:, :m],
+                   torch.empty(B, dtype=torch.int32, device=dev))
+        px, pl, status = out
+        for t, wd, name in ((px, n, "px"), (pl, m, "pl")):
+            if not (t.is_cuda and t.dtype == torch.float64 and t.shape == (B, wd) and t.stride(1) == 1):
+                raise ValueError(f"out {name} must be a float64 CUDA tensor of shape ({B}, {wd})")
+        if not (status.is_cuda and status.dtype == torch.int32 and status.shape == (B,) and status.is_contiguous()):
+            raise ValueError(f"out status must be a contiguous int32 CUDA tensor of shape ({B},)")
+        ld = lambda t, wd: t.stride(0) if B > 1 else wd
+        io = _KktIO()
+        io.hess, io.ldhess = hess.data_ptr(), ld(hess, self.nnz_hess)
+        io.jac, io.ldjac = jac.data_ptr(), ld(jac, self.nnz)
+        if sx is not None:
+            io.sx, io.ldsx = sx.data_ptr(), ld(sx, n)
+        io.dc, io.lddc = dc.data_ptr(), ld(dc, m)
+        io.r1, io.ldr1 = r1.data_ptr(), ld(r1, n)
+        io.r2, io.ldr2 = r2.data_ptr(), ld(r2, m)
+        io.px, io.ldpx = px.data_ptr(), ld(px, n)
+        io.pl, io.ldpl = pl.data_ptr(), ld(pl, m)
+        io.status = status.data_ptr()
+        s = torch.cuda.current_stream(dev) if stream is None else stream
+        _check(load_library().qlnlp_kkt_solve_batch_device(self._h, B, C.byref(io), C.c_void_p(s.cuda_stream)))
+        return px, pl, status
 
     def initialize(self, features: Iterable[str] = ()) -> None:
         return None                                       # moi.jl:30
