@@ -107,7 +107,10 @@ int qlnlp_devices(qlnlp_handle h, int* devices, int cap, int* ndev);
 int qlnlp_shard_bounds(int64_t B, int nshards, int shard, int64_t* lo, int64_t* hi);
 /* tuning knobs: "host_chunk" (evaluations per pipeline stage of the host-pointer path, default 512), "host_threads"
  * (row-builder threads per device, 0 = this handle's share of the CPUs the process may use), "pin_threads" (0/1),
- * "x_cache" (0/1: serve repeated single-evaluation callbacks at the same x from the last evaluation) */
+ * "x_cache" (0/1: serve repeated single-evaluation callbacks at the same x from the last evaluation), "compressible"
+ * (0/1, default 1: qlnlp_device_alloc asks for compressible memory where the device offers it; 0 gives cudaMalloc
+ * memory, for outputs that must be exported with cudaIpcGetMemHandle or shared through torch.multiprocessing, which
+ * cuMemCreate memory does not support; the Python layer's outputs follow it too) */
 int qlnlp_set_option(qlnlp_handle h, const char* name, int64_t value);
 
 /* num_primals / num_duals                                          nlp.jl:86-87
@@ -311,6 +314,25 @@ int qlnlp_host_unpin(void* ptr);
  * Free with qlnlp_host_free(ptr, same byte count). */
 int qlnlp_host_alloc(int64_t bytes, void** out);
 int qlnlp_host_free(void* ptr, int64_t bytes);
+/* Device memory for the evaluator's outputs on the handle's device (for a multi-device handle: the calling thread's
+ * current device, which must be one of the handle's).  Where the device reports CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_
+ * SUPPORTED the block is compressible (cuMemCreate with CU_MEM_ALLOCATION_COMP_GENERIC, rounded up to the allocation
+ * granularity): the compression is lossless and invisible to kernels and copies, and it cuts the DRAM traffic of
+ * zero-rich rows such as the SPARSE_BLOCK Jacobian's.  Otherwise, when the driver declines a compressible block
+ * (compressible backing is limited), or after qlnlp_set_option(h, "compressible", 0), the block is plain cudaMalloc
+ * memory.  A compressible block is mapped read-write for its device and for every device that can access it peer to
+ * peer, as cudaMalloc memory is; it cannot be exported with cudaIpcGetMemHandle (so neither shared through
+ * torch.multiprocessing).  Blocks are at least 256-byte aligned.  Each call is a driver allocation: callers that
+ * allocate per evaluation should keep and reuse their blocks (the Python layer draws its outputs from a caching pool
+ * over these blocks).  Caller-owned buffers behave exactly as before; callers who want the gain allocate their
+ * outputs here.  Returns QLNLP_ENODEVICE without a device. */
+int qlnlp_device_alloc(qlnlp_handle h, int64_t bytes, void** out);
+/* Frees a qlnlp_device_alloc block (NULL is a no-op).  Needs no handle: a block may outlive the handle it was
+ * allocated through.  Waits for the block's device, as cudaFree does.  QLNLP_EINVAL for any other pointer. */
+int qlnlp_device_free(void* ptr);
+/* For a pointer inside a qlnlp_device_alloc block: [0] 1 if the block is compressible, [1] its device, [2] its length
+ * in bytes.  QLNLP_EINVAL for any other pointer. */
+int qlnlp_device_alloc_info(const void* ptr, int64_t info[3]);
 /* host path facts: [0] row-builder threads per device, [1] Jacobian doubles per evaluation that cross PCIe,
  * [2] doubles per row, [3] 64-byte lines rewritten per registered row, [4] lines per row, [5] AVX-512 writer in use,
  * [6] rows assembled so far, [7] lines written so far */

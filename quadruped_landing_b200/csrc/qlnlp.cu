@@ -3,10 +3,13 @@
 // no CPU fallback: every evaluation entry point runs the CUDA kernels or fails.
 #include "../../include/qlnlp.h"
 
+#include <cuda.h>
+#include <cudaTypedefs.h>
 #include <cuda_runtime.h>
 #include <sys/mman.h>
 
 #include <algorithm>
+#include <atomic>
 #include <chrono>
 #include <cmath>
 #include <cstdarg>
@@ -176,6 +179,7 @@ struct qlnlp_handle_s {
     int64_t opt_host_threads = 0;      // 0: each device's share of the process's CPUs
     int64_t opt_pin_threads = 1;
     int64_t opt_x_cache = 1;
+    int64_t opt_compressible = 1;      // qlnlp_device_alloc: ask for compressible memory where the device has it
 };
 
 namespace {
@@ -1564,6 +1568,136 @@ int check_desc(const qlnlp_problem_desc* d, int jac_mode_flags)
     return QLNLP_OK;
 }
 
+// ---------------------------------------------------------------------------- device output allocator
+// The driver's virtual-memory calls, reached through the runtime so that the library does not link libcuda.
+struct DriverVmm {
+    bool ok = false;
+    PFN_cuDeviceGetAttribute_v2000 attr = nullptr;
+    PFN_cuMemGetAllocationGranularity_v10020 granularity = nullptr;
+    PFN_cuMemCreate_v10020 create = nullptr;
+    PFN_cuMemGetAllocationPropertiesFromHandle_v10020 props = nullptr;
+    PFN_cuMemRelease_v10020 release = nullptr;
+    PFN_cuMemAddressReserve_v10020 reserve = nullptr;
+    PFN_cuMemAddressFree_v10020 addr_free = nullptr;
+    PFN_cuMemMap_v10020 map = nullptr;
+    PFN_cuMemUnmap_v10020 unmap = nullptr;
+    PFN_cuMemSetAccess_v10020 access = nullptr;
+};
+
+const DriverVmm& driver_vmm()
+{
+    static const DriverVmm d = [] {
+        DriverVmm v;
+        auto get = [](const char* sym, int ver, auto& fn) {
+            void* p = nullptr;
+            cudaDriverEntryPointQueryResult q;
+            if (cudaGetDriverEntryPointByVersion(sym, &p, ver, cudaEnableDefault, &q) != cudaSuccess ||
+                q != cudaDriverEntryPointSuccess)
+                p = nullptr;
+            fn = reinterpret_cast<std::remove_reference_t<decltype(fn)>>(p);
+            return p != nullptr;
+        };
+        v.ok = get("cuDeviceGetAttribute", 2000, v.attr) & get("cuMemGetAllocationGranularity", 10020, v.granularity) &
+               get("cuMemCreate", 10020, v.create) & get("cuMemGetAllocationPropertiesFromHandle", 10020, v.props) &
+               get("cuMemRelease", 10020, v.release) & get("cuMemAddressReserve", 10020, v.reserve) &
+               get("cuMemAddressFree", 10020, v.addr_free) & get("cuMemMap", 10020, v.map) &
+               get("cuMemUnmap", 10020, v.unmap) & get("cuMemSetAccess", 10020, v.access);
+        cudaGetLastError();
+        return v;
+    }();
+    return d;
+}
+
+// One qlnlp_device_alloc block.  The table is process-wide, so a block can be freed after its handle is destroyed.
+struct DeviceBlock {
+    int device;
+    size_t bytes;                       // mapped length (rounded to the granularity) or the cudaMalloc request
+    bool vmm;                           // cuMemCreate + cuMemMap; otherwise cudaMalloc
+    bool compressible;
+    CUmemGenericAllocationHandle mem;
+};
+std::mutex g_blocks_mu;
+std::map<uintptr_t, DeviceBlock> g_blocks;
+std::atomic<int> g_refuse_compressible{0};   // tests: the next n compressible requests are refused as the driver would
+
+// cuMemCreate with generic compression on `device`, mapped read-write for that device.  Returns false (and leaves
+// nothing behind) whenever the driver declines: compressible backing is a limited resource, so a refusal is normal.
+bool compressible_alloc(int device, size_t bytes, void** out, DeviceBlock& blk)
+{
+    const DriverVmm& d = driver_vmm();
+    if (!d.ok) return false;
+    if (g_refuse_compressible.load() > 0 && g_refuse_compressible.fetch_sub(1) > 0) return false;
+    int vmm = 0, comp = 0;
+    if (d.attr(&vmm, CU_DEVICE_ATTRIBUTE_VIRTUAL_MEMORY_MANAGEMENT_SUPPORTED, device) != CUDA_SUCCESS || !vmm) return false;
+    if (d.attr(&comp, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, device) != CUDA_SUCCESS || !comp) return false;
+    CUmemAllocationProp prop = {};
+    prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    prop.location.id = device;
+    prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+    size_t gran = 0;
+    if (d.granularity(&gran, &prop, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED) != CUDA_SUCCESS || gran == 0) return false;
+    const size_t len = (bytes + gran - 1) / gran * gran;
+    CUmemGenericAllocationHandle mem = 0;
+    if (d.create(&mem, len, &prop, 0) != CUDA_SUCCESS) return false;
+    CUmemAllocationProp got = {};
+    CUdeviceptr va = 0;
+    bool mapped = false;
+    bool ok = d.props(&got, mem) == CUDA_SUCCESS && got.allocFlags.compressionType == CU_MEM_ALLOCATION_COMP_GENERIC &&
+              d.reserve(&va, len, gran, 0, 0) == CUDA_SUCCESS;
+    if (ok) ok = mapped = d.map(va, len, 0, mem, 0) == CUDA_SUCCESS;
+    if (ok) {
+        // read-write for the owning device and, as cudaMalloc memory would be, for every device that can reach it
+        // peer to peer; if the driver refuses the peers, the owner alone
+        std::vector<CUmemAccessDesc> acc(1);
+        acc[0].location = prop.location;
+        acc[0].flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+        int ndev = 0;
+        if (cudaGetDeviceCount(&ndev) != cudaSuccess) ndev = 0;
+        for (int peer = 0; peer < ndev; ++peer) {
+            int can = 0;
+            if (peer != device && cudaDeviceCanAccessPeer(&can, peer, device) == cudaSuccess && can) {
+                CUmemAccessDesc a = acc[0];
+                a.location.id = peer;
+                acc.push_back(a);
+            }
+        }
+        cudaGetLastError();
+        ok = d.access(va, len, acc.data(), acc.size()) == CUDA_SUCCESS ||
+             (acc.size() > 1 && d.access(va, len, acc.data(), 1) == CUDA_SUCCESS);
+    }
+    if (!ok) {
+        if (mapped) d.unmap(va, len);
+        if (va) d.addr_free(va, len);
+        d.release(mem);
+        return false;
+    }
+    blk = DeviceBlock{device, len, true, true, mem};
+    *out = reinterpret_cast<void*>(va);
+    return true;
+}
+
+// A block on `device`: compressible where offered and asked for, otherwise cudaMalloc.  Recorded in the block table.
+int device_block_alloc(int device, size_t bytes, bool compressible, void** out)
+{
+    DeviceGuard guard(device);
+    void* p = nullptr;
+    DeviceBlock blk{device, bytes, false, false, 0};
+    if (!(compressible && compressible_alloc(device, bytes, &p, blk))) {
+        blk = DeviceBlock{device, bytes, false, false, 0};
+        const cudaError_t e = cudaMalloc(&p, bytes);
+        if (e != cudaSuccess) {
+            cudaGetLastError();        // an out-of-memory must not linger as the thread's last error
+            return fail(e == cudaErrorMemoryAllocation ? QLNLP_ENOMEM : QLNLP_ECUDA, "cudaMalloc of %zu bytes: %s", bytes,
+                        cudaGetErrorString(e));
+        }
+    }
+    std::lock_guard<std::mutex> lk(g_blocks_mu);
+    g_blocks[reinterpret_cast<uintptr_t>(p)] = blk;
+    *out = p;
+    return QLNLP_OK;
+}
+
 }  // namespace
 
 // =============================================================================== C ABI
@@ -1699,6 +1833,7 @@ int qlnlp_set_option(qlnlp_handle h, const char* name, int64_t value)
     else if (n == "host_threads") { if (value < 0) return fail(QLNLP_EINVAL, "host_threads must be >= 0"); h->opt_host_threads = value; }
     else if (n == "pin_threads") h->opt_pin_threads = value != 0;
     else if (n == "x_cache") { h->opt_x_cache = value != 0; h->devs[0].one.valid = false; }
+    else if (n == "compressible") h->opt_compressible = value != 0;
     else return fail(QLNLP_EINVAL, "unknown option '%s'", name);
     if (n == "host_threads" || n == "pin_threads")          // the pools take both when they are made
         for (DeviceState& ds : h->devs) ds.pool.reset();
@@ -1891,6 +2026,84 @@ int qlnlp_host_free(void* ptr, int64_t bytes)
     const size_t len = ((size_t)bytes + huge - 1) / huge * huge;
     if (cudaHostUnregister(ptr) != cudaSuccess) cudaGetLastError();
     munmap(ptr, len);
+    return QLNLP_OK;
+}
+
+int qlnlp_device_alloc(qlnlp_handle h, int64_t bytes, void** out)
+{
+    if (int rc = check_handle(h)) return rc;
+    if (!out || bytes <= 0) return fail(QLNLP_EINVAL, "bad allocation request");
+    *out = nullptr;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        cudaGetLastError();
+        return fail(QLNLP_ENODEVICE, "no CUDA device available");
+    }
+    int device = h->devs[0].device;
+    if (h->multi) {                    // the caller's current device, which must be one of the handle's
+        if (cudaGetDevice(&device) != cudaSuccess) return fail(QLNLP_ECUDA, "cudaGetDevice failed");
+        if (std::none_of(h->devs.begin(), h->devs.end(), [&](const DeviceState& ds) { return ds.device == device; }))
+            return fail(QLNLP_EINVAL, "current device %d is not one of the handle's devices", device);
+    }
+    if (device < 0 || device >= ndev) return fail(QLNLP_EINVAL, "device %d out of range (0..%d)", device, ndev - 1);
+    return device_block_alloc(device, (size_t)bytes, h->opt_compressible != 0, out);
+}
+
+int qlnlp_device_free(void* ptr)
+{
+    if (!ptr) return QLNLP_OK;
+    DeviceBlock blk;
+    {
+        std::lock_guard<std::mutex> lk(g_blocks_mu);
+        auto it = g_blocks.find(reinterpret_cast<uintptr_t>(ptr));
+        if (it == g_blocks.end()) return fail(QLNLP_EINVAL, "%p was not returned by qlnlp_device_alloc", ptr);
+        blk = it->second;
+        g_blocks.erase(it);
+    }
+    DeviceGuard guard(blk.device);
+    if (!blk.vmm) {
+        CUDA_TRY(cudaFree(ptr));
+        return QLNLP_OK;
+    }
+    // cudaFree waits for the device's work; unmapping does not, so wait here as cudaFree would
+    CUDA_TRY(cudaDeviceSynchronize());
+    const DriverVmm& d = driver_vmm();
+    const CUdeviceptr va = reinterpret_cast<CUdeviceptr>(ptr);
+    if (d.unmap(va, blk.bytes) != CUDA_SUCCESS || d.addr_free(va, blk.bytes) != CUDA_SUCCESS || d.release(blk.mem) != CUDA_SUCCESS)
+        return fail(QLNLP_ECUDA, "releasing the mapping of %p failed", ptr);
+    return QLNLP_OK;
+}
+
+/* torch.cuda.CUDAPluggableAllocator entry points (evaluator.py): segments of the caching pool the Python layer draws
+ * its outputs from, so that outputs are reused in stream order instead of being allocated and freed per call.  Not part
+ * of the C ABI.  The pool frees a segment only when it releases its cache, with no work pending on it. */
+void* qlnlp_pool_alloc(ssize_t bytes, int device, void* /*stream*/)
+{
+    void* p = nullptr;
+    return (bytes > 0 && device_block_alloc(device, (size_t)bytes, true, &p) == QLNLP_OK) ? p : nullptr;
+}
+
+void qlnlp_pool_free(void* ptr, size_t /*bytes*/, int /*device*/, void* /*stream*/) { qlnlp_device_free(ptr); }
+
+/* tests: the next n compressible requests are refused as the driver refuses them when compressible backing runs out */
+int qlnlp_debug_refuse_compressible(int n)
+{
+    g_refuse_compressible.store(n < 0 ? 0 : n);
+    return QLNLP_OK;
+}
+
+int qlnlp_device_alloc_info(const void* ptr, int64_t info[3])
+{
+    if (!ptr || !info) return fail(QLNLP_EINVAL, "null argument");
+    std::lock_guard<std::mutex> lk(g_blocks_mu);
+    const uintptr_t a = reinterpret_cast<uintptr_t>(ptr);
+    auto it = g_blocks.upper_bound(a);
+    if (it == g_blocks.begin() || a >= std::prev(it)->first + std::prev(it)->second.bytes)
+        return fail(QLNLP_EINVAL, "%p is not inside a qlnlp_device_alloc block", ptr);
+    --it;
+    info[0] = it->second.compressible ? 1 : 0;
+    info[1] = it->second.device;
+    info[2] = (int64_t)it->second.bytes;
     return QLNLP_OK;
 }
 

@@ -43,9 +43,10 @@ EXPORTED_SYMBOLS = (
     "qlnlp_eval_constraint_jacobian_product", "qlnlp_eval_constraint_jacobian_transpose_product",
     "qlnlp_eval_hessian_lagrangian_product",
     "qlnlp_kkt_solve_batch_device",
+    "qlnlp_device_alloc", "qlnlp_device_free", "qlnlp_device_alloc_info",
 )
 _DEBUG_SYMBOLS = ("qlnlp_debug_segments", "qlnlp_debug_vals_map", "qlnlp_debug_build_rows", "qlnlp_debug_host_times",
-                  "qlnlp_debug_launch_geometry")
+                  "qlnlp_debug_launch_geometry", "qlnlp_debug_refuse_compressible")
 
 
 class QlnlpError(RuntimeError):
@@ -92,6 +93,7 @@ class _RaggedIO(C.Structure):
 
 
 _lib = None
+_lib_path = None
 
 
 def load_library(rebuild_if_stale: bool = True):
@@ -108,6 +110,8 @@ def load_library(rebuild_if_stale: bool = True):
         raise RuntimeError(f"{path} is missing: build it with `python -m quadruped_landing_b200.build` "
                            "(the evaluator has no CPU fallback)")
     L = C.CDLL(path)
+    global _lib_path
+    _lib_path = path
     vp, i64p = C.c_void_p, C.POINTER(C.c_int64)
     L.qlnlp_version.restype = C.c_int
     L.qlnlp_last_error.restype = C.c_char_p
@@ -156,6 +160,10 @@ def load_library(rebuild_if_stale: bool = True):
     L.qlnlp_kkt_solve_batch_device.argtypes = [vp, C.c_int64, C.POINTER(_KktIO), vp]
     L.qlnlp_host_alloc.argtypes = [C.c_int64, C.POINTER(vp)]
     L.qlnlp_host_free.argtypes = [vp, C.c_int64]
+    L.qlnlp_device_alloc.argtypes = [vp, C.c_int64, C.POINTER(vp)]
+    L.qlnlp_device_free.argtypes = [vp]
+    L.qlnlp_device_alloc_info.argtypes = [vp, i64p]
+    L.qlnlp_debug_refuse_compressible.argtypes = [C.c_int]
     for name in [n for n in EXPORTED_SYMBOLS if n not in ("qlnlp_version", "qlnlp_last_error")] + list(_DEBUG_SYMBOLS):
         getattr(L, name).restype = C.c_int
     _lib = L
@@ -211,6 +219,50 @@ def _np_ptr(a: Optional[np.ndarray]):
 def even_ld(n: int) -> int:
     """Leading dimension that keeps every row 16-byte aligned (what the TMA store path needs)."""
     return (n + 1) & ~1
+
+
+_pools = {}                                           # device -> torch.cuda.MemPool over qlnlp_pool_alloc / _free
+
+
+def _output_pool(device: int):
+    """The caching pool the library's outputs come from on ``cuda:device``: torch's caching allocator over segments
+    from ``qlnlp_pool_alloc`` (compressible where the device offers it).  Freed outputs return to the pool in stream
+    order and are reused; nothing is synchronised and no driver allocation happens once the pool holds the sizes a caller
+    uses.  The pools live for the process, so outputs outlive the handles that produced them."""
+    import torch
+
+    pool = _pools.get(device)
+    if pool is None:
+        load_library()
+        alloc = torch.cuda.memory.CUDAPluggableAllocator(_lib_path, "qlnlp_pool_alloc", "qlnlp_pool_free")
+        with torch.cuda.device(device):
+            pool = _pools[device] = (torch.cuda.MemPool(alloc.allocator()), alloc)
+    return pool[0]
+
+
+def device_alloc_info(t) -> Dict[str, int]:
+    """What ``qlnlp_device_alloc_info`` reports about the block holding tensor ``t`` (raises for other memory)."""
+    info = (C.c_int64 * 3)()
+    _check(load_library().qlnlp_device_alloc_info(C.c_void_p(t.data_ptr()), info))
+    return dict(zip(("compressible", "device", "bytes"), list(info)))
+
+
+def _device_empty(device: int, specs, compressible: bool = True) -> list:
+    """Output tensors on ``cuda:device``.  ``specs``: ``(rows, width, dtype)``; ``width=None`` gives a 1-D tensor of
+    ``rows`` entries, otherwise ``[rows, width]`` with rows padded to ``even_ld(width)`` (16-byte aligned rows).  They
+    come from the compressible output pool unless ``compressible`` is false or the current stream is being captured
+    into a CUDA graph (a capture keeps its allocations in its own pool, as torch.empty does)."""
+    import torch
+
+    def empty(rows, width, dtype):
+        t = torch.empty(rows if width is None else (rows, even_ld(width)), dtype=dtype, device=torch.device("cuda", device))
+        return t if width is None else t[:, :width]
+
+    with torch.cuda.device(device):
+        if not compressible or torch.cuda.is_current_stream_capturing():
+            return [empty(*s) for s in specs]
+        with torch.cuda.use_mem_pool(_output_pool(device), device):
+            return [empty(*s) for s in specs]
 
 
 class HybridNLP:
@@ -284,6 +336,7 @@ class HybridNLP:
             arr = (C.c_int * len(self.devices))(*self.devices)
             _check(L.qlnlp_create_multi(C.byref(d), arr, len(self.devices), flags, C.byref(self._h)))
         self._registered = {}
+        self._compressible = True
         self.hessian = False
         self.products = False
         nh = C.c_int64()
@@ -362,7 +415,7 @@ class HybridNLP:
             if not (t.is_cuda and t.dtype == torch.float64 and t.dim() == 2 and t.shape == (B, w) and t.stride(1) == 1):
                 raise ValueError(f"{name} must be a float64 CUDA tensor [B, {w}]")
         if out is None:
-            out = torch.empty((B, even_ld(self.nnz_hess)), dtype=torch.float64, device=Z.device)[:, :self.nnz_hess]
+            out, = _device_empty(Z.device.index, [(B, self.nnz_hess, torch.float64)], self._compressible)
         s = torch.cuda.current_stream(Z.device) if stream is None else stream
         ld = lambda t, w: t.stride(0) if B > 1 else even_ld(w)
         _check(load_library().qlnlp_eval_hessian_batch_device(
@@ -410,12 +463,13 @@ class HybridNLP:
             raise ValueError(f"Z lives on cuda:{Z.device.index}, the evaluator on cuda:{self.device}")
         out = {} if out is None else out
         dev = Z.device
+        missing = [k for k in ("f", "grad", "g") if k in want and out.get(k) is None]
+        missing += [k for k, v in (("jw", w), ("jty", y)) if v is not None and out.get(k) is None]
+        if missing:                                     # the library's output pool, compressible where offered
+            out.update(self.alloc_outputs(B, missing))
 
         def buf(name, width):
-            t = out.get(name)
-            if t is None:
-                t = torch.empty((B, even_ld(width)), dtype=torch.float64, device=dev)[:, :width]
-                out[name] = t
+            t = out[name]
             if not (t.is_cuda and t.dtype == torch.float64 and t.shape == (B, width) and t.stride(1) == 1):
                 raise ValueError(f"out[{name!r}] must be a float64 CUDA tensor of shape ({B}, {width})")
             return t
@@ -429,8 +483,6 @@ class HybridNLP:
                     raise ValueError(f"{name} must be a contiguous float64 CUDA tensor [B, 15]")
                 setattr(io, name, arr.data_ptr())
         if "f" in want:
-            if out.get("f") is None:
-                out["f"] = torch.empty(B, dtype=torch.float64, device=dev)
             io.f = out["f"].data_ptr()
         if "grad" in want:
             t = buf("grad", self.n_nlp)
@@ -460,7 +512,7 @@ class HybridNLP:
             if not (t.is_cuda and t.dtype == torch.float64 and t.dim() == 2 and t.shape == (B, wd) and t.stride(1) == 1):
                 raise ValueError(f"{name} must be a float64 CUDA tensor [B, {wd}]")
         if out is None:
-            out = torch.empty((B, even_ld(self.n_nlp)), dtype=torch.float64, device=Z.device)[:, :self.n_nlp]
+            out, = _device_empty(Z.device.index, [(B, self.n_nlp, torch.float64)], self._compressible)
         s = torch.cuda.current_stream(Z.device) if stream is None else stream
         ld = lambda t, wd: t.stride(0) if B > 1 else wd
         _check(load_library().qlnlp_eval_hessian_product_batch_device(
@@ -486,9 +538,8 @@ class HybridNLP:
                 raise ValueError(f"{name} must be a float64 CUDA tensor [B, {wd}] with unit inner stride")
         dev = hess.device
         if out is None:
-            out = (torch.empty((B, even_ld(n)), dtype=torch.float64, device=dev)[:, :n],
-                   torch.empty((B, even_ld(m)), dtype=torch.float64, device=dev)[:, :m],
-                   torch.empty(B, dtype=torch.int32, device=dev))
+            out = tuple(_device_empty(dev.index, [(B, n, torch.float64), (B, m, torch.float64), (B, None, torch.int32)],
+                                     self._compressible))
         px, pl, status = out
         for t, wd, name in ((px, n, "px"), (pl, m, "pl")):
             if not (t.is_cuda and t.dtype == torch.float64 and t.shape == (B, wd) and t.stride(1) == 1):
@@ -581,6 +632,8 @@ class HybridNLP:
 
     def set_option(self, name: str, value: int) -> None:
         _check(load_library().qlnlp_set_option(self._h, name.encode(), int(value)))
+        if name == "compressible":                      # the outputs this object allocates follow the handle's option
+            self._compressible = bool(value)
 
     # ---- host-pointer path helpers
     def register_host_output(self, jac: np.ndarray) -> None:
@@ -603,6 +656,26 @@ class HybridNLP:
                          "lines_per_row", "avx512", "rows_built", "lines_written"), list(info)))
 
     # ---- batched evaluation
+    def alloc_outputs(self, B: int, want: Sequence[str] = ("f", "grad", "g", "jac"), device: Optional[int] = None
+                      ) -> Dict[str, "object"]:
+        """The output arrays ``eval_batch`` (and ``eval_products_batch``: ``jw``, ``jty``) would allocate for a batch of
+        ``B`` on ``cuda:device`` (default: the evaluator's device, which is the only one a single-device evaluator
+        accepts), from the library's caching output pool: compressible where the device offers it, which cuts the DRAM
+        traffic of the zero-rich Jacobian rows.  Rows are padded to an even length (16-byte aligned).  Pass the dict as
+        ``out=`` to reuse it."""
+        import torch
+
+        widths = {"f": None, "grad": self.n_nlp, "g": self.m_nlp, "jac": self.nnz_batch, "jw": self.m_nlp,
+                  "jty": self.n_nlp}
+        names = [k for k in widths if k in want]
+        if any(k not in widths for k in want):
+            raise ValueError(f"want may name {sorted(widths)}, got {list(want)}")
+        dev = self.device if device is None else int(device)
+        if dev not in self.devices:
+            raise ValueError(f"device {dev} is not one of the evaluator's devices {self.devices}")
+        ts = _device_empty(dev, [(int(B), widths[k], torch.float64) for k in names], self._compressible)
+        return dict(zip(names, ts))
+
     def eval_batch(self, Z, *, x0=None, xf=None, want: Sequence[str] = ("f", "grad", "g", "jac"),
                    out: Optional[Dict[str, "object"]] = None, stream=None) -> Dict[str, "object"]:
         """Evaluate ``B`` decision vectors held in a CUDA tensor ``Z[B, ldz>=n_nlp]`` (fp64, row-major).
@@ -622,12 +695,12 @@ class HybridNLP:
         B = Z.shape[0]
         out = {} if out is None else out
         dev = Z.device
+        missing = [k for k in ("f", "grad", "g", "jac") if k in want and out.get(k) is None]
+        if missing:                                     # the library's output pool, compressible where offered
+            out.update(self.alloc_outputs(B, missing))
 
         def buf(name, width):
-            t = out.get(name)
-            if t is None:
-                t = torch.empty((B, even_ld(width)), dtype=torch.float64, device=dev)[:, :width]
-                out[name] = t
+            t = out[name]
             if not (t.is_cuda and t.dtype == torch.float64 and t.shape == (B, width) and t.stride(1) == 1):
                 raise ValueError(f"out[{name!r}] must be a float64 CUDA tensor of shape ({B}, {width})")
             return t
@@ -640,8 +713,6 @@ class HybridNLP:
                     raise ValueError(f"{name} must be a contiguous float64 CUDA tensor [B, 15]")
                 setattr(io, name, arr.data_ptr())
         if "f" in want:
-            if out.get("f") is None:
-                out["f"] = torch.empty(B, dtype=torch.float64, device=dev)
             io.f = out["f"].data_ptr()
         if "grad" in want:
             t = buf("grad", self.n_nlp)
@@ -680,17 +751,15 @@ class HybridNLP:
             io = ios[i]
             io.Z, io.ldz = Z.data_ptr(), Z.stride(0) if B > 1 else self.n_nlp
             widths = {"grad": self.n_nlp, "g": self.m_nlp, "jac": self.nnz_batch}
+            missing = [k for k in ("f", "grad", "g", "jac") if k in want and out.get(k) is None]
+            if missing:
+                out.update(self.alloc_outputs(B, missing, device=Z.device.index))
             if "f" in want:
-                if out.get("f") is None:
-                    out["f"] = torch.empty(B, dtype=torch.float64, device=Z.device)
                 io.f = out["f"].data_ptr()
             for name, w in widths.items():
                 if name not in want:
                     continue
-                t = out.get(name)
-                if t is None:
-                    t = torch.empty((B, even_ld(w)), dtype=torch.float64, device=Z.device)[:, :w]
-                    out[name] = t
+                t = out[name]
                 setattr(io, name, t.data_ptr())
                 setattr(io, "ld" + name, t.stride(0) if B > 1 else even_ld(w))
             streams[i] = torch.cuda.current_stream(Z.device).cuda_stream
@@ -716,7 +785,7 @@ class HybridNLP:
             base = torch.from_numpy(initial_guess(self.prob, dt)).to(x0.device)
             self._registered[key] = base
         if out is None:
-            out = torch.empty((B, even_ld(self.n_nlp)), dtype=torch.float64, device=x0.device)[:, :self.n_nlp]
+            out, = _device_empty(x0.device.index, [(B, self.n_nlp, torch.float64)], self._compressible)
         s = torch.cuda.current_stream(x0.device) if stream is None else stream
         _check(load_library().qlnlp_initial_guess_batch_device(self._h, B, C.c_void_p(base.data_ptr()), C.c_void_p(x0.data_ptr()),
                                                                C.c_void_p(out.data_ptr()), out.stride(0) if B > 1 else even_ld(self.n_nlp),

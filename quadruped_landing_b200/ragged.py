@@ -12,7 +12,7 @@ from typing import Dict, List, Sequence
 
 import numpy as np
 
-from .evaluator import HybridNLP
+from .evaluator import HybridNLP, _device_empty
 from .problem import ProblemData
 
 
@@ -88,12 +88,17 @@ class RaggedEvaluator:
         off = plan.off
         flat = {"Z": Z_flat}
         sizes = {"f": B, "grad": int(off["z_off"][-1]), "g": int(off["g_off"][-1]), "jac": int(off["j_off"][-1])}
+        missing = []
         for name in ("f", "grad", "g", "jac"):
             if name in want:
                 t = None if out is None else out.get(name)
                 if t is None or t.numel() != sizes[name] or t.device != dev:
-                    t = torch.empty(sizes[name], dtype=torch.float64, device=dev)
-                flat[name] = t
+                    missing.append(name)
+                else:
+                    flat[name] = t
+        if missing:                        # the library's output pool, compressible where the device offers it
+            ts = _device_empty(dev.index, [(sizes[k], None, torch.float64) for k in missing], self.nlps[0]._compressible)
+            flat.update(zip(missing, ts))
         HybridNLP.eval_ragged_classes(self.nlps, plan.order, plan.dclass, flat, plan.doff, z_padded=True)
         res = {k: v for k, v in flat.items() if k != "Z"}
         res.update(off)
