@@ -11,15 +11,18 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <climits>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <initializer_list>
 #include <map>
 #include <memory>
 #include <mutex>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "hostrows.h"
@@ -80,9 +83,16 @@ struct HostLane {
     double* stage = nullptr;    // pinned host rows of VALS values awaiting the row builder
 };
 
+// device memory that only grows (per-stream scratch, single-call slots)
+struct Scratch {
+    double* ptr = nullptr;
+    size_t cap = 0;             // doubles
+};
+
 // single evaluations (the four MOI callbacks): one launch per decision vector, results cached
 struct OneEval {
     cudaStream_t stream = nullptr;
+    Scratch slots;              // device rows of the other single calls (single_call)
     double* hx = nullptr;       // pinned, mapped: x(ldz_e) | f(2) grad(ldgrad_e) g(ldg_e) vals(ldv_e)
     double* hout = nullptr;
     double* mx = nullptr;       // device-side addresses of hx / hout: the kernel reads x and writes the results there
@@ -96,14 +106,12 @@ struct Registration {
     int64_t ld, rows;
 };
 
-// class table of a ragged launch (device copy of one QlRagClass per handle) + the launch geometry for its largest horizon
+// class table of a ragged launch (device copy of one QlRagClass per handle)
 struct RagTable {
     ql::QlRagClass* d_classes = nullptr;
     int ncls = 0;
     QlClass layout;                    // the class with the largest N: sizes the shared-memory carve-up
     bool fastdiv = false;
-    size_t smem[NJM] = {0, 0, 0, 0};
-    int blocks_per_sm[NJM] = {0, 0, 0, 0};
 };
 
 // The problem a handle evaluates: built once when the handle is created, host memory only, read-only afterwards.
@@ -131,8 +139,7 @@ struct DeviceState {
     std::string pci_bus_id;
     int sm_count = 0;
     size_t smem_per_sm = 0, smem_optin = 0;
-    int blocks_per_sm[NJM] = {0, 0, 0, 0};
-    size_t smem[NJM] = {0, 0, 0, 0};
+    std::map<std::pair<const void*, size_t>, int> blocks_per_sm;   // (kernel, dynamic smem) -> resident CTAs (kernel_geometry)
     double* d_cost = nullptr;
     double* d_x0xf = nullptr;          // x0[15] | xf[15]
     QlSeg* d_segs = nullptr;
@@ -144,19 +151,11 @@ struct DeviceState {
     std::map<cudaStream_t, unsigned*> tickets;   // work counters, one pair per stream the device has launched on
     unsigned* ticket_pool = nullptr;             // pre-zeroed counters (128 B apart) so that a launch needs no
     int ticket_pool_used = 0;                    // allocation: launches stay legal inside CUDA-graph capture
-    // Lagrangian Hessian (single evaluations on host pointers): device scratch x | lambda | values
-    double* d_hess_in = nullptr;
-    double* d_hess_out = nullptr;
-    int hess_blocks_per_sm = 0;
-    int prod_blocks_per_sm = 0;        // matrix-free products: resident CTAs of eval_prod_kernel / hess_prod_kernel
-    int hprod_blocks_per_sm = 0;
-    double* d_prod_one = nullptr;      // scratch of the three product callbacks: 5 rows
     int* d_kin_map = nullptr;          // caller-visible value order of the batch pattern -> scratch position or -(entry + 1)
-    std::map<cudaStream_t, std::pair<double*, int64_t>> kin_scratch;   // per stream: reference-order rows (device), capacity
+    std::map<cudaStream_t, Scratch> kin_scratch;                 // per stream: reference-order rows (device)
     std::map<std::vector<uint64_t>, RagTable> rag_tables;       // ragged launches led by this handle (key: the classes' serials)
     unsigned short* d_kkt_tab = nullptr;   // KKT solve: slot / column of every SPARSE_TRUE value, then row / column of every W value
-    int kkt_blocks_per_sm = 0;
-    std::map<cudaStream_t, double*> kkt_scratch;                 // per stream: factor scratch of every resident warp
+    std::map<cudaStream_t, Scratch> kkt_scratch;                 // per stream: factor scratch of every resident warp
     int64_t last_launch[5] = {0, 0, 0, 0, 0};
     std::unique_ptr<qlhost::Pool> pool;                                  // row builders of the host-pointer path
     int64_t stat_host_rows = 0, stat_host_lines = 0;                     // rows / 64-byte lines the row builder wrote
@@ -265,21 +264,54 @@ bool fastdiv_is_exact(double b)
     return true;
 }
 
-template <int JM>
-const void* kernel_fn_jm(bool fast, bool ragged)
+// ---- what the launcher knows about a kernel ----------------------------------------------------------------------
+// The launch policies, each measured on the B200.  One CTA is one warp.
+struct KernelSpec {
+    const void* fn;
+    size_t smem;        // dynamic shared memory per CTA at the problem's N
+    int warp_cap;       // most resident CTAs per SM (0: as many as fit)
+    bool carveout;      // the library sets the kernel's carve-out to what its resident CTAs need (else: driver default)
+    bool pad;           // launched with padded shared memory, so that one CTA more than asked for never fits
+    bool pdl;           // programmatic dependent launch
+};
+
+// eval_kernel<JM, FASTDIV, RAGGED>; RAGGED: rows addressed through offset tables (qlnlp_eval_ragged_device) instead of
+// leading dimensions.  JM_VALS serves the host-pointer path only and is never ragged.
+#define QL_EVAL_FNS(JM) {{(const void*)ql::eval_kernel<JM, false, false>, (const void*)ql::eval_kernel<JM, false, true>}, \
+                         {(const void*)ql::eval_kernel<JM, true, false>, (const void*)ql::eval_kernel<JM, true, true>}}
+const void* const EVAL_FN[NJM][2][2] = {
+    QL_EVAL_FNS(ql::JM_NONE), QL_EVAL_FNS(ql::JM_BLOCK), QL_EVAL_FNS(ql::JM_TRUE),
+    {{(const void*)ql::eval_kernel<ql::JM_VALS, false, false>, nullptr}, {(const void*)ql::eval_kernel<ql::JM_VALS, true, false>, nullptr}},
+};
+#undef QL_EVAL_FNS
+
+KernelSpec eval_spec(int N, int jm, bool fast, bool ragged)
 {
-    if (fast) return ragged ? (const void*)ql::eval_kernel<JM, true, true> : (const void*)ql::eval_kernel<JM, true, false>;
-    return ragged ? (const void*)ql::eval_kernel<JM, false, true> : (const void*)ql::eval_kernel<JM, false, false>;
+    // The SPARSE_BLOCK stream is store-bound and the memory system takes the output of a few fast warps better than
+    // that of all 8 that fit (occupancy sweeps in profiles/r01_ablation.md, section 7): at most 6 CTAs per SM (launch()
+    // narrows that to 5 or 6), with padded shared memory.  The other value streams run as many warps as the kernel was
+    // compiled for (its __launch_bounds__).
+    const bool block = jm == ql::JM_BLOCK;
+    const int cap = block ? 6 : jm == ql::JM_NONE ? QL_NONE_WARPS : QL_TRUE_WARPS;
+    return {EVAL_FN[jm][fast][ragged], ql::smem_bytes(N, jm), cap, true, block, true};
 }
-// ragged: rows addressed through offset tables (qlnlp_eval_ragged_device) instead of leading dimensions
-const void* kernel_fn(int jm, bool fast, bool ragged)
+
+KernelSpec prod_spec(const Problem& p)
 {
-    if (jm == ql::JM_BLOCK) return kernel_fn_jm<ql::JM_BLOCK>(fast, ragged);
-    if (jm == ql::JM_TRUE) return kernel_fn_jm<ql::JM_TRUE>(fast, ragged);
-    if (jm == ql::JM_VALS)      // host-pointer path only: never ragged
-        return fast ? (const void*)ql::eval_kernel<ql::JM_VALS, true, false> : (const void*)ql::eval_kernel<ql::JM_VALS, false, false>;
-    return kernel_fn_jm<ql::JM_NONE>(fast, ragged);
+    const void* fn = p.fastdiv ? (const void*)ql::eval_prod_kernel<true> : (const void*)ql::eval_prod_kernel<false>;
+    return {fn, ql::smem_bytes(p.cls.N, ql::JM_PROD), QL_TRUE_WARPS, true, false, true};
 }
+
+// the Hessian kernels have not been measured with programmatic dependent launch
+KernelSpec hess_spec(const Problem& p, bool prod)
+{
+    const void* fn = prod ? (p.fastdiv ? (const void*)ql::hess_prod_kernel<true> : (const void*)ql::hess_prod_kernel<false>)
+                          : (p.fastdiv ? (const void*)ql::hess_kernel<true> : (const void*)ql::hess_kernel<false>);
+    return {fn, ql::hess_smem_bytes(p.cls.N), 0, true, false, false};
+}
+
+// static shared memory only; its carve-out has not been measured, so the driver's default stays
+KernelSpec kkt_spec() { return {(const void*)ql::kkt_kernel, 0, 0, false, false, true}; }
 
 // the sparse pattern batched evaluations of this problem produce (DENSE handles batch in SPARSE_BLOCK)
 int batch_jm(const Problem& p) { return p.jac_mode == QLNLP_JAC_SPARSE_TRUE ? ql::JM_TRUE : ql::JM_BLOCK; }
@@ -287,7 +319,6 @@ int std_nnz(const Problem& p) { return p.jac_mode == QLNLP_JAC_SPARSE_TRUE ? p.c
 // what the caller sees: the kinematic rows add 8 entries per knot to either pattern and 2 rows per knot to g
 int batch_nnz(const Problem& p) { return std_nnz(p) + (p.kin ? 8 * p.cls.N : 0); }
 int m_rows(const Problem& p) { return p.cls.m_nlp + (p.kin ? 2 * p.cls.N : 0); }
-int jm_nnz(const QlClass& c, int jm) { return jm == ql::JM_TRUE ? c.nnz_true : jm == ql::JM_VALS ? c.nnz_vals : c.nnz; }
 
 // SPARSE_TRUE structure (1-based, value order): like sparse_block_structure restricted to structural non-zeros
 void sparse_true_structure(const QlClass& c, int64_t* rows, int64_t* cols)
@@ -484,28 +515,34 @@ int set_carveout(const void* fn, int resident_blocks, size_t smem_per_block, siz
     return QLNLP_OK;
 }
 
-// Launch geometry of the eval kernel `fn` (value stream `wj`) at `smem` bytes of dynamic shared memory per CTA on the
-// device `ds`: the resident CTAs per SM, and the L1 carve-out they leave.
-int kernel_geometry(const DeviceState& ds, const void* fn, int wj, size_t smem, int* blocks_per_sm)
+// Launch geometry of kernel `k` on the device `ds`: the resident CTAs per SM, and the L1 carve-out they leave.  Cached
+// per device on the first call.
+int kernel_geometry(DeviceState& ds, const KernelSpec& k, int* blocks_per_sm)
 {
-    // the attributes are per FUNCTION, shared by every handle of the process: always raise the limit to the device's,
-    // never to this handle's own (possibly smaller) requirement
-    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ds.smem_optin));
-    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    const auto key = std::make_pair(k.fn, k.smem);
+    auto it = ds.blocks_per_sm.find(key);
+    if (it != ds.blocks_per_sm.end()) { *blocks_per_sm = it->second; return QLNLP_OK; }
+    if (k.smem > ds.smem_optin) return fail(QLNLP_EINVAL, "the kernel needs %zu B of shared memory per warp (> %zu)", k.smem, ds.smem_optin);
+    if (k.carveout) {
+        // the attributes are per FUNCTION, shared by every handle of the process: always raise the limit to the
+        // device's, never to this handle's own (possibly smaller) requirement
+        CUDA_TRY(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ds.smem_optin));
+        CUDA_TRY(cudaFuncSetAttribute(k.fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    }
     int nb = 0;
-    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, QL_LANES, smem));
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k.fn, QL_LANES, k.smem));
     if (nb < 1) return fail(QLNLP_ECUDA, "kernel does not fit on an SM");
-    // never more resident warps than the kernel was compiled for (its __launch_bounds__)
-    if (wj == ql::JM_NONE) nb = std::min(nb, QL_NONE_WARPS);
-    else if (wj != ql::JM_BLOCK) nb = std::min(nb, QL_TRUE_WARPS);
+    if (k.warp_cap) nb = std::min(nb, k.warp_cap);
+    if (k.carveout) {
+        // Shared memory the resident warps really need: whatever the SM has beyond that serves as L1 (the cost table
+        // and the boundary states are re-read by every warp).  The attribute belongs to the FUNCTION, so it only ever
+        // grows (handles of other horizons share it).
+        const size_t per_block = k.pad ? padded_smem(ds.smem_per_sm, ds.smem_optin, nb, k.smem) : k.smem;
+        if (int rc = set_carveout(k.fn, nb, per_block, ds.smem_per_sm)) return rc;
+    }
+    ds.blocks_per_sm.emplace(key, nb);
     *blocks_per_sm = nb;
-    // Shared memory the resident warps really need: whatever the SM has beyond that serves as L1 (the cost table and
-    // the boundary states are re-read by every warp).  The attribute belongs to the FUNCTION, so it only ever grows
-    // (handles of other horizons share it).  launch() runs the SPARSE_BLOCK kernel on at most 6 CTAs per SM, each with
-    // its shared memory padded.
-    const int res = (wj == ql::JM_BLOCK) ? std::min(nb, 6) : nb;
-    const size_t per_block = (wj == ql::JM_BLOCK) ? padded_smem(ds.smem_per_sm, ds.smem_optin, res, smem) : smem;
-    return set_carveout(fn, res, per_block, ds.smem_per_sm);
+    return QLNLP_OK;
 }
 
 int check_handle(qlnlp_handle h)
@@ -546,17 +583,12 @@ int ensure_device(const Problem& p, DeviceState& ds)
     CUDA_TRY(cudaMalloc(&ds.d_seg_begin, p.seg_begin.size() * sizeof(int)));
     CUDA_TRY(cudaMemcpy(ds.d_seg_begin, p.seg_begin.data(), p.seg_begin.size() * sizeof(int), cudaMemcpyHostToDevice));
 
-    for (int wj = 0; wj < NJM; ++wj) {
-        ds.smem[wj] = ql::smem_bytes(p.cls.N, wj);
-        if (ds.smem[wj] > ds.smem_optin)
-            return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp (> %zu)", p.cls.N, ds.smem[wj], ds.smem_optin);
-        for (int rg = 0; rg < 2; ++rg) {
-            if (rg && wj == ql::JM_VALS) continue;
+    // the eval kernels' attributes are set here, at the first evaluation, whatever the handle launches later
+    for (int wj = 0; wj < NJM; ++wj)
+        for (int rg = 0; rg < (wj == ql::JM_VALS ? 1 : 2); ++rg) {
             int nb = 0;
-            if (int rc = kernel_geometry(ds, kernel_fn(wj, p.fastdiv, rg != 0), wj, ds.smem[wj], &nb)) return rc;
-            ds.blocks_per_sm[wj] = rg ? std::min(ds.blocks_per_sm[wj], nb) : nb;
+            if (int rc = kernel_geometry(ds, eval_spec(p.cls.N, wj, p.fastdiv, rg != 0), &nb)) return rc;
         }
-    }
     for (auto& ln : ds.lanes) {
         CUDA_TRY(cudaStreamCreateWithFlags(&ln.stream, cudaStreamNonBlocking));
         CUDA_TRY(cudaEventCreateWithFlags(&ln.done, cudaEventDisableTiming));
@@ -599,13 +631,100 @@ int stream_ticket(DeviceState& ds, cudaStream_t stream, unsigned** out)
     return QLNLP_OK;
 }
 
-int launch(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* io, cudaStream_t stream, int jm_force = -1,
-           const qlnlp_ragged_io* rg = nullptr, const RagTable* table = nullptr, const int32_t* class_of = nullptr)
+// The one launch of every kernel that hands out work with a ticket: B evaluations of record `P` on `stream`, on at most
+// `cap` resident CTAs per SM.  `info`: the launch_info record to fill (eval launches).
+template <typename R>
+int launch_kernel(DeviceState& ds, const KernelSpec& k, int64_t B, R& P, cudaStream_t stream, int cap = INT_MAX,
+                  int64_t* info = nullptr)
+{
+    int per_sm = 0;
+    if (int rc = kernel_geometry(ds, k, &per_sm)) return rc;
+    per_sm = std::min(per_sm, cap);
+    const int grid = (int)std::min<int64_t>(B, (int64_t)ds.sm_count * per_sm);
+    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
+    // With programmatic dependent launch the next grid's CTAs are placed as soon as an SM has room for one.  The
+    // SPARSE_BLOCK kernel runs on fewer CTAs per SM than would fit (5 or 6 of up to 7 by shared memory): a spare slot
+    // would take a CTA of the next grid while this grid is still running at full strength, and the next grid would
+    // start out unevenly spread over the SMs (measured: -5 % on the headline once another handle had raised the
+    // kernel's carve-out to 228 KB).  Ask for enough shared memory per CTA that per_sm + 1 of them never fit.
+    // (Only that kernel: the others are capped by their registers, and padding them would cost L1.)
+    const size_t smem = k.pad ? padded_smem(ds.smem_per_sm, ds.smem_optin, per_sm, k.smem) : k.smem;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(QL_LANES);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    // programmatic dependent launch: back-to-back launches on a stream overlap the next grid's start-up with this
+    // grid's drain (B = 4,096: +1 % full evaluation, +4..6 % for the compact-output kernels; the kernels wait for their
+    // predecessors before they touch any data, see griddepcontrol.wait in eval_kernel)
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = k.pdl ? 1 : 0;
+    void* args[] = {&P};
+    CUDA_TRY(cudaLaunchKernelExC(&cfg, k.fn, args));
+    if (info) {
+        info[0] = grid;
+        info[1] = QL_LANES;
+        info[2] = (int64_t)smem;
+        info[3] = per_sm;
+        info[4] = ds.sm_count;
+    }
+    return QLNLP_OK;
+}
+
+// The problem fields the launch records share
+template <typename R>
+void set_problem(R& P, const Problem& p, const DeviceState& ds)
+{
+    P.c = p.cls;
+    P.rmb = p.rmb; P.rmf = p.rmf; P.rIb = p.rIb;
+    P.cost = ds.d_cost;
+    P.npad = p.npad;
+    if constexpr (std::is_base_of<ql::Launch, R>::value) {
+        P.x0_def = ds.d_x0xf;
+        P.xf_def = ds.d_x0xf + QL_NX;
+    }
+}
+
+// Device scratch of at least n doubles for work on `stream`, grown only.  It cannot grow while the stream is being
+// captured into a graph: the call fails with `msg`.
+int grow_scratch(Scratch& sc, cudaStream_t stream, size_t n, const char* msg, double** out)
+{
+    if (sc.cap < n) {
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        cudaStreamIsCapturing(stream, &cap);
+        if (cap != cudaStreamCaptureStatusNone) return fail(QLNLP_EINVAL, "%s", msg);
+        if (sc.ptr) {
+            CUDA_TRY(cudaDeviceSynchronize());      // earlier launches may still use it
+            cudaFree(sc.ptr);
+            sc = Scratch();
+        }
+        CUDA_TRY(cudaMalloc(&sc.ptr, sizeof(double) * n));
+        sc.cap = n;
+    }
+    *out = sc.ptr;
+    return QLNLP_OK;
+}
+
+// End of a call that reads or writes caller-owned host memory: wait for `stream` whatever happened (copies may still be
+// in flight), and report the first error.
+int finish(cudaStream_t stream, int rc, const char* what)
+{
+    const std::string msg = g_err;
+    const cudaError_t e = cudaStreamSynchronize(stream);
+    if (rc == QLNLP_OK && e != cudaSuccess) return fail(QLNLP_ECUDA, "%s: %s", what, cudaGetErrorString(e));
+    g_err = msg;
+    return rc;
+}
+
+// Argument checks of a batch on device pointers (rg: a ragged batch) or, with `host`, on host pointers: host logic
+// only, before any device is touched.  The kernels read Z themselves; on host pointers the row builder writes jac.
+int check_batch(const Problem& p, int64_t B, const qlnlp_batch_io* io, const qlnlp_ragged_io* rg, bool host = false)
 {
     const QlClass& c = p.cls;
-    if (rg && !table) return fail(QLNLP_EINVAL, "internal: ragged launch without a class table");
     if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
-    if (B == 0) return QLNLP_OK;          // an empty shard is not an error (its pointers may be NULL)
     if (!io || !io->Z) return fail(QLNLP_EINVAL, "io->Z is required");
     if (rg) {
         if (!rg->z_off || (io->g && !rg->g_off) || (io->jac && !rg->jac_off))
@@ -613,23 +732,25 @@ int launch(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* i
     } else {
         if (io->ldz < c.n_nlp) return fail(QLNLP_EINVAL, "ldz %lld < n_nlp %d", (long long)io->ldz, c.n_nlp);
         if (io->grad && io->ldgrad < c.n_nlp) return fail(QLNLP_EINVAL, "ldgrad %lld < n_nlp %d", (long long)io->ldgrad, c.n_nlp);
-        if (io->g && io->ldg < c.m_nlp) return fail(QLNLP_EINVAL, "ldg %lld < m_nlp %d", (long long)io->ldg, c.m_nlp);
+        if (io->g && io->ldg < m_rows(p)) return fail(QLNLP_EINVAL, "ldg %lld < m_nlp %d", (long long)io->ldg, m_rows(p));
+        if (io->jac && io->ldjac < batch_nnz(p)) return fail(QLNLP_EINVAL, "ldjac %lld < nnz %d", (long long)io->ldjac, batch_nnz(p));
     }
-    const int jm_jac = jm_force >= 0 ? jm_force : batch_jm(p);
-    const int nnz_jac = jm_nnz(c, jm_jac);
-    if (!rg && io->jac && io->ldjac < nnz_jac) return fail(QLNLP_EINVAL, "ldjac %lld < nnz %d", (long long)io->ldjac, nnz_jac);
-    if ((reinterpret_cast<uintptr_t>(io->Z) & 7) != 0) return fail(QLNLP_EINVAL, "Z must be 8-byte aligned");
+    if (!host && (reinterpret_cast<uintptr_t>(io->Z) & 7) != 0) return fail(QLNLP_EINVAL, "Z must be 8-byte aligned");
+    if (host && io->jac && (reinterpret_cast<uintptr_t>(io->jac) & 7) != 0) return fail(QLNLP_EINVAL, "jac must be 8-byte aligned");
+    return QLNLP_OK;
+}
 
+// One launch of the evaluator over arguments that have passed check_batch (B > 0).  jm_force: the value stream to
+// write instead of the batch pattern's (JM_VALS for the host-pointer paths).
+int launch(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* io, cudaStream_t stream, int jm_force = -1,
+           const qlnlp_ragged_io* rg = nullptr, const RagTable* table = nullptr, const int32_t* class_of = nullptr)
+{
     ql::Launch P;
-    P.c = rg ? table->layout : c;
+    set_problem(P, p, ds);
+    if (rg) P.c = table->layout;
     P.classes = rg ? table->d_classes : nullptr;
     P.cls_of = rg ? reinterpret_cast<const int*>(class_of) : nullptr;
-    P.rmb = p.rmb; P.rmf = p.rmf; P.rIb = p.rIb;
-    P.cost = ds.d_cost;
-    P.npad = p.npad;
     P.nseg = (int)p.segs.size();
-    P.x0_def = ds.d_x0xf;
-    P.xf_def = ds.d_x0xf + QL_NX;
     P.segs = ds.d_segs;
     P.seg_begin = ds.d_seg_begin;
     P.Z = io->Z; P.ldz = io->ldz;
@@ -647,48 +768,14 @@ int launch(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* i
     if (rg) P.zbulk = ((reinterpret_cast<uintptr_t>(io->Z) & 15) == 0 && (rg->flags & QLNLP_RAGGED_Z_PADDED)) ? 1 : 0;
     else P.zbulk = ((reinterpret_cast<uintptr_t>(io->Z) & 15) == 0 && (io->ldz & 1) == 0) ? 1 : 0;   // ldz even > n_nlp (odd)
 
-    const int wj = io->jac ? jm_jac : ql::JM_NONE;
-    // Resident warps per SM.  The SPARSE_BLOCK stream is store-bound and the memory system takes the output of a
-    // few fast warps better than that of all 8 that fit (occupancy sweeps in profiles/r01_ablation.md, section 7):
-    // 5 per SM, 6 for short batches that also want the cost/gradient.
-    int per_sm = rg ? table->blocks_per_sm[wj] : ds.blocks_per_sm[wj];
-    const size_t smem = rg ? table->smem[wj] : ds.smem[wj];
-    const bool fast = rg ? table->fastdiv : p.fastdiv;
-    if (wj == ql::JM_BLOCK) {
-        const bool want_cost = io->f || io->grad;
-        const bool short_batch = B < 8 * (int64_t)ds.sm_count * 6;
-        per_sm = std::min(per_sm, (want_cost && short_batch) ? 6 : 5);
-    }
-    const int grid = (int)std::min<int64_t>(B, (int64_t)ds.sm_count * per_sm);
-    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
-    // With programmatic dependent launch the next grid's CTAs are placed as soon as an SM has room for one.  The
-    // SPARSE_BLOCK kernel runs on fewer CTAs per SM than would fit (5 or 6 of up to 7 by shared memory): a spare slot
-    // would take a CTA of the next grid while this grid is still running at full strength, and the next grid would
-    // start out unevenly spread over the SMs (measured: -5 % on the headline once another handle had raised the
-    // kernel's carve-out to 228 KB).  Ask for enough shared memory per CTA that per_sm + 1 of them never fit.
-    // (Only that kernel: the others are capped by their registers, and padding them would cost L1.)
-    const size_t smem_launch = (wj == ql::JM_BLOCK) ? padded_smem(ds.smem_per_sm, ds.smem_optin, per_sm, smem) : smem;
-    void* args[] = {&P};
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(QL_LANES);
-    cfg.dynamicSmemBytes = smem_launch;
-    cfg.stream = stream;
-    // programmatic dependent launch: back-to-back evaluations on a stream overlap the next grid's start-up with this
-    // grid's drain (B = 4,096: +1 % full evaluation, +4..6 % for the compact-output kernels; the kernel waits for its
-    // predecessors before it touches any data, see griddepcontrol.wait in eval_kernel)
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    CUDA_TRY(cudaLaunchKernelExC(&cfg, kernel_fn(wj, fast, rg != nullptr), args));
-    ds.last_launch[0] = grid;
-    ds.last_launch[1] = QL_LANES;
-    ds.last_launch[2] = (int64_t)smem_launch;
-    ds.last_launch[3] = per_sm;
-    ds.last_launch[4] = ds.sm_count;
-    return QLNLP_OK;
+    const int wj = io->jac ? (jm_force >= 0 ? jm_force : batch_jm(p)) : ql::JM_NONE;
+    int cap = INT_MAX;
+    if (!rg && wj != ql::JM_VALS)      // a plain launch runs on no more CTAs per SM than the ragged instantiation
+        if (int rc = kernel_geometry(ds, eval_spec(p.cls.N, wj, p.fastdiv, true), &cap)) return rc;
+    // SPARSE_BLOCK: 5 CTAs per SM, 6 for short batches that also want the cost/gradient (see eval_spec)
+    if (wj == ql::JM_BLOCK) cap = std::min(cap, (io->f || io->grad) && B < 8 * (int64_t)ds.sm_count * 6 ? 6 : 5);
+    const KernelSpec k = rg ? eval_spec(table->layout.N, wj, table->fastdiv, true) : eval_spec(p.cls.N, wj, p.fastdiv, false);
+    return launch_kernel(ds, k, B, P, stream, cap, ds.last_launch);
 }
 
 // The class table of a ragged launch over the single-device handles `hs` (all on one device, already bound to it),
@@ -730,12 +817,6 @@ int ragged_table(const qlnlp_handle* hs, int ncls, const RagTable** out)
     CUDA_TRY(cudaMemcpy(d, packed.data(), packed.size(), cudaMemcpyHostToDevice));
     CUDA_TRY(cudaDeviceSynchronize());
     t.d_classes = static_cast<ql::QlRagClass*>(d);
-    for (int wj = 0; wj < NJM; ++wj) {
-        if (wj == ql::JM_VALS) continue;
-        t.smem[wj] = ql::smem_bytes(t.layout.N, wj);
-        if (t.smem[wj] > lead.smem_optin) return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp", t.layout.N, t.smem[wj]);
-        if (int rc = kernel_geometry(lead, kernel_fn(wj, t.fastdiv, true), wj, t.smem[wj], &t.blocks_per_sm[wj])) return rc;
-    }
     *out = &lead.rag_tables.emplace(key, t).first->second;
     return QLNLP_OK;
 }
@@ -781,24 +862,13 @@ int ensure_kin(const Problem& p, DeviceState& ds)
 int launch_kin(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* io, cudaStream_t stream)
 {
     const QlClass& c = p.cls;
-    if (B == 0) return QLNLP_OK;
-    if (!io || !io->Z) return fail(QLNLP_EINVAL, "io->Z is required");
-    if (io->g && io->ldg < m_rows(p)) return fail(QLNLP_EINVAL, "ldg %lld < m_nlp %d", (long long)io->ldg, m_rows(p));
-    if (io->jac && io->ldjac < batch_nnz(p)) return fail(QLNLP_EINVAL, "ldjac %lld < nnz %d", (long long)io->ldjac, batch_nnz(p));
     if (int rc = ensure_kin(p, ds)) return rc;
     qlnlp_batch_io d = *io;
     const int64_t lds = (std_nnz(p) + 1) & ~1;
     if (io->jac) {
-        auto& sc = ds.kin_scratch[stream];
-        if (sc.second < B * lds) {
-            cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-            cudaStreamIsCapturing(stream, &cap);
-            if (cap != cudaStreamCaptureStatusNone) return fail(QLNLP_EINVAL, "kinematic rows: the scratch would have to grow during a graph capture");
-            if (sc.first) { CUDA_TRY(cudaDeviceSynchronize()); cudaFree(sc.first); sc.first = nullptr; sc.second = 0; }
-            CUDA_TRY(cudaMalloc(&sc.first, sizeof(double) * (size_t)(B * lds)));
-            sc.second = B * lds;
-        }
-        d.jac = sc.first;
+        if (int rc = grow_scratch(ds.kin_scratch[stream], stream, (size_t)(B * lds),
+                                  "kinematic rows: the scratch would have to grow during a graph capture", &d.jac))
+            return rc;
         d.ldjac = lds;
     }
     if (int rc = launch(p, ds, B, &d, stream)) return rc;
@@ -836,63 +906,56 @@ void hessian_structure(const QlClass& c, int64_t* rows, int64_t* cols)
     }
 }
 
-int launch_hessian(const Problem& p, DeviceState& ds, int64_t B, const double* Z, int64_t ldz, const double* sigma,
-                   double sigma0, const double* lam, int64_t ldlam, double* H, int64_t ldh, cudaStream_t stream)
+// Argument checks of the Hessian entry points: Z, the multipliers and one output row of `width` values per evaluation.
+// Host logic only, before any device is touched.
+int check_hessian(const Problem& p, int64_t B, const double* Z, int64_t ldz, const double* lam, int64_t ldlam,
+                  const double* out, int64_t ldout, int64_t width)
 {
     const QlClass& c = p.cls;
     if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
-    if (B == 0) return QLNLP_OK;
-    if (!Z || !lam || !H) return fail(QLNLP_EINVAL, "Z, lambda and H are required");
-    if (ldz < c.n_nlp || ldlam < c.m_nlp || ldh < ql_hess_nnz(c)) return fail(QLNLP_EINVAL, "leading dimension too small");
-    const void* fn = p.fastdiv ? (const void*)ql::hess_kernel<true> : (const void*)ql::hess_kernel<false>;
-    const size_t smem = ql::hess_smem_bytes(c.N);
-    if (!ds.hess_blocks_per_sm) {
-        if (smem > ds.smem_optin) return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp", c.N, smem);
-        CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ds.smem_optin));
-        int nb = 0;
-        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, QL_LANES, smem));
-        if (nb < 1) return fail(QLNLP_ECUDA, "Hessian kernel does not fit on an SM");
-        ds.hess_blocks_per_sm = nb;
-        if (int rc = set_carveout(fn, nb, smem, ds.smem_per_sm)) return rc;      // the rest of the SM's memory is L1 (cost table)
-    }
-    ql::HessLaunch P;
-    P.c = c;
-    P.rmb = p.rmb; P.rmf = p.rmf; P.rIb = p.rIb;
-    P.cost = ds.d_cost; P.npad = p.npad;
-    P.Z = Z; P.ldz = ldz;
-    P.lam = lam; P.ldlam = ldlam;
-    P.sigma = sigma; P.sigma0 = sigma0;
-    P.H = H; P.ldh = ldh;
-    P.B = B;
-    P.bulk = ((reinterpret_cast<uintptr_t>(H) & 15) == 0 && (ldh & 1) == 0) ? 1 : 0;
-    P.zbulk = ((reinterpret_cast<uintptr_t>(Z) & 15) == 0 && (ldz & 1) == 0) ? 1 : 0;
-    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
-    const int grid = (int)std::min<int64_t>(B, (int64_t)ds.sm_count * ds.hess_blocks_per_sm);
-    void* args[] = {&P};
-    CUDA_TRY(cudaLaunchKernel(fn, dim3(grid), dim3(QL_LANES), args, smem, stream));
+    if (!Z || !lam || !out) return fail(QLNLP_EINVAL, "Z, lambda and the output are required");
+    if (ldz < c.n_nlp || ldlam < c.m_nlp || ldout < width) return fail(QLNLP_EINVAL, "leading dimension too small");
     return QLNLP_OK;
 }
 
+template <typename R>
+void set_hessian(R& P, const Problem& p, const DeviceState& ds, int64_t B, const double* Z, int64_t ldz,
+                 const double* sigma, double sigma0, const double* lam, int64_t ldlam)
+{
+    set_problem(P, p, ds);
+    P.Z = Z; P.ldz = ldz;
+    P.lam = lam; P.ldlam = ldlam;
+    P.sigma = sigma; P.sigma0 = sigma0;
+    P.B = B;
+    P.zbulk = ((reinterpret_cast<uintptr_t>(Z) & 15) == 0 && (ldz & 1) == 0) ? 1 : 0;
+}
+
+int launch_hessian(const Problem& p, DeviceState& ds, int64_t B, const double* Z, int64_t ldz, const double* sigma,
+                   double sigma0, const double* lam, int64_t ldlam, double* H, int64_t ldh, cudaStream_t stream)
+{
+    ql::HessLaunch P;
+    set_hessian(P, p, ds, B, Z, ldz, sigma, sigma0, lam, ldlam);
+    P.H = H; P.ldh = ldh;
+    P.bulk = ((reinterpret_cast<uintptr_t>(H) & 15) == 0 && (ldh & 1) == 0) ? 1 : 0;
+    return launch_kernel(ds, hess_spec(p, false), B, P, stream);
+}
+
 // ---- matrix-free products (MOI :JacVec / :HessVec) ---------------------------------------------------------------
-// Argument checks of the batched product entry points: host logic only, before any device is touched.
 int check_products(const Problem& p, int64_t B, const qlnlp_batch_io* io, const qlnlp_product_io* pv)
 {
     const QlClass& c = p.cls;
     const int m = m_rows(p);
-    if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
-    if (!io || !pv || !io->Z) return fail(QLNLP_EINVAL, "io, pv and io->Z are required");
+    if (!pv) return fail(QLNLP_EINVAL, "pv is required");
+    if (int rc = check_batch(p, B, io, nullptr)) return rc;
     if (io->jac) return fail(QLNLP_EINVAL, "io->jac must be NULL: the product launch writes no Jacobian values");
     if (!pv->w && !pv->y) return fail(QLNLP_EINVAL, "pv->w or pv->y is required");
     if (!pv->w != !pv->jw) return fail(QLNLP_EINVAL, "pv->jw is required iff pv->w is set");
     if (!pv->y != !pv->jty) return fail(QLNLP_EINVAL, "pv->jty is required iff pv->y is set");
-    if (io->ldz < c.n_nlp) return fail(QLNLP_EINVAL, "ldz %lld < n_nlp %d", (long long)io->ldz, c.n_nlp);
-    if (io->grad && io->ldgrad < c.n_nlp) return fail(QLNLP_EINVAL, "ldgrad %lld < n_nlp %d", (long long)io->ldgrad, c.n_nlp);
-    if (io->g && io->ldg < m) return fail(QLNLP_EINVAL, "ldg %lld < m_nlp %d", (long long)io->ldg, m);
     if (pv->w && (pv->ldw < c.n_nlp || pv->ldjw < m))
         return fail(QLNLP_EINVAL, "ldw %lld < n_nlp %d or ldjw %lld < m_nlp %d", (long long)pv->ldw, c.n_nlp, (long long)pv->ldjw, m);
     if (pv->y && (pv->ldy < m || pv->ldjty < c.n_nlp))
         return fail(QLNLP_EINVAL, "ldy %lld < m_nlp %d or ldjty %lld < n_nlp %d", (long long)pv->ldy, m, (long long)pv->ldjty, c.n_nlp);
-    for (const void* a : {(const void*)io->Z, (const void*)pv->w, (const void*)pv->jw, (const void*)pv->y, (const void*)pv->jty})
+    for (const void* a : {(const void*)pv->w, (const void*)pv->jw, (const void*)pv->y, (const void*)pv->jty})
         if ((reinterpret_cast<uintptr_t>(a) & 7) != 0) return fail(QLNLP_EINVAL, "arrays must be 8-byte aligned");
     return QLNLP_OK;
 }
@@ -901,21 +964,9 @@ int check_products(const Problem& p, int64_t B, const qlnlp_batch_io* io, const 
 int launch_products(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* io, const qlnlp_product_io* pv,
                     cudaStream_t stream)
 {
-    const QlClass& c = p.cls;
-    const void* fn = p.fastdiv ? (const void*)ql::eval_prod_kernel<true> : (const void*)ql::eval_prod_kernel<false>;
-    const size_t smem = ql::smem_bytes(c.N, ql::JM_PROD);
-    if (!ds.prod_blocks_per_sm) {
-        if (smem > ds.smem_optin) return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp", c.N, smem);
-        if (int rc = kernel_geometry(ds, fn, ql::JM_PROD, smem, &ds.prod_blocks_per_sm)) return rc;
-    }
     ql::ProdLaunch P;
     std::memset(&P, 0, sizeof P);
-    P.c = c;
-    P.rmb = p.rmb; P.rmf = p.rmf; P.rIb = p.rIb;
-    P.cost = ds.d_cost;
-    P.npad = p.npad;
-    P.x0_def = ds.d_x0xf;
-    P.xf_def = ds.d_x0xf + QL_NX;
+    set_problem(P, p, ds);
     P.Z = io->Z; P.ldz = io->ldz;
     P.x0 = io->x0; P.xf = io->xf;
     P.f = io->f;
@@ -928,30 +979,15 @@ int launch_products(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_ba
     P.y = pv->y; P.ldy = pv->ldy;
     P.jty = pv->jty; P.ldjty = pv->ldjty;
     P.kin = p.kin ? 1 : 0;
-    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
-    const int grid = (int)std::min<int64_t>(B, (int64_t)ds.sm_count * ds.prod_blocks_per_sm);
-    void* args[] = {&P};
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(QL_LANES);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];         // programmatic dependent launch, as in launch()
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    CUDA_TRY(cudaLaunchKernelExC(&cfg, fn, args));
-    return QLNLP_OK;
+    return launch_kernel(ds, prod_spec(p), B, P, stream);
 }
 
 int check_hess_products(const Problem& p, int64_t B, const double* Z, int64_t ldz, const double* lam, int64_t ldlam,
                         const double* V, int64_t ldv, const double* HV, int64_t ldhv)
 {
-    const QlClass& c = p.cls;
-    if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
-    if (!Z || !lam || !V || !HV) return fail(QLNLP_EINVAL, "Z, lambda, V and HV are required");
-    if (ldz < c.n_nlp || ldlam < c.m_nlp || ldv < c.n_nlp || ldhv < c.n_nlp) return fail(QLNLP_EINVAL, "leading dimension too small");
+    if (int rc = check_hessian(p, B, Z, ldz, lam, ldlam, HV, ldhv, p.cls.n_nlp)) return rc;
+    if (!V) return fail(QLNLP_EINVAL, "V is required");
+    if (ldv < p.cls.n_nlp) return fail(QLNLP_EINVAL, "leading dimension too small");
     for (const void* a : {(const void*)Z, (const void*)lam, (const void*)V, (const void*)HV})
         if ((reinterpret_cast<uintptr_t>(a) & 7) != 0) return fail(QLNLP_EINVAL, "arrays must be 8-byte aligned");
     return QLNLP_OK;
@@ -961,35 +997,12 @@ int launch_hess_products(const Problem& p, DeviceState& ds, int64_t B, const dou
                          double sigma0, const double* lam, int64_t ldlam, const double* V, int64_t ldv, double* HV,
                          int64_t ldhv, cudaStream_t stream)
 {
-    const QlClass& c = p.cls;
-    const void* fn = p.fastdiv ? (const void*)ql::hess_prod_kernel<true> : (const void*)ql::hess_prod_kernel<false>;
-    const size_t smem = ql::hess_smem_bytes(c.N);
-    if (!ds.hprod_blocks_per_sm) {
-        if (smem > ds.smem_optin) return fail(QLNLP_EINVAL, "N=%d needs %zu B of shared memory per warp", c.N, smem);
-        CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ds.smem_optin));
-        int nb = 0;
-        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, QL_LANES, smem));
-        if (nb < 1) return fail(QLNLP_ECUDA, "Hessian-product kernel does not fit on an SM");
-        if (int rc = set_carveout(fn, nb, smem, ds.smem_per_sm)) return rc;
-        ds.hprod_blocks_per_sm = nb;
-    }
     ql::HessProdLaunch P;
     std::memset(&P, 0, sizeof P);
-    P.c = c;
-    P.rmb = p.rmb; P.rmf = p.rmf; P.rIb = p.rIb;
-    P.cost = ds.d_cost; P.npad = p.npad;
-    P.Z = Z; P.ldz = ldz;
-    P.lam = lam; P.ldlam = ldlam;
-    P.sigma = sigma; P.sigma0 = sigma0;
-    P.B = B;
-    P.zbulk = ((reinterpret_cast<uintptr_t>(Z) & 15) == 0 && (ldz & 1) == 0) ? 1 : 0;
+    set_hessian(P, p, ds, B, Z, ldz, sigma, sigma0, lam, ldlam);
     P.V = V; P.ldv = ldv;
     P.HV = HV; P.ldhv = ldhv;
-    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
-    const int grid = (int)std::min<int64_t>(B, (int64_t)ds.sm_count * ds.hprod_blocks_per_sm);
-    void* args[] = {&P};
-    CUDA_TRY(cudaLaunchKernel(fn, dim3(grid), dim3(QL_LANES), args, smem, stream));
-    return QLNLP_OK;
+    return launch_kernel(ds, hess_spec(p, true), B, P, stream);
 }
 
 // ---- batched KKT solve (qlnlp_kkt.cuh) --------------------------------------------------------------------------
@@ -1048,33 +1061,17 @@ int ensure_kkt_tables(const Problem& p, DeviceState& ds)
 int launch_kkt(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_kkt_io* io, cudaStream_t stream)
 {
     const QlClass& c = p.cls;
-    const void* fn = (const void*)ql::kkt_kernel;
     if (int rc = ensure_kkt_tables(p, ds)) return rc;
-    if (!ds.kkt_blocks_per_sm) {
-        int nb = 0;
-        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, QL_LANES, 0));
-        if (nb < 1) return fail(QLNLP_ECUDA, "KKT kernel does not fit on an SM");
-        ds.kkt_blocks_per_sm = nb;
-    }
-    const int64_t slots = (int64_t)ds.sm_count * ds.kkt_blocks_per_sm;
-    // the scratch holds one factor per resident warp (the most a launch of any B uses), allocated at the first call on
-    // a stream and never grown
-    double*& scratch = ds.kkt_scratch[stream];
-    if (!scratch) {
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        cudaStreamIsCapturing(stream, &cap);
-        if (cap != cudaStreamCaptureStatusNone) {
-            ds.kkt_scratch.erase(stream);
-            return fail(QLNLP_EINVAL, "KKT solve: the factor scratch of this stream would have to be allocated during a graph capture");
-        }
-        cudaError_t e = cudaMalloc(&scratch, sizeof(double) * (size_t)slots * c.N * ql::KKT_FSTRIDE);
-        if (e != cudaSuccess) {
-            ds.kkt_scratch.erase(stream);
-            return fail(e == cudaErrorMemoryAllocation ? QLNLP_ENOMEM : QLNLP_ECUDA, "KKT scratch: %s", cudaGetErrorString(e));
-        }
-    }
+    const KernelSpec k = kkt_spec();
+    int per_sm = 0;
+    if (int rc = kernel_geometry(ds, k, &per_sm)) return rc;
+    // the scratch holds one factor per resident warp (the most a launch of any B uses)
     ql::KktLaunch P;
     std::memset(&P, 0, sizeof P);
+    if (int rc = grow_scratch(ds.kkt_scratch[stream], stream, (size_t)ds.sm_count * per_sm * c.N * ql::KKT_FSTRIDE,
+                              "KKT solve: the factor scratch of this stream would have to be allocated during a graph capture",
+                              &P.scratch))
+        return rc;
     P.c = c;
     P.jtab = ds.d_kkt_tab;
     P.htab = ds.d_kkt_tab + c.nnz_true;
@@ -1087,53 +1084,50 @@ int launch_kkt(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_kkt_io*
     P.px = io->px; P.ldpx = io->ldpx;
     P.pl = io->pl; P.ldpl = io->ldpl;
     P.status = io->status;
-    P.scratch = scratch;
     P.B = B;
-    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
-    const int grid = (int)std::min<int64_t>(B, slots);
-    void* args[] = {&P};
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(QL_LANES);
-    cfg.dynamicSmemBytes = 0;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];         // programmatic dependent launch, as in launch()
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    CUDA_TRY(cudaLaunchKernelExC(&cfg, fn, args));
-    return QLNLP_OK;
+    return launch_kernel(ds, k, B, P, stream);
 }
 
-// The three MOI product callbacks: copy in, one launch of B = 1, copy out, on the single-evaluation stream of the
-// handle's first device.  `in[0..nin)` go to device slots 1.., x to slot 0; the result comes back from the last slot.
+// A row of a single call: n doubles, copied in from `in` before the launch and / or back to `out` after it
+struct Row {
+    const double* in;
+    double* out;
+    int64_t n;
+};
+
+// One call on host pointers (the MOI callbacks other than the cached evaluation), on the single-evaluation stream of
+// the handle's first device: the rows (at most 5) are copied into device slots, each padded to an even length ld[i],
+// run(ds, slot, ld, stream) launches on them, and the outputs come back before the call returns.
 template <typename RUN>
-int product_one(qlnlp_handle h, const double* x, const double* const* in, const int64_t* nin, int nslots, double* out,
-                int64_t nout, RUN run)
+int single_call(qlnlp_handle h, std::initializer_list<Row> rows, const char* what, RUN run)
 {
-    const Problem& p = h->prob;
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
-    if (int rc = ensure_device(p, ds)) return rc;
-    const int64_t ld = std::max(p.ldz_e, p.ldg_e);           // every slot holds a row of n_nlp or m_nlp (+ 2N) doubles
-    if (!ds.d_prod_one) CUDA_TRY(cudaMalloc(&ds.d_prod_one, sizeof(double) * 5 * ld));
+    if (int rc = ensure_device(h->prob, ds)) return rc;
+    const cudaStream_t s = ds.one.stream;
     double* slot[5];
-    for (int i = 0; i < 5; ++i) slot[i] = ds.d_prod_one + i * ld;
-    cudaStream_t s = ds.one.stream;
-    cudaError_t e = cudaMemcpyAsync(slot[0], x, sizeof(double) * p.cls.n_nlp, cudaMemcpyHostToDevice, s);
-    for (int i = 0; i < nslots - 2 && e == cudaSuccess; ++i)
-        e = cudaMemcpyAsync(slot[1 + i], in[i], sizeof(double) * nin[i], cudaMemcpyHostToDevice, s);
-    int rc = e == cudaSuccess ? run(p, ds, slot, ld, s) : fail(QLNLP_ECUDA, "product: %s", cudaGetErrorString(e));
-    if (rc == QLNLP_OK) {
-        e = cudaMemcpyAsync(out, slot[nslots - 1], sizeof(double) * nout, cudaMemcpyDeviceToHost, s);
-        if (e != cudaSuccess) rc = fail(QLNLP_ECUDA, "product: %s", cudaGetErrorString(e));
+    int64_t ld[5];
+    size_t total = 0;
+    int i = 0;
+    for (const Row& r : rows) total += ld[i++] = (r.n + 1) & ~1;
+    if (int rc = grow_scratch(ds.one.slots, s, total, what, &slot[0])) return rc;
+    cudaError_t e = cudaSuccess;
+    i = 0;
+    for (const Row& r : rows) {
+        if (i) slot[i] = slot[i - 1] + ld[i - 1];
+        if (r.in && e == cudaSuccess) e = cudaMemcpyAsync(slot[i], r.in, sizeof(double) * r.n, cudaMemcpyHostToDevice, s);
+        ++i;
     }
-    const std::string msg = g_err;
-    const cudaError_t es = cudaStreamSynchronize(s);      // also on the error path: the host arrays are caller-owned
-    if (rc == QLNLP_OK && es != cudaSuccess) return fail(QLNLP_ECUDA, "product: %s", cudaGetErrorString(es));
-    g_err = msg;
-    return rc;
+    int rc = e == cudaSuccess ? run(ds, slot, ld, s) : fail(QLNLP_ECUDA, "%s: %s", what, cudaGetErrorString(e));
+    i = 0;
+    for (const Row& r : rows) {
+        if (rc == QLNLP_OK && r.out) {
+            e = cudaMemcpyAsync(r.out, slot[i], sizeof(double) * r.n, cudaMemcpyDeviceToHost, s);
+            if (e != cudaSuccess) rc = fail(QLNLP_ECUDA, "%s: %s", what, cudaGetErrorString(e));
+        }
+        ++i;
+    }
+    return finish(s, rc, what);
 }
 
 void free_lane(HostLane& ln)
@@ -1304,27 +1298,18 @@ int eval_host(qlnlp_handle h, int dev, int64_t B, const qlnlp_batch_io* io)
 {
     const Problem& p = h->prob;
     DeviceState& ds = h->devs[(size_t)dev];
-    const QlClass& c = p.cls;
     if (B == 0) return QLNLP_OK;
-    if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
-    if (!io || !io->Z) return fail(QLNLP_EINVAL, "io->Z is required");
-    if (io->ldz < c.n_nlp) return fail(QLNLP_EINVAL, "ldz < n_nlp");
-    if (io->grad && io->ldgrad < c.n_nlp) return fail(QLNLP_EINVAL, "ldgrad < n_nlp");
-    if (io->g && io->ldg < m_rows(p)) return fail(QLNLP_EINVAL, "ldg < m_nlp");
-    if (io->jac && io->ldjac < batch_nnz(p)) return fail(QLNLP_EINVAL, "ldjac < nnz");
-    if (io->jac && (reinterpret_cast<uintptr_t>(io->jac) & 7) != 0) return fail(QLNLP_EINVAL, "jac must be 8-byte aligned");
+    if (int rc = check_batch(p, B, io, nullptr, true)) return rc;
     DeviceGuard guard(ds.device);
     if (int rc = ensure_device(p, ds)) return rc;
     const int rc = eval_host_impl(h, dev, B, io);
     if (rc != QLNLP_OK) {
         // copies into caller-owned host memory (and out of the pinned stage) may still be in flight: finish them
         // before the caller gets its buffers back
-        const std::string msg = g_err;
         if (ds.pool) ds.pool->finish();
         for (auto& ln : ds.lanes)
-            if (ln.stream) cudaStreamSynchronize(ln.stream);
+            if (ln.stream) finish(ln.stream, rc, "host pipeline");
         cudaGetLastError();
-        g_err = msg;
     }
     return rc;
 }
@@ -1383,36 +1368,25 @@ int eval_one(qlnlp_handle h, const double* x, double* f, double* grad, double* g
     if (int rc = check_handle(h)) return rc;
     if (!x) return fail(QLNLP_EINVAL, "null x");
     const Problem& p = h->prob;
-    DeviceState& ds = h->devs[0];
     const QlClass& c = p.cls;
-    DeviceGuard guard(ds.device);
-    if (int rc = ensure_device(p, ds)) return rc;
     if (p.kin) {
         // kinematic rows: the plain route -- copy x in, evaluate what was asked for, copy it out (no x cache)
-        HostLane& ln = ds.lanes[0];
-        if (int rc = reserve_lane(p, ln, 1)) return rc;
-        cudaStream_t s = ln.stream;
-        CUDA_TRY(cudaMemcpyAsync(ln.Z, x, sizeof(double) * c.n_nlp, cudaMemcpyHostToDevice, s));
-        qlnlp_batch_io d;
-        std::memset(&d, 0, sizeof d);
-        d.Z = ln.Z; d.ldz = p.ldz_e;
-        d.f = f ? ln.f : nullptr;
-        d.grad = grad ? ln.grad : nullptr; d.ldgrad = p.ldgrad_e;
-        d.g = g ? ln.g : nullptr; d.ldg = p.ldg_e;
-        d.jac = vals ? ln.jac : nullptr; d.ldjac = p.ldjac_e;
-        int rc = launch_kin(p, ds, 1, &d, s);
-        cudaError_t e = cudaSuccess;
-        if (rc == QLNLP_OK && f) e = cudaMemcpyAsync(f, ln.f, sizeof(double), cudaMemcpyDeviceToHost, s);
-        if (rc == QLNLP_OK && e == cudaSuccess && grad) e = cudaMemcpyAsync(grad, ln.grad, sizeof(double) * c.n_nlp, cudaMemcpyDeviceToHost, s);
-        if (rc == QLNLP_OK && e == cudaSuccess && g) e = cudaMemcpyAsync(g, ln.g, sizeof(double) * m_rows(p), cudaMemcpyDeviceToHost, s);
-        if (rc == QLNLP_OK && e == cudaSuccess && vals) e = cudaMemcpyAsync(vals, ln.jac, sizeof(double) * batch_nnz(p), cudaMemcpyDeviceToHost, s);
-        if (rc == QLNLP_OK && e != cudaSuccess) rc = fail(QLNLP_ECUDA, "single evaluation: %s", cudaGetErrorString(e));
-        const std::string msg = g_err;
-        const cudaError_t es = cudaStreamSynchronize(s);
-        if (rc == QLNLP_OK && es != cudaSuccess) return fail(QLNLP_ECUDA, "single evaluation: %s", cudaGetErrorString(es));
-        g_err = msg;
-        return rc;
+        return single_call(h, {{x, nullptr, c.n_nlp}, {nullptr, f, 1}, {nullptr, grad, c.n_nlp}, {nullptr, g, m_rows(p)},
+                               {nullptr, vals, batch_nnz(p)}}, "single evaluation",
+                           [&](DeviceState& ds, double* const* d, const int64_t* ld, cudaStream_t s) {
+                               qlnlp_batch_io io;
+                               std::memset(&io, 0, sizeof io);
+                               io.Z = d[0]; io.ldz = ld[0];
+                               io.f = f ? d[1] : nullptr;
+                               io.grad = grad ? d[2] : nullptr; io.ldgrad = ld[2];
+                               io.g = g ? d[3] : nullptr; io.ldg = ld[3];
+                               io.jac = vals ? d[4] : nullptr; io.ldjac = ld[4];
+                               return launch_kin(p, ds, 1, &io, s);
+                           });
     }
+    DeviceState& ds = h->devs[0];
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(p, ds)) return rc;
     OneEval& o = ds.one;
     if (int rc = reserve_one(p, o)) return rc;
     const bool hit = h->opt_x_cache && o.valid && std::memcmp(o.hx, x, sizeof(double) * c.n_nlp) == 0;
@@ -1479,11 +1453,7 @@ int eval_dense_jacobian(const Problem& p, DeviceState& ds, const double* x, doub
         if (e == cudaSuccess) e = cudaMemcpyAsync(vals, ds.d_dense, sizeof(double) * dense_n, cudaMemcpyDeviceToHost, s);
         if (e != cudaSuccess) rc = fail(QLNLP_ECUDA, "dense Jacobian: %s", cudaGetErrorString(e));
     }
-    const std::string msg = g_err;
-    const cudaError_t es = cudaStreamSynchronize(s);      // also on the error path: `vals` is caller-owned
-    if (rc == QLNLP_OK && es != cudaSuccess) return fail(QLNLP_ECUDA, "dense Jacobian: %s", cudaGetErrorString(es));
-    g_err = msg;
-    return rc;
+    return finish(s, rc, "dense Jacobian");
 }
 
 void destroy_device_state(DeviceState& ds)
@@ -1499,11 +1469,11 @@ void destroy_device_state(DeviceState& ds)
     }
     if (ds.one.stream) cudaStreamDestroy(ds.one.stream);
     if (ds.one.hx) cudaFreeHost(ds.one.hx);
-    cudaFree(ds.d_hess_in); cudaFree(ds.d_hess_out); cudaFree(ds.d_prod_one);
+    cudaFree(ds.one.slots.ptr);
     cudaFree(ds.d_kin_map);
-    for (auto& kv : ds.kin_scratch) cudaFree(kv.second.first);
+    for (auto& kv : ds.kin_scratch) cudaFree(kv.second.ptr);
     cudaFree(ds.d_kkt_tab);
-    for (auto& kv : ds.kkt_scratch) cudaFree(kv.second);
+    for (auto& kv : ds.kkt_scratch) cudaFree(kv.second.ptr);
     for (auto& kv : ds.rag_tables) cudaFree(kv.second.d_classes);
     cudaFree(ds.ticket_pool);
     cudaFree(ds.d_cost); cudaFree(ds.d_x0xf); cudaFree(ds.d_segs); cudaFree(ds.d_seg_begin);
@@ -1845,6 +1815,7 @@ int qlnlp_eval_batch_device(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io,
     if (int rc = check_handle(h)) return rc;
     if (h->multi) return fail(QLNLP_EINVAL, "multi-device handle: use qlnlp_eval_batch_device_multi");
     if (B == 0) return QLNLP_OK;
+    if (int rc = check_batch(h->prob, B, io, nullptr)) return rc;
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
     if (int rc = ensure_device(h->prob, ds)) return rc;
@@ -1857,6 +1828,9 @@ int qlnlp_eval_batch_device_multi(qlnlp_handle h, const int64_t* B, const qlnlp_
     if (int rc = check_handle(h)) return rc;
     if (!B || !io) return fail(QLNLP_EINVAL, "null argument");
     const Problem& p = h->prob;
+    for (size_t i = 0; i < h->devs.size(); ++i)
+        if (B[i] != 0)
+            if (int rc = check_batch(p, B[i], io + i, nullptr)) return rc;
     for (size_t i = 0; i < h->devs.size(); ++i) {
         DeviceState& ds = h->devs[i];
         if (B[i] == 0) continue;
@@ -1886,6 +1860,7 @@ int qlnlp_eval_ragged_device(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io
     if (!rg) return fail(QLNLP_EINVAL, "null ragged descriptor");
     if (h->prob.kin) return fail(QLNLP_EINVAL, "ragged launches do not carry the kinematic rows");
     if (B == 0) return QLNLP_OK;
+    if (int rc = check_batch(h->prob, B, io, rg)) return rc;
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
     if (int rc = ensure_device(h->prob, ds)) return rc;
@@ -1908,6 +1883,7 @@ int qlnlp_eval_ragged_classes(const qlnlp_handle* hs, int ncls, int64_t B, const
         if (hs[i]->prob.kin) return fail(QLNLP_EINVAL, "ragged launches do not carry the kinematic rows");
     }
     if (B == 0) return QLNLP_OK;
+    if (int rc = check_batch(hs[0]->prob, B, io, rg)) return rc;
     DeviceGuard guard(hs[0]->devs[0].device);
     for (int i = 0; i < ncls; ++i)
         if (int rc = ensure_device(hs[i]->prob, hs[i]->devs[0])) return rc;
@@ -2131,6 +2107,7 @@ int qlnlp_eval_hessian_batch_device(qlnlp_handle h, int64_t B, const double* Z, 
     if (h->multi) return fail(QLNLP_EINVAL, "multi-device handle: the Hessian takes a single-device handle");
     if (h->prob.kin) return fail(QLNLP_EINVAL, "the Hessian does not cover the kinematic rows");
     if (B == 0) return QLNLP_OK;
+    if (int rc = check_hessian(h->prob, B, Z, ldz, lambda, ldlambda, H, ldh, ql_hess_nnz(h->prob.cls))) return rc;
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
     if (int rc = ensure_device(h->prob, ds)) return rc;
@@ -2143,28 +2120,11 @@ int qlnlp_eval_hessian_lagrangian(qlnlp_handle h, const double* x, double sigma,
     if (!x || !lambda || !vals) return fail(QLNLP_EINVAL, "null argument");
     const Problem& p = h->prob;
     if (p.kin) return fail(QLNLP_EINVAL, "the Hessian does not cover the kinematic rows");
-    DeviceState& ds = h->devs[0];
     const QlClass& c = p.cls;
-    DeviceGuard guard(ds.device);
-    if (int rc = ensure_device(p, ds)) return rc;
-    const int64_t ldl = (c.m_nlp + 1) & ~1, ldh = (ql_hess_nnz(c) + 1) & ~1;
-    if (!ds.d_hess_in) {
-        CUDA_TRY(cudaMalloc(&ds.d_hess_in, sizeof(double) * (p.ldz_e + ldl)));
-        CUDA_TRY(cudaMalloc(&ds.d_hess_out, sizeof(double) * ldh));
-    }
-    cudaStream_t s = ds.one.stream;
-    CUDA_TRY(cudaMemcpyAsync(ds.d_hess_in, x, sizeof(double) * c.n_nlp, cudaMemcpyHostToDevice, s));
-    CUDA_TRY(cudaMemcpyAsync(ds.d_hess_in + p.ldz_e, lambda, sizeof(double) * c.m_nlp, cudaMemcpyHostToDevice, s));
-    int rc = launch_hessian(p, ds, 1, ds.d_hess_in, p.ldz_e, nullptr, sigma, ds.d_hess_in + p.ldz_e, ldl, ds.d_hess_out, ldh, s);
-    if (rc == QLNLP_OK) {
-        cudaError_t e = cudaMemcpyAsync(vals, ds.d_hess_out, sizeof(double) * ql_hess_nnz(c), cudaMemcpyDeviceToHost, s);
-        if (e != cudaSuccess) rc = fail(QLNLP_ECUDA, "Hessian: %s", cudaGetErrorString(e));
-    }
-    const std::string msg = g_err;
-    const cudaError_t es = cudaStreamSynchronize(s);      // also on the error path: x / lambda / vals are caller-owned
-    if (rc == QLNLP_OK && es != cudaSuccess) return fail(QLNLP_ECUDA, "Hessian: %s", cudaGetErrorString(es));
-    g_err = msg;
-    return rc;
+    return single_call(h, {{x, nullptr, c.n_nlp}, {lambda, nullptr, c.m_nlp}, {nullptr, vals, ql_hess_nnz(c)}}, "Hessian",
+                       [&](DeviceState& ds, double* const* d, const int64_t* ld, cudaStream_t s) {
+                           return launch_hessian(p, ds, 1, d[0], ld[0], nullptr, sigma, d[1], ld[1], d[2], ld[2], s);
+                       });
 }
 
 /* ---- matrix-free products (MOI :JacVec / :HessVec) ---- */
@@ -2212,24 +2172,23 @@ int qlnlp_kkt_solve_batch_device(qlnlp_handle h, int64_t B, const qlnlp_kkt_io* 
     return launch_kkt(h->prob, ds, B, io, static_cast<cudaStream_t>(stream));
 }
 
-// J w (transpose: J' y) at x for one evaluation: slot 1 holds the vector, slot 2 the result
+// J w (transpose: J' y) at x for one evaluation
 static int jacobian_product_one(qlnlp_handle h, const double* x, const double* v, double* out, bool transpose)
 {
     if (int rc = check_handle(h)) return rc;
     if (!x || !v || !out) return fail(QLNLP_EINVAL, "null argument");
     const Problem& p = h->prob;
     const int64_t n = p.cls.n_nlp, m = m_rows(p);
-    const int64_t nin = transpose ? m : n;
-    return product_one(h, x, &v, &nin, 3, out, transpose ? n : m,
-                       [&](const Problem& pp, DeviceState& ds, double* const* slot, int64_t ld, cudaStream_t s) {
+    return single_call(h, {{x, nullptr, n}, {v, nullptr, transpose ? m : n}, {nullptr, out, transpose ? n : m}}, "product",
+                       [&](DeviceState& ds, double* const* d, const int64_t* ld, cudaStream_t s) {
                            qlnlp_batch_io io;
                            std::memset(&io, 0, sizeof io);
-                           io.Z = slot[0]; io.ldz = ld;
+                           io.Z = d[0]; io.ldz = ld[0];
                            qlnlp_product_io pv;
                            std::memset(&pv, 0, sizeof pv);
-                           if (transpose) { pv.y = slot[1]; pv.ldy = ld; pv.jty = slot[2]; pv.ldjty = ld; }
-                           else { pv.w = slot[1]; pv.ldw = ld; pv.jw = slot[2]; pv.ldjw = ld; }
-                           return launch_products(pp, ds, 1, &io, &pv, s);
+                           if (transpose) { pv.y = d[1]; pv.ldy = ld[1]; pv.jty = d[2]; pv.ldjty = ld[2]; }
+                           else { pv.w = d[1]; pv.ldw = ld[1]; pv.jw = d[2]; pv.ldjw = ld[2]; }
+                           return launch_products(p, ds, 1, &io, &pv, s);
                        });
 }
 
@@ -2250,12 +2209,11 @@ int qlnlp_eval_hessian_lagrangian_product(qlnlp_handle h, const double* x, const
     if (!x || !v || !lambda || !hv) return fail(QLNLP_EINVAL, "null argument");
     const Problem& p = h->prob;
     if (p.kin) return fail(QLNLP_EINVAL, "the Hessian does not cover the kinematic rows");
-    const double* in[2] = {lambda, v};
-    const int64_t nin[2] = {p.cls.m_nlp, p.cls.n_nlp};
-    return product_one(h, x, in, nin, 4, hv, p.cls.n_nlp,
-                       [&](const Problem& pp, DeviceState& ds, double* const* slot, int64_t ld, cudaStream_t s) {
-                           return launch_hess_products(pp, ds, 1, slot[0], ld, nullptr, sigma, slot[1], ld, slot[2], ld,
-                                                       slot[3], ld, s);
+    const int64_t n = p.cls.n_nlp;
+    return single_call(h, {{x, nullptr, n}, {lambda, nullptr, p.cls.m_nlp}, {v, nullptr, n}, {nullptr, hv, n}}, "product",
+                       [&](DeviceState& ds, double* const* d, const int64_t* ld, cudaStream_t s) {
+                           return launch_hess_products(p, ds, 1, d[0], ld[0], nullptr, sigma, d[1], ld[1], d[2], ld[2],
+                                                       d[3], ld[3], s);
                        });
 }
 

@@ -151,6 +151,63 @@ def test_multi_device_handle_answers_like_a_plain_handle(devices):
         assert call() == ev.QLNLP_EINVAL and L.qlnlp_last_error().decode() == msg
 
 
+def test_batch_argument_checks_need_no_device():
+    """The batched entry points on device pointers check their arguments before they bind the device, so an invalid
+    call is refused the same way with or without a GPU."""
+    prob = ql.build_problem(N=5, k_trans=3)
+    L = ql.load_library()
+    nlp = ql.HybridNLP.from_problem(prob, hessian=True)
+    n, m, nnz, nh = nlp.n_nlp, nlp.m_nlp, nlp.nnz, nlp.nnz_hess
+    Z, g, jac, lam, H = np.zeros(n + 1), np.zeros(m + 1), np.zeros(nnz + 1), np.zeros(m + 1), np.zeros(nh + 1)
+    off = np.zeros(2, dtype=np.int64)
+
+    def io(**kw):
+        d = ev._BatchIO()
+        d.Z, d.ldz = Z.ctypes.data, n
+        for k, v in kw.items():
+            setattr(d, k, v)
+        return d
+
+    def rg(**kw):
+        r = ev._RaggedIO()
+        r.z_off = off.ctypes.data
+        for k, v in kw.items():
+            setattr(r, k, v)
+        return r
+
+    def batch(B, d):
+        return L.qlnlp_eval_batch_device(nlp._h, B, None if d is None else C.byref(d), None)
+
+    def ragged(B, d, r):
+        return L.qlnlp_eval_ragged_device(nlp._h, B, None if d is None else C.byref(d), C.byref(r), None)
+
+    def classes(B, d, r):
+        return L.qlnlp_eval_ragged_classes((C.c_void_p * 1)(nlp._h.value), 1, B, None if d is None else C.byref(d),
+                                           C.byref(r), None, None)
+
+    def hess(B, Zp=Z.ctypes.data, ldz=n, lp=lam.ctypes.data, ldl=m, hp=H.ctypes.data, ldh=nh):
+        return L.qlnlp_eval_hessian_batch_device(nlp._h, B, Zp, ldz, None, lp, ldl, hp, ldh, None)
+
+    invalid = [
+        lambda: batch(-1, io()), lambda: batch(1, None), lambda: batch(1, io(Z=None)), lambda: batch(2, io(ldz=n - 1)),
+        lambda: batch(2, io(g=g.ctypes.data, ldg=m - 1)), lambda: batch(2, io(jac=jac.ctypes.data, ldjac=nnz - 1)),
+        lambda: batch(1, io(Z=Z.ctypes.data + 4)),
+        lambda: ragged(-1, io(), rg()), lambda: ragged(1, None, rg()), lambda: ragged(1, io(), rg(z_off=None)),
+        lambda: ragged(1, io(g=g.ctypes.data), rg()), lambda: ragged(1, io(jac=jac.ctypes.data), rg()),
+        lambda: classes(-1, io(), rg()), lambda: classes(1, None, rg()), lambda: classes(1, io(), rg(z_off=None)),
+        lambda: classes(1, io(jac=jac.ctypes.data), rg()),
+        lambda: hess(-1), lambda: hess(1, Zp=None), lambda: hess(1, lp=None), lambda: hess(1, hp=None),
+        lambda: hess(2, ldz=n - 1), lambda: hess(2, ldl=m - 1), lambda: hess(2, ldh=nh - 1),
+    ]
+    for i, call in enumerate(invalid):
+        assert call() == ev.QLNLP_EINVAL, (i, L.qlnlp_last_error())
+    assert batch(0, None) == ev.QLNLP_OK and hess(0, Zp=None, lp=None, hp=None) == ev.QLNLP_OK
+    if not _has_gpu():                                     # valid arguments (host memory here) reach the device
+        for call in (lambda: batch(1, io()), lambda: ragged(1, io(), rg()), lambda: classes(1, io(), rg()),
+                     lambda: hess(1)):
+            assert call() == ev.QLNLP_ENODEVICE
+
+
 def _build_demo(tmp_path):
     import subprocess
     exe = str(tmp_path / "qlnlp_demo")

@@ -567,6 +567,62 @@ def test_launches_can_be_captured_in_a_cuda_graph(dflt, golden):
         assert torch.equal(out[k], eager[k]), k
 
 
+def test_every_launcher_can_be_captured_in_a_cuda_graph(dflt, golden):
+    """The products, the Hessian, the Hessian products, the KKT solve and a kinematic handle's evaluation launch
+    through the same path as the plain evaluation: once the capture stream has been used (its work counter, the
+    kinematic and KKT scratch), their launches can be captured into one graph whose replay equals the eager results."""
+    p = dflt[0]
+    nlp = ql.HybridNLP.from_problem(p, pattern="true", hessian=True)
+    kin = ql.HybridNLP.from_problem(p, kinematics=True)
+    B, n, m = 600, nlp.n_nlp, nlp.m_nlp
+    rng = np.random.default_rng(12)
+    cuda = lambda a: torch.from_numpy(np.ascontiguousarray(a)).cuda()
+    Z = cuda(perturbed_batch(p, _bases(p, golden), B, 1e-2, 12))
+    lam, sigma = cuda(1e-4 * rng.standard_normal((B, m))), cuda(np.full(B, 1e-4))
+    w, y, V = cuda(rng.standard_normal((B, n))), cuda(rng.standard_normal((B, m))), cuda(rng.standard_normal((B, n)))
+    dc, sx = cuda(rng.uniform(1e-2, 1.0, (B, m))), cuda(rng.uniform(1.0, 10.0, (B, n)))
+    r1, r2 = cuda(rng.standard_normal((B, n))), cuda(rng.standard_normal((B, m)))
+    jac = nlp.eval_batch(Z, want=("jac",))["jac"]
+
+    def run(out):
+        nlp.eval_products_batch(Z, w=w, y=y, want=("f", "g"), out=out["prod"])
+        nlp.eval_hessian_batch(Z, lam, sigma=sigma, out=out["hess"])
+        nlp.eval_hessian_product_batch(Z, lam, V, sigma=sigma, out=out["hv"])
+        nlp.kkt_solve_batch(out["hess"], jac, dc, r1, r2, sx=sx, out=out["kkt"])
+        kin.eval_batch(Z, out=out["kin"])
+
+    eager = {"prod": nlp.eval_products_batch(Z, w=w, y=y, want=("f", "g")), "hess": nlp.eval_hessian_batch(Z, lam, sigma=sigma),
+             "hv": nlp.eval_hessian_product_batch(Z, lam, V, sigma=sigma), "kin": kin.eval_batch(Z)}
+    eager["kkt"] = nlp.kkt_solve_batch(eager["hess"], jac, dc, r1, r2, sx=sx)
+    torch.cuda.synchronize()
+    assert not eager["kkt"][2].any()                    # every problem solved: the comparison covers real steps
+
+    def like(t):                                        # same row stride as the library's outputs
+        if t.dim() == 1:
+            return torch.zeros_like(t)
+        return torch.zeros((t.shape[0], t.stride(0)), dtype=t.dtype, device=t.device)[:, :t.shape[1]]
+
+    out = {"prod": {k: like(v) for k, v in eager["prod"].items()}, "hess": like(eager["hess"]), "hv": like(eager["hv"]),
+           "kkt": tuple(like(t) for t in eager["kkt"]), "kin": {k: like(v) for k, v in eager["kin"].items()}}
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):                       # warm the capture stream outside the capture
+        run(out)
+    torch.cuda.current_stream().wait_stream(side)
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g, stream=side):
+        run(out)
+    flat = lambda o: [*o["prod"].values(), o["hess"], o["hv"], *o["kkt"], *o["kin"].values()]
+    for t in flat(out):
+        t.zero_()
+    for _ in range(2):
+        g.replay()
+    torch.cuda.synchronize()
+    for i, (a, b) in enumerate(zip(flat(out), flat(eager))):
+        assert torch.equal(a, b), i
+
+
 def test_back_to_back_launches_respect_stream_order(dflt, golden):
     """Evaluations are launched with programmatic dependent launch: the next grid may be scheduled while the previous
     one drains, so the kernel itself has to wait for its predecessors before it touches data.  Queue, without any
