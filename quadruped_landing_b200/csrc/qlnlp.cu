@@ -287,12 +287,13 @@ const void* const EVAL_FN[NJM][2][2] = {
 
 KernelSpec eval_spec(int N, int jm, bool fast, bool ragged)
 {
-    // The SPARSE_BLOCK stream is store-bound and the memory system takes the output of a few fast warps better than
-    // that of all 8 that fit (occupancy sweeps in profiles/r01_ablation.md, section 7): at most 6 CTAs per SM (launch()
-    // narrows that to 5 or 6), with padded shared memory.  The other value streams run as many warps as the kernel was
-    // compiled for (its __launch_bounds__).
+    // SPARSE_BLOCK: all 8 CTAs per SM that fit (launch() narrows that to 7 for short batches), with padded shared
+    // memory.  Since the outputs live in compressible memory the stream no longer waits on DRAM but on the warps' own
+    // arithmetic, and more resident warps hide it (profiles/r05_occupancy_sweep.log; the 5-6 warps of
+    // profiles/r01_ablation.md section 7 were measured against plain memory).  The other value streams run as many
+    // warps as the kernel was compiled for (its __launch_bounds__).
     const bool block = jm == ql::JM_BLOCK;
-    const int cap = block ? 6 : jm == ql::JM_NONE ? QL_NONE_WARPS : QL_TRUE_WARPS;
+    const int cap = block ? 8 : jm == ql::JM_NONE ? QL_NONE_WARPS : QL_TRUE_WARPS;
     return {EVAL_FN[jm][fast][ragged], ql::smem_bytes(N, jm), cap, true, block, true};
 }
 
@@ -643,7 +644,7 @@ int launch_kernel(DeviceState& ds, const KernelSpec& k, int64_t B, R& P, cudaStr
     const int grid = (int)std::min<int64_t>(B, (int64_t)ds.sm_count * per_sm);
     if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
     // With programmatic dependent launch the next grid's CTAs are placed as soon as an SM has room for one.  The
-    // SPARSE_BLOCK kernel runs on fewer CTAs per SM than would fit (5 or 6 of up to 7 by shared memory): a spare slot
+    // SPARSE_BLOCK kernel can run on fewer CTAs per SM than would fit (7 of 8 for short batches): a spare slot
     // would take a CTA of the next grid while this grid is still running at full strength, and the next grid would
     // start out unevenly spread over the SMs (measured: -5 % on the headline once another handle had raised the
     // kernel's carve-out to 228 KB).  Ask for enough shared memory per CTA that per_sm + 1 of them never fit.
@@ -772,8 +773,9 @@ int launch(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* i
     int cap = INT_MAX;
     if (!rg && wj != ql::JM_VALS)      // a plain launch runs on no more CTAs per SM than the ragged instantiation
         if (int rc = kernel_geometry(ds, eval_spec(p.cls.N, wj, p.fastdiv, true), &cap)) return rc;
-    // SPARSE_BLOCK: 5 CTAs per SM, 6 for short batches that also want the cost/gradient (see eval_spec)
-    if (wj == ql::JM_BLOCK) cap = std::min(cap, (io->f || io->grad) && B < 8 * (int64_t)ds.sm_count * 6 ? 6 : 5);
+    // SPARSE_BLOCK: 8 CTAs per SM, 7 for short batches (fewer than 8 evaluations per warp).  B = 4,096 at 7 / 8 / the
+    // former 6 or 5: full 24.8 / 24.2 / 24.6, g+J 27.8 / 26.9 / 26.0 M evals/s (profiles/r05_occupancy_sweep.log)
+    if (wj == ql::JM_BLOCK) cap = std::min(cap, B < 8 * (int64_t)ds.sm_count * 7 ? 7 : 8);
     const KernelSpec k = rg ? eval_spec(table->layout.N, wj, table->fastdiv, true) : eval_spec(p.cls.N, wj, p.fastdiv, false);
     return launch_kernel(ds, k, B, P, stream, cap, ds.last_launch);
 }
