@@ -14,6 +14,17 @@
  *   - one handle may be driven by one host thread at a time (Ipopt calls back from one thread);
  *     different handles are independent;
  *   - every call leaves the calling thread's current CUDA device as it found it;
+ *   - streams and CUDA graphs (the *_device entry points): a handle may launch on any number of streams, and
+ *     launches on different streams may run at once.  Launches may be captured into CUDA graphs, and a graph may be
+ *     replayed on any stream, concurrently with anything else the handle does, including replays of other graphs
+ *     captured on the same stream and eager launches on the capture stream: each graph owns the work counter and
+ *     the scratch its launches use.  Up to 1,024 graphs per handle may hold launches at once (a capture beyond that
+ *     is refused with QLNLP_EINVAL); a graph gives its counter back when it and its executable instantiations are
+ *     destroyed, and must not outlive its handle.  Replay one executable instantiation of a graph at a time.
+ *     First-use set-up allocates and synchronises, which a capture cannot hold: the first call of a handle, its first
+ *     kinematic evaluation, its first KKT solve and the first ragged launch over a set of classes are refused with
+ *     QLNLP_EINVAL inside a capture (the caller's capture stays valid).  Warm the handle outside the capture by
+ *     making each kind of call it will capture once, on any stream;
  *   - there is NO CPU fallback: evaluation entry points fail with QLNLP_ENODEVICE when no
  *     sm_100 device / driver is present.  Structure, dimension and bound queries are pure host
  *     integer logic and work anywhere.
@@ -244,7 +255,8 @@ int qlnlp_eval_hessian_lagrangian_product(qlnlp_handle h, const double* x, const
  * One fixed operation order per problem: the bits do not depend on B, the batch position, leading dimensions,
  * alignment or the stream.  DEVICE pointers, 8-byte aligned (status 4-byte); enqueued on `stream`, not
  * synchronised.  Refused (QLNLP_EINVAL): SPARSE_BLOCK / DENSE handles, QLNLP_WITH_KINEMATICS handles, multi-device
- * handles.  The factor scratch (1,840 B per knot per resident warp) is allocated at the first call on a stream. */
+ * handles.  The factor scratch (1,840 B per knot per resident warp) is allocated at the first call on a stream; a
+ * captured solve allocates its own inside the graph. */
 typedef struct {
     const double* hess; int64_t ldhess;   /* [B][ldhess >= nnz_hess] */
     const double* jac;  int64_t ldjac;    /* [B][ldjac  >= nnz (SPARSE_TRUE)] */

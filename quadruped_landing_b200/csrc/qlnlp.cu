@@ -54,7 +54,8 @@ int fail(int code, const char* fmt, ...)
                         cudaGetErrorString(e_), __FILE__, __LINE__);                                \
     } while (0)
 
-constexpr int TICKET_POOL = 64;
+constexpr int TICKET_POOL = 64;       // work counters of streams (recycled once every one is taken)
+constexpr int GRAPH_TICKETS = 1024;   // work counters of captured graphs (each held until its graph is destroyed)
 constexpr int NJM = 4;                 // kernel value streams: JM_NONE, JM_BLOCK, JM_TRUE, JM_VALS
 constexpr int MAX_LANES = 4;           // pipeline depth of the host-pointer path
 constexpr int64_t COMPACT_MIN_B = 64;  // below this, host-pointer batches copy the pattern rows as they are
@@ -132,6 +133,30 @@ struct Problem {
     int64_t ldz_e = 0, ldgrad_e = 0, ldg_e = 0, ldjac_e = 0, ldv_e = 0;   // even leading dimensions of the scratch
 };
 
+// Work counters that captured graphs own: the GRAPH_TICKETS counters after the stream pool.  A capture sequence takes
+// one per stream at its first launch there, and its graph holds it through a CUDA user object until the graph (and
+// every executable instantiated from it) is destroyed.  The user object's destructor runs on a thread of the CUDA
+// runtime, may make no CUDA call and may run after the handle is gone: it only hands the counter back, under `mu`.
+struct GraphTickets {
+    std::mutex mu;
+    std::vector<int> free;                                                // counters no graph holds
+    std::map<std::pair<unsigned long long, cudaStream_t>, int> live;     // (capture sequence, stream) -> counter
+};
+
+struct GraphTicket {
+    std::shared_ptr<GraphTickets> pool;
+    std::pair<unsigned long long, cudaStream_t> key;
+    int index;
+};
+
+void release_graph_ticket(void* p)
+{
+    std::unique_ptr<GraphTicket> t(static_cast<GraphTicket*>(p));
+    std::lock_guard<std::mutex> lk(t->pool->mu);
+    t->pool->live.erase(t->key);
+    t->pool->free.push_back(t->index);        // zero again: the last CTA of every grid re-arms its counter
+}
+
 // What one device of a handle holds, created at its first evaluation (ensure_device).
 struct DeviceState {
     int device = 0;
@@ -151,6 +176,7 @@ struct DeviceState {
     std::map<cudaStream_t, unsigned*> tickets;   // work counters, one pair per stream the device has launched on
     unsigned* ticket_pool = nullptr;             // pre-zeroed counters (128 B apart) so that a launch needs no
     int ticket_pool_used = 0;                    // allocation: launches stay legal inside CUDA-graph capture
+    std::shared_ptr<GraphTickets> graph_tickets; // the counters after the TICKET_POOL stream counters
     int* d_kin_map = nullptr;          // caller-visible value order of the batch pattern -> scratch position or -(entry + 1)
     std::map<cudaStream_t, Scratch> kin_scratch;                 // per stream: reference-order rows (device)
     std::map<std::vector<uint64_t>, RagTable> rag_tables;       // ragged launches led by this handle (key: the classes' serials)
@@ -552,10 +578,28 @@ int check_handle(qlnlp_handle h)
     return QLNLP_OK;
 }
 
-// Binds one device of a handle (first call: tables, occupancy, streams).  The caller holds a DeviceGuard.
-int ensure_device(const Problem& p, DeviceState& ds)
+// Whether work on `stream` is being captured into a graph (the legacy default stream never is)
+bool capturing(cudaStream_t stream)
+{
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    return stream && cudaStreamIsCapturing(stream, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone;
+}
+
+// First-use set-up (allocations, blocking copies, a device synchronise) would invalidate a graph capture: the call
+// that needs it is refused before it makes any such call, and the caller's capture goes on.
+int refuse_setup_in_capture(cudaStream_t stream, const char* what)
+{
+    if (!capturing(stream)) return QLNLP_OK;
+    return fail(QLNLP_EINVAL, "%s: first use inside a CUDA-graph capture, which cannot allocate or synchronise; warm the "
+                "handle with one such call outside the capture before capturing", what);
+}
+
+// Binds one device of a handle (first call: tables, occupancy, streams).  The caller holds a DeviceGuard.  `stream`:
+// the stream the call launches on (set-up is refused while it is being captured).
+int ensure_device(const Problem& p, DeviceState& ds, cudaStream_t stream = nullptr)
 {
     if (ds.ready) return QLNLP_OK;
+    if (int rc = refuse_setup_in_capture(stream, "set-up of the handle")) return rc;
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
     if (e != cudaSuccess || ndev == 0)
@@ -595,8 +639,10 @@ int ensure_device(const Problem& p, DeviceState& ds)
         CUDA_TRY(cudaEventCreateWithFlags(&ln.done, cudaEventDisableTiming));
     }
     CUDA_TRY(cudaStreamCreateWithFlags(&ds.one.stream, cudaStreamNonBlocking));
-    CUDA_TRY(cudaMalloc(&ds.ticket_pool, 128 * TICKET_POOL));
-    CUDA_TRY(cudaMemset(ds.ticket_pool, 0, 128 * TICKET_POOL));
+    CUDA_TRY(cudaMalloc(&ds.ticket_pool, 128 * (TICKET_POOL + GRAPH_TICKETS)));
+    CUDA_TRY(cudaMemset(ds.ticket_pool, 0, 128 * (TICKET_POOL + GRAPH_TICKETS)));
+    ds.graph_tickets = std::make_shared<GraphTickets>();
+    for (int i = TICKET_POOL + GRAPH_TICKETS - 1; i >= TICKET_POOL; --i) ds.graph_tickets->free.push_back(i);
     // the set-up copies above ran on the legacy default stream and may still be in flight when cudaMemcpy returns
     // (pageable source); launches go to arbitrary, possibly non-blocking streams, so finish the set-up first
     CUDA_TRY(cudaDeviceSynchronize());
@@ -632,6 +678,55 @@ int stream_ticket(DeviceState& ds, cudaStream_t stream, unsigned** out)
     return QLNLP_OK;
 }
 
+// Work counter of a launch on `stream`.  An eager launch takes the stream's counter.  A launch captured into a graph
+// takes a counter its graph owns (GraphTickets), never a stream's: a replay may run on any stream, beside eager work
+// on the capture stream and beside replays of other graphs captured there, and each grid needs a counter no other
+// running grid draws from.  Launches of one capture sequence on one stream are ordered, so they share one.
+int launch_ticket(DeviceState& ds, cudaStream_t stream, unsigned** out)
+{
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    unsigned long long id = 0;
+    cudaGraph_t graph = nullptr;
+    if (cudaStreamGetCaptureInfo(stream, &cap, &id, &graph) != cudaSuccess || cap != cudaStreamCaptureStatusActive)
+        return stream_ticket(ds, stream, out);
+    GraphTickets& gt = *ds.graph_tickets;
+    const auto key = std::make_pair(id, stream);
+    int index = -1;
+    {
+        std::lock_guard<std::mutex> lk(gt.mu);
+        auto it = gt.live.find(key);
+        if (it != gt.live.end()) {
+            *out = ds.ticket_pool + 32 * it->second;
+            return QLNLP_OK;
+        }
+        if (gt.free.empty())
+            return fail(QLNLP_EINVAL, "%d captured graphs of this handle hold work counters: destroy some before capturing more",
+                        GRAPH_TICKETS);
+        index = gt.free.back();
+        gt.free.pop_back();
+        gt.live.emplace(key, index);
+    }
+    // the graph takes the only reference; the CUDA calls run outside the lock (a release may run the destructor)
+    GraphTicket* t = new (std::nothrow) GraphTicket{ds.graph_tickets, key, index};
+    if (!t) {
+        std::lock_guard<std::mutex> lk(gt.mu);
+        gt.live.erase(key);
+        gt.free.push_back(index);
+        return fail(QLNLP_ENOMEM, "out of host memory");
+    }
+    cudaUserObject_t obj = nullptr;
+    if (cudaError_t e = cudaUserObjectCreate(&obj, t, release_graph_ticket, 1, cudaUserObjectNoDestructorSync)) {
+        release_graph_ticket(t);
+        return fail(QLNLP_ECUDA, "cudaUserObjectCreate: %s", cudaGetErrorString(e));
+    }
+    if (cudaError_t e = cudaGraphRetainUserObject(graph, obj, 1, cudaGraphUserObjectMove)) {
+        cudaUserObjectRelease(obj, 1);
+        return fail(QLNLP_ECUDA, "cudaGraphRetainUserObject: %s", cudaGetErrorString(e));
+    }
+    *out = ds.ticket_pool + 32 * index;
+    return QLNLP_OK;
+}
+
 // The one launch of every kernel that hands out work with a ticket: B evaluations of record `P` on `stream`, on at most
 // `cap` resident CTAs per SM.  `info`: the launch_info record to fill (eval launches).
 template <typename R>
@@ -642,7 +737,7 @@ int launch_kernel(DeviceState& ds, const KernelSpec& k, int64_t B, R& P, cudaStr
     if (int rc = kernel_geometry(ds, k, &per_sm)) return rc;
     per_sm = std::min(per_sm, cap);
     const int grid = (int)std::min<int64_t>(B, (int64_t)ds.sm_count * per_sm);
-    if (int rc = stream_ticket(ds, stream, &P.ticket)) return rc;
+    if (int rc = launch_ticket(ds, stream, &P.ticket)) return rc;
     // With programmatic dependent launch the next grid's CTAs are placed as soon as an SM has room for one.  The
     // SPARSE_BLOCK kernel can run on fewer CTAs per SM than would fit (7 of 8 for short batches): a spare slot
     // would take a CTA of the next grid while this grid is still running at full strength, and the next grid would
@@ -689,14 +784,11 @@ void set_problem(R& P, const Problem& p, const DeviceState& ds)
     }
 }
 
-// Device scratch of at least n doubles for work on `stream`, grown only.  It cannot grow while the stream is being
-// captured into a graph: the call fails with `msg`.
-int grow_scratch(Scratch& sc, cudaStream_t stream, size_t n, const char* msg, double** out)
+// Device scratch of at least n doubles for eager work on one stream, grown only.  (A launch captured into a graph
+// takes scratch its graph owns instead: launch_scratch.)
+int grow_scratch(Scratch& sc, size_t n, double** out)
 {
     if (sc.cap < n) {
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        cudaStreamIsCapturing(stream, &cap);
-        if (cap != cudaStreamCaptureStatusNone) return fail(QLNLP_EINVAL, "%s", msg);
         if (sc.ptr) {
             CUDA_TRY(cudaDeviceSynchronize());      // earlier launches may still use it
             cudaFree(sc.ptr);
@@ -706,6 +798,26 @@ int grow_scratch(Scratch& sc, cudaStream_t stream, size_t n, const char* msg, do
         sc.cap = n;
     }
     *out = sc.ptr;
+    return QLNLP_OK;
+}
+
+// Scratch of n doubles for the launches of one call on `stream`.  Eager: the stream's grow-only block in `per_stream`.
+// Inside a graph capture: a block of the graph's own, allocated here and freed by end_scratch after the call's last
+// kernel (graph memory nodes).  A replay then shares no scratch with eager work or with other graphs, and no eager
+// call can free a block a graph still points to.
+int launch_scratch(std::map<cudaStream_t, Scratch>& per_stream, cudaStream_t stream, size_t n, double** out, bool* owned)
+{
+    *owned = capturing(stream);
+    if (*owned) {
+        CUDA_TRY(cudaMallocAsync(reinterpret_cast<void**>(out), sizeof(double) * n, stream));
+        return QLNLP_OK;
+    }
+    return grow_scratch(per_stream[stream], n, out);
+}
+
+int end_scratch(double* ptr, bool owned, cudaStream_t stream)
+{
+    if (owned) CUDA_TRY(cudaFreeAsync(ptr, stream));
     return QLNLP_OK;
 }
 
@@ -781,14 +893,15 @@ int launch(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* i
 }
 
 // The class table of a ragged launch over the single-device handles `hs` (all on one device, already bound to it),
-// cached in the device state of hs[0].
-int ragged_table(const qlnlp_handle* hs, int ncls, const RagTable** out)
+// cached in the device state of hs[0].  A new class set is refused while `stream` is being captured.
+int ragged_table(const qlnlp_handle* hs, int ncls, cudaStream_t stream, const RagTable** out)
 {
     DeviceState& lead = hs[0]->devs[0];
     std::vector<uint64_t> key((size_t)ncls);
     for (int i = 0; i < ncls; ++i) key[(size_t)i] = hs[i]->prob.serial;
     auto it = lead.rag_tables.find(key);
     if (it != lead.rag_tables.end()) { *out = &it->second; return QLNLP_OK; }
+    if (int rc = refuse_setup_in_capture(stream, "ragged launch over a new set of classes")) return rc;
     RagTable t;
     t.ncls = ncls;
     t.fastdiv = true;
@@ -846,9 +959,10 @@ void kin_structure(const Problem& p, std::vector<int64_t>& rows, std::vector<int
     for (size_t i = 0; i < all.size(); ++i) { rows[i] = all[i].row; cols[i] = all[i].col; map[i] = all[i].src; }
 }
 
-int ensure_kin(const Problem& p, DeviceState& ds)
+int ensure_kin(const Problem& p, DeviceState& ds, cudaStream_t stream)
 {
     if (ds.d_kin_map) return QLNLP_OK;
+    if (int rc = refuse_setup_in_capture(stream, "kinematic rows")) return rc;
     std::vector<int64_t> rows, cols;
     std::vector<int32_t> map;
     kin_structure(p, rows, cols, map);
@@ -864,13 +978,12 @@ int ensure_kin(const Problem& p, DeviceState& ds)
 int launch_kin(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* io, cudaStream_t stream)
 {
     const QlClass& c = p.cls;
-    if (int rc = ensure_kin(p, ds)) return rc;
+    if (int rc = ensure_kin(p, ds, stream)) return rc;
     qlnlp_batch_io d = *io;
     const int64_t lds = (std_nnz(p) + 1) & ~1;
+    bool owned = false;
     if (io->jac) {
-        if (int rc = grow_scratch(ds.kin_scratch[stream], stream, (size_t)(B * lds),
-                                  "kinematic rows: the scratch would have to grow during a graph capture", &d.jac))
-            return rc;
+        if (int rc = launch_scratch(ds.kin_scratch, stream, (size_t)(B * lds), &d.jac, &owned)) return rc;
         d.ldjac = lds;
     }
     if (int rc = launch(p, ds, B, &d, stream)) return rc;
@@ -887,7 +1000,7 @@ int launch_kin(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_i
             ds.d_kin_map, nnz_out, d.jac, lds, io->Z, io->ldz, io->jac, io->ldjac, B);
         CUDA_TRY(cudaGetLastError());
     }
-    return QLNLP_OK;
+    return end_scratch(d.jac, owned, stream);
 }
 
 // ---- Lagrangian Hessian ----------------------------------------------------------------------------------------
@@ -1034,9 +1147,10 @@ int check_kkt(const Problem& p, int64_t B, const qlnlp_kkt_io* io)
 // Per-value tables of the kernel, from the host structures: for every SPARSE_TRUE value its slot in the local Jacobian
 // of its knot (ql::kkt_slot_row) and its column inside the knot; then for every Hessian value its row and column inside
 // the knot (lower triangle).
-int ensure_kkt_tables(const Problem& p, DeviceState& ds)
+int ensure_kkt_tables(const Problem& p, DeviceState& ds, cudaStream_t stream)
 {
     if (ds.d_kkt_tab) return QLNLP_OK;
+    if (int rc = refuse_setup_in_capture(stream, "KKT solve")) return rc;
     const QlClass& c = p.cls;
     const int nh = ql_hess_nnz(c);
     std::vector<int64_t> rows(std::max(c.nnz_true, nh)), cols(rows.size());
@@ -1063,16 +1177,16 @@ int ensure_kkt_tables(const Problem& p, DeviceState& ds)
 int launch_kkt(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_kkt_io* io, cudaStream_t stream)
 {
     const QlClass& c = p.cls;
-    if (int rc = ensure_kkt_tables(p, ds)) return rc;
+    if (int rc = ensure_kkt_tables(p, ds, stream)) return rc;
     const KernelSpec k = kkt_spec();
     int per_sm = 0;
     if (int rc = kernel_geometry(ds, k, &per_sm)) return rc;
     // the scratch holds one factor per resident warp (the most a launch of any B uses)
     ql::KktLaunch P;
     std::memset(&P, 0, sizeof P);
-    if (int rc = grow_scratch(ds.kkt_scratch[stream], stream, (size_t)ds.sm_count * per_sm * c.N * ql::KKT_FSTRIDE,
-                              "KKT solve: the factor scratch of this stream would have to be allocated during a graph capture",
-                              &P.scratch))
+    bool owned = false;
+    if (int rc = launch_scratch(ds.kkt_scratch, stream, (size_t)ds.sm_count * per_sm * c.N * ql::KKT_FSTRIDE, &P.scratch,
+                                &owned))
         return rc;
     P.c = c;
     P.jtab = ds.d_kkt_tab;
@@ -1087,7 +1201,8 @@ int launch_kkt(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_kkt_io*
     P.pl = io->pl; P.ldpl = io->ldpl;
     P.status = io->status;
     P.B = B;
-    return launch_kernel(ds, k, B, P, stream);
+    if (int rc = launch_kernel(ds, k, B, P, stream)) return rc;
+    return end_scratch(P.scratch, owned, stream);
 }
 
 // A row of a single call: n doubles, copied in from `in` before the launch and / or back to `out` after it
@@ -1112,7 +1227,7 @@ int single_call(qlnlp_handle h, std::initializer_list<Row> rows, const char* wha
     size_t total = 0;
     int i = 0;
     for (const Row& r : rows) total += ld[i++] = (r.n + 1) & ~1;
-    if (int rc = grow_scratch(ds.one.slots, s, total, what, &slot[0])) return rc;
+    if (int rc = grow_scratch(ds.one.slots, total, &slot[0])) return rc;
     cudaError_t e = cudaSuccess;
     i = 0;
     for (const Row& r : rows) {
@@ -1820,7 +1935,7 @@ int qlnlp_eval_batch_device(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io,
     if (int rc = check_batch(h->prob, B, io, nullptr)) return rc;
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
-    if (int rc = ensure_device(h->prob, ds)) return rc;
+    if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
     if (h->prob.kin) return launch_kin(h->prob, ds, B, io, static_cast<cudaStream_t>(stream));
     return launch(h->prob, ds, B, io, static_cast<cudaStream_t>(stream));
 }
@@ -1837,8 +1952,8 @@ int qlnlp_eval_batch_device_multi(qlnlp_handle h, const int64_t* B, const qlnlp_
         DeviceState& ds = h->devs[i];
         if (B[i] == 0) continue;
         DeviceGuard guard(ds.device);
-        if (int rc = ensure_device(p, ds)) return rc;
         cudaStream_t st = streams ? static_cast<cudaStream_t>(streams[i]) : nullptr;
+        if (int rc = ensure_device(p, ds, st)) return rc;
         if (int rc = p.kin ? launch_kin(p, ds, B[i], io + i, st) : launch(p, ds, B[i], io + i, st)) return rc;
     }
     return QLNLP_OK;
@@ -1865,9 +1980,9 @@ int qlnlp_eval_ragged_device(qlnlp_handle h, int64_t B, const qlnlp_batch_io* io
     if (int rc = check_batch(h->prob, B, io, rg)) return rc;
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
-    if (int rc = ensure_device(h->prob, ds)) return rc;
+    if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
     const RagTable* table = nullptr;
-    if (int rc = ragged_table(&h, 1, &table)) return rc;
+    if (int rc = ragged_table(&h, 1, static_cast<cudaStream_t>(stream), &table)) return rc;
     return launch(h->prob, ds, B, io, static_cast<cudaStream_t>(stream), -1, rg, table, nullptr);
 }
 
@@ -1888,9 +2003,9 @@ int qlnlp_eval_ragged_classes(const qlnlp_handle* hs, int ncls, int64_t B, const
     if (int rc = check_batch(hs[0]->prob, B, io, rg)) return rc;
     DeviceGuard guard(hs[0]->devs[0].device);
     for (int i = 0; i < ncls; ++i)
-        if (int rc = ensure_device(hs[i]->prob, hs[i]->devs[0])) return rc;
+        if (int rc = ensure_device(hs[i]->prob, hs[i]->devs[0], static_cast<cudaStream_t>(stream))) return rc;
     const RagTable* table = nullptr;
-    if (int rc = ragged_table(hs, ncls, &table)) return rc;
+    if (int rc = ragged_table(hs, ncls, static_cast<cudaStream_t>(stream), &table)) return rc;
     return launch(hs[0]->prob, hs[0]->devs[0], B, io, static_cast<cudaStream_t>(stream), -1, rg, table, class_of);
 }
 
@@ -2112,7 +2227,7 @@ int qlnlp_eval_hessian_batch_device(qlnlp_handle h, int64_t B, const double* Z, 
     if (int rc = check_hessian(h->prob, B, Z, ldz, lambda, ldlambda, H, ldh, ql_hess_nnz(h->prob.cls))) return rc;
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
-    if (int rc = ensure_device(h->prob, ds)) return rc;
+    if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
     return launch_hessian(h->prob, ds, B, Z, ldz, sigma, 1.0, lambda, ldlambda, H, ldh, static_cast<cudaStream_t>(stream));
 }
 
@@ -2139,7 +2254,7 @@ int qlnlp_eval_jacobian_products_batch_device(qlnlp_handle h, int64_t B, const q
     if (int rc = check_products(h->prob, B, io, pv)) return rc;
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
-    if (int rc = ensure_device(h->prob, ds)) return rc;
+    if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
     return launch_products(h->prob, ds, B, io, pv, static_cast<cudaStream_t>(stream));
 }
 
@@ -2154,7 +2269,7 @@ int qlnlp_eval_hessian_product_batch_device(qlnlp_handle h, int64_t B, const dou
     if (int rc = check_hess_products(h->prob, B, Z, ldz, lambda, ldlambda, V, ldv, HV, ldhv)) return rc;
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
-    if (int rc = ensure_device(h->prob, ds)) return rc;
+    if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
     return launch_hess_products(h->prob, ds, B, Z, ldz, sigma, 1.0, lambda, ldlambda, V, ldv, HV, ldhv,
                                 static_cast<cudaStream_t>(stream));
 }
@@ -2170,7 +2285,7 @@ int qlnlp_kkt_solve_batch_device(qlnlp_handle h, int64_t B, const qlnlp_kkt_io* 
     if (int rc = check_kkt(h->prob, B, io)) return rc;
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
-    if (int rc = ensure_device(h->prob, ds)) return rc;
+    if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
     return launch_kkt(h->prob, ds, B, io, static_cast<cudaStream_t>(stream));
 }
 
@@ -2231,7 +2346,7 @@ int qlnlp_initial_guess_batch_device(qlnlp_handle h, int64_t B, const double* ba
     DeviceState& ds = h->devs[0];
     if (ldz < c.n_nlp) return fail(QLNLP_EINVAL, "ldz < n_nlp");
     DeviceGuard guard(ds.device);
-    if (int rc = ensure_device(h->prob, ds)) return rc;
+    if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
     const long long total = (long long)B * c.n_nlp;
     const int threads = 256;
     ql::initial_guess_kernel<<<(unsigned)((total + threads - 1) / threads), threads, 0, static_cast<cudaStream_t>(stream)>>>(
