@@ -168,31 +168,41 @@ def test_ragged_classes_with_their_own_tables_and_states():
                   sample_knots(p.N, p.k_trans))
 
 
-def test_hessian_batch(rnd):
+def test_hessian_batch(rnd, monkeypatch):
     """sigma given and default (1); an output with odd leading dimension (plain stores) and an even one, both with
-    guard rows; lambda rows wider than m_nlp; and the single host-pointer call."""
+    guard rows; lambda rows wider than m_nlp; and the single host-pointer call.  Both division instantiations: one
+    handle created without QLNLP_IEEE_DIV and one with it (the variable is read once, when a handle is created)."""
     p, Z, _, _ = rnd
-    nlp = ql.HybridNLP.from_problem(p, hessian=True)
-    rows, cols = nlp.hessian_structure_arrays()
-    B, guard, sentinel, nh = 6, 2, -7.25, nlp.nnz_hess
+    nlps = []
+    for ieee_div in (False, True):
+        monkeypatch.delenv("QLNLP_IEEE_DIV", raising=False)
+        if ieee_div:
+            monkeypatch.setenv("QLNLP_IEEE_DIV", "1")
+        nlps.append(ql.HybridNLP.from_problem(p, hessian=True))
+    monkeypatch.delenv("QLNLP_IEEE_DIV", raising=False)
+    B, guard, sentinel = 6, 2, -7.25
     rng = np.random.default_rng(9)
     lam_wide = dev(rng.standard_normal((B, p.m_nlp + 3)))
     lam = lam_wide[:, :p.m_nlp]                                  # ldlambda = m_nlp + 3
     sigma = rng.uniform(0.3, 1.7, size=B)
     knots = hess_knots(p.N, p.k_trans) + [5, 17]
     m = model(p, ("rnd", 1), x0=p.x0, xf=p.xf)
-    for sig in (sigma, None):
-        for pad in (nh % 2 + 1, 2 - nh % 2):                     # odd and even leading dimension
-            big = torch.full((B + 2 * guard, nh + pad), sentinel, dtype=torch.float64, device="cuda")
-            H = nlp.eval_hessian_batch(dev(Z[:B]), lam, None if sig is None else dev(sig), out=big[guard:guard + B, :nh])
-            torch.cuda.synchronize()
-            assert bool((big[:guard] == sentinel).all()) and bool((big[guard + B:] == sentinel).all())
-            assert bool((big[:, nh:] == sentinel).all()) and not bool((H == sentinel).any())
-            s = 1.0 if sig is None else sig[1]
-            check_hess(m, Z[1], s, lam[1].cpu().numpy(), H[1].cpu().numpy(), rows, cols, knots)
-    vals = np.empty(nh)
-    nlp.eval_hessian_lagrangian(vals, Z[1], sigma[1], lam[1].cpu().numpy())
-    check_hess(m, Z[1], sigma[1], lam[1].cpu().numpy(), vals, rows, cols, knots)
+    for nlp in nlps:
+        rows, cols = nlp.hessian_structure_arrays()
+        nh = nlp.nnz_hess
+        for sig in (sigma, None):
+            for pad in (nh % 2 + 1, 2 - nh % 2):                 # odd and even leading dimension
+                big = torch.full((B + 2 * guard, nh + pad), sentinel, dtype=torch.float64, device="cuda")
+                H = nlp.eval_hessian_batch(dev(Z[:B]), lam, None if sig is None else dev(sig),
+                                           out=big[guard:guard + B, :nh])
+                torch.cuda.synchronize()
+                assert bool((big[:guard] == sentinel).all()) and bool((big[guard + B:] == sentinel).all())
+                assert bool((big[:, nh:] == sentinel).all()) and not bool((H == sentinel).any())
+                s = 1.0 if sig is None else sig[1]
+                check_hess(m, Z[1], s, lam[1].cpu().numpy(), H[1].cpu().numpy(), rows, cols, knots)
+        vals = np.empty(nh)
+        nlp.eval_hessian_lagrangian(vals, Z[1], sigma[1], lam[1].cpu().numpy())
+        check_hess(m, Z[1], sigma[1], lam[1].cpu().numpy(), vals, rows, cols, knots)
 
 
 LARGE = [(128, 33, 1), (129, 129, 2), (257, 100, 1), (1024, 2, 2), (1024, 1000, 1)]

@@ -455,6 +455,26 @@ def test_non_finite_inputs_do_not_crash_and_stay_local(dflt):
     assert_same_bits(nlp, {k: v[clean] for k, v in got.items()}, {k: v[clean] for k, v in ref.items()})
     assert np.isnan(got["f"][3]) and np.isnan(got["g"][3]).any() and not np.isfinite(got["f"][5])
     assert np.isfinite(got["g"][3]).sum() > 900          # only the rows that touch knot 10/11 are affected
+    # B = 16,384: every resident warp evaluates several rows, clean ones after poisoned ones.  NaN or Inf in one entry
+    # of every fifth row; the clean rows must be the bits of a batch of the clean rows alone, in every value stream
+    # (none: no Jacobian; SPARSE_BLOCK; SPARSE_TRUE)
+    B = 16384
+    gen = torch.Generator(device="cuda").manual_seed(3)
+    Zd = torch.from_numpy(ql.initial_guess(p)).cuda().repeat(B, 1)
+    Zd += 1e-2 * torch.randn(Zd.shape, generator=gen, dtype=torch.float64, device="cuda")
+    Zd[:, 19::20].clamp_(1e-3, 2e-2)
+    bad = np.arange(4, B, 5)
+    for j, b in enumerate(bad.tolist()):
+        Zd[b, (20 * ((7 * j) % p.N) + j % 20) % p.n_nlp] = np.nan if j % 2 else np.inf
+    clean = torch.from_numpy(np.setdiff1d(np.arange(B), bad)).cuda()
+    true = ql.HybridNLP.from_problem(p, pattern="true")
+    for h, want in ((nlp, ("f", "grad", "g")), (nlp, ("f", "grad", "g", "jac")), (true, ("f", "grad", "g", "jac"))):
+        got, alone = h.eval_batch(Zd, want=want), h.eval_batch(Zd[clean], want=want)
+        torch.cuda.synchronize()
+        assert not bool(torch.isfinite(got["f"][torch.from_numpy(bad).cuda()]).any())
+        for k in want:
+            a, c = got[k][clean].contiguous(), alone[k].contiguous()
+            assert bool(torch.isfinite(c).all()) and torch.equal(a.view(torch.int64), c.view(torch.int64)), (want, k)
 
 
 def test_handles_of_different_sizes_coexist():

@@ -62,11 +62,16 @@ def test_unit_vectors_rebuild_the_matrices(N, kt, im):
     assert np.array_equal(hv.T, H)
 
 
+@pytest.mark.parametrize("ieee_div", [False, True])
 @pytest.mark.parametrize("N,kt,im", [(61, 21, 1), (65, 2, 1), (129, 129, 2), (257, 100, 1), (1024, 1000, 1)])
-def test_random_directions_are_the_fold_of_the_materialised_values(N, kt, im):
+def test_random_directions_are_the_fold_of_the_materialised_values(N, kt, im, ieee_div, monkeypatch):
     B = 6
     p, Z = _setup(N, kt, im, B, seed=3)
+    monkeypatch.delenv("QLNLP_IEEE_DIV", raising=False)
+    if ieee_div:
+        monkeypatch.setenv("QLNLP_IEEE_DIV", "1")
     nlp = ql.HybridNLP.from_problem(p, pattern="true", hessian=True, products=True)
+    monkeypatch.delenv("QLNLP_IEEE_DIV", raising=False)      # read once, when the handle is created
     rng = np.random.default_rng(N)
     w, y, v, lam = (rng.standard_normal((B, d)) for d in (nlp.n_nlp, nlp.m_nlp, nlp.n_nlp, nlp.m_nlp))
     sigma = rng.uniform(0.3, 1.7, B)
