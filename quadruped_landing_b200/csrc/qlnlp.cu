@@ -54,6 +54,62 @@ int fail(int code, const char* fmt, ...)
                         cudaGetErrorString(e_), __FILE__, __LINE__);                                \
     } while (0)
 
+// Owners of what a handle holds on the device.  device_alloc / pinned_alloc count a block in, its deleter counts it out.
+std::atomic<int> g_owned_blocks{0};
+std::atomic<int64_t> g_fail_alloc{-1};  // tests: allocations to go before one fails as out of memory (negative: none)
+struct CudaFree { void operator()(void* p) const { cudaFree(p); --g_owned_blocks; } };
+struct CudaFreeHost { void operator()(void* p) const { cudaFreeHost(p); --g_owned_blocks; } };
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+template <typename T> using DevPtr = std::unique_ptr<T, CudaFree>;
+template <typename T> using PinnedPtr = std::unique_ptr<T, CudaFreeHost>;
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamDestroy>;
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventDestroy>;
+
+// A failed allocation, mapped as CUDA_TRY maps it; an out-of-memory must not linger as the thread's last error.
+int alloc_failed(cudaError_t e, const char* what, size_t bytes)
+{
+    cudaGetLastError();
+    return fail(e == cudaErrorMemoryAllocation ? QLNLP_ENOMEM : QLNLP_ECUDA, "%s of %zu bytes: %s", what, bytes,
+                cudaGetErrorString(e));
+}
+
+template <typename T>
+int device_alloc(DevPtr<T>& out, size_t n)
+{
+    void* p = nullptr;
+    const cudaError_t e = g_fail_alloc.fetch_sub(1) == 0 ? cudaErrorMemoryAllocation : cudaMalloc(&p, sizeof(T) * n);
+    if (e != cudaSuccess) return alloc_failed(e, "cudaMalloc", sizeof(T) * n);
+    ++g_owned_blocks;
+    out.reset(static_cast<T*>(p));
+    return QLNLP_OK;
+}
+
+template <typename T>
+int pinned_alloc(PinnedPtr<T>& out, size_t n, unsigned flags)
+{
+    void* p = nullptr;
+    const cudaError_t e = g_fail_alloc.fetch_sub(1) == 0 ? cudaErrorMemoryAllocation : cudaHostAlloc(&p, sizeof(T) * n, flags);
+    if (e != cudaSuccess) return alloc_failed(e, "cudaHostAlloc", sizeof(T) * n);
+    ++g_owned_blocks;
+    out.reset(static_cast<T*>(p));
+    return QLNLP_OK;
+}
+
+// A device copy of n values, handed to `out` only once complete: a table is either absent or valid.  The copy may still
+// be in flight when cudaMemcpy returns (pageable source) and launches go to any stream, so `sync` waits for the device
+// before the hand-over; a set-up of several tables waits once, after the last.
+template <typename T>
+int upload(DevPtr<T>& out, const T* src, size_t n, bool sync = true)
+{
+    DevPtr<T> d;
+    if (int rc = device_alloc(d, n)) return rc;
+    CUDA_TRY(cudaMemcpy(d.get(), src, sizeof(T) * n, cudaMemcpyHostToDevice));
+    if (sync) CUDA_TRY(cudaDeviceSynchronize());
+    out = std::move(d);
+    return QLNLP_OK;
+}
+
 constexpr int TICKET_POOL = 64;       // work counters of streams (recycled once every one is taken)
 constexpr int GRAPH_TICKETS = 1024;   // work counters of captured graphs (each held until its graph is destroyed)
 constexpr int NJM = 4;                 // kernel value streams: JM_NONE, JM_BLOCK, JM_TRUE, JM_VALS
@@ -77,24 +133,24 @@ struct DeviceGuard {
 
 // per-stream scratch of the host-pointer pipeline
 struct HostLane {
-    cudaStream_t stream = nullptr;
-    cudaEvent_t done = nullptr; // the chunk's last copy has landed
+    Stream stream;
+    Event done;                 // the chunk's last copy has landed
     int64_t cap = 0;            // evaluations the buffers hold
-    double *Z = nullptr, *x0 = nullptr, *xf = nullptr, *f = nullptr, *grad = nullptr, *g = nullptr, *jac = nullptr;
-    double* stage = nullptr;    // pinned host rows of VALS values awaiting the row builder
+    DevPtr<double> Z, x0, xf, f, grad, g, jac;
+    PinnedPtr<double> stage;    // host rows of VALS values awaiting the row builder
 };
 
 // device memory that only grows (per-stream scratch, single-call slots)
 struct Scratch {
-    double* ptr = nullptr;
+    DevPtr<double> ptr;
     size_t cap = 0;             // doubles
 };
 
 // single evaluations (the four MOI callbacks): one launch per decision vector, results cached
 struct OneEval {
-    cudaStream_t stream = nullptr;
+    Stream stream;
     Scratch slots;              // device rows of the other single calls (single_call)
-    double* hx = nullptr;       // pinned, mapped: x(ldz_e) | f(2) grad(ldgrad_e) g(ldg_e) vals(ldv_e)
+    PinnedPtr<double> hx;       // mapped: x(ldz_e) | f(2) grad(ldgrad_e) g(ldg_e) vals(ldv_e)
     double* hout = nullptr;
     double* mx = nullptr;       // device-side addresses of hx / hout: the kernel reads x and writes the results there
     double* mout = nullptr;
@@ -109,8 +165,7 @@ struct Registration {
 
 // class table of a ragged launch (device copy of one QlRagClass per handle)
 struct RagTable {
-    ql::QlRagClass* d_classes = nullptr;
-    int ncls = 0;
+    DevPtr<unsigned char> d_classes;   // QL_RAGCLASS_BYTES per class
     QlClass layout;                    // the class with the largest N: sizes the shared-memory carve-up
     bool fastdiv = false;
 };
@@ -122,7 +177,7 @@ struct Problem {
     // opt-in kinematic rows (qlnlp_kin.cuh): 2N more constraints, 8N more entries in either sparse pattern
     bool kin = false;
     double leg_reach = 0;              // l1 + l2 + lb/2
-    double x0[QL_NX], xf[QL_NX];
+    double x0xf[2 * QL_NX];            // x0 | xf
     std::vector<double> cost;          // field-major [QL_NCOST][npad]
     int npad = 0;
     std::vector<QlSeg> segs;
@@ -165,22 +220,21 @@ struct DeviceState {
     int sm_count = 0;
     size_t smem_per_sm = 0, smem_optin = 0;
     std::map<std::pair<const void*, size_t>, int> blocks_per_sm;   // (kernel, dynamic smem) -> resident CTAs (kernel_geometry)
-    double* d_cost = nullptr;
-    double* d_x0xf = nullptr;          // x0[15] | xf[15]
-    QlSeg* d_segs = nullptr;
-    int* d_seg_begin = nullptr;
-    long long* d_dense_lin = nullptr;  // DENSE mode: linear index of every SPARSE_BLOCK value
-    double* d_dense = nullptr;         // DENSE mode: m x n grid
+    DevPtr<double> d_cost;
+    DevPtr<double> d_x0xf;             // x0[15] | xf[15]
+    DevPtr<QlSeg> d_segs;
+    DevPtr<int> d_seg_begin;
+    DevPtr<long long> d_dense_lin;     // DENSE mode: linear index of every SPARSE_BLOCK value
     HostLane lanes[MAX_LANES];
     OneEval one;
     std::map<cudaStream_t, unsigned*> tickets;   // work counters, one pair per stream the device has launched on
-    unsigned* ticket_pool = nullptr;             // pre-zeroed counters (128 B apart) so that a launch needs no
+    DevPtr<unsigned> ticket_pool;                // pre-zeroed counters (128 B apart) so that a launch needs no
     int ticket_pool_used = 0;                    // allocation: launches stay legal inside CUDA-graph capture
     std::shared_ptr<GraphTickets> graph_tickets; // the counters after the TICKET_POOL stream counters
-    int* d_kin_map = nullptr;          // caller-visible value order of the batch pattern -> scratch position or -(entry + 1)
+    DevPtr<int> d_kin_map;             // caller-visible value order of the batch pattern -> scratch position or -(entry + 1)
     std::map<cudaStream_t, Scratch> kin_scratch;                 // per stream: reference-order rows (device)
     std::map<std::vector<uint64_t>, RagTable> rag_tables;       // ragged launches led by this handle (key: the classes' serials)
-    unsigned short* d_kkt_tab = nullptr;   // KKT solve: slot / column of every SPARSE_TRUE value, then row / column of every W value
+    DevPtr<unsigned short> d_kkt_tab;  // KKT solve: slot / column of every SPARSE_TRUE value, then row / column of every W value
     std::map<cudaStream_t, Scratch> kkt_scratch;                 // per stream: factor scratch of every resident warp
     int64_t last_launch[5] = {0, 0, 0, 0, 0};
     std::unique_ptr<qlhost::Pool> pool;                                  // row builders of the host-pointer path
@@ -594,12 +648,14 @@ int refuse_setup_in_capture(cudaStream_t stream, const char* what)
                 "handle with one such call outside the capture before capturing", what);
 }
 
-// Binds one device of a handle (first call: tables, occupancy, streams).  The caller holds a DeviceGuard.  `stream`:
-// the stream the call launches on (set-up is refused while it is being captured).
-int ensure_device(const Problem& p, DeviceState& ds, cudaStream_t stream = nullptr)
+// Binds one device of a handle (first call: tables, occupancy, streams), all or nothing: a failed set-up releases what
+// it made (`state` is replaced once the set-up is complete).  The caller holds a DeviceGuard.  `stream`: the stream the
+// call launches on (set-up is refused while it is being captured).
+int ensure_device(const Problem& p, DeviceState& state, cudaStream_t stream = nullptr)
 {
-    if (ds.ready) return QLNLP_OK;
+    if (state.ready) return QLNLP_OK;
     if (int rc = refuse_setup_in_capture(stream, "set-up of the handle")) return rc;
+    DeviceState ds{state.device};
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
     if (e != cudaSuccess || ndev == 0)
@@ -618,15 +674,10 @@ int ensure_device(const Problem& p, DeviceState& ds, cudaStream_t stream = nullp
     char bus[32] = {0};
     if (cudaDeviceGetPCIBusId(bus, sizeof bus, ds.device) == cudaSuccess) ds.pci_bus_id = bus;
 
-    CUDA_TRY(cudaMalloc(&ds.d_cost, p.cost.size() * sizeof(double)));
-    CUDA_TRY(cudaMemcpy(ds.d_cost, p.cost.data(), p.cost.size() * sizeof(double), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMalloc(&ds.d_x0xf, 2 * QL_NX * sizeof(double)));
-    CUDA_TRY(cudaMemcpy(ds.d_x0xf, p.x0, QL_NX * sizeof(double), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(ds.d_x0xf + QL_NX, p.xf, QL_NX * sizeof(double), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMalloc(&ds.d_segs, p.segs.size() * sizeof(QlSeg)));
-    CUDA_TRY(cudaMemcpy(ds.d_segs, p.segs.data(), p.segs.size() * sizeof(QlSeg), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMalloc(&ds.d_seg_begin, p.seg_begin.size() * sizeof(int)));
-    CUDA_TRY(cudaMemcpy(ds.d_seg_begin, p.seg_begin.data(), p.seg_begin.size() * sizeof(int), cudaMemcpyHostToDevice));
+    if (int rc = upload(ds.d_cost, p.cost.data(), p.cost.size(), false)) return rc;
+    if (int rc = upload(ds.d_x0xf, p.x0xf, 2 * QL_NX, false)) return rc;
+    if (int rc = upload(ds.d_segs, p.segs.data(), p.segs.size(), false)) return rc;
+    if (int rc = upload(ds.d_seg_begin, p.seg_begin.data(), p.seg_begin.size(), false)) return rc;
 
     // the eval kernels' attributes are set here, at the first evaluation, whatever the handle launches later
     for (int wj = 0; wj < NJM; ++wj)
@@ -634,19 +685,24 @@ int ensure_device(const Problem& p, DeviceState& ds, cudaStream_t stream = nullp
             int nb = 0;
             if (int rc = kernel_geometry(ds, eval_spec(p.cls.N, wj, p.fastdiv, rg != 0), &nb)) return rc;
         }
+    cudaStream_t s = nullptr;
+    cudaEvent_t ev = nullptr;
     for (auto& ln : ds.lanes) {
-        CUDA_TRY(cudaStreamCreateWithFlags(&ln.stream, cudaStreamNonBlocking));
-        CUDA_TRY(cudaEventCreateWithFlags(&ln.done, cudaEventDisableTiming));
+        CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+        ln.stream.reset(s);
+        CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+        ln.done.reset(ev);
     }
-    CUDA_TRY(cudaStreamCreateWithFlags(&ds.one.stream, cudaStreamNonBlocking));
-    CUDA_TRY(cudaMalloc(&ds.ticket_pool, 128 * (TICKET_POOL + GRAPH_TICKETS)));
-    CUDA_TRY(cudaMemset(ds.ticket_pool, 0, 128 * (TICKET_POOL + GRAPH_TICKETS)));
+    CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    ds.one.stream.reset(s);
+    if (int rc = device_alloc(ds.ticket_pool, 32 * (TICKET_POOL + GRAPH_TICKETS))) return rc;
+    CUDA_TRY(cudaMemset(ds.ticket_pool.get(), 0, 128 * (TICKET_POOL + GRAPH_TICKETS)));
     ds.graph_tickets = std::make_shared<GraphTickets>();
     for (int i = TICKET_POOL + GRAPH_TICKETS - 1; i >= TICKET_POOL; --i) ds.graph_tickets->free.push_back(i);
-    // the set-up copies above ran on the legacy default stream and may still be in flight when cudaMemcpy returns
-    // (pageable source); launches go to arbitrary, possibly non-blocking streams, so finish the set-up first
-    CUDA_TRY(cudaDeviceSynchronize());
+    CUDA_TRY(cudaDeviceSynchronize());         // the set-up copies (upload)
     ds.ready = true;
+    ds.pool = std::move(state.pool);           // row builders started before the set-up (qlnlp_host_output_register)
+    state = std::move(ds);
     return QLNLP_OK;
 }
 
@@ -666,12 +722,12 @@ int stream_ticket(DeviceState& ds, cudaStream_t stream, unsigned** out)
             if (cap != cudaStreamCaptureStatusNone)
                 return fail(QLNLP_EINVAL, "more than %d streams used with this handle: cannot recycle work counters during a graph capture", TICKET_POOL);
             CUDA_TRY(cudaDeviceSynchronize());
-            CUDA_TRY(cudaMemset(ds.ticket_pool, 0, 128 * TICKET_POOL));
+            CUDA_TRY(cudaMemset(ds.ticket_pool.get(), 0, 128 * TICKET_POOL));
             CUDA_TRY(cudaDeviceSynchronize());
             ds.tickets.clear();
             ds.ticket_pool_used = 0;
         }
-        unsigned* d = ds.ticket_pool + 32 * ds.ticket_pool_used++;      // zeroed (and synchronised) at set-up
+        unsigned* d = ds.ticket_pool.get() + 32 * ds.ticket_pool_used++;      // zeroed (and synchronised) at set-up
         it = ds.tickets.emplace(stream, d).first;
     }
     *out = it->second;
@@ -696,7 +752,7 @@ int launch_ticket(DeviceState& ds, cudaStream_t stream, unsigned** out)
         std::lock_guard<std::mutex> lk(gt.mu);
         auto it = gt.live.find(key);
         if (it != gt.live.end()) {
-            *out = ds.ticket_pool + 32 * it->second;
+            *out = ds.ticket_pool.get() + 32 * it->second;
             return QLNLP_OK;
         }
         if (gt.free.empty())
@@ -723,7 +779,7 @@ int launch_ticket(DeviceState& ds, cudaStream_t stream, unsigned** out)
         cudaUserObjectRelease(obj, 1);
         return fail(QLNLP_ECUDA, "cudaGraphRetainUserObject: %s", cudaGetErrorString(e));
     }
-    *out = ds.ticket_pool + 32 * index;
+    *out = ds.ticket_pool.get() + 32 * index;
     return QLNLP_OK;
 }
 
@@ -776,11 +832,11 @@ void set_problem(R& P, const Problem& p, const DeviceState& ds)
 {
     P.c = p.cls;
     P.rmb = p.rmb; P.rmf = p.rmf; P.rIb = p.rIb;
-    P.cost = ds.d_cost;
+    P.cost = ds.d_cost.get();
     P.npad = p.npad;
     if constexpr (std::is_base_of<ql::Launch, R>::value) {
-        P.x0_def = ds.d_x0xf;
-        P.xf_def = ds.d_x0xf + QL_NX;
+        P.x0_def = ds.d_x0xf.get();
+        P.xf_def = ds.d_x0xf.get() + QL_NX;
     }
 }
 
@@ -789,15 +845,12 @@ void set_problem(R& P, const Problem& p, const DeviceState& ds)
 int grow_scratch(Scratch& sc, size_t n, double** out)
 {
     if (sc.cap < n) {
-        if (sc.ptr) {
-            CUDA_TRY(cudaDeviceSynchronize());      // earlier launches may still use it
-            cudaFree(sc.ptr);
-            sc = Scratch();
-        }
-        CUDA_TRY(cudaMalloc(&sc.ptr, sizeof(double) * n));
+        if (sc.ptr) CUDA_TRY(cudaDeviceSynchronize());      // earlier launches may still use it
+        sc = Scratch();
+        if (int rc = device_alloc(sc.ptr, n)) return rc;
         sc.cap = n;
     }
-    *out = sc.ptr;
+    *out = sc.ptr.get();
     return QLNLP_OK;
 }
 
@@ -861,11 +914,11 @@ int launch(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* i
     ql::Launch P;
     set_problem(P, p, ds);
     if (rg) P.c = table->layout;
-    P.classes = rg ? table->d_classes : nullptr;
+    P.classes = rg ? reinterpret_cast<const ql::QlRagClass*>(table->d_classes.get()) : nullptr;
     P.cls_of = rg ? reinterpret_cast<const int*>(class_of) : nullptr;
     P.nseg = (int)p.segs.size();
-    P.segs = ds.d_segs;
-    P.seg_begin = ds.d_seg_begin;
+    P.segs = ds.d_segs.get();
+    P.seg_begin = ds.d_seg_begin.get();
     P.Z = io->Z; P.ldz = io->ldz;
     P.x0 = io->x0; P.xf = io->xf;
     P.f = io->f;
@@ -903,36 +956,30 @@ int ragged_table(const qlnlp_handle* hs, int ncls, cudaStream_t stream, const Ra
     if (it != lead.rag_tables.end()) { *out = &it->second; return QLNLP_OK; }
     if (int rc = refuse_setup_in_capture(stream, "ragged launch over a new set of classes")) return rc;
     RagTable t;
-    t.ncls = ncls;
     t.fastdiv = true;
     t.layout = hs[0]->prob.cls;
-    std::vector<ql::QlRagClass> host((size_t)ncls);
+    // device records are QL_RAGCLASS_BYTES apart (the kernel copies whole slots)
+    std::vector<unsigned char> packed((size_t)ncls * QL_RAGCLASS_BYTES, 0);
     for (int i = 0; i < ncls; ++i) {
         const Problem& p = hs[i]->prob;
         const DeviceState& ds = hs[i]->devs[0];
-        ql::QlRagClass& r = host[(size_t)i];
+        ql::QlRagClass r;
         std::memset(&r, 0, sizeof r);
         r.c = p.cls;
         r.rmb = p.rmb; r.rmf = p.rmf; r.rIb = p.rIb;
-        r.cost = ds.d_cost;
-        r.x0_def = ds.d_x0xf;
-        r.xf_def = ds.d_x0xf + QL_NX;
-        r.segs = ds.d_segs;
-        r.seg_begin = ds.d_seg_begin;
+        r.cost = ds.d_cost.get();
+        r.x0_def = ds.d_x0xf.get();
+        r.xf_def = ds.d_x0xf.get() + QL_NX;
+        r.segs = ds.d_segs.get();
+        r.seg_begin = ds.d_seg_begin.get();
         r.npad = p.npad;
         r.nseg = (int)p.segs.size();
         t.fastdiv = t.fastdiv && p.fastdiv;
         if (p.cls.N > t.layout.N) t.layout = p.cls;
+        std::memcpy(packed.data() + (size_t)i * QL_RAGCLASS_BYTES, &r, sizeof r);
     }
-    // device records are QL_RAGCLASS_BYTES apart (the kernel copies whole slots)
-    std::vector<unsigned char> packed((size_t)ncls * QL_RAGCLASS_BYTES, 0);
-    for (int i = 0; i < ncls; ++i) std::memcpy(packed.data() + (size_t)i * QL_RAGCLASS_BYTES, &host[(size_t)i], sizeof(ql::QlRagClass));
-    void* d = nullptr;
-    CUDA_TRY(cudaMalloc(&d, packed.size()));
-    CUDA_TRY(cudaMemcpy(d, packed.data(), packed.size(), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaDeviceSynchronize());
-    t.d_classes = static_cast<ql::QlRagClass*>(d);
-    *out = &lead.rag_tables.emplace(key, t).first->second;
+    if (int rc = upload(t.d_classes, packed.data(), packed.size())) return rc;
+    *out = &lead.rag_tables.emplace(key, std::move(t)).first->second;
     return QLNLP_OK;
 }
 
@@ -966,10 +1013,7 @@ int ensure_kin(const Problem& p, DeviceState& ds, cudaStream_t stream)
     std::vector<int64_t> rows, cols;
     std::vector<int32_t> map;
     kin_structure(p, rows, cols, map);
-    CUDA_TRY(cudaMalloc(&ds.d_kin_map, sizeof(int) * map.size()));
-    CUDA_TRY(cudaMemcpy(ds.d_kin_map, map.data(), sizeof(int) * map.size(), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaDeviceSynchronize());
-    return QLNLP_OK;
+    return upload(ds.d_kin_map, map.data(), map.size());
 }
 
 // launch() for a problem with kinematic rows: io describes the CALLER's arrays (g rows of m_nlp + 2N, jac rows of
@@ -997,7 +1041,7 @@ int launch_kin(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_i
         const int nnz_out = batch_nnz(p);
         const long long total = (long long)B * nnz_out;
         ql::kin_expand_kernel<<<(unsigned)((total + threads - 1) / threads), threads, 0, stream>>>(
-            ds.d_kin_map, nnz_out, d.jac, lds, io->Z, io->ldz, io->jac, io->ldjac, B);
+            ds.d_kin_map.get(), nnz_out, d.jac, lds, io->Z, io->ldz, io->jac, io->ldjac, B);
         CUDA_TRY(cudaGetLastError());
     }
     return end_scratch(d.jac, owned, stream);
@@ -1168,10 +1212,7 @@ int ensure_kkt_tables(const Problem& p, DeviceState& ds, cudaStream_t stream)
         const int r = (int)((rows[e] - 1) % QL_NZK), q = (int)((cols[e] - 1) % QL_NZK);
         tab[(size_t)c.nnz_true + e] = (unsigned short)(std::max(r, q) | std::min(r, q) << 8);
     }
-    CUDA_TRY(cudaMalloc(&ds.d_kkt_tab, sizeof(unsigned short) * tab.size()));
-    CUDA_TRY(cudaMemcpy(ds.d_kkt_tab, tab.data(), sizeof(unsigned short) * tab.size(), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaDeviceSynchronize());
-    return QLNLP_OK;
+    return upload(ds.d_kkt_tab, tab.data(), tab.size());
 }
 
 int launch_kkt(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_kkt_io* io, cudaStream_t stream)
@@ -1189,8 +1230,8 @@ int launch_kkt(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_kkt_io*
                                 &owned))
         return rc;
     P.c = c;
-    P.jtab = ds.d_kkt_tab;
-    P.htab = ds.d_kkt_tab + c.nnz_true;
+    P.jtab = ds.d_kkt_tab.get();
+    P.htab = ds.d_kkt_tab.get() + c.nnz_true;
     P.hess = io->hess; P.ldhess = io->ldhess;
     P.jac = io->jac; P.ldjac = io->ldjac;
     P.sx = io->sx; P.ldsx = io->ldsx;
@@ -1221,7 +1262,7 @@ int single_call(qlnlp_handle h, std::initializer_list<Row> rows, const char* wha
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
     if (int rc = ensure_device(h->prob, ds)) return rc;
-    const cudaStream_t s = ds.one.stream;
+    const cudaStream_t s = ds.one.stream.get();
     double* slot[5];
     int64_t ld[5];
     size_t total = 0;
@@ -1247,27 +1288,15 @@ int single_call(qlnlp_handle h, std::initializer_list<Row> rows, const char* wha
     return finish(s, rc, what);
 }
 
-void free_lane(HostLane& ln)
-{
-    if (ln.stage) cudaFreeHost(ln.stage);
-    ln.stage = nullptr;
-    cudaFree(ln.Z); cudaFree(ln.x0); cudaFree(ln.xf); cudaFree(ln.f); cudaFree(ln.grad); cudaFree(ln.g); cudaFree(ln.jac);
-    ln.Z = ln.x0 = ln.xf = ln.f = ln.grad = ln.g = ln.jac = nullptr;
-    ln.cap = 0;
-}
-
 int reserve_lane(const Problem& p, HostLane& ln, int64_t cap)
 {
     if (ln.cap >= cap) return QLNLP_OK;
-    free_lane(ln);
-    CUDA_TRY(cudaMalloc(&ln.Z, sizeof(double) * cap * p.ldz_e));
-    CUDA_TRY(cudaMalloc(&ln.x0, sizeof(double) * cap * QL_NX));
-    CUDA_TRY(cudaMalloc(&ln.xf, sizeof(double) * cap * QL_NX));
-    CUDA_TRY(cudaMalloc(&ln.f, sizeof(double) * cap));
-    CUDA_TRY(cudaMalloc(&ln.grad, sizeof(double) * cap * p.ldgrad_e));
-    CUDA_TRY(cudaMalloc(&ln.g, sizeof(double) * cap * p.ldg_e));
-    CUDA_TRY(cudaMalloc(&ln.jac, sizeof(double) * cap * std::max(p.ldjac_e, p.ldv_e)));
-    CUDA_TRY(cudaHostAlloc(&ln.stage, sizeof(double) * cap * p.ldv_e, cudaHostAllocDefault));
+    ln = HostLane{std::move(ln.stream), std::move(ln.done)};      // the old buffers go before the new ones are made
+    const std::pair<DevPtr<double>*, int64_t> rows[] = {{&ln.Z, p.ldz_e}, {&ln.x0, QL_NX}, {&ln.xf, QL_NX}, {&ln.f, 1},
+        {&ln.grad, p.ldgrad_e}, {&ln.g, p.ldg_e}, {&ln.jac, std::max(p.ldjac_e, p.ldv_e)}};
+    for (auto& r : rows)
+        if (int rc = device_alloc(*r.first, (size_t)(cap * r.second))) return rc;
+    if (int rc = pinned_alloc(ln.stage, (size_t)(cap * p.ldv_e), cudaHostAllocDefault)) return rc;
     ln.cap = cap;
     return QLNLP_OK;
 }
@@ -1334,31 +1363,31 @@ int eval_host_impl(qlnlp_handle h, int dev, int64_t B, const qlnlp_batch_io* io)
         const double t0 = now();
         HostLane& ln = ds.lanes[i % nlanes];
         const int64_t b0 = i * chunk, nb = std::min(chunk, B - b0);
-        cudaStream_t s = ln.stream;
-        CUDA_TRY(copy_rows(ln.Z, ldz_d, io->Z + b0 * io->ldz, io->ldz, c.n_nlp, nb, cudaMemcpyHostToDevice, s));
-        if (io->x0) CUDA_TRY(cudaMemcpyAsync(ln.x0, io->x0 + b0 * QL_NX, sizeof(double) * nb * QL_NX, cudaMemcpyHostToDevice, s));
-        if (io->xf) CUDA_TRY(cudaMemcpyAsync(ln.xf, io->xf + b0 * QL_NX, sizeof(double) * nb * QL_NX, cudaMemcpyHostToDevice, s));
+        cudaStream_t s = ln.stream.get();
+        CUDA_TRY(copy_rows(ln.Z.get(), ldz_d, io->Z + b0 * io->ldz, io->ldz, c.n_nlp, nb, cudaMemcpyHostToDevice, s));
+        if (io->x0) CUDA_TRY(cudaMemcpyAsync(ln.x0.get(), io->x0 + b0 * QL_NX, sizeof(double) * nb * QL_NX, cudaMemcpyHostToDevice, s));
+        if (io->xf) CUDA_TRY(cudaMemcpyAsync(ln.xf.get(), io->xf + b0 * QL_NX, sizeof(double) * nb * QL_NX, cudaMemcpyHostToDevice, s));
         qlnlp_batch_io d;
         std::memset(&d, 0, sizeof d);
-        d.Z = ln.Z; d.ldz = ldz_d;
-        d.x0 = io->x0 ? ln.x0 : nullptr;
-        d.xf = io->xf ? ln.xf : nullptr;
-        d.f = io->f ? ln.f : nullptr;
-        d.grad = io->grad ? ln.grad : nullptr; d.ldgrad = ldgrad_d;
-        d.g = io->g ? ln.g : nullptr; d.ldg = ldg_d;
-        d.jac = io->jac ? ln.jac : nullptr; d.ldjac = compact ? p.ldv_e : ldjac_d;
+        d.Z = ln.Z.get(); d.ldz = ldz_d;
+        d.x0 = io->x0 ? ln.x0.get() : nullptr;
+        d.xf = io->xf ? ln.xf.get() : nullptr;
+        d.f = io->f ? ln.f.get() : nullptr;
+        d.grad = io->grad ? ln.grad.get() : nullptr; d.ldgrad = ldgrad_d;
+        d.g = io->g ? ln.g.get() : nullptr; d.ldg = ldg_d;
+        d.jac = io->jac ? ln.jac.get() : nullptr; d.ldjac = compact ? p.ldv_e : ldjac_d;
         if (int rc = p.kin ? launch_kin(p, ds, nb, &d, s) : launch(p, ds, nb, &d, s, compact ? ql::JM_VALS : -1)) return rc;
         // the staged values go first: the row builder only waits for them, f / grad / g land in the caller's arrays
         // by DMA while it works (the lanes are synchronised before the call returns)
         if (compact) {
-            CUDA_TRY(cudaMemcpyAsync(ln.stage, ln.jac, sizeof(double) * nb * p.ldv_e, cudaMemcpyDeviceToHost, s));
-            CUDA_TRY(cudaEventRecord(ln.done, s));
+            CUDA_TRY(cudaMemcpyAsync(ln.stage.get(), ln.jac.get(), sizeof(double) * nb * p.ldv_e, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(cudaEventRecord(ln.done.get(), s));
         }
-        if (io->f) CUDA_TRY(cudaMemcpyAsync(io->f + b0, ln.f, sizeof(double) * nb, cudaMemcpyDeviceToHost, s));
-        if (io->grad) CUDA_TRY(copy_rows(io->grad + b0 * io->ldgrad, io->ldgrad, ln.grad, ldgrad_d, c.n_nlp, nb, cudaMemcpyDeviceToHost, s));
-        if (io->g) CUDA_TRY(copy_rows(io->g + b0 * io->ldg, io->ldg, ln.g, ldg_d, m_out, nb, cudaMemcpyDeviceToHost, s));
+        if (io->f) CUDA_TRY(cudaMemcpyAsync(io->f + b0, ln.f.get(), sizeof(double) * nb, cudaMemcpyDeviceToHost, s));
+        if (io->grad) CUDA_TRY(copy_rows(io->grad + b0 * io->ldgrad, io->ldgrad, ln.grad.get(), ldgrad_d, c.n_nlp, nb, cudaMemcpyDeviceToHost, s));
+        if (io->g) CUDA_TRY(copy_rows(io->g + b0 * io->ldg, io->ldg, ln.g.get(), ldg_d, m_out, nb, cudaMemcpyDeviceToHost, s));
         if (!compact && io->jac)
-            CUDA_TRY(copy_rows(io->jac + b0 * io->ldjac, io->ldjac, ln.jac, ldjac_d, nnz_b, nb, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(copy_rows(io->jac + b0 * io->ldjac, io->ldjac, ln.jac.get(), ldjac_d, nnz_b, nb, cudaMemcpyDeviceToHost, s));
         ds.stat_t_enqueue += now() - t0;
         return QLNLP_OK;
     };
@@ -1380,14 +1409,14 @@ int eval_host_impl(qlnlp_handle h, int dev, int64_t B, const qlnlp_batch_io* io)
         if (handed == built && handed < enq) {
             HostLane& ln = ds.lanes[handed % nlanes];
             const double t0 = now();
-            cudaError_t q = may_block ? cudaEventSynchronize(ln.done) : cudaEventQuery(ln.done);
+            cudaError_t q = may_block ? cudaEventSynchronize(ln.done.get()) : cudaEventQuery(ln.done.get());
             ds.stat_t_wait += now() - t0;
             if (q == cudaErrorNotReady) return QLNLP_OK;
             if (q != cudaSuccess) return fail(QLNLP_ECUDA, "host pipeline: %s", cudaGetErrorString(q));
             const int64_t b0 = handed * chunk, nb = std::min(chunk, B - b0);
             double* rows = io->jac + b0 * io->ldjac;
             t_build0 = now();
-            h->plan->build_async(ds.pool.get(), ln.stage, p.ldv_e, rows, io->ldjac, nb, touched_only);
+            h->plan->build_async(ds.pool.get(), ln.stage.get(), p.ldv_e, rows, io->ldjac, nb, touched_only);
             ++handed;
             ds.stat_host_rows += nb;
             ds.stat_host_lines += nb * (touched_only ? h->plan->touched_lines((int)((reinterpret_cast<uintptr_t>(rows) >> 3) & 7))
@@ -1405,7 +1434,7 @@ int eval_host_impl(qlnlp_handle h, int dev, int64_t B, const qlnlp_batch_io* io)
     while (built < enq)
         if (int rc = progress(true)) return rc;
     const double t_sync = now();
-    for (int l = 0; l < nlanes; ++l) CUDA_TRY(cudaStreamSynchronize(ds.lanes[l].stream));
+    for (int l = 0; l < nlanes; ++l) CUDA_TRY(cudaStreamSynchronize(ds.lanes[l].stream.get()));
     ds.stat_t_wait += now() - t_sync;
     ds.stat_t_total += now() - t_begin;
     return QLNLP_OK;
@@ -1424,8 +1453,7 @@ int eval_host(qlnlp_handle h, int dev, int64_t B, const qlnlp_batch_io* io)
         // copies into caller-owned host memory (and out of the pinned stage) may still be in flight: finish them
         // before the caller gets its buffers back
         if (ds.pool) ds.pool->finish();
-        for (auto& ln : ds.lanes)
-            if (ln.stream) finish(ln.stream, rc, "host pipeline");
+        for (auto& ln : ds.lanes) finish(ln.stream.get(), rc, "host pipeline");
         cudaGetLastError();
     }
     return rc;
@@ -1464,10 +1492,10 @@ int reserve_one(const Problem& p, OneEval& o)
     o.total = o.o_vals + p.ldv_e;
     // One decision vector is latency-bound: with mapped pinned memory the kernel fetches x and stores its 41 KB of
     // results over PCIe itself, which saves the two copy calls.
-    if (!o.hx) CUDA_TRY(cudaHostAlloc(&o.hx, sizeof(double) * (p.ldz_e + o.total), cudaHostAllocMapped));
-    o.hout = o.hx + p.ldz_e;
+    if (int rc = pinned_alloc(o.hx, (size_t)(p.ldz_e + o.total), cudaHostAllocMapped)) return rc;
+    o.hout = o.hx.get() + p.ldz_e;
     void* dp = nullptr;
-    CUDA_TRY(cudaHostGetDevicePointer(&dp, o.hx, 0));
+    CUDA_TRY(cudaHostGetDevicePointer(&dp, o.hx.get(), 0));
     o.mx = static_cast<double*>(dp);
     o.mout = o.mx + p.ldz_e;
     o.valid = false;
@@ -1506,11 +1534,11 @@ int eval_one(qlnlp_handle h, const double* x, double* f, double* grad, double* g
     if (int rc = ensure_device(p, ds)) return rc;
     OneEval& o = ds.one;
     if (int rc = reserve_one(p, o)) return rc;
-    const bool hit = h->opt_x_cache && o.valid && std::memcmp(o.hx, x, sizeof(double) * c.n_nlp) == 0;
+    const bool hit = h->opt_x_cache && o.valid && std::memcmp(o.hx.get(), x, sizeof(double) * c.n_nlp) == 0;
     if (!hit) {
         o.valid = false;
-        std::memcpy(o.hx, x, sizeof(double) * c.n_nlp);
-        cudaStream_t s = o.stream;
+        std::memcpy(o.hx.get(), x, sizeof(double) * c.n_nlp);
+        cudaStream_t s = o.stream.get();
         qlnlp_batch_io d;
         std::memset(&d, 0, sizeof d);
         d.Z = o.mx; d.ldz = c.n_nlp;                                 // odd ld: plain (non-TMA) loads from host memory
@@ -1532,69 +1560,33 @@ int eval_one(qlnlp_handle h, const double* x, double* f, double* grad, double* g
     return QLNLP_OK;
 }
 
-// DENSE: evaluate SPARSE_BLOCK on the device, scatter into the zeroed m x n grid, copy back
-int eval_dense_jacobian(const Problem& p, DeviceState& ds, const double* x, double* vals)
+// DENSE: evaluate SPARSE_BLOCK (+ the kinematic entries) into a scratch row, scatter it into the zeroed m x n grid
+int eval_dense_jacobian(qlnlp_handle h, const double* x, double* vals)
 {
     if (!x) return fail(QLNLP_EINVAL, "null x");
-    DeviceGuard guard(ds.device);
-    if (int rc = ensure_device(p, ds)) return rc;
-    const QlClass& c = p.cls;
-    const int m = m_rows(p), nz = batch_nnz(p);          // DENSE handles batch in SPARSE_BLOCK (+ the kinematic entries)
-    const size_t dense_n = (size_t)m * c.n_nlp;
-    if (!ds.d_dense_lin) {
-        std::vector<int64_t> rows((size_t)nz), cols((size_t)nz);
-        if (p.kin) { std::vector<int32_t> map; kin_structure(p, rows, cols, map); }
-        else sparse_block_structure(c, rows.data(), cols.data());
-        std::vector<long long> lin((size_t)nz);
-        for (int i = 0; i < nz; ++i) lin[(size_t)i] = (rows[(size_t)i] - 1) + (long long)m * (cols[(size_t)i] - 1);
-        CUDA_TRY(cudaMalloc(&ds.d_dense_lin, sizeof(long long) * nz));
-        CUDA_TRY(cudaMemcpy(ds.d_dense_lin, lin.data(), sizeof(long long) * nz, cudaMemcpyHostToDevice));
-        CUDA_TRY(cudaMalloc(&ds.d_dense, sizeof(double) * dense_n));
-        CUDA_TRY(cudaDeviceSynchronize());     // set-up copy on the default stream before work on the lane's stream
-    }
-    HostLane& ln = ds.lanes[0];
-    if (int rc = reserve_lane(p, ln, 1)) return rc;
-    cudaStream_t s = ln.stream;
-    CUDA_TRY(cudaMemcpyAsync(ln.Z, x, sizeof(double) * c.n_nlp, cudaMemcpyHostToDevice, s));
-    qlnlp_batch_io d;
-    std::memset(&d, 0, sizeof d);
-    d.Z = ln.Z; d.ldz = p.ldz_e;
-    d.jac = ln.jac; d.ldjac = p.ldjac_e;
-    int rc = p.kin ? launch_kin(p, ds, 1, &d, s) : launch(p, ds, 1, &d, s);
-    if (rc == QLNLP_OK) {
-        cudaError_t e = cudaMemsetAsync(ds.d_dense, 0, sizeof(double) * dense_n, s);
-        if (e == cudaSuccess) {
-            ql::scatter_dense_kernel<<<(nz + 255) / 256, 256, 0, s>>>(ln.jac, ds.d_dense_lin, ds.d_dense, nz);
-            e = cudaGetLastError();
-        }
-        if (e == cudaSuccess) e = cudaMemcpyAsync(vals, ds.d_dense, sizeof(double) * dense_n, cudaMemcpyDeviceToHost, s);
-        if (e != cudaSuccess) rc = fail(QLNLP_ECUDA, "dense Jacobian: %s", cudaGetErrorString(e));
-    }
-    return finish(s, rc, "dense Jacobian");
-}
-
-void destroy_device_state(DeviceState& ds)
-{
-    if (!ds.ready) return;
-    DeviceGuard guard(ds.device);
-    cudaDeviceSynchronize();     // launches on caller streams may still use the handle's tables and counters
-    for (auto& ln : ds.lanes) {
-        if (ln.stream) cudaStreamSynchronize(ln.stream);
-        free_lane(ln);
-        if (ln.stream) cudaStreamDestroy(ln.stream);
-        if (ln.done) cudaEventDestroy(ln.done);
-    }
-    if (ds.one.stream) cudaStreamDestroy(ds.one.stream);
-    if (ds.one.hx) cudaFreeHost(ds.one.hx);
-    cudaFree(ds.one.slots.ptr);
-    cudaFree(ds.d_kin_map);
-    for (auto& kv : ds.kin_scratch) cudaFree(kv.second.ptr);
-    cudaFree(ds.d_kkt_tab);
-    for (auto& kv : ds.kkt_scratch) cudaFree(kv.second.ptr);
-    for (auto& kv : ds.rag_tables) cudaFree(kv.second.d_classes);
-    cudaFree(ds.ticket_pool);
-    cudaFree(ds.d_cost); cudaFree(ds.d_x0xf); cudaFree(ds.d_segs); cudaFree(ds.d_seg_begin);
-    cudaFree(ds.d_dense_lin); cudaFree(ds.d_dense);
+    const Problem& p = h->prob;
+    const int m = m_rows(p), nz = batch_nnz(p);
+    const int64_t dense_n = (int64_t)m * p.cls.n_nlp;
+    return single_call(h, {{x, nullptr, p.cls.n_nlp}, {nullptr, vals, dense_n}, {nullptr, nullptr, nz}}, "dense Jacobian",
+                       [&](DeviceState& ds, double* const* d, const int64_t* ld, cudaStream_t s) -> int {
+                           if (!ds.d_dense_lin) {          // the position in the grid of every value
+                               std::vector<int64_t> rows((size_t)nz), cols((size_t)nz);
+                               if (p.kin) { std::vector<int32_t> map; kin_structure(p, rows, cols, map); }
+                               else sparse_block_structure(p.cls, rows.data(), cols.data());
+                               std::vector<long long> lin((size_t)nz);
+                               for (int i = 0; i < nz; ++i) lin[(size_t)i] = (rows[(size_t)i] - 1) + (long long)m * (cols[(size_t)i] - 1);
+                               if (int rc = upload(ds.d_dense_lin, lin.data(), lin.size())) return rc;
+                           }
+                           qlnlp_batch_io io;
+                           std::memset(&io, 0, sizeof io);
+                           io.Z = d[0]; io.ldz = ld[0];
+                           io.jac = d[2]; io.ldjac = ld[2];
+                           if (int rc = p.kin ? launch_kin(p, ds, 1, &io, s) : launch(p, ds, 1, &io, s)) return rc;
+                           CUDA_TRY(cudaMemsetAsync(d[1], 0, sizeof(double) * dense_n, s));
+                           ql::scatter_dense_kernel<<<(nz + 255) / 256, 256, 0, s>>>(d[2], ds.d_dense_lin.get(), d[1], nz);
+                           CUDA_TRY(cudaGetLastError());
+                           return QLNLP_OK;
+                       });
 }
 
 // The problem of `d` on the devices `devices[0 .. ndev)`, which share the host cores.
@@ -1610,8 +1602,8 @@ int create_one(const qlnlp_problem_desc* d, const int* devices, int ndev, int ja
     p.jac_mode = jac_mode & ~QLNLP_WITH_KINEMATICS;
     p.kin = (jac_mode & QLNLP_WITH_KINEMATICS) != 0;
     p.leg_reach = d->model.l1 + d->model.l2 + d->model.lb / 2;
-    std::memcpy(p.x0, d->x0, sizeof p.x0);
-    std::memcpy(p.xf, d->xf, sizeof p.xf);
+    std::memcpy(p.x0xf, d->x0, sizeof d->x0);
+    std::memcpy(p.x0xf + QL_NX, d->xf, sizeof d->xf);
     const QlClass& c = p.cls;
     const int N = c.N;
     p.npad = (N + 31) & ~31;
@@ -1773,11 +1765,7 @@ int device_block_alloc(int device, size_t bytes, bool compressible, void** out)
     if (!(compressible && compressible_alloc(device, bytes, &p, blk))) {
         blk = DeviceBlock{device, bytes, false, false, 0};
         const cudaError_t e = cudaMalloc(&p, bytes);
-        if (e != cudaSuccess) {
-            cudaGetLastError();        // an out-of-memory must not linger as the thread's last error
-            return fail(e == cudaErrorMemoryAllocation ? QLNLP_ENOMEM : QLNLP_ECUDA, "cudaMalloc of %zu bytes: %s", bytes,
-                        cudaGetErrorString(e));
-        }
+        if (e != cudaSuccess) return alloc_failed(e, "cudaMalloc", bytes);
     }
     std::lock_guard<std::mutex> lk(g_blocks_mu);
     g_blocks[reinterpret_cast<uintptr_t>(p)] = blk;
@@ -1822,7 +1810,12 @@ int qlnlp_destroy(qlnlp_handle h)
     if (!h) return QLNLP_OK;
     for (auto& w : h->drivers) w->wait();
     h->drivers.clear();
-    for (DeviceState& ds : h->devs) destroy_device_state(ds);
+    for (DeviceState& ds : h->devs) {
+        if (!ds.ready) continue;       // nothing on the device: a failed set-up releases what it made
+        DeviceGuard guard(ds.device);
+        cudaDeviceSynchronize();       // launches on caller streams may still use the handle's tables and counters
+        ds = DeviceState();
+    }
     delete h;
     return QLNLP_OK;
 }
@@ -2185,6 +2178,11 @@ int qlnlp_debug_refuse_compressible(int n)
     return QLNLP_OK;
 }
 
+/* tests: the n-th device or pinned allocation of a handle from now fails as an out-of-memory cudaMalloc would (n < 0:
+ * none); returns the allocations the previous setting still had to go (-1: none armed).  And the blocks handles own. */
+int qlnlp_debug_fail_alloc(int n) { return (int)std::max<int64_t>(-1, g_fail_alloc.exchange(n < 0 ? -1 : n)); }
+int qlnlp_debug_owned_blocks(void) { return g_owned_blocks.load(); }
+
 int qlnlp_device_alloc_info(const void* ptr, int64_t info[3])
 {
     if (!ptr || !info) return fail(QLNLP_EINVAL, "null argument");
@@ -2350,7 +2348,7 @@ int qlnlp_initial_guess_batch_device(qlnlp_handle h, int64_t B, const double* ba
     const long long total = (long long)B * c.n_nlp;
     const int threads = 256;
     ql::initial_guess_kernel<<<(unsigned)((total + threads - 1) / threads), threads, 0, static_cast<cudaStream_t>(stream)>>>(
-        base, x0, ds.d_x0xf + QL_NX, Z, ldz, B, c.n_nlp, c.k_trans);
+        base, x0, ds.d_x0xf.get() + QL_NX, Z, ldz, B, c.n_nlp, c.k_trans);
     CUDA_TRY(cudaGetLastError());
     return QLNLP_OK;
 }
@@ -2360,7 +2358,7 @@ int qlnlp_eval_all(qlnlp_handle h, const double* x, double* f, double* grad, dou
     if (int rc = check_handle(h)) return rc;
     if (vals && h->prob.jac_mode == QLNLP_JAC_DENSE) {
         if (int rc = eval_one(h, x, f, grad, g, nullptr)) return rc;
-        return eval_dense_jacobian(h->prob, h->devs[0], x, vals);
+        return eval_dense_jacobian(h, x, vals);
     }
     return eval_one(h, x, f, grad, g, vals);
 }
@@ -2388,7 +2386,7 @@ int qlnlp_eval_constraint_jacobian(qlnlp_handle h, const double* x, double* vals
     if (int rc = check_handle(h)) return rc;
     if (!vals) return fail(QLNLP_EINVAL, "null output");
     if (h->prob.jac_mode != QLNLP_JAC_DENSE) return eval_one(h, x, nullptr, nullptr, nullptr, vals);
-    return eval_dense_jacobian(h->prob, h->devs[0], x, vals);
+    return eval_dense_jacobian(h, x, vals);
 }
 
 int qlnlp_launch_info(qlnlp_handle h, int64_t info[5])

@@ -46,7 +46,8 @@ EXPORTED_SYMBOLS = (
     "qlnlp_device_alloc", "qlnlp_device_free", "qlnlp_device_alloc_info",
 )
 _DEBUG_SYMBOLS = ("qlnlp_debug_segments", "qlnlp_debug_vals_map", "qlnlp_debug_build_rows", "qlnlp_debug_host_times",
-                  "qlnlp_debug_launch_geometry", "qlnlp_debug_refuse_compressible")
+                  "qlnlp_debug_launch_geometry", "qlnlp_debug_refuse_compressible", "qlnlp_debug_fail_alloc",
+                  "qlnlp_debug_owned_blocks")
 
 
 class QlnlpError(RuntimeError):
@@ -164,6 +165,8 @@ def load_library(rebuild_if_stale: bool = True):
     L.qlnlp_device_free.argtypes = [vp]
     L.qlnlp_device_alloc_info.argtypes = [vp, i64p]
     L.qlnlp_debug_refuse_compressible.argtypes = [C.c_int]
+    L.qlnlp_debug_fail_alloc.argtypes = [C.c_int]
+    L.qlnlp_debug_owned_blocks.argtypes = []
     for name in [n for n in EXPORTED_SYMBOLS if n not in ("qlnlp_version", "qlnlp_last_error")] + list(_DEBUG_SYMBOLS):
         getattr(L, name).restype = C.c_int
     _lib = L

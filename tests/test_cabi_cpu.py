@@ -112,6 +112,18 @@ def test_evaluation_fails_loudly_without_a_gpu():
         assert e.value.code == ev.QLNLP_ENODEVICE and f"error {ev.QLNLP_ENODEVICE}: device 0: no CUDA device" in str(e.value)
 
 
+def test_allocation_failure_hook_reports_what_it_had_left():
+    """qlnlp_debug_fail_alloc returns what the previous setting still had to go (-1: disarmed or used up), which is how
+    the GPU sweep over allocation points tells an injected failure from one it never reached.  Arming allocates nothing."""
+    L = ql.load_library()
+    blocks = L.qlnlp_debug_owned_blocks()
+    assert L.qlnlp_debug_fail_alloc(3) == -1
+    assert L.qlnlp_debug_fail_alloc(0) == 3
+    assert L.qlnlp_debug_fail_alloc(-7) == 0
+    assert L.qlnlp_debug_fail_alloc(-1) == -1
+    assert L.qlnlp_debug_owned_blocks() == blocks
+
+
 @pytest.mark.parametrize("devices", [[0], [0, 1]])
 def test_multi_device_handle_answers_like_a_plain_handle(devices):
     """qlnlp_create_multi needs no device until it evaluates: its host-side answers equal those of a plain handle, its
