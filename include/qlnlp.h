@@ -22,7 +22,8 @@
  *     is refused with QLNLP_EINVAL); a graph gives its counter back when it and its executable instantiations are
  *     destroyed, and must not outlive its handle.  Replay one executable instantiation of a graph at a time.
  *     First-use set-up allocates and synchronises, which a capture cannot hold: the first call of a handle, its first
- *     kinematic evaluation, its first KKT solve and the first ragged launch over a set of classes are refused with
+ *     kinematic evaluation, its first KKT call of any of the three kinds (one-shot solve, factor, factored solve) and
+ *     the first ragged launch over a set of classes are refused with
  *     QLNLP_EINVAL inside a capture (the caller's capture stays valid).  Warm the handle outside the capture by
  *     making each kind of call it will capture once, on any stream;
  *   - there is NO CPU fallback: evaluation entry points fail with QLNLP_ENODEVICE when no
@@ -269,6 +270,47 @@ typedef struct {
     int32_t* status;                      /* [B] */
 } qlnlp_kkt_io;
 int qlnlp_kkt_solve_batch_device(qlnlp_handle h, int64_t B, const qlnlp_kkt_io* io, void* stream);
+
+/* The same solve split in two: factorise once, then solve any number of right-hand sides against the kept factor
+ * (iterative refinement, predictor and corrector, second-order corrections).  A factor followed by a factored solve
+ * gives the bits qlnlp_kkt_solve_batch_device gives for the same inputs.
+ *
+ * A factor row holds, in a layout that belongs to the library, L_kk of every knot (210 doubles, packed), the 15x20
+ * off-diagonal factor X_k of every knot but the last (300), the problem's SPARSE_TRUE J values and dc, its status and
+ * a stamp of its class (N, k_trans, init_mode):
+ *     size = 4 + 210 N + 300 (N - 1) + nnz (SPARSE_TRUE) + m_nlp   doubles
+ * 36,747 doubles (293,976 B) per problem at the default instance (N = 61, k_trans = 21), 19.3 GB at B = 65,536.
+ * qlnlp_kkt_factor_size reports it.  A factor is self-contained: overwriting hess, jac, sx or dc after factorising
+ * changes no later solve.  A row with status 0 is written in full; entries beyond `size` are never written.  The handles qlnlp_kkt_solve_batch_device
+ * refuses are refused by the three calls below too.  Neither kernel needs scratch: the factor lives in caller memory. */
+int qlnlp_kkt_factor_size(qlnlp_handle h, int64_t* doubles);
+typedef struct {
+    const double* hess; int64_t ldhess;   /* [B][ldhess >= nnz_hess] */
+    const double* jac;  int64_t ldjac;    /* [B][ldjac  >= nnz (SPARSE_TRUE)] */
+    const double* sx;   int64_t ldsx;     /* [B][ldsx   >= n_nlp]   or NULL */
+    const double* dc;   int64_t lddc;     /* [B][lddc   >= m_nlp] */
+    double* factor;     int64_t ldfactor; /* [B][ldfactor >= qlnlp_kkt_factor_size] */
+    int32_t* status;                      /* [B] as qlnlp_kkt_solve_batch_device: 0, the failing knot k, or -1 */
+} qlnlp_kkt_factor_io;
+/* Factorises B problems (inputs as qlnlp_kkt_solve_batch_device).  DEVICE pointers, enqueued on `stream`. */
+int qlnlp_kkt_factor_batch_device(qlnlp_handle h, int64_t B, const qlnlp_kkt_factor_io* io, void* stream);
+typedef struct {
+    const double* factor; int64_t ldfactor; int64_t nfactor;   /* [nfactor][ldfactor]: rows of factors */
+    const int64_t* index;                 /* [R] factor row of each right-hand side, or NULL: row i uses factor i */
+    const double* r1;   int64_t ldr1;     /* [R][ldr1 >= n_nlp] */
+    const double* r2;   int64_t ldr2;     /* [R][ldr2 >= m_nlp] */
+    double* px;         int64_t ldpx;     /* [R][ldpx >= n_nlp] */
+    double* pl;         int64_t ldpl;     /* [R][ldpl >= m_nlp] */
+    int32_t* status;                      /* [R] */
+} qlnlp_kkt_rhs_io;
+/* Solves R right-hand sides; row i against the factor of row index[i] (or i), so several right-hand sides may share
+ * one factor and a subset of the problems may be solved alone.  status[i]:
+ *      0  success;
+ *      k > 0 or -1  the factor's own status, copied;
+ *     -2  index[i] (or i) outside [0, nfactor);
+ *     -3  the factor's class stamp is not this handle's class.
+ * px[i] and pl[i] of a row with status != 0 are written as NaN.  DEVICE pointers, enqueued on `stream`. */
+int qlnlp_kkt_solve_factored_batch_device(qlnlp_handle h, int64_t R, const qlnlp_kkt_rhs_io* io, void* stream);
 
 /* Ragged batches: problems of different size (several handles = several (N, k_trans, init_mode) classes) packed
  * back to back in flat arrays.  One call evaluates the B problems of THIS handle's class; the b-th of them is problem

@@ -393,6 +393,8 @@ KernelSpec hess_spec(const Problem& p, bool prod)
 
 // static shared memory only; its carve-out has not been measured, so the driver's default stays
 KernelSpec kkt_spec() { return {(const void*)ql::kkt_kernel, 0, 0, false, false, true}; }
+KernelSpec kkt_factor_spec() { return {(const void*)ql::kkt_factor_kernel, 0, 0, false, false, true}; }
+KernelSpec kkt_solve_factored_spec() { return {(const void*)ql::kkt_solve_factored_kernel, 0, 0, false, false, true}; }
 
 // the sparse pattern batched evaluations of this problem produce (DENSE handles batch in SPARSE_BLOCK)
 int batch_jm(const Problem& p) { return p.jac_mode == QLNLP_JAC_SPARSE_TRUE ? ql::JM_TRUE : ql::JM_BLOCK; }
@@ -1244,6 +1246,82 @@ int launch_kkt(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_kkt_io*
     P.B = B;
     if (int rc = launch_kernel(ds, k, B, P, stream)) return rc;
     return end_scratch(P.scratch, owned, stream);
+}
+
+int check_kkt_factor(const Problem& p, int64_t B, const qlnlp_kkt_factor_io* io)
+{
+    const QlClass& c = p.cls;
+    if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
+    if (!io || !io->hess || !io->jac || !io->dc || !io->factor || !io->status)
+        return fail(QLNLP_EINVAL, "io, hess, jac, dc, factor and status are required");
+    if (io->ldhess < ql_hess_nnz(c)) return fail(QLNLP_EINVAL, "ldhess %lld < nnz_hess %d", (long long)io->ldhess, ql_hess_nnz(c));
+    if (io->ldjac < c.nnz_true) return fail(QLNLP_EINVAL, "ldjac %lld < nnz %d", (long long)io->ldjac, c.nnz_true);
+    if (io->sx && io->ldsx < c.n_nlp) return fail(QLNLP_EINVAL, "ldsx %lld < n_nlp %d", (long long)io->ldsx, c.n_nlp);
+    if (io->lddc < c.m_nlp) return fail(QLNLP_EINVAL, "lddc %lld < m_nlp %d", (long long)io->lddc, c.m_nlp);
+    if (io->ldfactor < ql::kkt_factor_size(c))
+        return fail(QLNLP_EINVAL, "ldfactor %lld < factor size %lld", (long long)io->ldfactor, ql::kkt_factor_size(c));
+    for (const void* a : {(const void*)io->hess, (const void*)io->jac, (const void*)io->sx, (const void*)io->dc,
+                          (const void*)io->factor})
+        if ((reinterpret_cast<uintptr_t>(a) & 7) != 0) return fail(QLNLP_EINVAL, "arrays must be 8-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(io->status) & 3) != 0) return fail(QLNLP_EINVAL, "status must be 4-byte aligned");
+    return QLNLP_OK;
+}
+
+int check_kkt_rhs(const Problem& p, int64_t R, const qlnlp_kkt_rhs_io* io)
+{
+    const QlClass& c = p.cls;
+    if (R < 0) return fail(QLNLP_EINVAL, "negative batch");
+    if (!io || !io->factor || !io->r1 || !io->r2 || !io->px || !io->pl || !io->status)
+        return fail(QLNLP_EINVAL, "io, factor, r1, r2, px, pl and status are required");
+    if (io->nfactor < 0) return fail(QLNLP_EINVAL, "negative nfactor");
+    if (io->ldfactor < ql::kkt_factor_size(c))
+        return fail(QLNLP_EINVAL, "ldfactor %lld < factor size %lld", (long long)io->ldfactor, ql::kkt_factor_size(c));
+    if (io->ldr1 < c.n_nlp || io->ldpx < c.n_nlp)
+        return fail(QLNLP_EINVAL, "ldr1 %lld / ldpx %lld < n_nlp %d", (long long)io->ldr1, (long long)io->ldpx, c.n_nlp);
+    if (io->ldr2 < c.m_nlp || io->ldpl < c.m_nlp)
+        return fail(QLNLP_EINVAL, "ldr2 %lld / ldpl %lld < m_nlp %d", (long long)io->ldr2, (long long)io->ldpl, c.m_nlp);
+    for (const void* a : {(const void*)io->factor, (const void*)io->index, (const void*)io->r1, (const void*)io->r2,
+                          (const void*)io->px, (const void*)io->pl})
+        if ((reinterpret_cast<uintptr_t>(a) & 7) != 0) return fail(QLNLP_EINVAL, "arrays must be 8-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(io->status) & 3) != 0) return fail(QLNLP_EINVAL, "status must be 4-byte aligned");
+    return QLNLP_OK;
+}
+
+int launch_kkt_factor(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_kkt_factor_io* io, cudaStream_t stream)
+{
+    const QlClass& c = p.cls;
+    if (int rc = ensure_kkt_tables(p, ds, stream)) return rc;
+    ql::KktFactorLaunch P;
+    std::memset(&P, 0, sizeof P);
+    P.c = c;
+    P.jtab = ds.d_kkt_tab.get();
+    P.htab = ds.d_kkt_tab.get() + c.nnz_true;
+    P.hess = io->hess; P.ldhess = io->ldhess;
+    P.jac = io->jac; P.ldjac = io->ldjac;
+    P.sx = io->sx; P.ldsx = io->ldsx;
+    P.dc = io->dc; P.lddc = io->lddc;
+    P.factor = io->factor; P.ldfactor = io->ldfactor;
+    P.status = io->status;
+    P.B = B;
+    return launch_kernel(ds, kkt_factor_spec(), B, P, stream);
+}
+
+int launch_kkt_solve_factored(const Problem& p, DeviceState& ds, int64_t R, const qlnlp_kkt_rhs_io* io, cudaStream_t stream)
+{
+    if (int rc = ensure_kkt_tables(p, ds, stream)) return rc;
+    ql::KktSolveLaunch P;
+    std::memset(&P, 0, sizeof P);
+    P.c = p.cls;
+    P.jtab = ds.d_kkt_tab.get();
+    P.factor = io->factor; P.ldfactor = io->ldfactor; P.nfactor = io->nfactor;
+    P.index = reinterpret_cast<const long long*>(io->index);
+    P.r1 = io->r1; P.ldr1 = io->ldr1;
+    P.r2 = io->r2; P.ldr2 = io->ldr2;
+    P.px = io->px; P.ldpx = io->ldpx;
+    P.pl = io->pl; P.ldpl = io->ldpl;
+    P.status = io->status;
+    P.B = R;
+    return launch_kernel(ds, kkt_solve_factored_spec(), R, P, stream);
 }
 
 // A row of a single call: n doubles, copied in from `in` before the launch and / or back to `out` after it
@@ -2273,18 +2351,55 @@ int qlnlp_eval_hessian_product_batch_device(qlnlp_handle h, int64_t B, const dou
 }
 
 /* ---- batched KKT solve (qlnlp_kkt.cuh) ---- */
-int qlnlp_kkt_solve_batch_device(qlnlp_handle h, int64_t B, const qlnlp_kkt_io* io, void* stream)
+// the handles every KKT entry point takes
+static int check_kkt_handle(qlnlp_handle h)
 {
     if (int rc = check_handle(h)) return rc;
     if (h->multi) return fail(QLNLP_EINVAL, "multi-device handle: the KKT solve takes a single-device handle");
     if (h->prob.kin) return fail(QLNLP_EINVAL, "the KKT solve does not cover the kinematic rows");
     if (h->prob.jac_mode != QLNLP_JAC_SPARSE_TRUE) return fail(QLNLP_EINVAL, "the KKT solve takes a SPARSE_TRUE handle");
+    return QLNLP_OK;
+}
+
+int qlnlp_kkt_solve_batch_device(qlnlp_handle h, int64_t B, const qlnlp_kkt_io* io, void* stream)
+{
+    if (int rc = check_kkt_handle(h)) return rc;
     if (B == 0) return QLNLP_OK;
     if (int rc = check_kkt(h->prob, B, io)) return rc;
     DeviceState& ds = h->devs[0];
     DeviceGuard guard(ds.device);
     if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
     return launch_kkt(h->prob, ds, B, io, static_cast<cudaStream_t>(stream));
+}
+
+int qlnlp_kkt_factor_size(qlnlp_handle h, int64_t* doubles)
+{
+    if (int rc = check_kkt_handle(h)) return rc;
+    if (!doubles) return fail(QLNLP_EINVAL, "null output");
+    *doubles = ql::kkt_factor_size(h->prob.cls);
+    return QLNLP_OK;
+}
+
+int qlnlp_kkt_factor_batch_device(qlnlp_handle h, int64_t B, const qlnlp_kkt_factor_io* io, void* stream)
+{
+    if (int rc = check_kkt_handle(h)) return rc;
+    if (B == 0) return QLNLP_OK;
+    if (int rc = check_kkt_factor(h->prob, B, io)) return rc;
+    DeviceState& ds = h->devs[0];
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
+    return launch_kkt_factor(h->prob, ds, B, io, static_cast<cudaStream_t>(stream));
+}
+
+int qlnlp_kkt_solve_factored_batch_device(qlnlp_handle h, int64_t R, const qlnlp_kkt_rhs_io* io, void* stream)
+{
+    if (int rc = check_kkt_handle(h)) return rc;
+    if (R == 0) return QLNLP_OK;
+    if (int rc = check_kkt_rhs(h->prob, R, io)) return rc;
+    DeviceState& ds = h->devs[0];
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
+    return launch_kkt_solve_factored(h->prob, ds, R, io, static_cast<cudaStream_t>(stream));
 }
 
 // J w (transpose: J' y) at x for one evaluation

@@ -42,7 +42,8 @@ EXPORTED_SYMBOLS = (
     "qlnlp_eval_jacobian_products_batch_device", "qlnlp_eval_hessian_product_batch_device",
     "qlnlp_eval_constraint_jacobian_product", "qlnlp_eval_constraint_jacobian_transpose_product",
     "qlnlp_eval_hessian_lagrangian_product",
-    "qlnlp_kkt_solve_batch_device",
+    "qlnlp_kkt_solve_batch_device", "qlnlp_kkt_factor_size", "qlnlp_kkt_factor_batch_device",
+    "qlnlp_kkt_solve_factored_batch_device",
     "qlnlp_device_alloc", "qlnlp_device_free", "qlnlp_device_alloc_info",
 )
 _DEBUG_SYMBOLS = ("qlnlp_debug_segments", "qlnlp_debug_vals_map", "qlnlp_debug_build_rows", "qlnlp_debug_host_times",
@@ -83,6 +84,19 @@ class _ProductIO(C.Structure):
 class _KktIO(C.Structure):
     _fields_ = [("hess", C.c_void_p), ("ldhess", C.c_int64), ("jac", C.c_void_p), ("ldjac", C.c_int64),
                 ("sx", C.c_void_p), ("ldsx", C.c_int64), ("dc", C.c_void_p), ("lddc", C.c_int64),
+                ("r1", C.c_void_p), ("ldr1", C.c_int64), ("r2", C.c_void_p), ("ldr2", C.c_int64),
+                ("px", C.c_void_p), ("ldpx", C.c_int64), ("pl", C.c_void_p), ("ldpl", C.c_int64),
+                ("status", C.c_void_p)]
+
+
+class _KktFactorIO(C.Structure):
+    _fields_ = [("hess", C.c_void_p), ("ldhess", C.c_int64), ("jac", C.c_void_p), ("ldjac", C.c_int64),
+                ("sx", C.c_void_p), ("ldsx", C.c_int64), ("dc", C.c_void_p), ("lddc", C.c_int64),
+                ("factor", C.c_void_p), ("ldfactor", C.c_int64), ("status", C.c_void_p)]
+
+
+class _KktRhsIO(C.Structure):
+    _fields_ = [("factor", C.c_void_p), ("ldfactor", C.c_int64), ("nfactor", C.c_int64), ("index", C.c_void_p),
                 ("r1", C.c_void_p), ("ldr1", C.c_int64), ("r2", C.c_void_p), ("ldr2", C.c_int64),
                 ("px", C.c_void_p), ("ldpx", C.c_int64), ("pl", C.c_void_p), ("ldpl", C.c_int64),
                 ("status", C.c_void_p)]
@@ -159,6 +173,9 @@ def load_library(rebuild_if_stale: bool = True):
     L.qlnlp_eval_constraint_jacobian_transpose_product.argtypes = [vp, vp, vp, vp]
     L.qlnlp_eval_hessian_lagrangian_product.argtypes = [vp, vp, vp, C.c_double, vp, vp]
     L.qlnlp_kkt_solve_batch_device.argtypes = [vp, C.c_int64, C.POINTER(_KktIO), vp]
+    L.qlnlp_kkt_factor_size.argtypes = [vp, i64p]
+    L.qlnlp_kkt_factor_batch_device.argtypes = [vp, C.c_int64, C.POINTER(_KktFactorIO), vp]
+    L.qlnlp_kkt_solve_factored_batch_device.argtypes = [vp, C.c_int64, C.POINTER(_KktRhsIO), vp]
     L.qlnlp_host_alloc.argtypes = [C.c_int64, C.POINTER(vp)]
     L.qlnlp_host_free.argtypes = [vp, C.c_int64]
     L.qlnlp_device_alloc.argtypes = [vp, C.c_int64, C.POINTER(vp)]
@@ -266,6 +283,23 @@ def _device_empty(device: int, specs, compressible: bool = True) -> list:
             return [empty(*s) for s in specs]
         with torch.cuda.use_mem_pool(_output_pool(device), device):
             return [empty(*s) for s in specs]
+
+
+def _check_rows(B: int, specs) -> None:
+    """Each ``(tensor or None, width, name)`` is a float64 CUDA tensor ``[B, width]`` with unit inner stride."""
+    import torch
+
+    for t, wd, name in specs:
+        if t is not None and not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64
+                                  and t.dim() == 2 and t.shape == (B, wd) and t.stride(1) == 1):
+            raise ValueError(f"{name} must be a float64 CUDA tensor [{B}, {wd}] with unit inner stride")
+
+
+def _check_status(t, B: int) -> None:
+    import torch
+
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.int32 and t.shape == (B,) and t.is_contiguous()):
+        raise ValueError(f"out status must be a contiguous int32 CUDA tensor of shape ({B},)")
 
 
 class HybridNLP:
@@ -563,6 +597,79 @@ class HybridNLP:
         io.status = status.data_ptr()
         s = torch.cuda.current_stream(dev) if stream is None else stream
         _check(load_library().qlnlp_kkt_solve_batch_device(self._h, B, C.byref(io), C.c_void_p(s.cuda_stream)))
+        return px, pl, status
+
+    # The same solve split in two: factorise once, solve many right-hand sides (include/qlnlp.h).  A factor followed by
+    # a factored solve gives the bits of kkt_solve_batch.
+    @property
+    def kkt_factor_size(self) -> int:
+        """Doubles in one problem's factor row (``qlnlp_kkt_factor_size``)."""
+        v = C.c_int64()
+        _check(load_library().qlnlp_kkt_factor_size(self._h, C.byref(v)))
+        return v.value
+
+    def kkt_factor_batch(self, hess, jac, dc, sx=None, out=None, stream=None):
+        """Device tensors as ``kkt_solve_batch`` -> ``(factor[B, kkt_factor_size], status[B] int32)``.  The factor holds
+        everything a later solve reads: overwriting the inputs afterwards changes no solve.  ``out`` may give both
+        outputs.  Enqueued on the current torch stream (or ``stream``), not synchronised."""
+        import torch
+
+        B = hess.shape[0]
+        size = self.kkt_factor_size
+        _check_rows(B, ((hess, self.nnz_hess, "hess"), (jac, self.nnz, "jac"), (dc, self.m_nlp, "dc"),
+                        (sx, self.n_nlp, "sx")))
+        dev = hess.device
+        if out is None:
+            out = tuple(_device_empty(dev.index, [(B, size, torch.float64), (B, None, torch.int32)], self._compressible))
+        factor, status = out
+        _check_rows(B, ((factor, size, "out factor"),))
+        _check_status(status, B)
+        ld = lambda t, wd: t.stride(0) if B > 1 else wd
+        io = _KktFactorIO()
+        io.hess, io.ldhess = hess.data_ptr(), ld(hess, self.nnz_hess)
+        io.jac, io.ldjac = jac.data_ptr(), ld(jac, self.nnz)
+        if sx is not None:
+            io.sx, io.ldsx = sx.data_ptr(), ld(sx, self.n_nlp)
+        io.dc, io.lddc = dc.data_ptr(), ld(dc, self.m_nlp)
+        io.factor, io.ldfactor = factor.data_ptr(), ld(factor, size)
+        io.status = status.data_ptr()
+        s = torch.cuda.current_stream(dev) if stream is None else stream
+        _check(load_library().qlnlp_kkt_factor_batch_device(self._h, B, C.byref(io), C.c_void_p(s.cuda_stream)))
+        return factor, status
+
+    def kkt_solve_factored_batch(self, factor, r1, r2, index=None, out=None, stream=None):
+        """``factor[F, kkt_factor_size]`` (``kkt_factor_batch``), ``r1[R, n_nlp]``, ``r2[R, m_nlp]``, optional
+        ``index[R]`` int64 (the factor row of each right-hand side; default: row i uses factor i) -> ``(px[R, n_nlp],
+        pl[R, m_nlp], status[R] int32)``.  status: 0, the factor's own non-zero status, -2 for an index outside
+        ``[0, F)``, -3 for a factor of another class.  Enqueued on the current torch stream (or ``stream``)."""
+        import torch
+
+        R, F = r1.shape[0], factor.shape[0]
+        n, m, size = self.n_nlp, self.m_nlp, self.kkt_factor_size
+        _check_rows(F, ((factor, size, "factor"),))
+        _check_rows(R, ((r1, n, "r1"), (r2, m, "r2")))
+        if index is not None and not (isinstance(index, torch.Tensor) and index.is_cuda and index.dtype == torch.int64
+                                      and index.shape == (R,) and index.is_contiguous()):
+            raise ValueError(f"index must be a contiguous int64 CUDA tensor of shape ({R},)")
+        dev = r1.device
+        if out is None:
+            out = tuple(_device_empty(dev.index, [(R, n, torch.float64), (R, m, torch.float64), (R, None, torch.int32)],
+                                      self._compressible))
+        px, pl, status = out
+        _check_rows(R, ((px, n, "out px"), (pl, m, "out pl")))
+        _check_status(status, R)
+        io = _KktRhsIO()
+        io.factor, io.ldfactor, io.nfactor = factor.data_ptr(), factor.stride(0) if F > 1 else size, F
+        if index is not None:
+            io.index = index.data_ptr()
+        ld = lambda t, wd: t.stride(0) if R > 1 else wd
+        io.r1, io.ldr1 = r1.data_ptr(), ld(r1, n)
+        io.r2, io.ldr2 = r2.data_ptr(), ld(r2, m)
+        io.px, io.ldpx = px.data_ptr(), ld(px, n)
+        io.pl, io.ldpl = pl.data_ptr(), ld(pl, m)
+        io.status = status.data_ptr()
+        s = torch.cuda.current_stream(dev) if stream is None else stream
+        _check(load_library().qlnlp_kkt_solve_factored_batch_device(self._h, R, C.byref(io), C.c_void_p(s.cuda_stream)))
         return px, pl, status
 
     def initialize(self, features: Iterable[str] = ()) -> None:

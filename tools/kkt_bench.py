@@ -1,6 +1,9 @@
 """Throughput of the batched KKT solve (kkt_kernel) at the default instance (N = 61, k_trans = 21) on one GPU, next to
 a CPU baseline in the same process: scipy factorising the same problems one by one (splu of the assembled sparse KKT
-matrix) on all host cores, over a sample.
+matrix) on all host cores, over a sample.  Then the factor / solve split in the same process: kkt_factor_kernel alone,
+kkt_solve_factored_kernel with one right-hand side per factor (R = B) and with four per factor through `index`
+(R = 4B), each launch alternating with a one-shot solve, and one factorisation plus two factored solves against two
+one-shot solves.
 
 Inputs: C3-style decision vectors (device-built guesses of the drop-height x pitch sweep, perturbed), seeded
 multipliers (scale 1e-4), objective factor 1e-4 (at 1 the objective's x-h second derivatives make these M
@@ -62,6 +65,46 @@ def kernel_flops(N):
     return total
 
 
+def _knot_flops(N, k):
+    """Operations of knot k by step, from the loops of qlnlp_kkt.cuh (see kernel_flops)."""
+    S = 34
+    nk = 20 if k < N else 15
+    T = nk * (nk + 1) // 2
+    return {
+        "mkk": T * (1 + 3 * S) + (15 * 20 + 120 * (2 * 20 + 1) if k > 1 else 0),         # M_kk, E, rank-15 update
+        "chol": sum(1 + (nk - 1 - j) + sum(2 * (i - j) for i in range(j + 1, nk)) for j in range(nk)),
+        "xk": 15 * sum(1 + 2 * j + 1 for j in range(20)) if k < N else 0,                  # X_k = D^-1 A_k L^-T
+        "bk": nk + nk * (S * 3 + 1) + (15 * (2 * 20 + 1) if k > 1 else 0),                 # b_k - X_(k-1) y_(k-1)
+        "yk": sum(1 + 2 * (nk - 1 - j) for j in range(nk)),                                # y_k = L^-1 b
+        "back": (20 * 15 * 4 + sum(1 + 2 * (19 - j) for j in range(20)) + 20 if k < N else 0)
+                + sum(1 + 2 * j for j in range(nk)) + S * (2 * nk + 4),                    # x_k and the pl rows
+        "rdc": S,                                                                          # 1/dc per slot, one gather
+    }
+
+
+def factor_flops(N):
+    """kkt_factor_kernel per problem: M_kk, Cholesky and X_k of every knot."""
+    return sum(t["mkk"] + t["chol"] + t["xk"] + t["rdc"] for t in (_knot_flops(N, k) for k in range(1, N + 1)))
+
+
+def solve_flops(N):
+    """kkt_solve_factored_kernel per right-hand side: b_k, y_k, the backward sweep (1/dc in both sweeps' gathers)."""
+    return sum(t["bk"] + t["yk"] + t["back"] + 2 * t["rdc"] for t in (_knot_flops(N, k) for k in range(1, N + 1)))
+
+
+def factor_bytes(nlp):
+    """kkt_factor_kernel per problem: W, J, sx, dc read once, the factor row written once."""
+    n, m = nlp.n_nlp, nlp.m_nlp
+    return 8 * (nlp.nnz_hess + nlp.nnz + n + m) + 8 * nlp.kkt_factor_size
+
+
+def solve_bytes(nlp):
+    """kkt_solve_factored_kernel per right-hand side: the factor row read once (the backward sweep's second read of
+    L_kk, J and dc not counted), r1, r2 read, y_k written to px and read back, px and pl written."""
+    n, m = nlp.n_nlp, nlp.m_nlp
+    return 8 * nlp.kkt_factor_size + 8 * (n + m) + 16 * n + 8 * (n + m)
+
+
 def _cpu_solve(args):
     hs, hv, js, jv, sx, dc, r1, r2 = args
     n, m = len(sx), len(dc)
@@ -77,6 +120,59 @@ def _cpu_solve(args):
 
 def _cpu_batch(chunk):
     return [_cpu_solve(a) for a in chunk]
+
+
+def split(a, log, nlp, B, hess, jac, dc, sx, r1, r2, out, gen):
+    """The factor / solve split at batch B, each new launch alternating with a one-shot solve in one stream."""
+    n, m = nlp.n_nlp, nlp.m_nlp
+    R4 = 4 * B
+    q1 = torch.randn((R4, n), generator=gen, device="cuda", dtype=torch.float64)
+    q2 = torch.randn((R4, m), generator=gen, device="cuda", dtype=torch.float64)
+    index = torch.arange(B, dtype=torch.int64, device="cuda").repeat_interleave(4)
+    fac = nlp.kkt_factor_batch(hess, jac, dc, sx=sx)
+    one = nlp.kkt_solve_factored_batch(fac[0], r1, r2)
+    four = nlp.kkt_solve_factored_batch(fac[0], q1, q2, index=index)
+    torch.cuda.synchronize()
+    same = all(torch.equal(x, y) for x, y in zip(one, out))
+    calls = {
+        "one-shot": lambda: nlp.kkt_solve_batch(hess, jac, dc, r1, r2, sx=sx, out=out),
+        "factor": lambda: nlp.kkt_factor_batch(hess, jac, dc, sx=sx, out=fac),
+        "solve R=B": lambda: nlp.kkt_solve_factored_batch(fac[0], r1, r2, out=one),
+        "solve R=4B": lambda: nlp.kkt_solve_factored_batch(fac[0], q1, q2, index=index, out=four),
+    }
+    for f in calls.values():
+        f()
+    torch.cuda.synchronize()
+    ev = {k: [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(a.iters)]
+          for k in calls}
+    for i in range(a.iters):
+        for k, f in calls.items():
+            e0, e1 = ev[k][i]
+            e0.record()
+            f()
+            e1.record()
+    torch.cuda.synchronize()
+    med = {}
+    for k in calls:
+        ms = sorted(e0.elapsed_time(e1) for e0, e1 in ev[k])
+        med[k] = ms[len(ms) // 2]
+        rows = R4 if k == "solve R=4B" else B
+        per = {"one-shot": (stream_bytes(nlp) + scratch_bytes(nlp.N), kernel_flops(nlp.N)),
+               "factor": (factor_bytes(nlp), factor_flops(nlp.N))}.get(k, (solve_bytes(nlp), solve_flops(nlp.N)))
+        rate = rows / (med[k] * 1e-3)
+        bw, fr = per[0] * rate / 1e12, per[1] * rate / 1e12
+        log(f"  B={B} {k:>10}: {med[k]:.3f} ms median (min {ms[0]:.3f}, max {ms[-1]:.3f}) over {a.iters} alternating "
+            f"launches; {rate / 1e6:.3f} M rows/s; {bw:.3f} TB/s ({100 * bw / HBM_TBS:.1f} % of HBM), {fr:.3f} TFLOP/s "
+            f"({100 * fr / FP64_TFLOPS:.1f} % of DFMA)")
+    st = [t.cpu().numpy() for t in (fac[1], one[2], four[2])]
+    log(f"  B={B}: factored solve R=B equals the one-shot bits: {same}; status 0: factor {int((st[0] == 0).sum())}, "
+        f"R=B {int((st[1] == 0).sum())} of {B}, R=4B {int((st[2] == 0).sum())} of {R4}")
+    two = 2 * med["one-shot"]
+    split_ms = med["factor"] + 2 * med["solve R=B"]
+    log(f"  B={B}: factor + 2 factored solves {split_ms:.3f} ms vs 2 one-shot solves {two:.3f} ms "
+        f"({'faster' if split_ms < two else 'NOT faster'}: {two / split_ms:.2f}x); a factored solve costs "
+        f"{med['solve R=B'] / med['one-shot']:.3f} of a one-shot solve, the factor {med['factor'] / med['one-shot']:.3f}")
+    del fac, one, four, q1, q2
 
 
 def main():
@@ -102,6 +198,9 @@ def main():
         f"nnz_hess={nlp.nnz_hess}")
     log(f"per problem: streams {sb:,} B, factor scratch {fb:,} B (write + read), kernel flops {fl:,} "
         f"({fl / N:,.0f} per knot)")
+    log(f"factor row {nlp.kkt_factor_size:,} doubles ({8 * nlp.kkt_factor_size:,} B); factor: {factor_bytes(nlp):,} B, "
+        f"{factor_flops(N):,} flops per problem; factored solve: {solve_bytes(nlp):,} B, {solve_flops(N):,} flops per "
+        f"right-hand side")
     log(f"host cores: {os.cpu_count()}")
     gen = torch.Generator(device="cuda").manual_seed(0)
     for B in (4096, 65536):
@@ -160,6 +259,7 @@ def main():
             log(f"  CPU baseline (scipy splu, one problem at a time, {ncpu} processes, {len(idx)} problems): "
                 f"{cpu_rate:,.0f} solves/s; GPU / CPU = {rate / cpu_rate:,.0f}x; max relative difference of the steps "
                 f"{rel.max():.2e}")
+        split(a, log, nlp, B, hess, jac, dc, sx, r1, r2, out, gen)
         del out, hess, jac, Z, lam, dc, sx, r1, r2
         torch.cuda.empty_cache()
     if a.out:
