@@ -22,7 +22,9 @@
 #include <mutex>
 #include <new>
 #include <string>
+#include <tuple>
 #include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "hostrows.h"
@@ -170,6 +172,13 @@ struct RagTable {
     bool fastdiv = false;
 };
 
+// One SPARSE_BLOCK value of the block plan (block_plan)
+struct BlockEntry {
+    int32_t row, col;                  // 1-based
+    double konst;                      // the constant image: what the value is where it does not depend on Z, else 0
+    bool vals;                         // depends on Z: part of the VALS stream
+};
+
 // The problem a handle evaluates: built once when the handle is created, host memory only, read-only afterwards.
 struct Problem {
     QlClass cls;
@@ -180,6 +189,7 @@ struct Problem {
     double x0xf[2 * QL_NX];            // x0 | xf
     std::vector<double> cost;          // field-major [QL_NCOST][npad]
     int npad = 0;
+    std::vector<BlockEntry> block;     // every SPARSE_BLOCK value in value order: the one source of every host pattern table
     std::vector<QlSeg> segs;
     std::vector<int> seg_begin;
     double rmb = 0, rmf = 0, rIb = 0;  // reciprocals of the divisors
@@ -264,15 +274,29 @@ struct qlnlp_handle_s {
 namespace {
 
 // ---------------------------------------------------------------------------- host planner
-// SPARSE_BLOCK structure in value order, straight from the closed-form layout (1-based output).
-void sparse_block_structure(const QlClass& c, int64_t* rows, int64_t* cols)
+struct ModePattern { int nvar; const unsigned char *vi, *vj; int ncon; const unsigned char *ci, *cj; const double* cv; };
+ModePattern mode_pattern(int mode)
 {
+    if (mode == 1) return {QL_NJ_MODE1, QL_PAT_I_MODE1, QL_PAT_J_MODE1, QL_NJC_MODE1, QL_CPAT_I_MODE1, QL_CPAT_J_MODE1, QL_CPAT_V_MODE1};
+    if (mode == 2) return {QL_NJ_MODE2, QL_PAT_I_MODE2, QL_PAT_J_MODE2, QL_NJC_MODE2, QL_CPAT_I_MODE2, QL_CPAT_J_MODE2, QL_CPAT_V_MODE2};
+    return {QL_NJ_MODE3, QL_PAT_I_MODE3, QL_PAT_J_MODE3, QL_NJC_MODE3, QL_CPAT_I_MODE3, QL_CPAT_J_MODE3, QL_CPAT_V_MODE3};
+}
+// rows the jump Jacobian keeps (planar_quadruped.jl:262-263)
+const int JUMP_KEEP[QL_NX] = {1, 1, 1, 1, 0, 1, 0, 1, 1, 1, 0, 0, 0, 0, 0};
+
+// The block plan of a class: every SPARSE_BLOCK value in value order, with its row and column (the closed-form
+// layout), its constant (everything jac_c! assigns that does not depend on Z; 0 elsewhere) and whether it is in the
+// VALS stream (layout.h: ql_vals_run_off; the kernel's writer is ql_vals_write_run in true_run.h).  SPARSE_TRUE is the
+// sub-sequence of values that are not structural zeros: a non-zero constant, or value-dependent.
+int block_plan(const QlClass& c, std::vector<BlockEntry>& plan)
+{
+    plan.assign((size_t)c.nnz, BlockEntry{});
     int64_t n = 0;
     for (int k = 1; k <= c.N; ++k) {
         const int ncol = (k < c.N) ? QL_NZK : QL_NX;
         for (int j = 0; j < ncol; ++j) {
-            const int64_t col = (int64_t)QL_NZK * (k - 1) + j + 1;
-            auto put = [&](int64_t row0) { rows[n] = row0 + 1; cols[n] = col; ++n; };
+            const int col = QL_NZK * (k - 1) + j + 1;
+            auto put = [&](int row0) { plan[(size_t)n].row = row0 + 1; plan[(size_t)n].col = col; ++n; };
             if (j < QL_NX) {
                 if (k == 1) for (int i = 0; i < QL_NX; ++i) put(i);                              // init rows
                 if (k == c.N) for (int i = 0; i < QL_NX - 1; ++i) put(c.c_term + i);             // term rows
@@ -288,12 +312,46 @@ void sparse_block_structure(const QlClass& c, int64_t* rows, int64_t* cols)
             }
         }
     }
+    std::vector<double> image((size_t)c.nnz, 0.0);
+    std::vector<int32_t> vals_pos;             // in VALS order
+    vals_pos.reserve((size_t)c.nnz_vals);
+    for (int k = 1; k <= c.N; ++k) {
+        const int base = ql_run_off(c, k);
+        ql_write_run_constants(c, k, image.data() + base);
+        const int theta = base + ql_theta_pos(c, k);
+        if (k == c.N) { vals_pos.push_back(theta); continue; }
+        const bool jump = (k == c.k_trans - 1);
+        const ModePattern mp = mode_pattern(k >= c.k_trans ? 3 : c.init_mode);
+        for (int e = 0; e < mp.ncon; ++e)
+            image[(size_t)(base + ql_rk4_pos(c, k, mp.ci[e], mp.cj[e]))] = (jump && !JUMP_KEEP[mp.ci[e]]) ? 0.0 : mp.cv[e];
+        bool theta_done = false;
+        for (int e = 0; e < mp.nvar; ++e) {
+            if (jump && !JUMP_KEEP[mp.vi[e]]) continue;          // constant zero at the jump knot: stays in the image
+            if (mp.vj[e] >= 3 && !theta_done) { vals_pos.push_back(theta); theta_done = true; }
+            vals_pos.push_back(base + ql_rk4_pos(c, k, mp.vi[e], mp.vj[e]));
+        }
+        if (!theta_done) vals_pos.push_back(theta);
+    }
+    // the VALS stream is the value-dependent entries in value order: a mark per entry says all of it
+    if ((int)vals_pos.size() != c.nnz_vals) return fail(QLNLP_ECUDA, "internal: VALS map has %zu entries, layout says %d", vals_pos.size(), c.nnz_vals);
+    for (size_t i = 1; i < vals_pos.size(); ++i)
+        if (vals_pos[i] <= vals_pos[i - 1]) return fail(QLNLP_ECUDA, "internal: VALS map is not ascending at %zu", i);
+    for (int32_t q : vals_pos) plan[(size_t)q].vals = true;
+    int nnz_true = 0;
+    for (size_t i = 0; i < plan.size(); ++i) {
+        plan[i].konst = image[i];
+        nnz_true += plan[i].konst != 0.0 || plan[i].vals;
+    }
+    if (nnz_true != c.nnz_true) return fail(QLNLP_ECUDA, "internal: SPARSE_TRUE has %d entries, layout says %d", nnz_true, c.nnz_true);
+    return QLNLP_OK;
 }
 
-// Segment plan: per pass, consecutive knots paired; template ids from the constant-image signature.
-void plan_segments(const QlClass& c, std::vector<QlSeg>& segs, std::vector<int>& seg_begin)
+// Segment plan: per pass, consecutive knots paired.  Two segments share a template id exactly when their staging
+// buffers hold the same image once the owner lanes have patched it: the same parity of `start` (the image's offset in
+// the buffer), the same knot count, and the same constants and value-dependent positions over [start, end).
+void plan_segments(const QlClass& c, const std::vector<BlockEntry>& block, std::vector<QlSeg>& segs, std::vector<int>& seg_begin)
 {
-    std::map<std::vector<int>, int> ids;
+    std::map<std::tuple<int, int, std::vector<std::pair<double, bool>>>, int> ids;
     segs.clear();
     seg_begin.assign(1, 0);
     for (int p = 0; p < c.npass; ++p) {
@@ -306,20 +364,9 @@ void plan_segments(const QlClass& c, std::vector<QlSeg>& segs, std::vector<int>&
             s.nk = (signed char)nk;
             s.start = ql_run_off(c, k);
             s.end = (k + nk > c.N) ? c.nnz : ql_run_off(c, k + nk);
-            // everything that determines the constant image of the segment
-            std::vector<int> sig{s.start & 1, nk};
-            for (int q = k; q < k + nk; ++q) {
-                sig.push_back(q == 1);
-                sig.push_back(q == c.N - 1);
-                sig.push_back(q == c.N);
-                sig.push_back(ql_e4(c, q));
-                sig.push_back(ql_e6(c, q));
-                sig.push_back(q >= c.k_trans);          // RK4 block constants of mode 3 vs the initial mode
-                sig.push_back(q == c.k_trans - 1);      // jump knot: masked rows hold 0 instead of 1
-            }
-            auto it = ids.find(sig);
-            if (it == ids.end()) it = ids.emplace(sig, (int)ids.size()).first;
-            s.tmpl = (short)it->second;
+            std::vector<std::pair<double, bool>> image;
+            for (int i = s.start; i < s.end; ++i) image.emplace_back(block[(size_t)i].konst, block[(size_t)i].vals);
+            s.tmpl = (short)ids.emplace(std::make_tuple(s.start & 1, nk, std::move(image)), (int)ids.size()).first->second;
             s.buf = 0;      // unused: the kernel alternates the staging buffers with a running counter (ql_seg_buffer)
             segs.push_back(s);
         }
@@ -403,112 +450,44 @@ int std_nnz(const Problem& p) { return p.jac_mode == QLNLP_JAC_SPARSE_TRUE ? p.c
 int batch_nnz(const Problem& p) { return std_nnz(p) + (p.kin ? 8 * p.cls.N : 0); }
 int m_rows(const Problem& p) { return p.cls.m_nlp + (p.kin ? 2 * p.cls.N : 0); }
 
-// SPARSE_TRUE structure (1-based, value order): like sparse_block_structure restricted to structural non-zeros
-void sparse_true_structure(const QlClass& c, int64_t* rows, int64_t* cols)
-{
-    int64_t n = 0;
-    for (int k = 1; k <= c.N; ++k) {
-        const int ncol = (k < c.N) ? QL_NZK : QL_NX;
-        const int mode = (k >= c.k_trans) ? 3 : c.init_mode;
-        const QlTruePattern pat = ql_true_pattern(mode, k < c.N && k == c.k_trans - 1);
-        for (int j = 0; j < ncol; ++j) {
-            const int64_t col = (int64_t)QL_NZK * (k - 1) + j + 1;
-            auto put = [&](int64_t row0) { rows[n] = row0 + 1; cols[n] = col; ++n; };
-            if (j < QL_NX) {
-                if (k == 1) put(j);                                              // init diagonal
-                if (k == c.N && j < QL_NX - 1) put(c.c_term + j);                // term diagonal
-                if (k >= 2) put(c.c_dyn + QL_NX * (k - 2) + j);                  // -I diagonal
-            }
-            if (k < c.N)
-                for (int e = 0; e < pat.n; ++e)
-                    if (pat.J[e] == j) put(c.c_dyn + QL_NX * (k - 1) + pat.I[e]);
-            if (j < QL_NX) {
-                const int jf = (c.init_mode == 1) ? 4 : 6, jo = (c.init_mode == 1) ? 6 : 4;
-                if (j == jf) put(c.c_cfirst + (k - 1));
-                if (j == jo && k >= c.k_trans) put(c.c_cother + (k - c.k_trans));
-                if (j == 1 || j == 2) put(c.c_body + (k - 1));
-            } else if (k == c.N - 1 && (j == 16 || j == 18)) {
-                put(c.c_fctrl);
-            }
-        }
-    }
-}
+// One value of the Jacobian row a batched evaluation of the handle returns
+struct BatchEntry {
+    BlockEntry v;      // a kinematic entry: a constant 0 outside the VALS stream (its rows never take the VALS route)
+    int32_t src;       // position in the kernel's row (SPARSE_BLOCK or SPARSE_TRUE order), or -(8 (k-1) + e + 1) for
+                       // the kinematic entry e of knot k (qlnlp_kin.cuh)
+};
 
-// ---- what a host-side row is made of ----------------------------------------------------------------------
-// Position of every SPARSE_TRUE value inside a SPARSE_BLOCK row (both column-major sorted; TRUE is a sub-sequence).
-std::vector<int32_t> true_to_block(const QlClass& c)
-{
-    std::vector<int64_t> rb(c.nnz), cb(c.nnz), rt(c.nnz_true), ct(c.nnz_true);
-    sparse_block_structure(c, rb.data(), cb.data());
-    sparse_true_structure(c, rt.data(), ct.data());
-    std::vector<int32_t> map(c.nnz_true);
-    int64_t j = 0;
-    for (int64_t i = 0; i < c.nnz_true; ++i) {
-        while (rb[j] != rt[i] || cb[j] != ct[i]) ++j;
-        map[i] = (int32_t)j;
-    }
-    return map;
-}
-
-struct ModePattern { int nvar; const unsigned char *vi, *vj; int ncon; const unsigned char *ci, *cj; const double* cv; };
-ModePattern mode_pattern(int mode)
-{
-    if (mode == 1) return {QL_NJ_MODE1, QL_PAT_I_MODE1, QL_PAT_J_MODE1, QL_NJC_MODE1, QL_CPAT_I_MODE1, QL_CPAT_J_MODE1, QL_CPAT_V_MODE1};
-    if (mode == 2) return {QL_NJ_MODE2, QL_PAT_I_MODE2, QL_PAT_J_MODE2, QL_NJC_MODE2, QL_CPAT_I_MODE2, QL_CPAT_J_MODE2, QL_CPAT_V_MODE2};
-    return {QL_NJ_MODE3, QL_PAT_I_MODE3, QL_PAT_J_MODE3, QL_NJC_MODE3, QL_CPAT_I_MODE3, QL_CPAT_J_MODE3, QL_CPAT_V_MODE3};
-}
-// rows the jump Jacobian keeps (planar_quadruped.jl:262-263)
-const int JUMP_KEEP[QL_NX] = {1, 1, 1, 1, 0, 1, 0, 1, 1, 1, 0, 0, 0, 0, 0};
-
-// The constant image of a SPARSE_BLOCK row (everything jac_c! assigns that does not depend on Z; 0 elsewhere) and
-// the position of every VALS element inside the row, in VALS order (layout.h: ql_vals_run_off; the kernel's writer
-// is ql_vals_write_run in true_run.h).
-void block_image_and_vals_map(const QlClass& c, std::vector<double>& image, std::vector<int32_t>& vals_pos)
-{
-    image.assign((size_t)c.nnz, 0.0);
-    vals_pos.clear();
-    vals_pos.reserve((size_t)c.nnz_vals);
-    for (int k = 1; k <= c.N; ++k) {
-        const int base = ql_run_off(c, k);
-        ql_write_run_constants(c, k, image.data() + base);
-        const int theta = base + ql_theta_pos(c, k);
-        if (k == c.N) { vals_pos.push_back(theta); continue; }
-        const bool jump = (k == c.k_trans - 1);
-        const ModePattern mp = mode_pattern(k >= c.k_trans ? 3 : c.init_mode);
-        for (int e = 0; e < mp.ncon; ++e)
-            image[(size_t)(base + ql_rk4_pos(c, k, mp.ci[e], mp.cj[e]))] = (jump && !JUMP_KEEP[mp.ci[e]]) ? 0.0 : mp.cv[e];
-        bool theta_done = false;
-        for (int e = 0; e < mp.nvar; ++e) {
-            if (jump && !JUMP_KEEP[mp.vi[e]]) continue;          // constant zero at the jump knot: stays in the image
-            if (mp.vj[e] >= 3 && !theta_done) { vals_pos.push_back(theta); theta_done = true; }
-            vals_pos.push_back(base + ql_rk4_pos(c, k, mp.vi[e], mp.vj[e]));
-        }
-        if (!theta_done) vals_pos.push_back(theta);
-    }
-}
-
-// The constant image and the VALS positions of a row of the problem's batch pattern (SPARSE_BLOCK, or SPARSE_TRUE as a
-// sub-sequence of it).
-int batch_image_and_vals_map(const Problem& p, std::vector<double>& image, std::vector<int32_t>& pos)
+// The Jacobian pattern the caller of the handle sees, in value order: the block plan (DENSE handles batch in
+// SPARSE_BLOCK) or its SPARSE_TRUE sub-sequence, with the kinematic rows' 8 entries per knot merged in column-major.
+std::vector<BatchEntry> batch_pattern(const Problem& p)
 {
     const QlClass& c = p.cls;
-    block_image_and_vals_map(c, image, pos);
-    if ((int)pos.size() != c.nnz_vals) return fail(QLNLP_ECUDA, "internal: VALS map has %zu entries, layout says %d", pos.size(), c.nnz_vals);
-    for (size_t i = 1; i < pos.size(); ++i)
-        if (pos[i] <= pos[i - 1]) return fail(QLNLP_ECUDA, "internal: VALS map is not ascending at %zu", i);
-    if (batch_jm(p) == ql::JM_TRUE) {
-        const std::vector<int32_t> t2b = true_to_block(c);
-        std::vector<int32_t> b2t((size_t)c.nnz, -1);
-        for (size_t t = 0; t < t2b.size(); ++t) b2t[(size_t)t2b[t]] = (int32_t)t;
-        std::vector<double> timage(t2b.size());
-        for (size_t t = 0; t < t2b.size(); ++t) timage[t] = image[(size_t)t2b[t]];
-        for (auto& q : pos) {
-            if (b2t[(size_t)q] < 0) return fail(QLNLP_ECUDA, "internal: value-dependent entry outside SPARSE_TRUE");
-            q = b2t[(size_t)q];
-        }
-        image.swap(timage);
+    std::vector<BatchEntry> out;
+    out.reserve((size_t)batch_nnz(p));
+    for (const BlockEntry& e : p.block)
+        if (batch_jm(p) == ql::JM_BLOCK || e.konst != 0.0 || e.vals) out.push_back({e, (int32_t)out.size()});
+    if (p.kin) {
+        static const int COL[8] = {0, 1, 3, 4, 0, 1, 5, 6};
+        for (int k = 1; k <= c.N; ++k)
+            for (int e = 0; e < 8; ++e)
+                out.push_back({{c.m_nlp + 2 * (k - 1) + (e >> 2) + 1, QL_NZK * (k - 1) + COL[e] + 1, 0.0, false}, -(8 * (k - 1) + e + 1)});
+        std::sort(out.begin(), out.end(), [](const BatchEntry& a, const BatchEntry& b) {
+            return a.v.col != b.v.col ? a.v.col < b.v.col : a.v.row < b.v.row;
+        });
     }
-    return QLNLP_OK;
+    return out;
+}
+
+// The constant image and the VALS positions of a row of the handle's batch pattern
+void batch_image_and_vals_map(const Problem& p, std::vector<double>& image, std::vector<int32_t>& pos)
+{
+    const std::vector<BatchEntry> pat = batch_pattern(p);
+    image.resize(pat.size());
+    pos.clear();
+    for (size_t i = 0; i < pat.size(); ++i) {
+        image[i] = pat[i].v.konst;
+        if (pat[i].v.vals) pos.push_back((int32_t)i);
+    }
 }
 
 // Row plan of the handle's batch pattern.
@@ -517,7 +496,7 @@ int ensure_plan(qlnlp_handle h)
     if (h->plan) return QLNLP_OK;
     std::vector<double> image;
     std::vector<int32_t> pos;
-    if (int rc = batch_image_and_vals_map(h->prob, image, pos)) return rc;
+    batch_image_and_vals_map(h->prob, image, pos);
     h->plan.reset(new (std::nothrow) qlhost::RowPlan((int64_t)image.size(), image.data(), (int64_t)pos.size(), pos.data()));
     if (!h->plan) return fail(QLNLP_ENOMEM, "out of host memory");
     return QLNLP_OK;
@@ -986,35 +965,12 @@ int ragged_table(const qlnlp_handle* hs, int ncls, cudaStream_t stream, const Ra
 }
 
 // ---- opt-in kinematic rows (qlnlp_kin.cuh) ---------------------------------------------------------------------
-// The caller-visible structure of a problem with kinematic rows: the reference's entries + 8 per knot, column-major.
-// map[o] = position in the reference-order row, or -(8 (k-1) + e + 1) for a kinematic entry.
-void kin_structure(const Problem& p, std::vector<int64_t>& rows, std::vector<int64_t>& cols, std::vector<int32_t>& map)
-{
-    const QlClass& c = p.cls;
-    const int n0 = std_nnz(p);
-    std::vector<int64_t> r0((size_t)n0), c0((size_t)n0);
-    if (p.jac_mode == QLNLP_JAC_SPARSE_TRUE) sparse_true_structure(c, r0.data(), c0.data());
-    else sparse_block_structure(c, r0.data(), c0.data());
-    struct Ent { int64_t col, row; int32_t src; };
-    std::vector<Ent> all;
-    all.reserve((size_t)n0 + 8 * (size_t)c.N);
-    for (int i = 0; i < n0; ++i) all.push_back({c0[(size_t)i], r0[(size_t)i], i});
-    static const int COL[8] = {0, 1, 3, 4, 0, 1, 5, 6};
-    for (int k = 1; k <= c.N; ++k)
-        for (int e = 0; e < 8; ++e)
-            all.push_back({(int64_t)QL_NZK * (k - 1) + COL[e] + 1, (int64_t)c.m_nlp + 2 * (k - 1) + (e >> 2) + 1, -(8 * (k - 1) + e + 1)});
-    std::sort(all.begin(), all.end(), [](const Ent& a, const Ent& b) { return a.col != b.col ? a.col < b.col : a.row < b.row; });
-    rows.resize(all.size()); cols.resize(all.size()); map.resize(all.size());
-    for (size_t i = 0; i < all.size(); ++i) { rows[i] = all[i].row; cols[i] = all[i].col; map[i] = all[i].src; }
-}
-
 int ensure_kin(const Problem& p, DeviceState& ds, cudaStream_t stream)
 {
     if (ds.d_kin_map) return QLNLP_OK;
     if (int rc = refuse_setup_in_capture(stream, "kinematic rows")) return rc;
-    std::vector<int64_t> rows, cols;
     std::vector<int32_t> map;
-    kin_structure(p, rows, cols, map);
+    for (const BatchEntry& e : batch_pattern(p)) map.push_back(e.src);
     return upload(ds.d_kin_map, map.data(), map.size());
 }
 
@@ -1199,20 +1155,20 @@ int ensure_kkt_tables(const Problem& p, DeviceState& ds, cudaStream_t stream)
     if (int rc = refuse_setup_in_capture(stream, "KKT solve")) return rc;
     const QlClass& c = p.cls;
     const int nh = ql_hess_nnz(c);
-    std::vector<int64_t> rows(std::max(c.nnz_true, nh)), cols(rows.size());
-    std::vector<unsigned short> tab((size_t)c.nnz_true + nh);
-    sparse_true_structure(c, rows.data(), cols.data());
-    for (int e = 0; e < c.nnz_true; ++e) {
-        const int k = (int)((cols[e] - 1) / QL_NZK) + 1, j = (int)((cols[e] - 1) % QL_NZK);
+    const std::vector<BatchEntry> jac = batch_pattern(p);       // SPARSE_TRUE: the only pattern the KKT solve takes
+    std::vector<unsigned short> tab(jac.size() + nh);
+    for (size_t e = 0; e < jac.size(); ++e) {
+        const int k = (jac[e].v.col - 1) / QL_NZK + 1, j = (jac[e].v.col - 1) % QL_NZK;
         int s = 0;
-        while (s < ql::KKT_SLOTS && ql::kkt_slot_row(c, k, s) != rows[e] - 1) ++s;
-        if (s == ql::KKT_SLOTS) return fail(QLNLP_ECUDA, "internal: Jacobian row %lld has no slot at knot %d", (long long)rows[e], k);
+        while (s < ql::KKT_SLOTS && ql::kkt_slot_row(c, k, s) != jac[e].v.row - 1) ++s;
+        if (s == ql::KKT_SLOTS) return fail(QLNLP_ECUDA, "internal: Jacobian row %d has no slot at knot %d", jac[e].v.row, k);
         tab[e] = (unsigned short)(s | j << 8);
     }
+    std::vector<int64_t> rows(nh), cols(nh);
     hessian_structure(c, rows.data(), cols.data());
     for (int e = 0; e < nh; ++e) {
         const int r = (int)((rows[e] - 1) % QL_NZK), q = (int)((cols[e] - 1) % QL_NZK);
-        tab[(size_t)c.nnz_true + e] = (unsigned short)(std::max(r, q) | std::min(r, q) << 8);
+        tab[jac.size() + e] = (unsigned short)(std::max(r, q) | std::min(r, q) << 8);
     }
     return upload(ds.d_kkt_tab, tab.data(), tab.size());
 }
@@ -1648,11 +1604,8 @@ int eval_dense_jacobian(qlnlp_handle h, const double* x, double* vals)
     return single_call(h, {{x, nullptr, p.cls.n_nlp}, {nullptr, vals, dense_n}, {nullptr, nullptr, nz}}, "dense Jacobian",
                        [&](DeviceState& ds, double* const* d, const int64_t* ld, cudaStream_t s) -> int {
                            if (!ds.d_dense_lin) {          // the position in the grid of every value
-                               std::vector<int64_t> rows((size_t)nz), cols((size_t)nz);
-                               if (p.kin) { std::vector<int32_t> map; kin_structure(p, rows, cols, map); }
-                               else sparse_block_structure(p.cls, rows.data(), cols.data());
-                               std::vector<long long> lin((size_t)nz);
-                               for (int i = 0; i < nz; ++i) lin[(size_t)i] = (rows[(size_t)i] - 1) + (long long)m * (cols[(size_t)i] - 1);
+                               std::vector<long long> lin;
+                               for (const BatchEntry& e : batch_pattern(p)) lin.push_back((e.v.row - 1) + (long long)m * (e.v.col - 1));
                                if (int rc = upload(ds.d_dense_lin, lin.data(), lin.size())) return rc;
                            }
                            qlnlp_batch_io io;
@@ -1697,7 +1650,11 @@ int create_one(const qlnlp_problem_desc* d, const int* devices, int ndev, int ja
         }
         p.cost[(size_t)40 * p.npad + k] = d->c[k];
     }
-    plan_segments(c, p.segs, p.seg_begin);
+    if (int rc = block_plan(c, p.block)) {
+        delete h;
+        return rc;
+    }
+    plan_segments(c, p.block, p.segs, p.seg_begin);
     p.rmb = 1.0 / c.mb;
     p.rmf = 1.0 / c.mf;
     p.rIb = 1.0 / c.Ib;
@@ -1936,16 +1893,8 @@ int qlnlp_jacobian_structure(qlnlp_handle h, int64_t* rows, int64_t* cols)
         int64_t n = 0;
         for (int64_t col = 1; col <= p.cls.n_nlp; ++col)
             for (int64_t row = 1; row <= m_rows(p); ++row) { rows[n] = row; cols[n] = col; ++n; }
-    } else if (p.kin) {
-        std::vector<int64_t> r, c;
-        std::vector<int32_t> map;
-        kin_structure(p, r, c, map);
-        std::copy(r.begin(), r.end(), rows);
-        std::copy(c.begin(), c.end(), cols);
-    } else if (p.jac_mode == QLNLP_JAC_SPARSE_TRUE) {
-        sparse_true_structure(p.cls, rows, cols);
     } else {
-        sparse_block_structure(p.cls, rows, cols);
+        for (const BatchEntry& e : batch_pattern(p)) { *rows++ = e.v.row; *cols++ = e.v.col; }
     }
     return QLNLP_OK;
 }
@@ -2579,7 +2528,7 @@ int qlnlp_debug_vals_map(qlnlp_handle h, int32_t* pos, int64_t cap, int64_t* n)
     if (int rc = check_handle(h)) return rc;
     std::vector<double> image;
     std::vector<int32_t> p;
-    if (int rc = batch_image_and_vals_map(h->prob, image, p)) return rc;
+    batch_image_and_vals_map(h->prob, image, p);
     if (n) *n = (int64_t)p.size();
     if (pos)
         for (size_t i = 0; i < p.size() && (int64_t)i < cap; ++i) pos[i] = p[i];
