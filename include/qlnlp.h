@@ -312,6 +312,48 @@ typedef struct {
  * px[i] and pl[i] of a row with status != 0 are written as NaN.  DEVICE pointers, enqueued on `stream`. */
 int qlnlp_kkt_solve_factored_batch_device(qlnlp_handle h, int64_t R, const qlnlp_kkt_rhs_io* io, void* stream);
 
+/* Accuracy.  The step comes from the condensed form M, which loses what W + diag(sx) holds below eps ||J' D^-1 J||: px
+ * loses digits when dc is small relative to ||J||^2 / ||W + diag(sx)||, and pl with it.  Measured on a B200 against an
+ * extended-precision solve of K (tests/test_gpu_kkt_accuracy.py, DESIGN.md section 5), errors relative to the largest
+ * entry of each block, N = 2 .. 1024:
+ *   normwise backward error ||r - K z||_inf / (||K||_inf ||z||_inf + ||r||_inf), z = [px; pl]: <= 1e-13 with dc_eq >=
+ *     1e-6 and inequality dc in [1e-2, 1]; up to 5e-12 at smaller dc_eq, and up to 7e-11 when the inequality dc span
+ *     1e-10 .. 1e2 (an active set).  The one-shot and factored solves are not backward stable at such scalings.
+ *   px: 1e-14 at dc >= 1e-2 (sx in [1, 10]); 3e-10 at dc_eq = 1e-6; 2e-6 at dc_eq = 1e-8 with sx over 1e-8 .. 1e8;
+ *     4e-4 at dc_eq = 1e-12, and no digit at all with an active set and wide sx.
+ * Iterative refinement with the residual below and the kept factor (HybridNLP.kkt_solve_refined_batch, 3 steps) brings
+ * px and pl to 1e-14 and the componentwise backward error to 3.2e-16 wherever dc_eq >= 1e-8 (2 steps: up to 4.9e-14).
+ * At dc_eq <= 1e-10 each step gains only 1 .. 3 digits although Skeel's condition of K times eps is 1e-15 there: the
+ * condensed factor, not K, limits it.  Where the factor is too far from K (dc_eq = 1e-12 with an active set and wide sx)
+ * refinement diverges; the refined solve keeps a step only when it halves the componentwise backward error, so it
+ * returns the unrefined step there, which has no correct digit.
+ *
+ * Residual of the system: s1 = r1 - (W + diag(sx)) px - J' pl,  s2 = r2 - J px + dc .* pl, for B problems, with W, J,
+ * sx, dc as the solve takes them.  Each entry is the left fold, starting from r, of fused multiply-adds
+ * acc = RN(acc - a * v), one per term, in this order:
+ *   s1_i  the row of i's knot block of W (mirrored) in ascending column order, its diagonal entry rounded once as
+ *         RN(W_ii + sx_i); then J' pl over the rows that touch i's knot in the order of kkt_slot_row (qlnlp_kkt.cuh);
+ *   s2_r  row r's entries in ascending column order (a defect row: the RK4 block's 20 columns, then -x_(k+1)), then
+ *         + dc_r pl_r.
+ * The knot-local blocks may hold structural zeros; they add exact zeros for finite px and pl.  The result is within
+ * gamma_t (|r| + |K| |z|) of the exact residual, t = 1 + the structural terms of the entry (at most 56 in s1, 23 in
+ * s2), and its bits do not depend on B, the batch position, leading dimensions or alignment.  NaN in px or pl (a failed
+ * solve's rows) gives NaN residual rows.  DEVICE pointers, 8-byte aligned, enqueued on `stream`; the handles the KKT
+ * solve refuses are refused. */
+typedef struct {
+    const double* hess; int64_t ldhess;   /* [B][ldhess >= nnz_hess] */
+    const double* jac;  int64_t ldjac;    /* [B][ldjac  >= nnz (SPARSE_TRUE)] */
+    const double* sx;   int64_t ldsx;     /* [B][ldsx   >= n_nlp]   or NULL */
+    const double* dc;   int64_t lddc;     /* [B][lddc   >= m_nlp] */
+    const double* r1;   int64_t ldr1;     /* [B][ldr1   >= n_nlp] */
+    const double* r2;   int64_t ldr2;     /* [B][ldr2   >= m_nlp] */
+    const double* px;   int64_t ldpx;     /* [B][ldpx   >= n_nlp] */
+    const double* pl;   int64_t ldpl;     /* [B][ldpl   >= m_nlp] */
+    double* s1;         int64_t lds1;     /* [B][lds1   >= n_nlp] */
+    double* s2;         int64_t lds2;     /* [B][lds2   >= m_nlp] */
+} qlnlp_kkt_residual_io;
+int qlnlp_kkt_residual_batch_device(qlnlp_handle h, int64_t B, const qlnlp_kkt_residual_io* io, void* stream);
+
 /* Ragged batches: problems of different size (several handles = several (N, k_trans, init_mode) classes) packed
  * back to back in flat arrays.  One call evaluates the B problems of THIS handle's class; the b-th of them is problem
  * number i = index[b] (or b when index is NULL) of the flat batch and its rows start at

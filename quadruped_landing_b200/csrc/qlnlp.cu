@@ -442,6 +442,7 @@ KernelSpec hess_spec(const Problem& p, bool prod)
 KernelSpec kkt_spec() { return {(const void*)ql::kkt_kernel, 0, 0, false, false, true}; }
 KernelSpec kkt_factor_spec() { return {(const void*)ql::kkt_factor_kernel, 0, 0, false, false, true}; }
 KernelSpec kkt_solve_factored_spec() { return {(const void*)ql::kkt_solve_factored_kernel, 0, 0, false, false, true}; }
+KernelSpec kkt_residual_spec() { return {(const void*)ql::kkt_residual_kernel, 0, 0, false, false, true}; }
 
 // the sparse pattern batched evaluations of this problem produce (DENSE handles batch in SPARSE_BLOCK)
 int batch_jm(const Problem& p) { return p.jac_mode == QLNLP_JAC_SPARSE_TRUE ? ql::JM_TRUE : ql::JM_BLOCK; }
@@ -1278,6 +1279,52 @@ int launch_kkt_solve_factored(const Problem& p, DeviceState& ds, int64_t R, cons
     P.status = io->status;
     P.B = R;
     return launch_kernel(ds, kkt_solve_factored_spec(), R, P, stream);
+}
+
+int check_kkt_residual(const Problem& p, int64_t B, const qlnlp_kkt_residual_io* io)
+{
+    const QlClass& c = p.cls;
+    if (B < 0) return fail(QLNLP_EINVAL, "negative batch");
+    if (!io || !io->hess || !io->jac || !io->dc || !io->r1 || !io->r2 || !io->px || !io->pl || !io->s1 || !io->s2)
+        return fail(QLNLP_EINVAL, "io, hess, jac, dc, r1, r2, px, pl, s1 and s2 are required");
+    const int64_t n = c.n_nlp, m = c.m_nlp;
+    if (io->ldhess < ql_hess_nnz(c)) return fail(QLNLP_EINVAL, "ldhess %lld < nnz_hess %d", (long long)io->ldhess, ql_hess_nnz(c));
+    if (io->ldjac < c.nnz_true) return fail(QLNLP_EINVAL, "ldjac %lld < nnz %d", (long long)io->ldjac, c.nnz_true);
+    if (io->sx && io->ldsx < n) return fail(QLNLP_EINVAL, "ldsx %lld < n_nlp %lld", (long long)io->ldsx, (long long)n);
+    if (io->ldr1 < n || io->ldpx < n || io->lds1 < n)
+        return fail(QLNLP_EINVAL, "ldr1 %lld / ldpx %lld / lds1 %lld < n_nlp %lld", (long long)io->ldr1, (long long)io->ldpx,
+                    (long long)io->lds1, (long long)n);
+    if (io->lddc < m || io->ldr2 < m || io->ldpl < m || io->lds2 < m)
+        return fail(QLNLP_EINVAL, "lddc %lld / ldr2 %lld / ldpl %lld / lds2 %lld < m_nlp %lld", (long long)io->lddc,
+                    (long long)io->ldr2, (long long)io->ldpl, (long long)io->lds2, (long long)m);
+    for (const void* a : {(const void*)io->hess, (const void*)io->jac, (const void*)io->sx, (const void*)io->dc,
+                          (const void*)io->r1, (const void*)io->r2, (const void*)io->px, (const void*)io->pl,
+                          (const void*)io->s1, (const void*)io->s2})
+        if ((reinterpret_cast<uintptr_t>(a) & 7) != 0) return fail(QLNLP_EINVAL, "arrays must be 8-byte aligned");
+    return QLNLP_OK;
+}
+
+int launch_kkt_residual(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_kkt_residual_io* io, cudaStream_t stream)
+{
+    const QlClass& c = p.cls;
+    if (int rc = ensure_kkt_tables(p, ds, stream)) return rc;
+    ql::KktResidualLaunch P;
+    std::memset(&P, 0, sizeof P);
+    P.c = c;
+    P.jtab = ds.d_kkt_tab.get();
+    P.htab = ds.d_kkt_tab.get() + c.nnz_true;
+    P.hess = io->hess; P.ldhess = io->ldhess;
+    P.jac = io->jac; P.ldjac = io->ldjac;
+    P.sx = io->sx; P.ldsx = io->ldsx;
+    P.dc = io->dc; P.lddc = io->lddc;
+    P.r1 = io->r1; P.ldr1 = io->ldr1;
+    P.r2 = io->r2; P.ldr2 = io->ldr2;
+    P.px = io->px; P.ldpx = io->ldpx;
+    P.pl = io->pl; P.ldpl = io->ldpl;
+    P.s1 = io->s1; P.lds1 = io->lds1;
+    P.s2 = io->s2; P.lds2 = io->lds2;
+    P.B = B;
+    return launch_kernel(ds, kkt_residual_spec(), B, P, stream);
 }
 
 // A row of a single call: n doubles, copied in from `in` before the launch and / or back to `out` after it
@@ -2349,6 +2396,17 @@ int qlnlp_kkt_solve_factored_batch_device(qlnlp_handle h, int64_t R, const qlnlp
     DeviceGuard guard(ds.device);
     if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
     return launch_kkt_solve_factored(h->prob, ds, R, io, static_cast<cudaStream_t>(stream));
+}
+
+int qlnlp_kkt_residual_batch_device(qlnlp_handle h, int64_t B, const qlnlp_kkt_residual_io* io, void* stream)
+{
+    if (int rc = check_kkt_handle(h)) return rc;
+    if (B == 0) return QLNLP_OK;
+    if (int rc = check_kkt_residual(h->prob, B, io)) return rc;
+    DeviceState& ds = h->devs[0];
+    DeviceGuard guard(ds.device);
+    if (int rc = ensure_device(h->prob, ds, static_cast<cudaStream_t>(stream))) return rc;
+    return launch_kkt_residual(h->prob, ds, B, io, static_cast<cudaStream_t>(stream));
 }
 
 // J w (transpose: J' y) at x for one evaluation

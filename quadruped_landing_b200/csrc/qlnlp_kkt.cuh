@@ -112,6 +112,24 @@ struct KktSolveLaunch {
     unsigned* ticket;
 };
 
+struct KktResidualLaunch {
+    QlClass c;
+    const unsigned short* jtab;
+    const unsigned short* htab;
+    const double* hess; long long ldhess;
+    const double* jac; long long ldjac;
+    const double* sx; long long ldsx;    // or nullptr: 0
+    const double* dc; long long lddc;
+    const double* r1; long long ldr1;
+    const double* r2; long long ldr2;
+    const double* px; long long ldpx;
+    const double* pl; long long ldpl;
+    double* s1; long long lds1;
+    double* s2; long long lds2;
+    long long B;
+    unsigned* ticket;
+};
+
 // The warp's working set of one knot: references to the kernel's own __shared__ arrays (QL_KKT_SHARED).  Declared
 // as separate arrays, not as one struct, so that kkt_kernel keeps the shared-memory layout and the register
 // allocation it had before the per-knot steps became functions (one struct: 108 registers instead of 168).
@@ -543,6 +561,72 @@ __global__ void __launch_bounds__(QL_LANES, 8) kkt_solve_factored_kernel(const _
         if (status != 0) kkt_fill_nan(c, px, pl, lane);
         if (lane == 0) P.status[b] = status;
         __syncwarp();
+        b = take_get(tkt);
+    }
+    kkt_rearm(P.ticket, lane);
+}
+
+// Residual of the system a solve was asked for, with the matrix the solve read (qlnlp_kkt_residual_batch_device):
+//   s1 = r1 - (W + diag(sx)) px - J' pl,   s2 = r2 - J px + dc .* pl.
+// Knots from N down to 1, as the backward sweep: knot k's G and W block gathered (with pl in place of r2, so r2s holds
+// pl of each slot), lane a folds s1 of knot k's variable a, and the rows that close at knot k (kkt_backward's) fold s2,
+// a defect row of step k taking the -I of knot k+1 from en, kept from the previous knot.  Each entry is a left fold of
+// fused multiply-adds from r, in the order include/qlnlp.h states; W_aa + sx_a is rounded once first, as K holds it.
+__global__ void __launch_bounds__(QL_LANES, 8) kkt_residual_kernel(const __grid_constant__ KktResidualLaunch P)
+{
+    QL_KKT_SHARED(S);
+    const QlClass& c = P.c;
+    const int lane = threadIdx.x;
+    const unsigned full = 0xffffffffu;
+
+    auto take_issue = [&]() -> unsigned { return lane == 0 ? atomicAdd(P.ticket, 1u) : 0u; };
+    auto take_get = [&](unsigned t) -> long long { return (long long)__shfl_sync(full, t, 0); };
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    long long b = take_get(take_issue());
+    while (b < P.B) {
+        const unsigned tkt = take_issue();
+        const double* const W = P.hess + b * P.ldhess;
+        const double* const J = P.jac + b * P.ldjac;
+        const double* const sx = P.sx ? P.sx + b * P.ldsx : nullptr;
+        const double* const dc = P.dc + b * P.lddc;
+        const double* const r1 = P.r1 + b * P.ldr1;
+        const double* const r2 = P.r2 + b * P.ldr2;
+        const double* const px = P.px + b * P.ldpx;
+        const double* const pl = P.pl + b * P.ldpl;
+        double* const s1 = P.s1 + b * P.lds1;
+        double* const s2 = P.s2 + b * P.lds2;
+
+        for (int k = c.N; k >= 1; --k) {
+            const int nk = k < c.N ? QL_NZK : QL_NX;
+            const int z0 = QL_NZK * (k - 1);
+            kkt_gather<true>(S, c, P.jtab, P.htab, J, dc, pl, W, k, lane);
+            if (lane < nk) S.xv[lane] = px[z0 + lane];
+            __syncwarp();
+            if (lane < nk) {               // s1: W row (mirrored, diagonal with sx), then J' column, slot by slot
+                double acc = r1[z0 + lane];
+                for (int j = 0; j < nk; ++j) {
+                    double w = j <= lane ? S.Ms[lane][j] : S.Ms[j][lane];
+                    if (j == lane && sx) w = __dadd_rn(w, sx[z0 + j]);
+                    acc = __fma_rn(-w, S.xv[j], acc);
+                }
+                for (int s = 0; s < KKT_SLOTS; ++s) acc = __fma_rn(-S.G[s][lane], S.r2s[s], acc);
+                s1[z0 + lane] = acc;
+            }
+#pragma unroll 1
+            for (int s = lane; s < KKT_SLOTS; s += QL_LANES) {     // s2: knot k's columns, the -I of knot k+1, dc pl
+                const int r = (s < QL_NX || s >= 2 * QL_NX || k == 1) ? kkt_slot_row(c, k, s) : -1;
+                if (r >= 0) {
+                    double acc = r2[r];
+                    for (int j = 0; j < nk; ++j) acc = __fma_rn(-S.G[s][j], S.xv[j], acc);
+                    if (s < QL_NX && k < c.N) acc = __fma_rn(-S.en[s], px[z0 + QL_NZK + s], acc);
+                    s2[r] = __fma_rn(S.dcs[s], S.r2s[s], acc);
+                }
+            }
+            __syncwarp();
+            if (lane < QL_NX) S.en[lane] = S.G[QL_NX + lane][lane];
+            __syncwarp();
+        }
         b = take_get(tkt);
     }
     kkt_rearm(P.ticket, lane);

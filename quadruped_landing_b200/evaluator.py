@@ -43,7 +43,7 @@ EXPORTED_SYMBOLS = (
     "qlnlp_eval_constraint_jacobian_product", "qlnlp_eval_constraint_jacobian_transpose_product",
     "qlnlp_eval_hessian_lagrangian_product",
     "qlnlp_kkt_solve_batch_device", "qlnlp_kkt_factor_size", "qlnlp_kkt_factor_batch_device",
-    "qlnlp_kkt_solve_factored_batch_device",
+    "qlnlp_kkt_solve_factored_batch_device", "qlnlp_kkt_residual_batch_device",
     "qlnlp_device_alloc", "qlnlp_device_free", "qlnlp_device_alloc_info",
 )
 _DEBUG_SYMBOLS = ("qlnlp_debug_segments", "qlnlp_debug_vals_map", "qlnlp_debug_build_rows", "qlnlp_debug_host_times",
@@ -100,6 +100,14 @@ class _KktRhsIO(C.Structure):
                 ("r1", C.c_void_p), ("ldr1", C.c_int64), ("r2", C.c_void_p), ("ldr2", C.c_int64),
                 ("px", C.c_void_p), ("ldpx", C.c_int64), ("pl", C.c_void_p), ("ldpl", C.c_int64),
                 ("status", C.c_void_p)]
+
+
+class _KktResidualIO(C.Structure):
+    _fields_ = [("hess", C.c_void_p), ("ldhess", C.c_int64), ("jac", C.c_void_p), ("ldjac", C.c_int64),
+                ("sx", C.c_void_p), ("ldsx", C.c_int64), ("dc", C.c_void_p), ("lddc", C.c_int64),
+                ("r1", C.c_void_p), ("ldr1", C.c_int64), ("r2", C.c_void_p), ("ldr2", C.c_int64),
+                ("px", C.c_void_p), ("ldpx", C.c_int64), ("pl", C.c_void_p), ("ldpl", C.c_int64),
+                ("s1", C.c_void_p), ("lds1", C.c_int64), ("s2", C.c_void_p), ("lds2", C.c_int64)]
 
 
 class _RaggedIO(C.Structure):
@@ -176,6 +184,7 @@ def load_library(rebuild_if_stale: bool = True):
     L.qlnlp_kkt_factor_size.argtypes = [vp, i64p]
     L.qlnlp_kkt_factor_batch_device.argtypes = [vp, C.c_int64, C.POINTER(_KktFactorIO), vp]
     L.qlnlp_kkt_solve_factored_batch_device.argtypes = [vp, C.c_int64, C.POINTER(_KktRhsIO), vp]
+    L.qlnlp_kkt_residual_batch_device.argtypes = [vp, C.c_int64, C.POINTER(_KktResidualIO), vp]
     L.qlnlp_host_alloc.argtypes = [C.c_int64, C.POINTER(vp)]
     L.qlnlp_host_free.argtypes = [vp, C.c_int64]
     L.qlnlp_device_alloc.argtypes = [vp, C.c_int64, C.POINTER(vp)]
@@ -670,6 +679,91 @@ class HybridNLP:
         io.status = status.data_ptr()
         s = torch.cuda.current_stream(dev) if stream is None else stream
         _check(load_library().qlnlp_kkt_solve_factored_batch_device(self._h, R, C.byref(io), C.c_void_p(s.cuda_stream)))
+        return px, pl, status
+
+    def kkt_residual_batch(self, hess, jac, dc, px, pl, r1, r2, sx=None, out=None, stream=None):
+        """Device tensors as ``kkt_solve_batch``, with a step ``px[B, n_nlp]``, ``pl[B, m_nlp]`` -> ``(s1[B, n_nlp],
+        s2[B, m_nlp])``, the residual ``s1 = r1 - (W + diag(sx)) px - J' pl``, ``s2 = r2 - J px + dc * pl`` in the fixed
+        summation order of include/qlnlp.h.  ``out`` may give both outputs.  Enqueued on the current torch stream (or
+        ``stream``), not synchronised."""
+        import torch
+
+        B = hess.shape[0]
+        n, m = self.n_nlp, self.m_nlp
+        _check_rows(B, ((hess, self.nnz_hess, "hess"), (jac, self.nnz, "jac"), (dc, m, "dc"), (px, n, "px"),
+                        (pl, m, "pl"), (r1, n, "r1"), (r2, m, "r2"), (sx, n, "sx")))
+        dev = hess.device
+        if out is None:
+            out = tuple(_device_empty(dev.index, [(B, n, torch.float64), (B, m, torch.float64)], self._compressible))
+        s1, s2 = out
+        _check_rows(B, ((s1, n, "out s1"), (s2, m, "out s2")))
+        ld = lambda t, wd: t.stride(0) if B > 1 else wd
+        io = _KktResidualIO()
+        io.hess, io.ldhess = hess.data_ptr(), ld(hess, self.nnz_hess)
+        io.jac, io.ldjac = jac.data_ptr(), ld(jac, self.nnz)
+        if sx is not None:
+            io.sx, io.ldsx = sx.data_ptr(), ld(sx, n)
+        io.dc, io.lddc = dc.data_ptr(), ld(dc, m)
+        io.r1, io.ldr1 = r1.data_ptr(), ld(r1, n)
+        io.r2, io.ldr2 = r2.data_ptr(), ld(r2, m)
+        io.px, io.ldpx = px.data_ptr(), ld(px, n)
+        io.pl, io.ldpl = pl.data_ptr(), ld(pl, m)
+        io.s1, io.lds1 = s1.data_ptr(), ld(s1, n)
+        io.s2, io.lds2 = s2.data_ptr(), ld(s2, m)
+        s = torch.cuda.current_stream(dev) if stream is None else stream
+        _check(load_library().qlnlp_kkt_residual_batch_device(self._h, B, C.byref(io), C.c_void_p(s.cuda_stream)))
+        return s1, s2
+
+    def kkt_solve_refined_batch(self, hess, jac, dc, r1, r2, sx=None, steps=3, out=None, stream=None):
+        """The step of ``kkt_solve_batch`` followed by ``steps`` rounds of iterative refinement against the kept factor:
+        factored solve of the residual of K (``kkt_residual_batch``), ``px + dpx``, ``pl + dpl``.  The condensed solve
+        loses digits of px when dc is small (include/qlnlp.h, "Accuracy"); refinement restores them where the factor is
+        close enough to K.  Where it is not, refinement can diverge, so each row keeps its new iterate only when that
+        iterate's componentwise backward error max_i |r - K z|_i / (|r| + |K| |z|)_i is at most half the kept one's (a
+        rejected row then repeats the same step; near convergence only steps at rounding level are refused): the
+        result's is never larger than the unrefined step's.  The
+        denominator comes from the residual kernel on absolute values, one more launch per step, and takes copies of
+        |hess| and |jac| for the call.  With ``steps = 0`` the result has the bits
+        of ``kkt_solve_batch``.  Same arguments and outputs as ``kkt_solve_batch``; status is the factor's, and rows with
+        a non-zero status stay NaN.  Everything is enqueued on the current torch stream (or ``stream``) with no host
+        synchronisation, so the chain can be captured in a graph."""
+        import torch
+
+        if steps < 0:
+            raise ValueError("steps must be >= 0")
+        B = hess.shape[0]
+        n, m = self.n_nlp, self.m_nlp
+        dev = hess.device
+        s = torch.cuda.current_stream(dev) if stream is None else stream
+        with torch.cuda.stream(s):
+            factor, _ = self.kkt_factor_batch(hess, jac, dc, sx=sx, stream=s)
+            px, pl, status = self.kkt_solve_factored_batch(factor, r1, r2, out=out, stream=s)
+            if steps:
+                s1, s2, dpx, dpl, qx, ql, t1, t2, a1, a2 = (torch.empty((B, w), dtype=torch.float64, device=dev)
+                                                            for w in (n, m, n, m, n, m, n, m, n, m))
+                dst = torch.empty((B,), dtype=torch.int32, device=dev)
+                # |r| + |K| |z| by the same kernel: with |W|, |J|, -dc, -|px|, -|pl|, |r1|, |r2| every term of its fold
+                # is non-negative (the diagonal is RN(|W_ii| + sx_i) >= |W_ii + sx_i|)
+                ah, aj, ndc, ar1, ar2 = hess.abs(), jac.abs(), -dc, r1.abs(), r2.abs()
+
+                def omega(x, y, u, v):
+                    """componentwise backward error max_i |s_i| / (|r| + |K| |z|)_i of z = [x; y] with residual [u; v]"""
+                    self.kkt_residual_batch(ah, aj, ndc, -x.abs(), -y.abs(), ar1, ar2, sx=sx, out=(a1, a2), stream=s)
+                    return torch.maximum((u.abs() / a1.clamp_min(1e-300)).amax(dim=1),
+                                         (v.abs() / a2.clamp_min(1e-300)).amax(dim=1))
+
+                self.kkt_residual_batch(hess, jac, dc, px, pl, r1, r2, sx=sx, out=(s1, s2), stream=s)
+                kept = omega(px, pl, s1, s2)
+                for _ in range(steps):
+                    self.kkt_solve_factored_batch(factor, s1, s2, out=(dpx, dpl, dst), stream=s)
+                    torch.add(px, dpx, out=qx)
+                    torch.add(pl, dpl, out=ql)
+                    self.kkt_residual_batch(hess, jac, dc, qx, ql, r1, r2, sx=sx, out=(t1, t2), stream=s)
+                    new = omega(qx, ql, t1, t2)
+                    take = new < 0.5 * kept             # False for NaN rows: a failed factor's rows stay NaN
+                    for old, cand in ((px, qx), (pl, ql), (s1, t1), (s2, t2)):
+                        old.copy_(torch.where(take[:, None], cand, old))
+                    kept = torch.where(take, new, kept)
         return px, pl, status
 
     def initialize(self, features: Iterable[str] = ()) -> None:

@@ -61,6 +61,8 @@ class Case:
 @pytest.mark.parametrize("N,kt,im", [(2, 2, 1), (2, 1, 2), (5, 3, 1), (33, 1, 2), (61, 21, 1), (61, 21, 2),
                                      (1024, 1000, 1)])
 def test_step_solves_the_kkt_system(N, kt, im):
+    """At Case's mild scalings (dc in [1e-2, 1], sx in [1, 10]), where the one-shot step's normwise backward error is
+    1e-12 or better.  It is not at interior-point scalings: tests/test_gpu_kkt_accuracy.py has that envelope."""
     B = 3 if N > 100 else 8
     cs = Case(N, kt, im, B, seed=N + kt)
     px, pl, st = cs.solve()

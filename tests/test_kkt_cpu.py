@@ -72,6 +72,46 @@ def test_argument_checks_need_no_device():
         assert call(1, sx=None, ldsx=0) == ev.QLNLP_ENODEVICE                          # sx is optional
 
 
+def test_residual_argument_checks_need_no_device():
+    """qlnlp_kkt_residual_batch_device: the solve's inputs plus px, pl in and s1, s2 out, each with its own leading
+    dimension; the handles the KKT solve refuses are refused."""
+    prob = build_problem(N=5, k_trans=3)
+    nlp = HybridNLP.from_problem(prob, pattern="true")
+    L = ql.load_library()
+    n, m = nlp.n_nlp, nlp.m_nlp
+    widths = (("hess", nlp.nnz_hess), ("jac", nlp.nnz), ("sx", n), ("dc", m), ("r1", n), ("r2", m), ("px", n), ("pl", m),
+              ("s1", n), ("s2", m))
+    arrays = {name: np.zeros(w + 2) for name, w in widths}
+
+    def call(B, h=nlp, **kw):
+        io = ev._KktResidualIO(*[v for name, w in widths for v in (_ptr(arrays[name]), w)])
+        for k, v in kw.items():
+            setattr(io, k, v)
+        return L.qlnlp_kkt_residual_batch_device(h._h, B, C.byref(io), None)
+
+    assert L.qlnlp_kkt_residual_batch_device(nlp._h, 0, None, None) == ev.QLNLP_OK
+    assert L.qlnlp_kkt_residual_batch_device(nlp._h, 1, None, None) == ev.QLNLP_EINVAL
+    assert call(-1) == ev.QLNLP_EINVAL
+    for name in ("hess", "jac", "dc", "r1", "r2", "px", "pl", "s1", "s2"):
+        assert call(1, **{name: None}) == ev.QLNLP_EINVAL, name
+    for name, w in widths:
+        assert call(2, **{"ld" + name: w - 1}) == ev.QLNLP_EINVAL, name
+        assert "ld" + name in L.qlnlp_last_error().decode(), name
+    for name, _ in widths:
+        assert call(1, **{name: _ptr(arrays[name]) + 4}) == ev.QLNLP_EINVAL, name       # misaligned
+    block = HybridNLP.from_problem(prob, pattern="block")
+    dense = HybridNLP.from_problem(prob, use_sparse_jacobian=False)
+    kin = HybridNLP.from_problem(prob, pattern="true", kinematics=True)
+    multi = HybridNLP.from_problem(prob, pattern="true", devices=[0])
+    for h, what in ((block, "SPARSE_TRUE"), (dense, "SPARSE_TRUE"), (kin, "kinematic"), (multi, "multi-device")):
+        assert call(1, h=h) == ev.QLNLP_EINVAL
+        assert what in L.qlnlp_last_error().decode()
+        assert call(0, h=h) == ev.QLNLP_EINVAL
+    if not _has_gpu():
+        assert call(1) == ev.QLNLP_ENODEVICE
+        assert call(1, sx=None, ldsx=0) == ev.QLNLP_ENODEVICE
+
+
 def _random_problem(nlp, seed, sigma_scale=1.0):
     """W and J with random values on the handle's structures, and positive diagonals."""
     rng = np.random.default_rng(seed)

@@ -3,7 +3,8 @@ a CPU baseline in the same process: scipy factorising the same problems one by o
 matrix) on all host cores, over a sample.  Then the factor / solve split in the same process: kkt_factor_kernel alone,
 kkt_solve_factored_kernel with one right-hand side per factor (R = B) and with four per factor through `index`
 (R = 4B), each launch alternating with a one-shot solve, and one factorisation plus two factored solves against two
-one-shot solves.
+one-shot solves.  The cost of one refinement step of kkt_solve_refined_batch: kkt_residual_kernel alone, and residual +
+factored solve + the two device adds (px += dpx, pl += dpl) as one timed call.
 
 Inputs: C3-style decision vectors (device-built guesses of the drop-height x pitch sweep, perturbed), seeded
 multipliers (scale 1e-4), objective factor 1e-4 (at 1 the objective's x-h second derivatives make these M
@@ -105,6 +106,18 @@ def solve_bytes(nlp):
     return 8 * nlp.kkt_factor_size + 8 * (n + m) + 16 * n + 8 * (n + m)
 
 
+def residual_flops(N, m):
+    """kkt_residual_kernel per problem: one fused multiply-add per term of every entry (2 flops), the knot-local
+    structural zeros included: s1 folds its knot's W row and 34 slots, s2 at most 20 columns + the -I + dc."""
+    return sum(2 * nk * (nk + 34 + 1) for nk in [20] * (N - 1) + [15]) + 2 * m * 22
+
+
+def residual_bytes(nlp):
+    """kkt_residual_kernel per problem: W, J, sx, dc, r1, r2, px, pl read once, s1, s2 written once."""
+    n, m = nlp.n_nlp, nlp.m_nlp
+    return 8 * (nlp.nnz_hess + nlp.nnz + n + m) + 8 * 3 * (n + m)
+
+
 def _cpu_solve(args):
     hs, hv, js, jv, sx, dc, r1, r2 = args
     n, m = len(sx), len(dc)
@@ -132,13 +145,25 @@ def split(a, log, nlp, B, hess, jac, dc, sx, r1, r2, out, gen):
     fac = nlp.kkt_factor_batch(hess, jac, dc, sx=sx)
     one = nlp.kkt_solve_factored_batch(fac[0], r1, r2)
     four = nlp.kkt_solve_factored_batch(fac[0], q1, q2, index=index)
+    res = nlp.kkt_residual_batch(hess, jac, dc, one[0], one[1], r1, r2, sx=sx)
+    cor = nlp.kkt_solve_factored_batch(fac[0], res[0], res[1])
+    px, pl = one[0].clone(), one[1].clone()
     torch.cuda.synchronize()
     same = all(torch.equal(x, y) for x, y in zip(one, out))
+
+    def refine_step():
+        nlp.kkt_residual_batch(hess, jac, dc, px, pl, r1, r2, sx=sx, out=res)
+        nlp.kkt_solve_factored_batch(fac[0], res[0], res[1], out=cor)
+        px.add_(cor[0])
+        pl.add_(cor[1])
+
     calls = {
         "one-shot": lambda: nlp.kkt_solve_batch(hess, jac, dc, r1, r2, sx=sx, out=out),
         "factor": lambda: nlp.kkt_factor_batch(hess, jac, dc, sx=sx, out=fac),
         "solve R=B": lambda: nlp.kkt_solve_factored_batch(fac[0], r1, r2, out=one),
         "solve R=4B": lambda: nlp.kkt_solve_factored_batch(fac[0], q1, q2, index=index, out=four),
+        "residual": lambda: nlp.kkt_residual_batch(hess, jac, dc, one[0], one[1], r1, r2, sx=sx, out=res),
+        "refine step": refine_step,
     }
     for f in calls.values():
         f()
@@ -158,7 +183,11 @@ def split(a, log, nlp, B, hess, jac, dc, sx, r1, r2, out, gen):
         med[k] = ms[len(ms) // 2]
         rows = R4 if k == "solve R=4B" else B
         per = {"one-shot": (stream_bytes(nlp) + scratch_bytes(nlp.N), kernel_flops(nlp.N)),
-               "factor": (factor_bytes(nlp), factor_flops(nlp.N))}.get(k, (solve_bytes(nlp), solve_flops(nlp.N)))
+               "factor": (factor_bytes(nlp), factor_flops(nlp.N)),
+               "residual": (residual_bytes(nlp), residual_flops(nlp.N, nlp.m_nlp)),
+               "refine step": (residual_bytes(nlp) + solve_bytes(nlp) + 8 * 3 * (nlp.n_nlp + nlp.m_nlp),
+                               residual_flops(nlp.N, nlp.m_nlp) + solve_flops(nlp.N))}.get(
+                   k, (solve_bytes(nlp), solve_flops(nlp.N)))
         rate = rows / (med[k] * 1e-3)
         bw, fr = per[0] * rate / 1e12, per[1] * rate / 1e12
         log(f"  B={B} {k:>10}: {med[k]:.3f} ms median (min {ms[0]:.3f}, max {ms[-1]:.3f}) over {a.iters} alternating "
@@ -172,7 +201,11 @@ def split(a, log, nlp, B, hess, jac, dc, sx, r1, r2, out, gen):
     log(f"  B={B}: factor + 2 factored solves {split_ms:.3f} ms vs 2 one-shot solves {two:.3f} ms "
         f"({'faster' if split_ms < two else 'NOT faster'}: {two / split_ms:.2f}x); a factored solve costs "
         f"{med['solve R=B'] / med['one-shot']:.3f} of a one-shot solve, the factor {med['factor'] / med['one-shot']:.3f}")
-    del fac, one, four, q1, q2
+    log(f"  B={B}: one refinement step (residual + factored solve + 2 adds) {med['refine step']:.3f} ms = "
+        f"{med['refine step'] / med['one-shot']:.3f} of a one-shot solve; the residual alone {med['residual']:.3f} ms; "
+        f"3-step refined solve ~ factor + {1 + 3} factored solves + 3 residuals = "
+        f"{med['factor'] + med['solve R=B'] + 3 * med['refine step']:.3f} ms")
+    del fac, one, four, q1, q2, res, cor, px, pl
 
 
 def main():
