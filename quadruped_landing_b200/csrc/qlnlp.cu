@@ -901,12 +901,7 @@ int launch(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_batch_io* i
     P.nseg = (int)p.segs.size();
     P.segs = ds.d_segs.get();
     P.seg_begin = ds.d_seg_begin.get();
-    P.Z = io->Z; P.ldz = io->ldz;
-    P.x0 = io->x0; P.xf = io->xf;
-    P.f = io->f;
-    P.grad = io->grad; P.ldgrad = io->ldgrad;
-    P.g = io->g; P.ldg = io->ldg;
-    P.jac = io->jac; P.ldjac = io->ldjac;
+    P.io = *io;
     P.B = B;
     P.index = rg ? reinterpret_cast<const long long*>(rg->index) : nullptr;
     P.z_off = rg ? reinterpret_cast<const long long*>(rg->z_off) : nullptr;
@@ -1085,17 +1080,10 @@ int launch_products(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_ba
     ql::ProdLaunch P;
     std::memset(&P, 0, sizeof P);
     set_problem(P, p, ds);
-    P.Z = io->Z; P.ldz = io->ldz;
-    P.x0 = io->x0; P.xf = io->xf;
-    P.f = io->f;
-    P.grad = io->grad; P.ldgrad = io->ldgrad;
-    P.g = io->g; P.ldg = io->ldg;
+    P.io = *io;
     P.B = B;
     P.zbulk = ((reinterpret_cast<uintptr_t>(io->Z) & 15) == 0 && (io->ldz & 1) == 0) ? 1 : 0;
-    P.w = pv->w; P.ldw = pv->ldw;
-    P.jw = pv->jw; P.ldjw = pv->ldjw;
-    P.y = pv->y; P.ldy = pv->ldy;
-    P.jty = pv->jty; P.ldjty = pv->ldjty;
+    P.pv = *pv;
     P.kin = p.kin ? 1 : 0;
     return launch_kernel(ds, prod_spec(p), B, P, stream);
 }
@@ -1191,15 +1179,7 @@ int launch_kkt(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_kkt_io*
     P.c = c;
     P.jtab = ds.d_kkt_tab.get();
     P.htab = ds.d_kkt_tab.get() + c.nnz_true;
-    P.hess = io->hess; P.ldhess = io->ldhess;
-    P.jac = io->jac; P.ldjac = io->ldjac;
-    P.sx = io->sx; P.ldsx = io->ldsx;
-    P.dc = io->dc; P.lddc = io->lddc;
-    P.r1 = io->r1; P.ldr1 = io->ldr1;
-    P.r2 = io->r2; P.ldr2 = io->ldr2;
-    P.px = io->px; P.ldpx = io->ldpx;
-    P.pl = io->pl; P.ldpl = io->ldpl;
-    P.status = io->status;
+    P.io = *io;
     P.B = B;
     if (int rc = launch_kernel(ds, k, B, P, stream)) return rc;
     return end_scratch(P.scratch, owned, stream);
@@ -1253,12 +1233,7 @@ int launch_kkt_factor(const Problem& p, DeviceState& ds, int64_t B, const qlnlp_
     P.c = c;
     P.jtab = ds.d_kkt_tab.get();
     P.htab = ds.d_kkt_tab.get() + c.nnz_true;
-    P.hess = io->hess; P.ldhess = io->ldhess;
-    P.jac = io->jac; P.ldjac = io->ldjac;
-    P.sx = io->sx; P.ldsx = io->ldsx;
-    P.dc = io->dc; P.lddc = io->lddc;
-    P.factor = io->factor; P.ldfactor = io->ldfactor;
-    P.status = io->status;
+    P.io = *io;
     P.B = B;
     return launch_kernel(ds, kkt_factor_spec(), B, P, stream);
 }
@@ -1270,13 +1245,7 @@ int launch_kkt_solve_factored(const Problem& p, DeviceState& ds, int64_t R, cons
     std::memset(&P, 0, sizeof P);
     P.c = p.cls;
     P.jtab = ds.d_kkt_tab.get();
-    P.factor = io->factor; P.ldfactor = io->ldfactor; P.nfactor = io->nfactor;
-    P.index = reinterpret_cast<const long long*>(io->index);
-    P.r1 = io->r1; P.ldr1 = io->ldr1;
-    P.r2 = io->r2; P.ldr2 = io->ldr2;
-    P.px = io->px; P.ldpx = io->ldpx;
-    P.pl = io->pl; P.ldpl = io->ldpl;
-    P.status = io->status;
+    P.io = *io;
     P.B = R;
     return launch_kernel(ds, kkt_solve_factored_spec(), R, P, stream);
 }
@@ -1313,16 +1282,7 @@ int launch_kkt_residual(const Problem& p, DeviceState& ds, int64_t B, const qlnl
     P.c = c;
     P.jtab = ds.d_kkt_tab.get();
     P.htab = ds.d_kkt_tab.get() + c.nnz_true;
-    P.hess = io->hess; P.ldhess = io->ldhess;
-    P.jac = io->jac; P.ldjac = io->ldjac;
-    P.sx = io->sx; P.ldsx = io->ldsx;
-    P.dc = io->dc; P.lddc = io->lddc;
-    P.r1 = io->r1; P.ldr1 = io->ldr1;
-    P.r2 = io->r2; P.ldr2 = io->ldr2;
-    P.px = io->px; P.ldpx = io->ldpx;
-    P.pl = io->pl; P.ldpl = io->ldpl;
-    P.s1 = io->s1; P.lds1 = io->lds1;
-    P.s2 = io->s2; P.lds2 = io->lds2;
+    P.io = *io;
     P.B = B;
     return launch_kernel(ds, kkt_residual_spec(), B, P, stream);
 }

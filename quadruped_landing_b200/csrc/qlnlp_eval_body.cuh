@@ -40,8 +40,8 @@
 
     const bool zbulk = P.zbulk != 0;      // ragged launches: only when the caller guarantees aligned, padded Z rows
     auto zrow_of = [&](long long t) -> const double* {
-        if (RAGGED) return P.Z + __ldg(P.z_off + (P.index ? __ldg(P.index + t) : t));
-        return P.Z + t * P.ldz;
+        if (RAGGED) return P.io.Z + __ldg(P.z_off + (P.index ? __ldg(P.index + t) : t));
+        return P.io.Z + t * P.io.ldz;
     };
     unsigned zphase = 0;                 // parity of the mbarrier phase the next wait completes
     if (zbulk) {
@@ -86,7 +86,7 @@
         // With a cost / gradient part the ticket is only DRAWN here and read after the first pass's cost section, when
         // the atomic has returned.  The short g-only evaluation reads it at once: reading it late made that launch
         // bimodal (265 or 349 M evals/s from one process to the next, profiles/r02_kernel_ab.md), at once it is steady.
-        const bool late_ticket = JM != JM_BLOCK && (P.f || P.grad);
+        const bool late_ticket = JM != JM_BLOCK && (P.io.f || P.io.grad);
         unsigned tkt = 0;
         if (JM != JM_BLOCK) tkt = take_issue();
         if (JM != JM_BLOCK && !late_ticket) nb = take_get(tkt);
@@ -115,16 +115,16 @@
             cost = rc->cost; x0_def = rc->x0_def; xf_def = rc->xf_def; seg_begin = rc->seg_begin; npad = rc->npad;
         }
         const bool first_is_y1 = (c.init_mode == 1);    // contact-first reads y1 (mode 1) or y2 (mode 2)
-        double* const grow = P.g ? P.g + (RAGGED ? __ldg(P.g_off + pi) : b * P.ldg) : nullptr;
-        double* const gradrow = P.grad ? P.grad + (RAGGED ? __ldg(P.z_off + pi) : b * P.ldgrad) : nullptr;
-        double* const jrow = (WITH_JAC && JM != JM_PROD) ? P.jac + (RAGGED ? __ldg(P.j_off + pi) : b * P.ldjac) : nullptr;
+        double* const grow = P.io.g ? P.io.g + (RAGGED ? __ldg(P.g_off + pi) : b * P.io.ldg) : nullptr;
+        double* const gradrow = P.io.grad ? P.io.grad + (RAGGED ? __ldg(P.z_off + pi) : b * P.io.ldgrad) : nullptr;
+        double* const jrow = (WITH_JAC && JM != JM_PROD) ? P.io.jac + (RAGGED ? __ldg(P.j_off + pi) : b * P.io.ldjac) : nullptr;
         // TMA bulk stores need 16-byte aligned rows: a launch-wide property for strided batches, per row when ragged
         const bool bulk = P.bulk != 0 && (!RAGGED || (reinterpret_cast<uintptr_t>(jrow) & 15) == 0);
 
         if (grow) {
             // boundary rows (constraints.jl:149-150) straight from the staged vector, one lane per row
-            const double* x0 = P.x0 ? P.x0 + pi * QL_NX : x0_def;
-            const double* xf = P.xf ? P.xf + pi * QL_NX : xf_def;
+            const double* x0 = P.io.x0 ? P.io.x0 + pi * QL_NX : x0_def;
+            const double* xf = P.io.xf ? P.io.xf + pi * QL_NX : xf_def;
             if (lane < QL_NX) QL_GST(grow + lane, __dsub_rn(zbuf[lane], __ldg(x0 + lane)));
             if (lane < QL_NX - 1) QL_GST(grow + c.c_term + lane, __dsub_rn(zbuf[(c.N - 1) * QL_NZK + lane], __ldg(xf + lane)));
             __syncwarp();
@@ -137,7 +137,7 @@
             double* const zk = zbuf + (k - 1) * QL_NZK;
             // costs.jl:9-15 accumulates J knot by knot: the 32 terms of the PREVIOUS pass are added here, in order,
             // where few registers are live (every lane adds up the same sequence; only lane 0's copy is stored)
-            if (P.f && p > 0) fsum = f_chain(fsum, fbuf);
+            if (P.io.f && p > 0) fsum = f_chain(fsum, fbuf);
 
             // ---- 1. my knot's slice of Z: x_k, u_k, x_{k+1} = zk[0..34], fetched with 128-bit shared loads (the knot
             // stride of 160 B makes 64-bit loads 4-way bank conflicted; 16-byte loads halve the wavefronts)
@@ -160,7 +160,7 @@
 
             // ---- 2. cost and gradient (costs.jl:6-34, quadratic_cost.jl:44-52); gradient in place over Z
             double lane_term = -0.0;                // lanes without a knot add -0.0: x + (-0.0) == x bit for bit
-            if (act && (P.f || gradrow)) {
+            if (act && (P.io.f || gradrow)) {
                 const double* ct = cost + (k - 1);
                 const int np = npad;
                 double cq[QL_NCOST];                // all loads first: their latency overlaps
@@ -210,7 +210,7 @@
                 }
                 lane_term = term;
             }
-            if (P.f) {
+            if (P.io.f) {
                 __syncwarp();                       // the previous pass's terms have been read by every lane
                 fbuf[lane] = lane_term;             // read back in the next pass, or after the last one (below)
             }
@@ -411,9 +411,9 @@
         }
 
         // ---- 6. cost (accumulated in the reference's order above)
-        if (P.f) {
+        if (P.io.f) {
             fsum = f_chain(fsum, fbuf);          // the last pass's terms
-            if (lane == 0) QL_GST(P.f + pi, fsum);
+            if (lane == 0) QL_GST(P.io.f + pi, fsum);
         }
         b = nb;
     }

@@ -32,6 +32,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/qlnlp.h"
 #include "layout.h"
 #include "qlnlp_kin.cuh"
 
@@ -191,13 +192,7 @@ struct Launch {
     const double* xf_def;      // [15]  desc.xf
     const QlSeg* segs;         // segment plan, all passes
     const int* seg_begin;      // [npass + 1]
-    const double* Z; long long ldz;
-    const double* x0;          // [B][15] or nullptr
-    const double* xf;          // [B][15] or nullptr
-    double* f;
-    double* grad; long long ldgrad;
-    double* g; long long ldg;
-    double* jac; long long ldjac;
+    qlnlp_batch_io io;         // the caller's arrays, as the entry point took them
     long long B;
     // RAGGED instantiation only: the b-th evaluation of the launch is problem index[b] (or b) of a flat, mixed-size
     // batch; its rows start at Z + z_off[i], grad + z_off[i], g + g_off[i], jac + j_off[i]; f, x0, xf are indexed by i
@@ -262,13 +257,10 @@ __device__ __forceinline__ double f_chain(double fsum, const double* fbuf)
     return fsum;
 }
 
-// The Jacobian-product launch (JM_PROD): the Launch fields keep their meaning (jac must be null), the products'
+// The Jacobian-product launch (JM_PROD): the Launch fields keep their meaning (io.jac must be null), the products'
 // vectors and outputs come on top.  Rows are [B][ld]; a null w (or y) skips J w (or J' y).
 struct ProdLaunch : Launch {
-    const double* w; long long ldw;        // [B][ldw >= n_nlp]
-    double* jw; long long ldjw;            // [B][ldjw >= m_nlp (+ 2N kinematic rows)]
-    const double* y; long long ldy;        // [B][ldy >= m_nlp (+ 2N)]
-    double* jty; long long ldjty;          // [B][ldjty >= n_nlp]
+    qlnlp_product_io pv;                   // jw and y rows hold m_nlp + 2N entries with kinematic rows
     int kin;                               // 1: the handle's kinematic rows (rows m_nlp + 2(k-1) + foot) are part of J and g
 };
 
@@ -296,16 +288,16 @@ __device__ __forceinline__ void prod_pass(const ProdLaunch& P, const QlClass& c,
             kv[f][1] = __ddiv_rn(dy, n);
             kv[f][2] = __ddiv_rn(-dx, n);
             kv[f][3] = __ddiv_rn(-dy, n);
-            if (P.g) gst<true>(P.g + b * P.ldg + c.m_nlp + 2 * (k - 1) + f, n);
+            if (P.io.g) gst<true>(P.io.g + b * P.io.ldg + c.m_nlp + 2 * (k - 1) + f, n);
         }
     }
-    if (P.jw) {
-        double* const jwrow = P.jw + b * P.ldjw;
+    if (P.pv.jw) {
+        double* const jwrow = P.pv.jw + b * P.pv.ldjw;
         double* const ddst = jwrow + c.c_dyn + p * QL_LANES * QL_NX;
         const int dpar = (int)((reinterpret_cast<uintptr_t>(ddst) >> 3) & 1);
         __syncwarp();                                   // the previous flush has read jb
         if (act) {
-            const double* const wk = P.w + b * P.ldw + (long long)QL_NZK * (k - 1);
+            const double* const wk = P.pv.w + b * P.pv.ldw + (long long)QL_NZK * (k - 1);
             double wv[QL_NZK];
 #pragma unroll
             for (int j = 0; j < QL_NZK; ++j) wv[j] = (j < QL_NX || has_u) ? __ldg(wk + j) : 0.0;
@@ -351,11 +343,11 @@ __device__ __forceinline__ void prod_pass(const ProdLaunch& P, const QlClass& c,
         if (lane == 0 && a > j0 && ndyn > 0) gst<true>(ddst, jb[j0]);
         if (lane == 1 && e < j1 && e >= a) gst<true>(ddst + (e - dpar), jb[e]);
     }
-    if (P.jty) {
-        double* const jtyrow = P.jty + b * P.ldjty;
+    if (P.pv.jty) {
+        double* const jtyrow = P.pv.jty + b * P.pv.ldjty;
         __syncwarp();                                   // the J w flush has read jb
         if (act) {
-            const double* const yr = P.y + b * P.ldy;
+            const double* const yr = P.pv.y + b * P.pv.ldy;
             double a[QL_NX], o[QL_NZK];
             // rows above the RK4 block in each state column: init (k = 1) or term (k = N), then knot k-1's -I block
 #pragma unroll

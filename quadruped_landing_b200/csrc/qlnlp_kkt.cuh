@@ -29,6 +29,7 @@
 
 #include <float.h>
 
+#include "../../include/qlnlp.h"
 #include "layout.h"
 
 namespace ql {
@@ -70,15 +71,7 @@ struct KktLaunch {
     QlClass c;
     const unsigned short* jtab;          // [nnz_true]  slot | local column << 8 of every SPARSE_TRUE value
     const unsigned short* htab;          // [nnz_hess]  local row | local column << 8 (row >= column) of every W value
-    const double* hess; long long ldhess;
-    const double* jac; long long ldjac;
-    const double* sx; long long ldsx;    // or nullptr: 0
-    const double* dc; long long lddc;
-    const double* r1; long long ldr1;
-    const double* r2; long long ldr2;
-    double* px; long long ldpx;
-    double* pl; long long ldpl;
-    int* status;
+    qlnlp_kkt_io io;
     double* scratch;                     // [gridDim.x][N][KKT_FSTRIDE]: one factor per resident warp
     long long B;
     unsigned* ticket;                    // work counter of the stream (shared with the other kernels' launches)
@@ -88,12 +81,7 @@ struct KktFactorLaunch {
     QlClass c;
     const unsigned short* jtab;
     const unsigned short* htab;
-    const double* hess; long long ldhess;
-    const double* jac; long long ldjac;
-    const double* sx; long long ldsx;    // or nullptr: 0
-    const double* dc; long long lddc;
-    double* factor; long long ldfactor;  // [B][ldfactor >= kkt_factor_size]
-    int* status;
+    qlnlp_kkt_factor_io io;
     long long B;
     unsigned* ticket;
 };
@@ -101,13 +89,7 @@ struct KktFactorLaunch {
 struct KktSolveLaunch {
     QlClass c;
     const unsigned short* jtab;
-    const double* factor; long long ldfactor; long long nfactor;
-    const long long* index;              // [B] factor row of each right-hand side, or nullptr: the row's own
-    const double* r1; long long ldr1;
-    const double* r2; long long ldr2;
-    double* px; long long ldpx;
-    double* pl; long long ldpl;
-    int* status;
+    qlnlp_kkt_rhs_io io;
     long long B;
     unsigned* ticket;
 };
@@ -116,16 +98,7 @@ struct KktResidualLaunch {
     QlClass c;
     const unsigned short* jtab;
     const unsigned short* htab;
-    const double* hess; long long ldhess;
-    const double* jac; long long ldjac;
-    const double* sx; long long ldsx;    // or nullptr: 0
-    const double* dc; long long lddc;
-    const double* r1; long long ldr1;
-    const double* r2; long long ldr2;
-    const double* px; long long ldpx;
-    const double* pl; long long ldpl;
-    double* s1; long long lds1;
-    double* s2; long long lds2;
+    qlnlp_kkt_residual_io io;
     long long B;
     unsigned* ticket;
 };
@@ -394,14 +367,14 @@ __global__ void __launch_bounds__(QL_LANES, 8) kkt_kernel(const __grid_constant_
     long long b = take_get(take_issue());
     while (b < P.B) {
         const unsigned tkt = take_issue();
-        const double* const W = P.hess + b * P.ldhess;
-        const double* const J = P.jac + b * P.ldjac;
-        const double* const sx = P.sx ? P.sx + b * P.ldsx : nullptr;
-        const double* const dc = P.dc + b * P.lddc;
-        const double* const r1 = P.r1 + b * P.ldr1;
-        const double* const r2 = P.r2 + b * P.ldr2;
-        double* const px = P.px + b * P.ldpx;
-        double* const pl = P.pl + b * P.ldpl;
+        const double* const W = P.io.hess + b * P.io.ldhess;
+        const double* const J = P.io.jac + b * P.io.ldjac;
+        const double* const sx = P.io.sx ? P.io.sx + b * P.io.ldsx : nullptr;
+        const double* const dc = P.io.dc + b * P.io.lddc;
+        const double* const r1 = P.io.r1 + b * P.io.ldr1;
+        const double* const r2 = P.io.r2 + b * P.io.ldr2;
+        double* const px = P.io.px + b * P.io.ldpx;
+        double* const pl = P.io.pl + b * P.io.ldpl;
 
         int status = kkt_dc_status(c, dc, lane);
 
@@ -435,7 +408,7 @@ __global__ void __launch_bounds__(QL_LANES, 8) kkt_kernel(const __grid_constant_
             kkt_backward(S, c, k, nk, z0, px, pl, lane);
         }
         if (status != 0) kkt_fill_nan(c, px, pl, lane);
-        if (lane == 0) P.status[b] = status;
+        if (lane == 0) P.io.status[b] = status;
         __syncwarp();
         b = take_get(tkt);
     }
@@ -458,11 +431,11 @@ __global__ void __launch_bounds__(QL_LANES, 8) kkt_factor_kernel(const __grid_co
     long long b = take_get(take_issue());
     while (b < P.B) {
         const unsigned tkt = take_issue();
-        const double* const W = P.hess + b * P.ldhess;
-        const double* const J = P.jac + b * P.ldjac;
-        const double* const sx = P.sx ? P.sx + b * P.ldsx : nullptr;
-        const double* const dc = P.dc + b * P.lddc;
-        double* const F = P.factor + b * P.ldfactor;
+        const double* const W = P.io.hess + b * P.io.ldhess;
+        const double* const J = P.io.jac + b * P.io.ldjac;
+        const double* const sx = P.io.sx ? P.io.sx + b * P.io.ldsx : nullptr;
+        const double* const dc = P.io.dc + b * P.io.lddc;
+        double* const F = P.io.factor + b * P.io.ldfactor;
 
         double* const Fj = F + kkt_factor_jac(c);
         double* const Fd = F + kkt_factor_dc(c);
@@ -495,7 +468,7 @@ __global__ void __launch_bounds__(QL_LANES, 8) kkt_factor_kernel(const __grid_co
             F[1] = (double)c.N;
             F[2] = (double)c.k_trans;
             F[3] = (double)c.init_mode;
-            P.status[b] = status;
+            P.io.status[b] = status;
         }
         __syncwarp();
         b = take_get(tkt);
@@ -518,15 +491,15 @@ __global__ void __launch_bounds__(QL_LANES, 8) kkt_solve_factored_kernel(const _
     long long b = take_get(take_issue());
     while (b < P.B) {
         const unsigned tkt = take_issue();
-        const double* const r1 = P.r1 + b * P.ldr1;
-        const double* const r2 = P.r2 + b * P.ldr2;
-        double* const px = P.px + b * P.ldpx;
-        double* const pl = P.pl + b * P.ldpl;
-        const long long f = P.index ? P.index[b] : b;
-        const double* F = P.factor;
+        const double* const r1 = P.io.r1 + b * P.io.ldr1;
+        const double* const r2 = P.io.r2 + b * P.io.ldr2;
+        double* const px = P.io.px + b * P.io.ldpx;
+        double* const pl = P.io.pl + b * P.io.ldpl;
+        const long long f = P.io.index ? P.io.index[b] : b;
+        const double* F = P.io.factor;
         int status = -2;
-        if (f >= 0 && f < P.nfactor) {
-            F += f * P.ldfactor;
+        if (f >= 0 && f < P.io.nfactor) {
+            F += f * P.io.ldfactor;
             const bool same = F[1] == (double)c.N && F[2] == (double)c.k_trans && F[3] == (double)c.init_mode;
             status = same ? (int)F[0] : -3;
         }
@@ -559,7 +532,7 @@ __global__ void __launch_bounds__(QL_LANES, 8) kkt_solve_factored_kernel(const _
             kkt_backward(S, c, k, nk, z0, px, pl, lane);
         }
         if (status != 0) kkt_fill_nan(c, px, pl, lane);
-        if (lane == 0) P.status[b] = status;
+        if (lane == 0) P.io.status[b] = status;
         __syncwarp();
         b = take_get(tkt);
     }
@@ -586,16 +559,16 @@ __global__ void __launch_bounds__(QL_LANES, 8) kkt_residual_kernel(const __grid_
     long long b = take_get(take_issue());
     while (b < P.B) {
         const unsigned tkt = take_issue();
-        const double* const W = P.hess + b * P.ldhess;
-        const double* const J = P.jac + b * P.ldjac;
-        const double* const sx = P.sx ? P.sx + b * P.ldsx : nullptr;
-        const double* const dc = P.dc + b * P.lddc;
-        const double* const r1 = P.r1 + b * P.ldr1;
-        const double* const r2 = P.r2 + b * P.ldr2;
-        const double* const px = P.px + b * P.ldpx;
-        const double* const pl = P.pl + b * P.ldpl;
-        double* const s1 = P.s1 + b * P.lds1;
-        double* const s2 = P.s2 + b * P.lds2;
+        const double* const W = P.io.hess + b * P.io.ldhess;
+        const double* const J = P.io.jac + b * P.io.ldjac;
+        const double* const sx = P.io.sx ? P.io.sx + b * P.io.ldsx : nullptr;
+        const double* const dc = P.io.dc + b * P.io.lddc;
+        const double* const r1 = P.io.r1 + b * P.io.ldr1;
+        const double* const r2 = P.io.r2 + b * P.io.ldr2;
+        const double* const px = P.io.px + b * P.io.ldpx;
+        const double* const pl = P.io.pl + b * P.io.ldpl;
+        double* const s1 = P.io.s1 + b * P.io.lds1;
+        double* const s2 = P.io.s2 + b * P.io.lds2;
 
         for (int k = c.N; k >= 1; --k) {
             const int nk = k < c.N ? QL_NZK : QL_NX;
