@@ -99,7 +99,11 @@ typedef struct qlnlp_handle_s* qlnlp_handle;
 
 /* HybridNLP(model, obj, init_mode, k_trans, N, x0, xf)            nlp.jl:33-83
  * `device` is the CUDA ordinal used by every later call on the handle (bound lazily, at the first
- * evaluation).  `jac_mode` selects what qlnlp_eval_constraint_jacobian / jacobian_structure report. */
+ * evaluation).  `jac_mode` selects what qlnlp_eval_constraint_jacobian / jacobian_structure report.
+ * Values: divisions by the model constants go through a reciprocal (csrc/fastdiv.h), exact while every numerator
+ * has |a| >= 2^-969 and a/mf, a/Ib ... stay clear of overflow (all of the landing problem's range).  Inputs that
+ * drive values to the ends of the double range may see one ulp, +0 for -0, or NaN where IEEE division gives +-Inf;
+ * with the environment variable QLNLP_IEEE_DIV=1 set when the handle is created, the kernels divide IEEE-exactly. */
 int qlnlp_create(const qlnlp_problem_desc* desc, int device, int jac_mode, qlnlp_handle* out);
 int qlnlp_destroy(qlnlp_handle h);
 

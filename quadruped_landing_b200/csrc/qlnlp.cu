@@ -374,23 +374,6 @@ void plan_segments(const QlClass& c, const std::vector<BlockEntry>& block, std::
     }
 }
 
-// q = a*r; q' = fma(fma(-q, b, a), r, q) is the correctly rounded a/b for r = RN(1/b) (Markstein) unless b's
-// significand is all ones.  Verify per divisor on pseudo-random numerators; any miss disables the fast path.
-bool fastdiv_is_exact(double b)
-{
-    if (!(std::isfinite(b)) || b == 0.0) return false;
-    const double r = 1.0 / b;
-    unsigned long long s = 88172645463325252ULL;
-    for (int i = 0; i < 200000; ++i) {
-        s ^= s << 13; s ^= s >> 7; s ^= s << 17;
-        const double m = 1.0 + (double)(s >> 12) * (1.0 / 4503599627370496.0);
-        const double a = std::ldexp((s & 1) ? -m : m, (int)((s >> 3) % 81) - 40);
-        const double q = a * r;
-        if (std::fma(std::fma(-q, b, a), r, q) != a / b) return false;
-    }
-    return true;
-}
-
 // ---- what the launcher knows about a kernel ----------------------------------------------------------------------
 // The launch policies, each measured on the B200.  One CTA is one warp.
 struct KernelSpec {
@@ -1665,8 +1648,9 @@ int create_one(const qlnlp_problem_desc* d, const int* devices, int ndev, int ja
     p.rmb = 1.0 / c.mb;
     p.rmf = 1.0 / c.mf;
     p.rIb = 1.0 / c.Ib;
-    p.fastdiv = fastdiv_is_exact(c.mb) && fastdiv_is_exact(c.mf) && fastdiv_is_exact(c.Ib) &&
-                fastdiv_is_exact(6.0) && !std::getenv("QLNLP_IEEE_DIV");   // env: force the IEEE-division kernels
+    p.fastdiv = !std::getenv("QLNLP_IEEE_DIV") &&     // env: force the IEEE-division kernels
+                ql::fastdiv_is_exact(c.mb) && ql::fastdiv_is_exact(c.mf) && ql::fastdiv_is_exact(c.Ib) &&
+                ql::fastdiv_is_exact(6.0);
     p.ldz_e = (c.n_nlp + 1) & ~1;
     p.ldgrad_e = p.ldz_e;
     p.ldg_e = (m_rows(p) + 1) & ~1;

@@ -24,15 +24,18 @@
 // All arithmetic is fp64 with explicit round-to-nearest add/mul/div (no FMA contraction) in the
 // reference's operation order, so f, g, grad and the Jacobian values are bit-identical to the CPU
 // oracle (sin/cos aside); the cost is accumulated knot by knot in the reference's sequential order.
-// Divisions by the model constants use q = a*r, q' = fma(fma(-q, b, a), r, q) with r = RN(1/b), which is
-// the correctly rounded quotient (Markstein); the host verifies this per divisor at create time and falls
-// back to IEEE division (template parameter FASTDIV = false) otherwise.
+// Divisions by the model constants use fastdiv.h: q = a*r, q' = fma(fma(-q, b, a), r, q) with r = RN(1/b), the
+// correctly rounded quotient (Markstein) in the domain |a| >= 2^-969, a*r finite.  Outside it q' can miss by an ulp
+// (0 < |a| < 2^-969), is +0 for a = -0, and NaN where a*r overflows; fastdiv.h states this exactly and why the
+// kernels do not guard it.  The host verifies the domain per divisor at create time on every binade and falls back
+// to IEEE division (template parameter FASTDIV = false, or QLNLP_IEEE_DIV) otherwise.
 #pragma once
 
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 #include "../../include/qlnlp.h"
+#include "fastdiv.h"
 #include "layout.h"
 #include "qlnlp_kin.cuh"
 
@@ -129,16 +132,13 @@ __device__ __forceinline__ void mbar_wait(unsigned mbar, unsigned parity)
 // make generic-proxy shared-memory writes visible to the async (TMA) proxy
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-// model constants + their reciprocals; division by a constant, correctly rounded
+// model constants + their reciprocals; division by a constant, correctly rounded (fastdiv.h)
 template <bool FAST>
 struct Consts {
     double g, mb, mf, Ib, rmb, rmf, rIb;
     __device__ __forceinline__ static double div(double a, double b, double r)
     {
-        if (FAST) {
-            const double q = __dmul_rn(a, r);
-            return __fma_rn(__fma_rn(-q, b, a), r, q);
-        }
+        if (FAST) return fastdiv(a, b, r);
         return __ddiv_rn(a, b);
     }
     __device__ __forceinline__ double div_mb(double a) const { return div(a, mb, rmb); }

@@ -241,6 +241,14 @@ def _check(rc: int):
         raise QlnlpError(rc, load_library().qlnlp_last_error().decode())
 
 
+def _check_sigma(sigma, B):
+    """The C ABI reads sigma as B consecutive doubles: a strided view would hand it other rows' weights."""
+    import torch
+    if sigma is not None and not (sigma.is_cuda and sigma.dtype == torch.float64 and tuple(sigma.shape) == (B,)
+                                  and (B <= 1 or sigma.stride(0) == 1)):
+        raise ValueError(f"sigma must be a contiguous float64 CUDA tensor [{B}]")
+
+
 def _np_ptr(a: Optional[np.ndarray]):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
@@ -460,6 +468,7 @@ class HybridNLP:
         for t, w, name in ((Z, self.n_nlp, "Z"), (mu, self.m_nlp, "mu")):
             if not (t.is_cuda and t.dtype == torch.float64 and t.dim() == 2 and t.shape == (B, w) and t.stride(1) == 1):
                 raise ValueError(f"{name} must be a float64 CUDA tensor [B, {w}]")
+        _check_sigma(sigma, B)
         if out is None:
             out, = _device_empty(Z.device.index, [(B, self.nnz_hess, torch.float64)], self._compressible)
         s = torch.cuda.current_stream(Z.device) if stream is None else stream
@@ -557,6 +566,7 @@ class HybridNLP:
         for t, wd, name in ((Z, self.n_nlp, "Z"), (mu, self.m_nlp, "mu"), (V, self.n_nlp, "V")):
             if not (t.is_cuda and t.dtype == torch.float64 and t.dim() == 2 and t.shape == (B, wd) and t.stride(1) == 1):
                 raise ValueError(f"{name} must be a float64 CUDA tensor [B, {wd}]")
+        _check_sigma(sigma, B)
         if out is None:
             out, = _device_empty(Z.device.index, [(B, self.n_nlp, torch.float64)], self._compressible)
         s = torch.cuda.current_stream(Z.device) if stream is None else stream

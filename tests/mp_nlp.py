@@ -283,8 +283,9 @@ class Model:
     # ---- Lagrangian Hessian
     def hess_knot(self, z, k, sigma, lam):
         """The 20x20 (15x15 at k = N) block of sigma Hess f + sum_r lam_r Hess g_r at knot k: the true second
-        derivatives (d/dh of h * stagecost included).  Linear rows contribute nothing; the body row contributes
-        lam * lb/2 |sin(theta)| at (theta, theta)."""
+        derivatives (d/dh of h * stagecost included).  Linear rows contribute nothing; the body row contributes the
+        theta-derivative of its Q4 Jacobian entry at (theta, theta): lam * lb/2 sin(theta) if theta > 0, else
+        -lam * lb/2 sin(theta).  That is lam * lb/2 |sin(theta)| while |theta| < pi, and differs from it beyond."""
         assert not self.kin, "the Hessian covers the NLP without kinematic rows"
         lam = np.asarray(lam, dtype=np.float64)
         lk = np.concatenate([lam[self.c_dyn + 15 * (k - 1):self.c_dyn + 15 * k] if k < self.N else [], lam[self.c_body + k - 1:][:1]])
@@ -318,7 +319,8 @@ class Model:
             for i in range(nv):
                 for j in range(i + 1):
                     H[i, j] = H[j, i] = float((at(i, j) - p1[i] - p1[j] + p0) / (_E2 * _E2))
-            H[2, 2] += float(mp.mpf(float(lam[self.c_body + k - 1])) * self.half_lb * abs(mp.sin(v[2])))
+            th = v[2]
+            H[2, 2] += float(mp.mpf(float(lam[self.c_body + k - 1])) * self.half_lb * (mp.sin(th) if th > 0 else -mp.sin(th)))
         return H
 
 

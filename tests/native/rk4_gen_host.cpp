@@ -6,6 +6,7 @@
 
 #include <cmath>
 #include "host_consts.h"
+#include "../../quadruped_landing_b200/csrc/fastdiv.h"
 #include "../../quadruped_landing_b200/csrc/rk4_dual_gen.h"
 
 extern "C" {
@@ -33,25 +34,15 @@ void host_rk4(int mode, const double* x, const double* u, double g, double mb, d
     else ql_rk4_mode3(x, u, K, xn);
 }
 
-// The kernel divides by the model constants with a precomputed reciprocal and two FMAs
-// (q = a*r; e = fma(-q, b, a); q' = fma(e, r, q)).  Counts how many of n pseudo-random numerators give a
-// result different from the IEEE quotient a / b (expected: 0).
-long long host_count_fastdiv_mismatches(double b, long long n, unsigned long long seed)
+// The kernels divide by the model constants with csrc/fastdiv.h.  Sweeps per_binade numerators of each binade of the
+// double range plus the special values: returns how many inside the formula's domain give bits different from the IEEE
+// quotient a / b, and counts those outside it, and those of them that break the documented behaviour there.
+long long host_count_fastdiv_mismatches(double b, int per_binade, unsigned long long seed, long long* outside,
+                                        long long* outside_bad)
 {
-    const double r = 1.0 / b;
-    long long bad = 0;
-    unsigned long long s = seed ? seed : 88172645463325252ULL;
-    for (long long i = 0; i < n; ++i) {
-        s ^= s << 13; s ^= s >> 7; s ^= s << 17;
-        // random sign, mantissa and an exponent in [-40, 40]
-        const double m = 1.0 + (double)(s >> 12) * (1.0 / 4503599627370496.0);
-        const int e = (int)((s >> 3) % 81) - 40;
-        const double a = std::ldexp((s & 1) ? -m : m, e);
-        const double q = a * r;
-        const double rem = std::fma(-q, b, a);
-        const double q1 = std::fma(rem, r, q);
-        if (q1 != a / b) ++bad;
-    }
-    return bad;
+    return ql::fastdiv_misses(b, per_binade, seed, outside, outside_bad);
 }
+
+// the create-time decision of qlnlp_create: may the kernels divide by b with the reciprocal?
+int host_fastdiv_is_exact(double b) { return ql::fastdiv_is_exact(b); }
 }

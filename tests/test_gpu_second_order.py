@@ -302,3 +302,21 @@ def test_poisoned_rows_stay_local_in_long_batches():
         t, _ = kinds[j]
         for k in hits[t]:
             assert not bool(torch.isfinite(got[k][b]).all()), (t, k)
+
+
+def test_sigma_must_be_one_contiguous_weight_per_row():
+    """The C ABI reads sigma as B consecutive doubles: a strided view (every second entry of a longer vector) would
+    weight row b with another row's sigma, so the binders refuse it, as they refuse a wrong length or type."""
+    p = ql.default_problem()
+    nlp = ql.HybridNLP.from_problem(p, hessian=True, products=True)
+    B, n, m = 4, p.n_nlp, p.m_nlp
+    Z = _cuda(perturbed_batch(p, [ql.initial_guess(p)], B, 1e-2, 1))
+    lam, v = _cuda(np.ones((B, m))), _cuda(np.ones((B, n)))
+    good = torch.full((2 * B,), 0.5, dtype=F64, device="cuda")
+    for bad in (good[::2], good, good[:B].float(), good[:B].cpu(), good[:B].reshape(B, 1)):
+        with pytest.raises(ValueError, match="sigma"):
+            nlp.eval_hessian_batch(Z, lam, bad)
+        with pytest.raises(ValueError, match="sigma"):
+            nlp.eval_hessian_product_batch(Z, lam, v, bad)
+    h = nlp.eval_hessian_batch(Z, lam, good[::2].contiguous())
+    assert _same_bits(h, nlp.eval_hessian_batch(Z, lam, good[:B]))

@@ -63,13 +63,22 @@ def test_other_model_constants(rk4_host_lib):
 
 @pytest.mark.parametrize("b", [10.0, 0.1, 10.0 * (0.5 * 0.5) / 12, 6.0, 7.3, 0.23, 3.0, 1.9999999999999998])
 def test_reciprocal_fma_division_is_correctly_rounded(rk4_host_lib, b):
-    """The kernel divides by model constants as q = a*r, q' = fma(fma(-q, b, a), r, q) with r = RN(1/b);
-    it must equal the IEEE quotient the reference computes (also re-checked at qlnlp_create)."""
+    """The kernel divides by model constants with csrc/fastdiv.h: q' = fma(fma(-q, b, a), r, q) for q = a*r and
+    r = RN(1/b).  Whenever the create-time check (fastdiv_is_exact) accepts b, q' must have the bits of the IEEE
+    quotient the reference computes for 2,000 numerators of every binade inside the domain |a| >= 2^-969, a*r finite
+    (signed zeros and Inf included), and do what fastdiv.h states outside it: one ulp at most below 2^-969, +0 for a
+    zero numerator, NaN where a*r overflows.  The check must refuse 1.9999999999999998, whose significand is all ones."""
     import ctypes as C
     fn = rk4_host_lib.host_count_fastdiv_mismatches
     fn.restype = C.c_longlong
-    fn.argtypes = [C.c_double, C.c_longlong, C.c_ulonglong]
-    assert fn(b, 3_000_000, 2024) == 0
+    fn.argtypes = [C.c_double, C.c_int, C.c_ulonglong, C.c_void_p, C.c_void_p]
+    rk4_host_lib.host_fastdiv_is_exact.argtypes = [C.c_double]
+    exact = bool(rk4_host_lib.host_fastdiv_is_exact(b))
+    assert exact == (b != 1.9999999999999998)
+    if exact:
+        outside, outside_bad = C.c_longlong(0), C.c_longlong(0)
+        assert fn(b, 2000, 2024, C.addressof(outside), C.addressof(outside_bad)) == 0
+        assert outside.value >= 2000 * 53 and outside_bad.value == 0, (outside.value, outside_bad.value)
 
 
 def test_committed_header_is_up_to_date(tmp_path):
